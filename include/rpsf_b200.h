@@ -151,6 +151,14 @@ int rpsf_isolate_cores(double* patches, int64_t n_patches, int patch_size, int d
  * workspace. */
 int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int height, int width, int pad_mode, int row_begin,
                      int row_end, int max_batch);
+/* A plan whose rpsf_apply computes the transpose of the plan rpsf_plan_create(t, H, W, pad_mode, 0, H, .) would run
+ * (no saturation): input = `batch` (H, W) frames of output gradients, output = (H, W) frames of input gradients.
+ * It runs the three default kernels on the bounding box of the patch footprints (zero-bordered copy of the input,
+ * conj of the transfer kernel, built at the first adjoint plan of `t`) and folds the box onto the frame along the
+ * np.pad index map (pad_mode 0..4; RPSF_PAD_MATERIALIZED is RPSF_E_UNSUPPORTED).  rpsf_apply takes whole frames
+ * (img_row0 = out_row0 = 0, img_rows = H); rpsf_apply_stages and rpsf_apply_host, a finite saturation threshold,
+ * output mirrors and the opt-in fused / paired / single-CTA paths are RPSF_E_UNSUPPORTED on it. */
+int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int height, int width, int pad_mode, int max_batch);
 int rpsf_plan_destroy(rpsf_plan* p);
 /* info[0]=active patches, [1]=colours, [2]=workspace bytes, [3]=first frame row read,
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,

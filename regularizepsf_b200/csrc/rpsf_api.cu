@@ -24,6 +24,7 @@
 #include "rpsf_ops.h"
 #include "rpsf_saturation.cuh"
 #include "rpsf_builder.cuh"
+#include "rpsf_adjoint.cuh"
 
 namespace rpsf {
 const Ops* ops_for(int P) {
@@ -354,7 +355,30 @@ struct rpsf_transform {
   bool own_win = false;            // the window table belongs to this transform (embedded sizes), not to the shared cache
   bool has_kernel = false;
   int sm_count = 148;
+  // conj of kmain / knyq: the transfer kernel of the transpose (rpsf_plan_create_adjoint); allocated at the first
+  // adjoint plan, refreshed by every rpsf_transform_set_kernel after that
+  void* kconj_main = nullptr;
+  void* kconj_nyq = nullptr;
 };
+
+namespace {
+// kconj_* = conj(kmain / knyq), stream-ordered after whatever wrote kmain on `s`
+int refresh_conj_kernel(rpsf_transform* t, cudaStream_t s) {
+  if (!t->kconj_main || t->n_kept == 0) return RPSF_OK;
+  const long long main_reals = (long long)t->n_kept * t->P * (t->P / 2) * 2, nyq_reals = (long long)t->n_kept * t->P * 2;
+  const unsigned blocks = (unsigned)t->sm_count * 8;
+  if (t->dtype == RPSF_F32) {
+    conj_spectrum<float><<<blocks, 256, 0, s>>>((const float*)t->kmain, (float*)t->kconj_main, main_reals);
+    conj_spectrum<float><<<blocks, 256, 0, s>>>((const float*)t->knyq, (float*)t->kconj_nyq, nyq_reals);
+  } else {
+    conj_spectrum<double><<<blocks, 256, 0, s>>>((const double*)t->kmain, (double*)t->kconj_main, main_reals);
+    conj_spectrum<double><<<blocks, 256, 0, s>>>((const double*)t->knyq, (double*)t->kconj_nyq, nyq_reals);
+  }
+  g_launches.fetch_add(2, std::memory_order_relaxed);
+  const cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? RPSF_OK : fail(RPSF_E_CUDA, "conjugate kernel launch failed: %s", cudaGetErrorString(e));
+}
+}  // namespace
 
 struct rpsf_plan {
   rpsf_transform* tr = nullptr;
@@ -428,6 +452,16 @@ struct rpsf_plan {
   int* sat_flags = nullptr;               // [2*max_batch]: any-masked flags, fill tickets
   // fused slab gather: peer buffers K3 stores to as well (same layout as `out`)
   std::vector<void*> mirrors;
+  // transpose (rpsf_plan_create_adjoint): this plan is the forward plan of the box [box_y0, box_y0 + H) x
+  // [box_x0, box_x0 + W) of the frame coordinates; rpsf_apply copies the frame of output gradients into box_in (zero
+  // margins), runs the three kernels with the conjugated transfer kernel into box_out and folds box_out onto the
+  // frame (fold_pad_adjoint)
+  bool adjoint = false;
+  int frame_H = 0, frame_W = 0, box_y0 = 0, box_x0 = 0;
+  long long box_pitch = 0;            // elements, a multiple of 16 bytes (K1's bulk row copies)
+  void* box_in = nullptr; void* box_out = nullptr;
+  int* fold_rows = nullptr;           // [frame_H + 1 offsets | box row indices], CSR preimages of the row pad map
+  int* fold_cols = nullptr;           // the same for columns
   // per-stage timing (bench only)
   bool timing = false;
   std::vector<cudaEvent_t> events;   // 4 per recorded apply call
@@ -530,6 +564,7 @@ int rpsf_transform_destroy(rpsf_transform* t) {
   if (!t) return RPSF_OK;
   DeviceGuard guard(t->device);
   cudaFree(t->kmain); cudaFree(t->knyq);
+  cudaFree(t->kconj_main); cudaFree(t->kconj_nyq);
   if (t->own_win) cudaFree(t->win);
   delete t;
   return RPSF_OK;
@@ -584,11 +619,11 @@ int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int ke
     release();
     if (e) return fail(RPSF_E_CUDA, "kernel layout launch failed: %s", cudaGetErrorString((cudaError_t)e));
     t->has_kernel = true;
-    return RPSF_OK;
+    return refresh_conj_kernel(t, s);
   }
   if (t->n_kept > 0) LAUNCH(t->ops->prep(t->dtype, kernel_dtype, kernel_full, t->kmain, t->knyq, t->n_kept, s));
   t->has_kernel = true;
-  return RPSF_OK;
+  return refresh_conj_kernel(t, s);
 }
 
 int rpsf_construct_kernel(const void* S, const void* Tg, void* K, int64_t count, int dtype, double alpha,
@@ -832,6 +867,7 @@ int rpsf_isolate_cores(double* patches, int64_t n_patches, int P, int device, vo
 
 int rpsf_plan_set_output_mirrors(rpsf_plan* p, int n, void* const* ptrs) {
   if (!p || n < 0 || n > 7 || (n > 0 && !ptrs)) return fail(RPSF_E_INVALID_ARGUMENT, "0..7 mirror buffers");
+  if (p->adjoint && n > 0) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan has no output mirrors");
   p->mirrors.assign(ptrs, ptrs + n);
   return RPSF_OK;
 }
@@ -868,8 +904,31 @@ int rpsf_ipc_close(void* ptr, int device) {
   return RPSF_OK;
 }
 
-int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int row_begin, int row_end,
-                     int max_batch) {
+}  // extern "C"
+
+namespace {
+// The reference pads 2P per side and slices [c+2P, c+3P) (transform.py:119-123,141-149); a corner outside [-2P, dim+P]
+// makes that slice short and numpy raises.  Reject it up front.  (P here is the true patch size; an embedded
+// transform's FFT length t->P is larger.)
+int check_corners(const rpsf_transform* t, int H, int W) {
+  const int P = t->win_len;
+  for (int i = 0; i < t->n; ++i) {
+    const int2 c = t->corners[i];
+    if (c.x < -2 * P || c.x + P > H + 2 * P || c.y < -2 * P || c.y + P > W + 2 * P)
+      return fail(RPSF_E_INVALID_COORDINATE,
+                  "patch corner (%d, %d) lies outside the 2*P padded frame of shape (%d, %d)", c.x, c.y, H, W);
+  }
+  return RPSF_OK;
+}
+
+// Where the plan of a transpose sits: the frame coordinates of box pixel (0, 0) and the frame shape.
+struct AdjointBox { int y0, x0, frame_H, frame_W; };
+
+// The forward plan of an H x W frame.  With `box`, the "frame" is the box of an adjoint plan: patch corners are shifted
+// into box coordinates, a patch takes part when it touches the real frame (exactly the patches the forward reads), and
+// only the default three-kernel path is prepared — the opt-in paths do not read the conjugated kernel.
+int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int row_begin, int row_end,
+               int max_batch, const AdjointBox* box) {
   // RPSF_PLAN_TIMING=1 prints where the planning time goes (host-side work lists and their uploads)
   const bool plan_timing = getenv("RPSF_PLAN_TIMING") != nullptr;
   auto plan_t0 = std::chrono::steady_clock::now();
@@ -887,15 +946,15 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
     return fail(RPSF_E_INVALID_ARGUMENT, "row band [%d,%d) outside frame of %d rows", row_begin, row_end, H);
   if (max_batch < 1) return fail(RPSF_E_INVALID_ARGUMENT, "max_batch must be >= 1");
   const int P = t->P;
-  // The reference pads 2P per side and slices [c+2P, c+3P) (transform.py:119-123,141-149); a
-  // corner outside [-2P, dim+P] makes that slice short and numpy raises.  Reject it up front.
-  // (P here is the true patch size; an embedded transform's FFT length t->P is larger.)
-  for (int i = 0; i < t->n; ++i) {
-    const int2 c = t->corners[i];
-    const int P = t->win_len;
-    if (c.x < -2 * P || c.x + P > H + 2 * P || c.y < -2 * P || c.y + P > W + 2 * P)
-      return fail(RPSF_E_INVALID_COORDINATE,
-                  "patch corner (%d, %d) lies outside the 2*P padded frame of shape (%d, %d)", c.x, c.y, H, W);
+  if (!box)
+    if (int rc = check_corners(t, H, W)) return rc;
+  const bool adjoint = box != nullptr;
+  std::vector<int2> tcorners(t->corners);
+  // the region a patch must touch to take part, in plan coordinates: the owned band, or the real frame inside the box
+  int reach_r0 = row_begin, reach_r1 = row_end, reach_c0 = 0, reach_c1 = W;
+  if (box) {
+    for (int2& c : tcorners) { c.x -= box->y0; c.y -= box->x0; }
+    reach_r0 = -box->y0; reach_r1 = box->frame_H - box->y0; reach_c0 = -box->x0; reach_c1 = box->frame_W - box->x0;
   }
   DeviceGuard guard(t->device);
   auto* p = new rpsf_plan;
@@ -914,16 +973,17 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   // bands of the fused pipeline), and the row kernels walk the frame top to bottom
   std::vector<int> order;
   for (int i = 0; i < t->n; ++i) {
-    const int2 c = t->corners[i];
-    if (std::max(c.x, row_begin) >= std::min(c.x + t->win_len, row_end) || std::max(c.y, 0) >= std::min(c.y + t->win_len, W)) continue;
+    const int2 c = tcorners[i];
+    if (std::max(c.x, reach_r0) >= std::min(c.x + t->win_len, reach_r1) ||
+        std::max(c.y, reach_c0) >= std::min(c.y + t->win_len, reach_c1)) continue;
     order.push_back(i);                                       // contributes to the owned band
   }
   std::stable_sort(order.begin(), order.end(), [&](int u, int v) {
-    const int2 cu = t->corners[u], cv = t->corners[v];
+    const int2 cu = tcorners[u], cv = tcorners[v];
     return cu.x != cv.x ? cu.x < cv.x : cu.y < cv.y;
   });
   for (int i : order) {
-    const int2 c = t->corners[i];
+    const int2 c = tcorners[i];
     const int r0 = std::max(c.x, row_begin), r1 = std::min(c.x + t->win_len, row_end);
     const int c0 = std::max(c.y, 0), c1 = std::min(c.y + t->win_len, W);
     const int a = (int)active.size();
@@ -1081,7 +1141,7 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   tick("streaming overlap-add tables");
   // ---- small patches: output tiles of P/2 x P/2 and the patches that cover each, in list order (the reference's `+=` order)
   if (const char* v = getenv("RPSF_SMALL")) p->small_mode = strcmp(v, "0") == 0 ? 1 : strcmp(v, "1") == 0 ? 2 : 0;
-  if (!embedded && p->n_active > 0 && P % 2 == 0 && t->ops->small_ok(t->dtype) && row_end > row_begin) {
+  if (!adjoint && !embedded && p->n_active > 0 && P % 2 == 0 && t->ops->small_ok(t->dtype) && row_end > row_begin) {
     const int ts = P / 2;
     bool aligned = true;
     for (const int2& c : corners) aligned = aligned && (((c.x % ts) + ts) % ts == 0) && (((c.y % ts) + ts) % ts == 0);
@@ -1124,7 +1184,7 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   tick("single-CTA tile lists");
   // ---- paired column pass: chains of active patches that share a corner column, corner rows P/2 apart
   if (const char* v = getenv("RPSF_PAIRED")) p->column_mode = strcmp(v, "1") == 0 ? 2 : 0;
-  if (p->stream_ok && !embedded && t->ops->chain_ok(t->dtype) && (P / 2) % 2 == 0) {
+  if (!adjoint && p->stream_ok && !embedded && t->ops->chain_ok(t->dtype) && (P / 2) % 2 == 0) {
     std::map<int, std::vector<int>> by_col;                       // corner column -> active patches, by corner row
     for (int a = 0; a < p->n_active; ++a) by_col[corners[a].y].push_back(a);
     bool ok = true;
@@ -1195,7 +1255,7 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   // is slower than the three stand-alone kernels, so it is opt-in: RPSF_FUSED=1 or rpsf_plan_set_fused(plan, 2).
   const char* fenv = getenv("RPSF_FUSED");
   if (fenv && strcmp(fenv, "1") == 0) p->fused_mode = 2;
-  if (finfo[0] && p->stream_ok && !(fenv && strcmp(fenv, "0") == 0)) {
+  if (!adjoint && finfo[0] && p->stream_ok && !(fenv && strcmp(fenv, "0") == 0)) {
     std::vector<int2> slots(p->n_active);
     std::vector<int> band_size;
     for (int a = 0; a < p->n_active; ++a) {
@@ -1279,6 +1339,87 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   return RPSF_OK;
 }
 
+// CSR preimages of the np.pad index map of one axis of length n, restricted to the box positions [b0, b0 + nb) (frame
+// coordinates): offsets [n + 1] then box indices, ascending per pixel
+std::vector<int> fold_table(int n, int b0, int nb, int pad_mode) {
+  std::vector<std::vector<int>> pre(n);
+  for (int k = 0; k < nb; ++k) {
+    const int src = pad_index(b0 + k, n, pad_mode);
+    if (src >= 0) pre[src].push_back(k);
+  }
+  std::vector<int> csr(1, 0);
+  for (const auto& v : pre) csr.push_back(csr.back() + (int)v.size());
+  for (const auto& v : pre) csr.insert(csr.end(), v.begin(), v.end());
+  return csr;
+}
+}  // namespace
+
+extern "C" {
+
+int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int row_begin, int row_end,
+                     int max_batch) {
+  return plan_build(out, t, H, W, pad_mode, row_begin, row_end, max_batch, nullptr);
+}
+
+int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int max_batch) {
+  if (!out || !t) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (H <= 0 || W <= 0) return fail(RPSF_E_INCORRECT_SHAPE, "frame shape must be positive, got (%d, %d)", H, W);
+  if (pad_mode < 0 || pad_mode >= RPSF_PAD_MATERIALIZED)
+    return fail(RPSF_E_UNSUPPORTED, "the transpose needs a pad mode with an index map (0..4), got %d", pad_mode);
+  if (max_batch < 1) return fail(RPSF_E_INVALID_ARGUMENT, "max_batch must be >= 1");
+  if (int rc = check_corners(t, H, W)) return rc;
+  // the box: bounding box of the footprints of the patches that touch the frame (a 1 x 1 box when none does)
+  const int L = t->win_len;
+  int y0 = INT_MAX, x0 = INT_MAX, y1 = INT_MIN, x1 = INT_MIN;
+  for (const int2& c : t->corners) {
+    if (std::max(c.x, 0) >= std::min(c.x + L, H) || std::max(c.y, 0) >= std::min(c.y + L, W)) continue;
+    y0 = std::min(y0, c.x); x0 = std::min(x0, c.y); y1 = std::max(y1, c.x + L); x1 = std::max(x1, c.y + L);
+  }
+  if (y0 == INT_MAX) { y0 = 0; x0 = 0; y1 = 1; x1 = 1; }
+  const int Hb = y1 - y0, Wb = x1 - x0;
+  const AdjointBox box{y0, x0, H, W};
+  rpsf_plan* p = nullptr;
+  // the box holds every patch it serves whole, so the index map is never consulted there; constant is the cheapest
+  if (int rc = plan_build(&p, t, Hb, Wb, RPSF_PAD_CONSTANT, 0, Hb, max_batch, &box)) return rc;
+  DeviceGuard guard(t->device);
+  p->adjoint = true;
+  p->frame_H = H; p->frame_W = W; p->box_y0 = y0; p->box_x0 = x0;
+  const size_t rs = real_size(t->dtype), align = 16 / rs;
+  p->box_pitch = (long long)((Wb + align - 1) / align * align);
+  const size_t box_bytes = (size_t)max_batch * Hb * p->box_pitch * rs;
+  const std::vector<int> rows = fold_table(H, y0, Hb, pad_mode), cols = fold_table(W, x0, Wb, pad_mode);
+  auto bail = [&](const char* what) {
+    const cudaError_t e = cudaGetLastError();
+    rpsf_plan_destroy(p);
+    return fail(RPSF_E_CUDA, "adjoint plan: %s failed: %s", what, cudaGetErrorString(e));
+  };
+  if (cudaMalloc(&p->box_in, box_bytes) != cudaSuccess || cudaMalloc(&p->box_out, box_bytes) != cudaSuccess)
+    return bail("box buffers");
+  if (cudaMemset(p->box_in, 0, box_bytes) != cudaSuccess) return bail("zeroing the box");     // margins stay zero
+  if (cudaMalloc(&p->fold_rows, sizeof(int) * rows.size()) != cudaSuccess ||
+      cudaMalloc(&p->fold_cols, sizeof(int) * cols.size()) != cudaSuccess)
+    return bail("fold tables");
+  if (cudaMemcpy(p->fold_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(p->fold_cols, cols.data(), sizeof(int) * cols.size(), cudaMemcpyHostToDevice) != cudaSuccess)
+    return bail("fold table upload");
+  if (!t->kconj_main && t->n_kept > 0) {
+    const size_t cs = 2 * rs;
+    if (cudaMalloc(&t->kconj_main, (size_t)t->n_kept * t->P * (t->P / 2) * cs) != cudaSuccess ||
+        cudaMalloc(&t->kconj_nyq, (size_t)t->n_kept * t->P * cs) != cudaSuccess) {
+      cudaFree(t->kconj_main); cudaFree(t->kconj_nyq); t->kconj_main = t->kconj_nyq = nullptr;
+      return bail("conjugated transfer kernel");
+    }
+    if (t->has_kernel) {
+      // kmain may still be written on another stream by rpsf_transform_set_kernel: order by the device
+      if (cudaDeviceSynchronize() != cudaSuccess) return bail("synchronise before conjugating");
+      if (int rc = refresh_conj_kernel(t, nullptr)) { rpsf_plan_destroy(p); return rc; }
+      if (cudaDeviceSynchronize() != cudaSuccess) return bail("conjugating the transfer kernel");
+    }
+  }
+  *out = p;
+  return RPSF_OK;
+}
+
 int rpsf_plan_destroy(rpsf_plan* p) {
   if (!p) return RPSF_OK;
   DeviceGuard guard(p->tr->device);
@@ -1300,6 +1441,7 @@ int rpsf_plan_destroy(rpsf_plan* p) {
   cudaFree(p->ftasks_dev); cudaFree(p->fcodes_dev);
   cudaFree(p->sat_pf); cudaFree(p->sat_mask[0]); cudaFree(p->sat_mask[1]); cudaFree(p->sat_list);
   cudaFree(p->sat_rows); cudaFree(p->sat_flags);
+  cudaFree(p->box_in); cudaFree(p->box_out); cudaFree(p->fold_rows); cudaFree(p->fold_cols);
   for (int* d : p->items_dev) cudaFree(d);
   for (cudaEvent_t e : p->events) cudaEventDestroy(e);
   delete p;
@@ -1453,6 +1595,8 @@ int rpsf_plan_set_saturation(rpsf_plan* p, double threshold, int dilation, int n
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (threshold != threshold) return fail(RPSF_E_INVALID_ARGUMENT, "saturation threshold is NaN");
   if (neighborhood_width < 0) return fail(RPSF_E_INVALID_ARGUMENT, "neighborhood_width must be >= 0");
+  if (p->adjoint && threshold < INFINITY)
+    return fail(RPSF_E_UNSUPPORTED, "an adjoint plan has no saturation branch (the mask depends on the image)");
   p->sat_threshold = threshold;
   p->sat_dilation = dilation;
   p->sat_width = neighborhood_width;
@@ -1530,14 +1674,10 @@ int sat_restore_launch(rpsf_plan* p, const void* image, void* out, int64_t out_p
   LAUNCH((int)cudaGetLastError());
   return RPSF_OK;
 }
-}  // namespace
 
-extern "C" {
-
-int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
-                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
-                      int batch, int stages, void* stream_v) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                 int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
+                 int batch, int stages, void* stream_v) {
   if (p->row_end == p->row_begin && stages >= 3) return RPSF_OK;      // an empty band (more ranks than half-patch rows): nothing to write
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   rpsf_transform* t = p->tr;
@@ -1669,7 +1809,8 @@ int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
     if (ev) CU(cudaEventRecord(ev[3], s));
     return restore();
   }
-  LAUNCH(t->ops->k2(t->dtype, p->workspace, t->kmain, t->knyq, p->active_dev, t->tw, g, batch, t->sm_count, s));
+  LAUNCH(t->ops->k2(t->dtype, p->workspace, p->adjoint ? t->kconj_main : t->kmain, p->adjoint ? t->kconj_nyq : t->knyq,
+                    p->active_dev, t->tw, g, batch, t->sm_count, s));
   if (ev) CU(cudaEventRecord(ev[2], s));
   if (stages < 3) return RPSF_OK;
   if (!p->mirrors.empty() && (!use_stream || sat))
@@ -1702,6 +1843,57 @@ int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
   return restore();
 }
 
+// Aᵀ y: y (whole frames) -> interior of the zero-bordered box, the forward kernels on the box with conj(Kh), fold
+template <typename T>
+int apply_adjoint(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                  int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                  cudaStream_t s) {
+  rpsf_transform* t = p->tr;
+  if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (!t->has_kernel) return fail(RPSF_E_NO_KERNEL, "transfer kernel not loaded (call rpsf_transform_set_kernel)");
+  if (batch < 1 || batch > p->max_batch)
+    return fail(RPSF_E_INVALID_ARGUMENT, "batch %d outside [1, max_batch=%d]", batch, p->max_batch);
+  if (img_row0 != 0 || img_rows != p->frame_H || out_row0 != 0)
+    return fail(RPSF_E_INVALID_ARGUMENT, "an adjoint plan takes and writes whole frames (row0 = 0, rows = %d)", p->frame_H);
+  if (img_pitch < p->frame_W || out_pitch < p->frame_W) return fail(RPSF_E_INCORRECT_SHAPE, "row pitch smaller than frame width");
+  DeviceGuard guard(t->device);
+  const int H = p->frame_H, W = p->frame_W;
+  const long long box_stride = (long long)p->H * p->box_pitch;
+  // the part of the frame inside the box; the rest of y meets no patch
+  const int r0 = std::max(0, p->box_y0), r1 = std::min(H, p->box_y0 + p->H);
+  const int c0 = std::max(0, p->box_x0), c1 = std::min(W, p->box_x0 + p->W);
+  if (r1 > r0 && c1 > c0) {
+    const dim3 grid((unsigned)((c1 - c0 + 255) / 256), (unsigned)std::min(r1 - r0, 1024), (unsigned)batch);
+    adjoint_copy_in<T><<<grid, 256, 0, s>>>((const T*)image + (long long)r0 * img_pitch + c0, img_pitch, img_frame_stride,
+                                            r1 - r0, c1 - c0,
+                                            (T*)p->box_in + (long long)(r0 - p->box_y0) * p->box_pitch + (c0 - p->box_x0),
+                                            p->box_pitch, box_stride);
+    LAUNCH((int)cudaGetLastError());
+  }
+  if (int rc = apply_stages(p, p->box_in, p->box_pitch, box_stride, 0, p->H, p->box_out, p->box_pitch, box_stride, 0,
+                            batch, 3, s))
+    return rc;
+  const int* rows = p->fold_rows;
+  const int* cols = p->fold_cols;
+  const dim3 grid((unsigned)((W + 255) / 256), (unsigned)std::min(H, 1024), (unsigned)batch);
+  fold_pad_adjoint<T><<<grid, 256, 0, s>>>((const T*)p->box_out, p->box_pitch, box_stride, rows, rows + H + 1, cols,
+                                           cols + W + 1, (T*)out, out_pitch, out_frame_stride, H, W);
+  LAUNCH((int)cudaGetLastError());
+  return RPSF_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
+                      int batch, int stages, void* stream) {
+  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (p->adjoint) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan runs whole (rpsf_apply)");
+  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
+                      out_row0, batch, stages, stream);
+}
+
 int rpsf_plan_enable_timing(rpsf_plan* p, int enabled) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   p->timing = enabled != 0;
@@ -1729,7 +1921,12 @@ int rpsf_plan_read_timing(rpsf_plan* p, double ms[3], int* calls) {
 int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
                int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
                void* stream) {
-  return rpsf_apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch,
+  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (p->adjoint)
+    return (p->tr->dtype == RPSF_F32 ? apply_adjoint<float> : apply_adjoint<double>)(
+        p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride, out_row0, batch,
+        (cudaStream_t)stream);
+  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch,
                            out_frame_stride, out_row0, batch, 3, stream);
 }
 
@@ -1826,6 +2023,7 @@ extern "C" {
 
 int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out, int out_dtype, int batch) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (p->adjoint) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan takes device pointers (rpsf_apply)");
   if (batch < 1) return fail(RPSF_E_INVALID_ARGUMENT, "batch must be >= 1");
   if (p->row_end == p->row_begin) return RPSF_OK;                      // empty band: no bytes to produce
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");

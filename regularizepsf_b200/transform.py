@@ -82,15 +82,17 @@ class _NativeTransform:
     #: workspaces (75.8 MB per 2048^2 / 256-px frame), so an unbounded cache is an HBM leak
     MAX_PLANS = 6
 
-    def plan(self, height: int, width: int, pad_mode: int, row_begin: int, row_end: int, max_batch: int) -> int:
-        """Plan for this geometry able to take ``max_batch`` frames per call.
+    def plan(self, height: int, width: int, pad_mode: int, row_begin: int, row_end: int, max_batch: int,
+             adjoint: bool = False) -> int:
+        """Plan for this geometry able to take ``max_batch`` frames per call (``adjoint``: the transpose of the
+        whole-frame plan, ``rpsf_plan_create_adjoint``; it has workspaces of its own).
 
         A cached plan of the same geometry is reused when its capacity is in [max_batch, 2 * max_batch]
         (``rpsf_apply`` accepts any batch up to the plan's; the factor keeps a single-frame call off a plan
         whose work lists were cut for large batches).  Plans are evicted least-recently-used beyond
         ``MAX_PLANS``; eviction calls ``rpsf_plan_destroy`` (its ``cudaFree`` waits for work in flight).
         """
-        geometry = (height, width, pad_mode, row_begin, row_end)
+        geometry = (height, width, pad_mode, row_begin, row_end, adjoint)
         exact = geometry + (max_batch,)
         if exact in self._plans:
             if next(reversed(self._plans)) != exact:
@@ -98,15 +100,19 @@ class _NativeTransform:
             return self._plans[exact]
         best = None
         for key in self._plans:
-            if key[:5] == geometry and max_batch <= key[5] <= 2 * max_batch and (best is None or key[5] < best[5]):
+            if key[:-1] == geometry and max_batch <= key[-1] <= 2 * max_batch and (best is None or key[-1] < best[-1]):
                 best = key
         if best is not None:
             plan = self._plans.pop(best)
             self._plans[best] = plan                      # most recently used last
             return plan
         out = ctypes.c_void_p()
-        _native.check(self.lib.rpsf_plan_create(ctypes.byref(out), self.handle, height, width, pad_mode,
-                                                row_begin, row_end, max_batch))
+        if adjoint:
+            _native.check(self.lib.rpsf_plan_create_adjoint(ctypes.byref(out), self.handle, height, width, pad_mode,
+                                                            max_batch))
+        else:
+            _native.check(self.lib.rpsf_plan_create(ctypes.byref(out), self.handle, height, width, pad_mode,
+                                                    row_begin, row_end, max_batch))
         self._plans[geometry + (max_batch,)] = out.value
         while len(self._plans) > self.MAX_PLANS:
             oldest = next(iter(self._plans))
@@ -293,6 +299,8 @@ class ArrayPSFTransform:
         device-to-host copy, which is what bounds a host-to-host call (DESIGN.md section 5).
         """
         del workers
+        if _is_torch_tensor(image) and image.requires_grad and _native.require_cuda().is_grad_enabled():
+            return self._apply_differentiable(image, pad_mode, saturation_threshold, dtype, adjoint=False)
         if (pad_mode == "symmetric" and saturation_threshold == math.inf and dtype is None and out_dtype is None
                 and _is_torch_tensor(image)):
             # the common device-resident call: nothing to normalise (the host side of such a call costs as much as
@@ -316,6 +324,45 @@ class ArrayPSFTransform:
         if image.ndim not in (2, 3):
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {image.shape}")
         return self._apply_host(image, dtype_name, _native.PAD_MODES[pad_mode], out_dtype=out_np.type, sat=sat)
+
+    def apply_adjoint(self, image, pad_mode: str = "symmetric", *, dtype=None):
+        """The transpose of ``apply`` without saturation, a linear map of the image: ``<apply(x), y> = <x,
+        apply_adjoint(y)>``.  For forward modelling and iterative solvers (Landweber, CG on the normal equations), and
+        the backward of ``apply`` under autograd.
+
+        Takes what ``apply`` takes: a numpy array (any real dtype; returns float64) or a CUDA tensor (returns the
+        compute dtype ``dtype``, "float32" by default), shaped (H, W) or (B, H, W).  ``pad_mode`` is one of the five
+        modes with an index map ("symmetric", "reflect", "edge", "wrap", "constant").  A tensor that requires grad
+        gives a differentiable result whose backward is ``apply``.
+        """
+        if pad_mode not in _native.PAD_MODES:
+            raise NotImplementedError(f"apply_adjoint supports the pad modes {sorted(_native.PAD_MODES)}, got {pad_mode!r}")
+        if self._shard_keep is not None:
+            raise NotImplementedError("apply_adjoint needs the kernels of every patch; a sharded transform holds a subset")
+        if _is_torch_tensor(image):
+            if image.requires_grad and _native.require_cuda().is_grad_enabled():
+                return self._apply_differentiable(image, pad_mode, math.inf, dtype, adjoint=True)
+            return self._apply_device(image, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
+        torch = _native.require_cuda()
+        host = np.asarray(image)
+        if host.ndim not in (2, 3):
+            raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {host.shape}")
+        dev = torch.from_numpy(np.ascontiguousarray(host, dtype=np.float64)).to(f"cuda:{torch.cuda.current_device()}")
+        out = self._apply_device(dev, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
+        return out.cpu().numpy().astype(np.float64, copy=False)
+
+    def _apply_differentiable(self, image, pad_mode: str, saturation_threshold: float, dtype, adjoint: bool):
+        """``apply`` / ``apply_adjoint`` of a CUDA tensor that requires grad: a linear map whose backward is the other."""
+        if not (saturation_threshold == math.inf or math.isnan(saturation_threshold)):
+            raise NotImplementedError("apply is not differentiable with a finite saturation_threshold: the mask and "
+                                      "the restored pixels depend on the image")
+        if pad_mode not in _native.PAD_MODES:
+            raise NotImplementedError(f"apply is differentiable for the pad modes {sorted(_native.PAD_MODES)} only; "
+                                      f"{pad_mode!r} is computed by np.pad on the host")
+        if self._shard_keep is not None:
+            raise NotImplementedError("a sharded transform is not differentiable: its transpose needs every patch's kernel")
+        from regularizepsf_b200._autograd import LinearMap
+        return LinearMap.apply(image, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
 
     _NO_SAT = (math.inf, 1, 7)
     _PAD_MATERIALIZED = 5                                  # RPSF_PAD_MATERIALIZED
@@ -372,18 +419,22 @@ class ArrayPSFTransform:
 
     def _apply_device(self, image, dtype_name: str, pad_code: int, row_range: tuple[int, int] | None = None,
                       out=None, sat: tuple = _NO_SAT, mirrors: list[int] | None = None,
-                      frame_rows: tuple[int, int] | None = None):
+                      frame_rows: tuple[int, int] | None = None, adjoint: bool = False):
         """``frame_rows = (first, height)``: ``image`` holds only rows [first, first + image.shape[-2]) of frames that
-        are ``height`` rows tall (a row slab keeps just the rows its patches read: ``plan_info()["rows_read"]``)."""
+        are ``height`` rows tall (a row slab keeps just the rows its patches read: ``plan_info()["rows_read"]``).
+        ``adjoint``: run the transpose (whole frames, no saturation)."""
         torch = _native.require_cuda()
         if not image.is_cuda:
             raise ValueError("apply() takes a numpy array or a CUDA tensor; move the tensor to the GPU first")
         if image.device.index == torch._C._cuda_getDevice():
-            return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows)
+            return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
+                                         adjoint)
         with torch.cuda.device(image.device):             # plans, streams and launches follow the image's device
-            return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows)
+            return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
+                                         adjoint)
 
-    def _apply_device_on(self, torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows=None):
+    def _apply_device_on(self, torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows=None,
+                         adjoint=False):
         nt = self._native_transform(dtype_name, image.device.index)
         want = torch.float32 if dtype_name == "float32" else torch.float64
         squeeze = image.dim() == 2
@@ -409,7 +460,7 @@ class ArrayPSFTransform:
                                           f"stride, got {out.dtype} {tuple(out.shape)}")
         if r1 <= r0:                                       # an empty band: nothing to compute, no native call
             return out[0] if squeeze else out
-        plan = nt.plan(h, w, pad_code, r0, r1, b)
+        plan = nt.plan(h, w, pad_code, r0, r1, b, adjoint=adjoint)
         nt.set_saturation(plan, sat)
         if mirrors:        # device pointers of peer buffers laid out like `out` (distributed.PeerFrames)
             import ctypes
