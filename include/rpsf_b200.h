@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define RPSF_ABI_VERSION 1
+#define RPSF_ABI_VERSION 2
 
 /* status codes */
 #define RPSF_OK 0
@@ -156,15 +156,14 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int height, int width, 
  * It runs the three default kernels on the bounding box of the patch footprints (zero-bordered copy of the input,
  * conj of the transfer kernel, built at the first adjoint plan of `t`) and folds the box onto the frame along the
  * np.pad index map (pad_mode 0..4; RPSF_PAD_MATERIALIZED is RPSF_E_UNSUPPORTED).  rpsf_apply takes whole frames
- * (img_row0 = out_row0 = 0, img_rows = H); rpsf_apply_stages and rpsf_apply_host, a finite saturation threshold,
- * output mirrors and the opt-in fused / paired / single-CTA paths are RPSF_E_UNSUPPORTED on it. */
+ * (img_row0 = out_row0 = 0, img_rows = H); rpsf_apply_stages and rpsf_apply_host, a finite saturation threshold and
+ * output mirrors are RPSF_E_UNSUPPORTED on it. */
 int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int height, int width, int pad_mode, int max_batch);
 int rpsf_plan_destroy(rpsf_plan* p);
 /* info[0]=active patches, [1]=colours, [2]=workspace bytes, [3]=first frame row read,
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,
  * [6]=overlap-add kernel: 2 = streaming chains (registers only), 1 = single-launch row-pair gather
- *      through a shared-memory plane, 0 = one launch per colour class; + 8 when apply runs as the fused
- *      persistent pipeline (rpsf_plan_set_fused),
+ *      through a shared-memory plane, 0 = one launch per colour class,
  * [7]=teams per CTA of the row-pair gather */
 int rpsf_plan_info(const rpsf_plan* p, int64_t info[8]);
 /* overlap-add kernel choice: 0 = automatic (streaming chains when every owned row pair is a chain of
@@ -176,43 +175,10 @@ int rpsf_plan_set_overlap_mode(rpsf_plan* p, int mode);
  * one-row-pair-per-team kernel with direct loads (test hook; same arithmetic up to rounding) */
 int rpsf_plan_set_gather_mode(rpsf_plan* p, int mode);
 
-/* Patches whose packed half-spectrum fits one SM's shared memory (P <= 128 in float32, P <= 64 in float64) and whose
- * corners lie on multiples of P/2 (every calculate_covering grid) take a two-launch path: one CTA carries a patch of a
- * frame through gather, window, both FFT axes, the transfer multiply, both inverse axes and the second window without
- * its spectrum ever leaving shared memory, writes the corrected P x P plane, and an elementwise kernel adds the planes
- * that cover each output tile in list order — the reference's own `+=` order (transform.py:167-169).  Measured at
- * 1024^2 / 128 px: 29.0 us per frame at 8 frames per call against 22.2 for the three kernels, 39.8 against 41.0 for one
- * frame: opt-in.  0 = automatic and 1 = never select the three kernels, 2 = this path or RPSF_E_UNSUPPORTED;
- * RPSF_SMALL=1 makes 2 the default of new plans that have the tables. */
-int rpsf_plan_set_small_mode(rpsf_plan* p, int mode);
-
-/* column pass choice.  2 = the PAIRED pass (k2_chain; coverings, else RPSF_E_UNSUPPORTED): a CTA walks the patches that
- * share a corner column top to bottom and writes, per band of P/2 output rows, the row-windowed sum of the two patches
- * that overlap there, so the column pass writes half as much and the overlap-add reads half as much.  Measured at 2048^2
- * / 256 px: 21 % less DRAM traffic, 2-5 % more throughput from 8 frames per call, slower below; the chain kernel is no
- * longer HBM-bound (0.54 of the peak), so 0 = automatic and 1 = classic both select the in-place column pass with the
- * pair sum in the overlap-add kernel.  The two agree to rounding (different association of the same sum).
- * RPSF_PAIRED=1 makes 2 the default of new plans that have the tables.
- * rpsf_plan_column_info: info[0] = 1 if the next apply of this plan takes the paired pass, info[1] = bytes of the
- * paired workspace per frame (0 if the plan has none). */
-int rpsf_plan_set_column_mode(rpsf_plan* p, int mode);
+/* column pass: info[0] = 0 (the in-place column pass over the spectrum workspace, the only one there is) and
+ * info[1] = 0 (bytes per frame of a column-pass workspace of its own: none).  Kept so that callers that report
+ * the column pass keep working. */
 int rpsf_plan_column_info(const rpsf_plan* p, int64_t info[2]);
-
-/* pipeline choice.  2 = run apply as ONE persistent cooperative launch whose spectrum hand-overs stay in L2
- * (rpsf_fused.cuh; coverings with 256-px patches in float32 — RPSF_E_UNSUPPORTED otherwise): DRAM traffic falls from
- * 346 to 121 MB per 2048^2 frame, bit-identical results, but measured slower than the three stand-alone kernels
- * (DESIGN.md section 4), which 0 = automatic and 1 = never therefore both select today.  RPSF_FUSED=1 in the
- * environment makes 2 the default of new plans, RPSF_FUSED=0 leaves the pipeline's tables out of the plan. */
-int rpsf_plan_set_fused(rpsf_plan* p, int mode);
-/* pipeline statistics of the fused launch (diagnostics; a few atomics per wait when enabled).  Reads and resets the
- * counters into out[8] (may be NULL), then switches collection on or off: [0..2] SM cycles the roles K1 / K2 / K3 spent
- * waiting on a producer / consumer counter (one sample per warp or column group), [3..5] cycles from role start to
- * role end summed over the role's warps, [6] column units whose tile could not be prefetched, [7] column units. */
-int rpsf_plan_fused_stats(rpsf_plan* p, int enable, uint64_t out[8]);
-/* timeline of the fused launch (diagnostics): reads into out[3][max_batch * n_bands] the %globaltimer nanoseconds at
- * which every band (frame-major sequence) was completed by role K1, by K2 and freed by K3 during the LAST launch, then
- * clears the record and switches collection on or off.  out may be NULL. */
-int rpsf_plan_fused_trace(rpsf_plan* p, int enable, uint64_t* out, int64_t out_len);
 
 /* ---- saturation arguments of apply (transform.py:88-90,125-138,171-172) ---------------------
  * threshold = +inf (the default) disables the branch.  Otherwise every apply on this plan pads

@@ -51,12 +51,7 @@ SIGNATURES = {
     "rpsf_plan_info": (_i, [_vp, ctypes.POINTER(_i64)]),
     "rpsf_plan_set_overlap_mode": (_i, [_vp, _i]),
     "rpsf_plan_set_gather_mode": (_i, [_vp, _i]),
-    "rpsf_plan_set_small_mode": (_i, [_vp, _i]),
-    "rpsf_plan_set_column_mode": (_i, [_vp, _i]),
     "rpsf_plan_column_info": (_i, [_vp, ctypes.POINTER(_i64)]),
-    "rpsf_plan_set_fused": (_i, [_vp, _i]),
-    "rpsf_plan_fused_stats": (_i, [_vp, _i, ctypes.POINTER(ctypes.c_uint64)]),
-    "rpsf_plan_fused_trace": (_i, [_vp, _i, ctypes.POINTER(ctypes.c_uint64), _i64]),
     "rpsf_plan_set_saturation": (_i, [_vp, _d, _i, _i]),
     "rpsf_plan_set_output_mirrors": (_i, [_vp, _i, ctypes.POINTER(_vp)]),
     "rpsf_ipc_alloc": (_i, [ctypes.POINTER(_vp), _i64, _i, ctypes.c_char_p]),

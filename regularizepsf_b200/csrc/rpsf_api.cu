@@ -201,15 +201,8 @@ struct StreamTables {
   bool ok = false;
 };
 
-// `slots` (fused pipeline only): per active patch (band, index in band).  Then tasks are ordered row-pair major
-// (a warp item = the same chunk of `tpw` consecutive row pairs), chains are cut into `fused_chunks` pieces, item
-// codes name ring slots (FUSED_*_SHIFT) and every task carries the first / last band it reads in pad0 / pad1.
 StreamTables build_stream_tables(const std::vector<int2>& corners, const std::vector<int>& colours, int P, int W,
-                                 int row_begin, int row_end, int tpw, long long team_slots, int max_batch,
-                                 const std::vector<int2>* slots = nullptr, int fused_chunks = 0,
-                                 const std::vector<int>* paired_band = nullptr) {
-  // `paired_band` (paired column pass, k2_chain): per active patch the band of the paired workspace that holds its
-  // UPPER half (the lower half is in the next band).  A group then is one item, code = band * P/4 + row pair in band.
+                                 int row_begin, int row_end, int tpw, long long team_slots, int max_batch) {
   StreamTables st;
   const int half = P / 2;
   if (corners.empty() || row_end <= row_begin) return st;
@@ -264,22 +257,8 @@ StreamTables build_stream_tables(const std::vector<int2>& corners, const std::ve
     }
   }
   std::vector<std::vector<int>> shape;        // per task: items per computed group
-  if (slots) chunks = std::max<long long>(1, std::min<long long>(fused_chunks, (long long)min_groups));
-  // visiting order of (chunk, row pair): chunk major for the stand-alone kernel; for the fused pipeline blocks of
-  // `tpw` row pairs, chunk by chunk, so that work becomes ready top to bottom
-  std::vector<std::pair<long long, int>> visit;
-  if (!slots) {
-    for (long long chn = 0; chn < chunks; ++chn)
-      for (int rp = 0; rp < n_rp; ++rp) visit.push_back({chn, rp});
-  } else {
-    for (int rp0 = 0; rp0 < n_rp; rp0 += tpw)
-      for (long long chn = 0; chn < chunks; ++chn)
-        for (int rp = rp0; rp < std::min(n_rp, rp0 + tpw); ++rp) visit.push_back({chn, rp});
-  }
-  for (const auto& vis : visit) {
-    {
-      const long long chn = vis.first;
-      const int rp = vis.second;
+  for (long long chn = 0; chn < chunks; ++chn) {
+    for (int rp = 0; rp < n_rp; ++rp) {
       const auto& ch = chains[rp];
       const size_t n_g = ch.size();
       const size_t gb = n_g * chn / chunks, ge = n_g * (chn + 1) / chunks;
@@ -291,34 +270,9 @@ StreamTables build_stream_tables(const std::vector<int2>& corners, const std::ve
       t.item_begin = (int)st.codes.size();
       t.flags = (gb > 0 ? TASK_SEAM : 0) | (ge == n_g ? TASK_LAST : 0);
       std::vector<int> sh;
-      if (slots) {
-        int lo = INT_MAX, hi = INT_MIN;
-        for (size_t gi = g0; gi < ge; ++gi)
-          for (int item : ch[gi].items) {
-            const int band = (*slots)[item / half].x;
-            lo = std::min(lo, band); hi = std::max(hi, band);
-          }
-        if (hi - lo > 7) return StreamTables{};                // the item code has 3 bits for the band offset
-        t.pad0 = lo; t.pad1 = hi;
-      }
       for (size_t gi = g0; gi < ge; ++gi) {
-        if (paired_band) {
-          const int item = ch[gi].items[0], a = item / half, pair = item % half;
-          const bool upper = 2 * pair < half;
-          const unsigned code = (unsigned)(((*paired_band)[a] + (upper ? 0 : 1)) * (half / 2) + (upper ? pair : pair - half / 2));
-          st.codes.push_back(code | ITEM_LAST_OF_GROUP);
-          sh.push_back(1);
-          continue;
-        }
-        for (size_t k = 0; k < ch[gi].items.size(); ++k) {
-          unsigned code = (unsigned)ch[gi].items[k];
-          if (slots) {
-            const int2 sl = (*slots)[ch[gi].items[k] / half];
-            code = (unsigned)(ch[gi].items[k] % half) | ((unsigned)sl.y << FUSED_IDX_SHIFT) |
-                   ((unsigned)(sl.x - t.pad0) << FUSED_BAND_SHIFT);
-          }
-          st.codes.push_back(code | (k + 1 == ch[gi].items.size() ? ITEM_LAST_OF_GROUP : 0u));
-        }
+        for (size_t k = 0; k < ch[gi].items.size(); ++k)
+          st.codes.push_back((unsigned)ch[gi].items[k] | (k + 1 == ch[gi].items.size() ? ITEM_LAST_OF_GROUP : 0u));
         sh.push_back((int)ch[gi].items.size());
       }
       t.n_steps = (int)st.codes.size() - t.item_begin;
@@ -405,32 +359,8 @@ struct rpsf_plan {
   StreamTask* stasks_dev = nullptr;
   unsigned* scodes_dev = nullptr;
   int n_warp_items = 0;
-  void* workspace = nullptr;       // allocated at the first unfused apply (the fused pipeline only needs its ring)
+  void* workspace = nullptr;       // allocated at the first apply
   size_t workspace_bytes = 0;
-  // small patches (rpsf_small.cuh): one CTA per patch-frame + overlap-add of the patch planes
-  bool small_ok = false;
-  int small_mode = 0;              // 0 = automatic (= the three kernels today), 1 = never, 2 = the single-CTA path
-  SmallTile* small_tiles_dev = nullptr; int* small_cover_dev = nullptr; int small_n_tiles = 0, small_max_cover = 0;
-  void* planes = nullptr; size_t planes_bytes = 0;
-  // paired column pass (k2_chain + k3_stream_paired): chains of patches sharing a corner column, the workspace of
-  // their band sums, and overlap-add tables with one item per group
-  bool paired_ok = false;
-  int column_mode = 0;             // 0 = automatic (= classic today), 1 = classic in-place column pass, 2 = paired
-  ChainDesc* chains_dev = nullptr; int n_segments = 0;
-  int* chain_patches_dev = nullptr;
-  long long bands_total = 0;
-  void* paired = nullptr; size_t paired_bytes = 0;
-  StreamTask* ptasks_dev = nullptr; unsigned* pcodes_dev = nullptr; int p_warp_items = 0;
-  // fused persistent pipeline (rpsf_fused.cuh): ring of band slots in place of the workspace, counters, its own
-  // overlap-add tables (row-pair major, item codes that name ring slots)
-  bool fused_ok = false;
-  int fused_mode = 0;              // 0 = automatic (the three kernels: they are faster), 1 = never, 2 = the fused pipeline
-  FusedGeom fg{};
-  void* ring = nullptr; size_t ring_bytes = 0;
-  uint64_t* fstats = nullptr; uint64_t* ftrace = nullptr;
-  int* fcounters = nullptr; size_t fcounter_ints = 0;
-  int2* fslot_dev = nullptr; int* fbands_dev = nullptr;   // fbands: [band_units | band_tasks]
-  StreamTask* ftasks_dev = nullptr; unsigned* fcodes_dev = nullptr; int f_warp_items = 0;
   int img_lo = 0, img_hi = 0;      // resident frame rows needed: [img_lo, img_hi)
   // host path: a ring of HOST_SLOTS chunk buffers so the upload of chunk i+1, the kernels of
   // chunk i and the download of chunk i-1 run concurrently on three streams (two copy engines)
@@ -948,7 +878,6 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
   const int P = t->P;
   if (!box)
     if (int rc = check_corners(t, H, W)) return rc;
-  const bool adjoint = box != nullptr;
   std::vector<int2> tcorners(t->corners);
   // the region a patch must touch to take part, in plan coordinates: the owned band, or the real frame inside the box
   int reach_r0 = row_begin, reach_r1 = row_end, reach_c0 = 0, reach_c1 = W;
@@ -969,8 +898,7 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
   std::vector<std::vector<int>> items(std::max(t->n_colours, 1));
   long long colour0_area = 0;
   int lo = H, hi = 0;
-  // active patches in (corner row, corner column) order: patches that share a corner row are consecutive (the
-  // bands of the fused pipeline), and the row kernels walk the frame top to bottom
+  // active patches in (corner row, corner column) order: the row kernels walk the frame top to bottom
   std::vector<int> order;
   for (int i = 0; i < t->n; ++i) {
     const int2 c = tcorners[i];
@@ -1139,202 +1067,9 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
     }
   }
   tick("streaming overlap-add tables");
-  // ---- small patches: output tiles of P/2 x P/2 and the patches that cover each, in list order (the reference's `+=` order)
-  if (const char* v = getenv("RPSF_SMALL")) p->small_mode = strcmp(v, "0") == 0 ? 1 : strcmp(v, "1") == 0 ? 2 : 0;
-  if (!adjoint && !embedded && p->n_active > 0 && P % 2 == 0 && t->ops->small_ok(t->dtype) && row_end > row_begin) {
-    const int ts = P / 2;
-    bool aligned = true;
-    for (const int2& c : corners) aligned = aligned && (((c.x % ts) + ts) % ts == 0) && (((c.y % ts) + ts) % ts == 0);
-    if (aligned) {
-      // every patch covers the 2 x 2 tiles under it (corners are tile-aligned): one pass over the patches
-      const int ty0 = row_begin / ts, ty1 = (row_end + ts - 1) / ts, ntx = (W + ts - 1) / ts;
-      std::vector<std::vector<std::pair<int, int>>> hits((size_t)(ty1 - ty0) * ntx);      // (list index, active index)
-      for (int a = 0; a < p->n_active; ++a) {
-        const int cy = (int)std::floor((double)corners[a].x / ts), cx = (int)std::floor((double)corners[a].y / ts);
-        for (int dy = 0; dy < 2; ++dy)
-          for (int dx = 0; dx < 2; ++dx) {
-            const int ty = cy + dy, tx = cx + dx;
-            if (ty >= ty0 && ty < ty1 && tx >= 0 && tx < ntx) hits[(size_t)(ty - ty0) * ntx + tx].push_back({active[a], a});
-          }
-      }
-      std::vector<SmallTile> tiles;
-      std::vector<std::vector<int>> cover;
-      size_t most = 0;
-      for (int ty = ty0; ty < ty1; ++ty)
-        for (int tx = 0; tx < ntx; ++tx) {
-          auto& h = hits[(size_t)(ty - ty0) * ntx + tx];
-          std::sort(h.begin(), h.end());
-          tiles.push_back(SmallTile{ty * ts, tx * ts});
-          cover.emplace_back();
-          for (auto& e : h) cover.back().push_back(e.second);
-          most = std::max(most, h.size());
-        }
-      const int mc = (int)std::max<size_t>(most, 1);
-      std::vector<int> flat(tiles.size() * (size_t)mc, -1);
-      for (size_t i = 0; i < tiles.size(); ++i) std::copy(cover[i].begin(), cover[i].end(), flat.begin() + i * mc);
-      if (cudaMalloc(&p->small_tiles_dev, sizeof(SmallTile) * tiles.size()) != cudaSuccess) return destroy_fail("output tiles");
-      if (cudaMalloc(&p->small_cover_dev, sizeof(int) * flat.size()) != cudaSuccess) return destroy_fail("tile cover lists");
-      if (cudaMemcpy(p->small_tiles_dev, tiles.data(), sizeof(SmallTile) * tiles.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      if (cudaMemcpy(p->small_cover_dev, flat.data(), sizeof(int) * flat.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      p->small_n_tiles = (int)tiles.size(); p->small_max_cover = mc;
-      p->planes_bytes = (size_t)max_batch * p->n_active * P * P * real_size(t->dtype);
-      p->small_ok = true;
-    }
-  }
-  tick("single-CTA tile lists");
-  // ---- paired column pass: chains of active patches that share a corner column, corner rows P/2 apart
-  if (const char* v = getenv("RPSF_PAIRED")) p->column_mode = strcmp(v, "1") == 0 ? 2 : 0;
-  if (!adjoint && p->stream_ok && !embedded && t->ops->chain_ok(t->dtype) && (P / 2) % 2 == 0) {
-    std::map<int, std::vector<int>> by_col;                       // corner column -> active patches, by corner row
-    for (int a = 0; a < p->n_active; ++a) by_col[corners[a].y].push_back(a);
-    bool ok = true;
-    std::vector<int> chain_patches, band_upper(p->n_active, 0);
-    struct Chain { int first, length, band0; };
-    std::vector<Chain> chains;
-    long long bands = 0;
-    size_t min_len = SIZE_MAX;
-    for (auto& kv : by_col) {
-      const auto& list = kv.second;
-      for (size_t i = 1; i < list.size() && ok; ++i) ok = corners[list[i]].x == corners[list[i - 1]].x + P / 2;
-      if (!ok) break;
-      chains.push_back({(int)chain_patches.size(), (int)list.size(), (int)bands});
-      for (size_t i = 0; i < list.size(); ++i) { band_upper[list[i]] = (int)(bands + (long long)i); chain_patches.push_back(list[i]); }
-      bands += (long long)list.size() + 1;
-      min_len = std::min(min_len, list.size());
-    }
-    ok = ok && !chains.empty() && bands * (P / 4) < (1LL << 30);
-    StreamTables pt;
-    if (ok) {
-      std::vector<int> colours(active.size());
-      for (size_t a = 0; a < active.size(); ++a) colours[a] = t->colour[active[a]];
-      const int tpw = t->ops->stream_tpw();
-      pt = build_stream_tables(corners, colours, P, W, row_begin, row_end, tpw, (long long)t->sm_count * 16 * tpw, max_batch,
-                               nullptr, 0, &band_upper);
-      ok = pt.ok;
-    }
-    if (ok) {
-      // segments per chain: a segment that does not start its chain recomputes one patch for its carry; pick the count
-      // that minimises (steps per segment) x (rounds of CTAs over the 2-per-SM slots)
-      const int C = std::min(16, P / 2), n1 = P == 16 || P == 32 ? 4 : P == 64 || P == 128 ? 8 : 16;
-      const int slots_per_cta = std::max(1, 256 / (C * n1)), tg = std::max(1, (P / 2) / C / slots_per_cta);
-      const long long cta_slots = 2LL * t->sm_count;
-      long long segs = 1, best = LLONG_MAX;
-      for (long long sgm = 1; sgm <= (long long)min_len; ++sgm) {
-        const long long steps = ((long long)min_len + sgm - 1) / sgm + (sgm > 1 ? 1 : 0);
-        const long long rounds = ((long long)chains.size() * sgm * tg * max_batch + cta_slots - 1) / cta_slots;
-        if (steps * rounds < best) { best = steps * rounds; segs = sgm; }
-      }
-      if (const char* v = getenv("RPSF_CHAIN_SEGMENTS")) segs = std::max(1, std::min(atoi(v), (int)min_len));
-      std::vector<ChainDesc> descs;
-      for (const Chain& c : chains)
-        for (long long sgm = 0; sgm < segs; ++sgm) {
-          const int b = (int)((long long)c.length * sgm / segs), e = (int)((long long)c.length * (sgm + 1) / segs);
-          if (e > b) descs.push_back(ChainDesc{c.first, c.length, c.band0, b, e - b});
-        }
-      if (cudaMalloc(&p->chains_dev, sizeof(ChainDesc) * descs.size()) != cudaSuccess) return destroy_fail("chain table");
-      if (cudaMalloc(&p->chain_patches_dev, sizeof(int) * chain_patches.size()) != cudaSuccess) return destroy_fail("chain patches");
-      if (cudaMalloc(&p->ptasks_dev, sizeof(StreamTask) * pt.tasks.size()) != cudaSuccess) return destroy_fail("paired tasks");
-      if (cudaMalloc(&p->pcodes_dev, sizeof(unsigned) * pt.codes.size()) != cudaSuccess) return destroy_fail("paired item codes");
-      if (cudaMemcpy(p->chains_dev, descs.data(), sizeof(ChainDesc) * descs.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      if (cudaMemcpy(p->chain_patches_dev, chain_patches.data(), sizeof(int) * chain_patches.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      if (cudaMemcpy(p->ptasks_dev, pt.tasks.data(), sizeof(StreamTask) * pt.tasks.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      if (cudaMemcpy(p->pcodes_dev, pt.codes.data(), sizeof(unsigned) * pt.codes.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-      p->n_segments = (int)descs.size();
-      p->bands_total = bands;
-      p->p_warp_items = pt.n_warp_items;
-      p->paired_bytes = (size_t)max_batch * bands * (P / 2) * (P / 2) * 2 * real_size(t->dtype);
-      p->paired_ok = true;
-    }
-  }
   p->workspace_bytes = (size_t)max_batch * p->n_active * P * (P / 2) * 2 * real_size(t->dtype);
-  tick("paired column tables");
-  // ---- fused persistent pipeline: bands = runs of equal corner row in the (sorted) active list
-  int finfo[4] = {0, 0, 0, 0};
-  t->ops->fused_info(t->dtype, finfo);
-  // Measured (profiles/r02_fused_*.txt): the fused pipeline cuts DRAM traffic from 346 to 121 MB per 2048^2 frame but
-  // is slower than the three stand-alone kernels, so it is opt-in: RPSF_FUSED=1 or rpsf_plan_set_fused(plan, 2).
-  const char* fenv = getenv("RPSF_FUSED");
-  if (fenv && strcmp(fenv, "1") == 0) p->fused_mode = 2;
-  if (!adjoint && finfo[0] && p->stream_ok && !(fenv && strcmp(fenv, "0") == 0)) {
-    std::vector<int2> slots(p->n_active);
-    std::vector<int> band_size;
-    for (int a = 0; a < p->n_active; ++a) {
-      if (a == 0 || corners[a].x != corners[a - 1].x) band_size.push_back(0);
-      slots[a] = make_int2((int)band_size.size() - 1, band_size.back()++);
-    }
-    const int n_bands = (int)band_size.size();
-    const int band_cap = *std::max_element(band_size.begin(), band_size.end());
-    const int min_band = *std::min_element(band_size.begin(), band_size.end());
-    const size_t patch_bytes = (size_t)P * (P / 2) * 2 * real_size(t->dtype);
-    int ring = 8, chunks = 4, split[3] = {0, 0, 0};
-    if (const char* v = getenv("RPSF_FUSED_RING")) ring = atoi(v);
-    if (const char* v = getenv("RPSF_FUSED_CHUNKS")) chunks = atoi(v);
-    if (const char* v = getenv("RPSF_FUSED_SPLIT")) sscanf(v, "%d,%d,%d", &split[0], &split[1], &split[2]);
-    if (split[0] <= 0 || split[1] <= 0 || split[2] <= 0 || split[0] + split[1] + split[2] > t->sm_count) {
-      // shares of the three roles measured on the stand-alone kernels (about 0.30 : 0.42 : 0.28)
-      split[0] = std::max(1, (int)std::lround(t->sm_count * 0.31));
-      split[2] = std::max(1, (int)std::lround(t->sm_count * 0.27));
-      split[1] = t->sm_count - split[0] - split[2];
-    }
-    // A K1 warp holds up to `stages` + 1 items it has not published yet while it asks for the slot of the next
-    // one, and a group of items is published when its slowest warp is through: what the role holds that way must
-    // stay inside the ring's slack, or a warp could wait for a slot that only its own CTA's unfinished items can free
-    const long long ahead_items = (long long)(finfo[3] + finfo[3] / 2) * split[0];
-    const long long ahead_bands = (ahead_items + (long long)min_band * finfo[1] - 1) / ((long long)min_band * finfo[1]) + 1;
-    while (ring < ahead_bands + 2 && ring < 1024) ring *= 2;
-    bool ok = (ring & (ring - 1)) == 0 && ring >= 4 && (size_t)ring * band_cap * patch_bytes <= (size_t)96 << 20 &&
-              band_cap < (1 << (FUSED_BAND_SHIFT - FUSED_IDX_SHIFT)) && t->sm_count >= 12 && ahead_bands <= ring - 2;
-    StreamTables ft;
-    if (ok) {
-      std::vector<int> colours(active.size());
-      for (size_t a = 0; a < active.size(); ++a) colours[a] = t->colour[active[a]];
-      ft = build_stream_tables(corners, colours, P, W, row_begin, row_end, t->ops->stream_tpw(), 0, max_batch, &slots,
-                               std::max(chunks, 1));
-      ok = ft.ok;
-    }
-    if (ok) {
-      std::vector<int> bands(2 * (size_t)n_bands, 0);            // [band_units | band_tasks]
-      for (int b = 0; b < n_bands; ++b) bands[b] = band_size[b] * finfo[2];
-      int span = 0;
-      for (const StreamTask& tk : ft.tasks)
-        if (tk.n_steps > 0) {
-          for (int b = tk.pad0; b <= tk.pad1; ++b) ++bands[n_bands + b];
-          span = std::max(span, tk.pad1 - tk.pad0 + 1);
-        }
-      ok = span + 2 <= ring;                                      // a task's bands, the band in K2 and the band K1 fills
-      for (int b = 0; b < n_bands && ok; ++b) ok = bands[n_bands + b] > 0;   // every band is read (else its slot never frees)
-      if (ok) {
-        p->ring_bytes = (size_t)ring * band_cap * patch_bytes;
-        p->fcounter_ints = (size_t)max_batch * (p->n_active + 2 * (size_t)n_bands) + 4;
-        if (cudaMalloc(&p->ring, p->ring_bytes) != cudaSuccess) return destroy_fail("spectrum ring");
-        if (cudaMalloc(&p->fcounters, p->fcounter_ints * sizeof(int)) != cudaSuccess) return destroy_fail("pipeline counters");
-        if (cudaMalloc(&p->fslot_dev, sizeof(int2) * slots.size()) != cudaSuccess) return destroy_fail("band slots");
-        if (cudaMalloc(&p->fbands_dev, sizeof(int) * bands.size()) != cudaSuccess) return destroy_fail("band targets");
-        if (cudaMalloc(&p->ftasks_dev, sizeof(StreamTask) * ft.tasks.size()) != cudaSuccess) return destroy_fail("fused tasks");
-        if (cudaMalloc(&p->fcodes_dev, sizeof(unsigned) * ft.codes.size()) != cudaSuccess) return destroy_fail("fused item codes");
-        if (cudaMemcpy(p->fslot_dev, slots.data(), sizeof(int2) * slots.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-        if (cudaMemcpy(p->fbands_dev, bands.data(), sizeof(int) * bands.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-        if (cudaMemcpy(p->ftasks_dev, ft.tasks.data(), sizeof(StreamTask) * ft.tasks.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-        if (cudaMemcpy(p->fcodes_dev, ft.codes.data(), sizeof(unsigned) * ft.codes.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
-        p->f_warp_items = ft.n_warp_items;
-        FusedGeom& fg = p->fg;
-        fg.n_bands = n_bands; fg.ring_mask = ring - 1; fg.band_cap = band_cap;
-        fg.n1 = split[0]; fg.n2 = split[1]; fg.n3 = split[2];
-        fg.units_per_patch = finfo[2]; fg.n_active = p->n_active; fg.stats = nullptr; fg.trace = nullptr; fg.trace_stride = 0;
-        fg.solo = 0;
-        if (const char* v = getenv("RPSF_FUSED_SOLO")) fg.solo = atoi(v);
-        fg.slot = p->fslot_dev; fg.band_units = p->fbands_dev; fg.band_tasks = p->fbands_dev + n_bands;
-        fg.ready1 = p->fcounters;
-        fg.ready2 = fg.ready1 + (size_t)max_batch * p->n_active;
-        fg.done3 = fg.ready2 + (size_t)max_batch * n_bands;
-        fg.ticket = reinterpret_cast<unsigned*>(fg.done3 + (size_t)max_batch * n_bands);
-        p->fused_ok = true;
-      }
-    }
-  }
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { rpsf_plan_destroy(p); return fail(RPSF_E_CUDA, "plan upload failed: %s", cudaGetErrorString(e)); }
-  tick("fused pipeline tables");
   *out = p;
   return RPSF_OK;
 }
@@ -1435,10 +1170,6 @@ int rpsf_plan_destroy(rpsf_plan* p) {
   cudaFree(p->active_dev); cudaFree(p->corners_dev); cudaFree(p->workspace);
   cudaFree(p->tiles_dev); cudaFree(p->groups_dev); cudaFree(p->gitems_dev);
   cudaFree(p->stasks_dev); cudaFree(p->scodes_dev);
-  cudaFree(p->small_tiles_dev); cudaFree(p->small_cover_dev); cudaFree(p->planes);
-  cudaFree(p->chains_dev); cudaFree(p->chain_patches_dev); cudaFree(p->paired); cudaFree(p->ptasks_dev); cudaFree(p->pcodes_dev);
-  cudaFree(p->ring); cudaFree(p->fstats); cudaFree(p->ftrace); cudaFree(p->fcounters); cudaFree(p->fslot_dev); cudaFree(p->fbands_dev);
-  cudaFree(p->ftasks_dev); cudaFree(p->fcodes_dev);
   cudaFree(p->sat_pf); cudaFree(p->sat_mask[0]); cudaFree(p->sat_mask[1]); cudaFree(p->sat_list);
   cudaFree(p->sat_rows); cudaFree(p->sat_flags);
   cudaFree(p->box_in); cudaFree(p->box_out); cudaFree(p->fold_rows); cudaFree(p->fold_cols);
@@ -1467,7 +1198,6 @@ int rpsf_plan_info(const rpsf_plan* p, int64_t info[8]) {
   if (!p || !info) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   const bool stream = p->stream_ok && p->k3_stream && !p->force_phases && !p->force_gather;
   info[6] = stream ? 2 : (p->gather && !p->force_phases) ? 1 : 0; info[7] = p->teams;
-  if (stream && p->fused_ok && p->fused_mode == 2 && p->k1_stream) info[6] += 8;
   info[0] = p->n_active; info[1] = p->tr->n_colours; info[2] = (int64_t)p->workspace_bytes;
   info[3] = p->img_lo; info[4] = p->img_hi; info[5] = p->colour0_covers ? 1 : 0;
   return RPSF_OK;
@@ -1490,74 +1220,9 @@ int rpsf_plan_workspace(const rpsf_plan* p, void** ptr, int64_t* bytes) {
   return RPSF_OK;
 }
 
-int rpsf_plan_fused_stats(rpsf_plan* p, int enable, uint64_t out[8]) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (!p->fused_ok) return fail(RPSF_E_UNSUPPORTED, "this plan has no fused pipeline");
-  DeviceGuard guard(p->tr->device);
-  if (out) {
-    for (int i = 0; i < 8; ++i) out[i] = 0;
-    if (p->fstats) {
-      CU(cudaDeviceSynchronize());
-      CU(cudaMemcpy(out, p->fstats, 8 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-      CU(cudaMemset(p->fstats, 0, 8 * sizeof(uint64_t)));
-    }
-  }
-  if (enable && !p->fstats) {
-    CU(cudaMalloc((void**)&p->fstats, 8 * sizeof(uint64_t)));
-    CU(cudaMemset(p->fstats, 0, 8 * sizeof(uint64_t)));
-  }
-  p->fg.stats = enable ? reinterpret_cast<unsigned long long*>(p->fstats) : nullptr;
-  return RPSF_OK;
-}
-
-int rpsf_plan_fused_trace(rpsf_plan* p, int enable, uint64_t* out, int64_t out_len) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (!p->fused_ok) return fail(RPSF_E_UNSUPPORTED, "this plan has no fused pipeline");
-  DeviceGuard guard(p->tr->device);
-  const size_t stride = (size_t)p->max_batch * p->fg.n_bands, n = 4 * stride;
-  if (out) {
-    if (!p->ftrace || out_len < (int64_t)(3 * stride)) return fail(RPSF_E_INVALID_ARGUMENT, "trace is off or the buffer is too small (%zu needed)", 3 * stride);
-    CU(cudaDeviceSynchronize());
-    CU(cudaMemcpy(out, p->ftrace, 3 * stride * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-  }
-  if (enable && !p->ftrace) CU(cudaMalloc((void**)&p->ftrace, n * sizeof(uint64_t)));
-  if (p->ftrace) CU(cudaMemset(p->ftrace, 0, n * sizeof(uint64_t)));
-  p->fg.trace = enable ? reinterpret_cast<unsigned long long*>(p->ftrace) : nullptr;
-  p->fg.trace_stride = (int)stride;
-  return RPSF_OK;
-}
-
-int rpsf_plan_set_small_mode(rpsf_plan* p, int mode) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (mode < 0 || mode > 2) return fail(RPSF_E_INVALID_ARGUMENT, "small-patch mode must be 0, 1 or 2");
-  if (mode == 2 && !p->small_ok)
-    return fail(RPSF_E_UNSUPPORTED, "this plan has no single-CTA path (needs patches of at most 128 px with corners on multiples of P/2)");
-  p->small_mode = mode;
-  return RPSF_OK;
-}
-
 int rpsf_plan_column_info(const rpsf_plan* p, int64_t info[2]) {
   if (!p || !info) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  const bool stream = p->stream_ok && p->k3_stream && !p->force_phases && !p->force_gather;
-  const bool want = p->column_mode == 2;
-  info[0] = (p->paired_ok && want && stream) ? 1 : 0;
-  info[1] = p->paired_ok ? (int64_t)(p->paired_bytes / (size_t)std::max(p->max_batch, 1)) : 0;
-  return RPSF_OK;
-}
-
-int rpsf_plan_set_column_mode(rpsf_plan* p, int mode) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (mode < 0 || mode > 2) return fail(RPSF_E_INVALID_ARGUMENT, "column mode must be 0, 1 or 2");
-  if (mode == 2 && !p->paired_ok) return fail(RPSF_E_UNSUPPORTED, "this plan has no paired column pass (needs a covering)");
-  p->column_mode = mode;
-  return RPSF_OK;
-}
-
-int rpsf_plan_set_fused(rpsf_plan* p, int mode) {
-  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (mode < 0 || mode > 2) return fail(RPSF_E_INVALID_ARGUMENT, "pipeline mode must be 0, 1 or 2");
-  if (mode == 2 && !p->fused_ok) return fail(RPSF_E_UNSUPPORTED, "this plan has no fused pipeline (needs a covering, 256-px patches, float32)");
-  p->fused_mode = mode;
+  info[0] = 0; info[1] = 0;       // there is one column pass, and it needs no workspace of its own
   return RPSF_OK;
 }
 
@@ -1606,9 +1271,6 @@ int rpsf_plan_set_saturation(rpsf_plan* p, double threshold, int dilation, int n
 }  // extern "C"
 
 namespace {
-// output mirrors are only offered without the saturation branch (checked again on the classic path)
-inline bool sat_blocks_mirrors(const rpsf_plan* p, bool sat) { return sat && !p->mirrors.empty(); }
-
 // Saturation pre-fill on the stream: pad + mask, dilate, compact in raster order, ordered fill.
 // On return *filled points at padded pixel (2P, 2P) of frame 0, i.e. at unpadded (0, 0).
 template <typename T>
@@ -1739,35 +1401,6 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
                : sat_restore_launch<double>(p, image, out, out_pitch, out_frame_stride, out_row0, batch, s, sg);
   };
   if (p->n_active == 0) return restore();
-  const size_t rsz0 = real_size(t->dtype);
-  const int bulk_ok0 = ((reinterpret_cast<uintptr_t>(k1_image) & 15) == 0 && ((size_t)g1.img_pitch * rsz0) % 16 == 0 &&
-                        ((size_t)g1.img_frame_stride * rsz0) % 16 == 0) ? 1 : 0;
-  if (p->fused_ok && p->fused_mode == 2 && stages >= 3 && use_stream && p->k1_stream && p->mirrors.empty() &&
-      (long long)batch * p->n_active * (t->P / 2) < (1LL << 30)) {
-    // one persistent launch: the spectrum goes from role to role through a ring that stays in L2
-    CU(cudaMemsetAsync(p->fcounters, 0, p->fcounter_ints * sizeof(int), s));
-    LAUNCH(t->ops->fused(t->dtype, k1_image, p->ring, out, p->corners_dev, p->active_dev, t->kmain, t->knyq, p->ftasks_dev,
-                         p->fcodes_dev, p->f_warp_items, t->tw, t->win, g1, g, batch, bulk_ok0, p->fg, s));
-    if (ev) { CU(cudaEventRecord(ev[1], s)); CU(cudaEventRecord(ev[2], s)); CU(cudaEventRecord(ev[3], s)); }
-    return restore();
-  }
-  if (p->small_ok && p->small_mode == 2 && stages >= 3 && p->mirrors.empty() && !p->force_phases && !p->force_gather) {
-    // Opt-in (rpsf_plan_set_small_mode(plan, 2) / RPSF_SMALL=1): the whole per-patch transform inside one CTA (the
-    // half-spectrum fits shared memory), then the planes are added.  Measured at config 1: 29.0 us per frame at 8 frames
-    // against 22.2 for the three kernels, 39.8 against 41.0 for a single frame — its phases are each slower than the
-    // tuned stand-alone kernels, which outweighs the HBM passes it saves.
-    if (!p->planes) {
-      if (cudaMalloc(&p->planes, p->planes_bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(RPSF_E_CUDA, "out of device memory for the patch planes (%zu bytes)", p->planes_bytes);
-      }
-    }
-    LAUNCH(t->ops->small(t->dtype, k1_image, p->planes, out, p->corners_dev, p->active_dev, t->kmain, t->knyq, t->tw, t->win,
-                         p->small_tiles_dev, p->small_n_tiles, p->small_cover_dev, p->small_max_cover, t->P / 2, g1, g, batch, bulk_ok0, s));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    if (ev) { CU(cudaEventRecord(ev[1], s)); CU(cudaEventRecord(ev[2], s)); CU(cudaEventRecord(ev[3], s)); }
-    return restore();
-  }
   if (int rc = ensure_workspace(p)) return rc;
   if (p->k1_stream && (long long)batch * p->n_active * (t->P / 2) < (1LL << 30)) {
     // bulk (1-D TMA) row copies need 16-byte aligned rows; the kernel still checks each patch's column offset
@@ -1781,34 +1414,6 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   }
   if (ev) CU(cudaEventRecord(ev[1], s));
   if (stages < 2) return RPSF_OK;
-  // Opt-in (rpsf_plan_set_column_mode(plan, 2) / RPSF_PAIRED=1).  Measured at config 2: 21 % less DRAM traffic and 2 % (8
-  // frames) to 5 % (32 frames) more throughput, slower below 8 frames; but the chain kernel is bound by shared-memory
-  // instruction issue and latency at 16 warps per SM, not by HBM any more (0.54 of the peak against 0.80 for the
-  // classic pass), so the classic pass stays the automatic choice.
-  const bool want_paired = p->column_mode == 2;
-  if (p->paired_ok && want_paired && use_stream && stages >= 3 && !sat_blocks_mirrors(p, sat)) {
-    // paired column pass: the two patches that overlap on a band of rows are summed right after the column IFFT, so
-    // the column pass writes half as much and the overlap-add reads half as much
-    if (!p->paired) {
-      if (cudaMalloc(&p->paired, p->paired_bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(RPSF_E_CUDA, "out of device memory for the paired workspace (%zu bytes)", p->paired_bytes);
-      }
-    }
-    LAUNCH(t->ops->k2c(t->dtype, p->workspace, p->paired, t->kmain, t->knyq, p->active_dev, p->chains_dev, p->n_segments,
-                       p->chain_patches_dev, t->tw, t->win, batch, p->n_active, p->bands_total, s));
-    if (ev) CU(cudaEventRecord(ev[2], s));
-    OutMirrors mir{};
-    mir.n = (int)p->mirrors.size();
-    for (int d = 0; d < mir.n; ++d) {
-      mir.delta[d] = (long long)((char*)p->mirrors[d] - (char*)out);
-      if (mir.delta[d] & 15) return fail(RPSF_E_INVALID_ARGUMENT, "mirror %d is not 16-byte congruent with out", d);
-    }
-    LAUNCH(t->ops->k3p(t->dtype, p->paired, out, p->ptasks_dev, p->pcodes_dev, p->p_warp_items, t->tw, t->win, g, batch,
-                       t->sm_count, mir.n ? &mir : nullptr, p->bands_total, s));
-    if (ev) CU(cudaEventRecord(ev[3], s));
-    return restore();
-  }
   LAUNCH(t->ops->k2(t->dtype, p->workspace, p->adjoint ? t->kconj_main : t->kmain, p->adjoint ? t->kconj_nyq : t->knyq,
                     p->active_dev, t->tw, g, batch, t->sm_count, s));
   if (ev) CU(cudaEventRecord(ev[2], s));

@@ -30,15 +30,6 @@ template <typename T> constexpr size_t fft2_row_smem() {
   return sizeof(cplx<T>) * P + sizeof(cplx<T>) * size_t(TL::TEAMS) * TL::SCR;
 }
 
-template <typename T> constexpr size_t chain_smem() {
-  return sizeof(cplx<T>) * P + sizeof(T) * P + 2 * sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C +
-         sizeof(cplx<T>) * size_t(TL::K2_THREADS) * (TL::N2 / 2);
-}
-// two CTAs per SM must fit, as for k2_pipelined
-template <typename T> constexpr bool use_chain() {
-  return use_col_pipe<T>() && 2 * chain_smem<T>() <= 220 * 1024 && TL::NTILE % TL::SLOTS == 0 && TL::NTILE >= TL::SLOTS;
-}
-
 // Launch one of the chained kernels (k1_stream -> k2_pipelined -> k3_stream -> the next call's k1_stream) so that its
 // CTAs may start while the kernel before it in the stream drains (programmatic dependent launch; the kernels wait in
 // grid_dependency_wait() before they touch anything a predecessor wrote).  RPSF_PDL=0 launches them the plain way.
@@ -79,8 +70,6 @@ int init() {
   if ((e = set_smem(k3_stream<P, double, false>, Stream<P, double>::SMEM))) return e;
   if ((e = set_smem(k3_stream<P, float, true>, Stream<P, float>::SMEM))) return e;
   if ((e = set_smem(k3_stream<P, double, true>, Stream<P, double>::SMEM))) return e;
-  if constexpr (Fused<P, float>::OK)
-    if ((e = set_smem(fused_apply<P, float>, Fused<P, float>::SMEM))) return e;
   if ((e = set_smem(k2_colfft_mul_colifft<P, float>, col_smem<float>()))) return e;
   if ((e = set_smem(k2_colfft_mul_colifft<P, double>, col_smem<double>()))) return e;
   if ((e = set_smem(k2_colfft_mul_colifft<P, float, true>, col_smem<float>()))) return e;
@@ -101,20 +90,6 @@ int init() {
     if ((e = set_smem(k2_pipelined<P, float, 4>, col_pipe_smem<float>()))) return e;
   if constexpr (use_col_pipe<double>() && TL::SLOTS == 1 && TL::NTILE % 4 == 0)
     if ((e = set_smem(k2_pipelined<P, double, 4>, col_pipe_smem<double>()))) return e;
-  if constexpr (Small<P, float>::OK)
-    if ((e = set_smem(small_patch<P, float>, Small<P, float>::SMEM))) return e;
-  if constexpr (Small<P, double>::OK)
-    if ((e = set_smem(small_patch<P, double>, Small<P, double>::SMEM))) return e;
-  if constexpr (use_chain<float>()) {
-    if ((e = set_smem(k2_chain<P, float>, chain_smem<float>()))) return e;
-    if ((e = set_smem(k3_stream_paired<P, float, false>, Stream<P, float>::SMEM))) return e;
-    if ((e = set_smem(k3_stream_paired<P, float, true>, Stream<P, float>::SMEM))) return e;
-  }
-  if constexpr (use_chain<double>()) {
-    if ((e = set_smem(k2_chain<P, double>, chain_smem<double>()))) return e;
-    if ((e = set_smem(k3_stream_paired<P, double, false>, Stream<P, double>::SMEM))) return e;
-    if ((e = set_smem(k3_stream_paired<P, double, true>, Stream<P, double>::SMEM))) return e;
-  }
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, float>, row_smem<float>()))) return e;
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, double>, row_smem<double>()))) return e;
   if ((e = set_smem(k3_rowpair_gather<P, float>, K3G_SMEM_MAX))) return e;
@@ -269,114 +244,7 @@ int k3s(int dt, const void* spec, void* out, const StreamTask* tasks, const unsi
   return dt == DT_F32 ? k3s_t<float>(spec, out, tasks, codes, n_warp_items, tw, win, g, batch, sm_count, mirrors, s)
                       : k3s_t<double>(spec, out, tasks, codes, n_warp_items, tw, win, g, batch, sm_count, mirrors, s);
 }
-template <typename T>
-int k2c_t(const void* spec, void* paired, const void* kmain, const void* knyq, const int* active, const ChainDesc* chains,
-          int n_segments, const int* patches, const void* tw, const void* win, int batch, int n_active, long long bands_total,
-          cudaStream_t s) {
-  if constexpr (use_chain<T>()) {
-    const long long ctas = (long long)n_segments * (TL::NTILE / TL::SLOTS) * batch;
-    if (ctas == 0) return 0;
-    k2_chain<P, T><<<(unsigned)ctas, TL::K2_THREADS, chain_smem<T>(), s>>>(
-        (const cplx<T>*)spec, (cplx<T>*)paired, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, chains, patches,
-        (const cplx<T>*)tw, (const T*)win, batch, n_active, bands_total);
-    return (int)cudaGetLastError();
-  } else {
-    return (int)cudaErrorInvalidValue;
-  }
-}
-int k2c(int dt, const void* spec, void* paired, const void* kmain, const void* knyq, const int* active, const ChainDesc* chains,
-        int n_segments, const int* patches, const void* tw, const void* win, int batch, int n_active, long long bands_total,
-        cudaStream_t s) {
-  return dt == DT_F32 ? k2c_t<float>(spec, paired, kmain, knyq, active, chains, n_segments, patches, tw, win, batch, n_active, bands_total, s)
-                      : k2c_t<double>(spec, paired, kmain, knyq, active, chains, n_segments, patches, tw, win, batch, n_active, bands_total, s);
-}
-template <typename T>
-int k3p_t(const void* paired, void* out, const StreamTask* tasks, const unsigned* codes, int n_warp_items, const void* tw,
-          const void* win, const ApplyGeom& g, int batch, int sm_count, const OutMirrors* mirrors, long long bands_total,
-          cudaStream_t s) {
-  if constexpr (use_chain<T>()) {
-    using ST = Stream<P, T>;
-    const long long items = (long long)n_warp_items * batch;
-    if (items == 0) return 0;
-    const long long ctas = (items + ST::WARPS - 1) / ST::WARPS;
-    const unsigned grid = (unsigned)(ctas < sm_count ? ctas : sm_count);
-    const long long ipf = bands_total * (P / 4);
-    if (mirrors && mirrors->n > 0)
-      k3_stream_paired<P, T, true><<<grid, ST::THREADS, ST::SMEM, s>>>((const cplx<T>*)paired, (T*)out, tasks, codes, n_warp_items,
-                                                                       (const cplx<T>*)tw, (const T*)win, g, batch, *mirrors, ipf);
-    else
-      k3_stream_paired<P, T, false><<<grid, ST::THREADS, ST::SMEM, s>>>((const cplx<T>*)paired, (T*)out, tasks, codes, n_warp_items,
-                                                                        (const cplx<T>*)tw, (const T*)win, g, batch, OutMirrors{}, ipf);
-    return (int)cudaGetLastError();
-  } else {
-    return (int)cudaErrorInvalidValue;
-  }
-}
-int k3p(int dt, const void* paired, void* out, const StreamTask* tasks, const unsigned* codes, int n_warp_items, const void* tw,
-        const void* win, const ApplyGeom& g, int batch, int sm_count, const OutMirrors* mirrors, long long bands_total,
-        cudaStream_t s) {
-  return dt == DT_F32 ? k3p_t<float>(paired, out, tasks, codes, n_warp_items, tw, win, g, batch, sm_count, mirrors, bands_total, s)
-                      : k3p_t<double>(paired, out, tasks, codes, n_warp_items, tw, win, g, batch, sm_count, mirrors, bands_total, s);
-}
-template <typename T>
-int small_t(const void* image, void* planes, void* out, const int2* corners, const int* active, const void* kmain,
-            const void* knyq, const void* tw, const void* win, const SmallTile* tiles, int n_tiles, const int* tile_patches,
-            int max_cover, int tile_size, const ApplyGeom& g_in, const ApplyGeom& g_out, int batch, int bulk_ok, cudaStream_t s) {
-  if constexpr (Small<P, T>::OK) {
-    if (g_in.n_active > 0) {
-      small_patch<P, T><<<(unsigned)(g_in.n_active * batch), Small<P, T>::THREADS, Small<P, T>::SMEM, s>>>(
-          (const T*)image, (T*)planes, corners, active, (const cplx<T>*)kmain, (const cplx<T>*)knyq, (const cplx<T>*)tw,
-          (const T*)win, g_in, batch, bulk_ok);
-      int e = (int)cudaGetLastError();
-      if (e) return e;
-    }
-    if (n_tiles > 0) {
-      small_overlap_add<P, T><<<dim3((unsigned)n_tiles, (unsigned)batch), 256, 0, s>>>(
-          (const T*)planes, (T*)out, tiles, tile_patches, max_cover, corners, tile_size, g_out);
-    }
-    return (int)cudaGetLastError();
-  } else {
-    return (int)cudaErrorInvalidValue;
-  }
-}
-int small(int dt, const void* image, void* planes, void* out, const int2* corners, const int* active, const void* kmain,
-          const void* knyq, const void* tw, const void* win, const SmallTile* tiles, int n_tiles, const int* tile_patches,
-          int max_cover, int tile_size, const ApplyGeom& g_in, const ApplyGeom& g_out, int batch, int bulk_ok, cudaStream_t s) {
-  return dt == DT_F32 ? small_t<float>(image, planes, out, corners, active, kmain, knyq, tw, win, tiles, n_tiles, tile_patches,
-                                       max_cover, tile_size, g_in, g_out, batch, bulk_ok, s)
-                      : small_t<double>(image, planes, out, corners, active, kmain, knyq, tw, win, tiles, n_tiles, tile_patches,
-                                        max_cover, tile_size, g_in, g_out, batch, bulk_ok, s);
-}
-int small_ok(int dt) { return dt == DT_F32 ? (Small<P, float>::OK ? 1 : 0) : (Small<P, double>::OK ? 1 : 0); }
-int chain_ok(int dt) { return dt == DT_F32 ? (use_chain<float>() ? 1 : 0) : (use_chain<double>() ? 1 : 0); }
 int stream_tpw() { return Stream<P, float>::TPW; }
-
-void fused_info(int dt, int info[4]) {
-  info[0] = (dt == DT_F32 && Fused<P, float>::OK) ? 1 : 0;
-  info[1] = Stream<P, float>::IPP;
-  info[2] = TL::NTILE / TL::SLOTS;
-  info[3] = Stream<P, float>::WARPS * Stream<P, float>::STAGES;     // issued ahead + the item published one iteration late
-}
-int fused(int dt, const void* image, void* ring, void* out, const int2* corners, const int* active, const void* kmain,
-          const void* knyq, const StreamTask* tasks, const unsigned* codes, int n_warp_items, const void* tw,
-          const void* win, const ApplyGeom& g_in, const ApplyGeom& g_out, int batch, int bulk_ok, const FusedGeom& fg,
-          cudaStream_t s) {
-  if constexpr (Fused<P, float>::OK) {
-    if (dt != DT_F32) return (int)cudaErrorInvalidValue;
-    using T = float;
-    const T* image_t = (const T*)image; cplx<T>* ring_t = (cplx<T>*)ring; T* out_t = (T*)out;
-    const cplx<T>* kmain_t = (const cplx<T>*)kmain; const cplx<T>* knyq_t = (const cplx<T>*)knyq;
-    const cplx<T>* tw_t = (const cplx<T>*)tw; const T* win_t = (const T*)win;
-    ApplyGeom gi = g_in, go = g_out; FusedGeom f = fg;
-    void* args[] = {&image_t, &ring_t, &out_t, &corners, &active, &kmain_t, &knyq_t, &tasks, &codes, &n_warp_items,
-                    &tw_t, &win_t, &gi, &go, &batch, &bulk_ok, &f};
-    // cooperative: every CTA of the three roles must be resident at once (they wait on each other's counters)
-    return (int)cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(fused_apply<P, T>), dim3(fg.n1 + fg.n2 + fg.n3),
-                                            dim3(Fused<P, T>::THREADS), args, Fused<P, T>::SMEM, s);
-  } else {
-    return (int)cudaErrorInvalidValue;
-  }
-}
 
 template <typename T, typename TK>
 int prep_t(const void* full, void* kmain, void* knyq, int n, cudaStream_t s) {
@@ -411,7 +279,7 @@ int fft2(int dt, int in_dt, const void* values, void* out, const void* tw, long 
   return dt == DT_F32 ? fft2_t<float>(values, out, tw, n, s) : fft2_t<double>(values, out, tw, n, s);
 }
 
-const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, k2c, k3p, chain_ok, small_ok, small, stream_tpw, fused_info, fused, k3g_smem, prep, fft2};
+const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2};
 
 }  // namespace
 

@@ -551,173 +551,6 @@ k2_pipelined(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kmain, cons
     k2_frames<P, T, false, TPC, PRUNED>(spec, kp, kn, tw, stage0, valid, special, a, tile, c, n1, slot, lt, f_begin, f_end, g);
 }
 
-// ---------------------------------------------------------------------------- K2, paired (round 2)
-// The overlap-add sums, for every output row, the two patches whose rows contain it (corner rows P/2 apart, same
-// corner column), and K3 does that in the frequency domain before its row IFFT (transform.py:165-169 is linear in the
-// patch).  The same sum can be formed one step earlier, right after the column IFFT, and then the column pass writes
-// HALF as much and K3 reads half as much: a CTA walks a CHAIN of patches that share a corner column, top to bottom,
-// for one tile of bins and one frame; thread (c, n1) holds rows n1 + N1*j of its column, rows below P/2 in j >= N2/2
-// and the matching rows of the next patch (P/2 further down) in j - N2/2, so the pairing needs no communication:
-//     band k of the chain = rowwin[r] * upper half of patch k  +  rowwin[P/2 + r] * lower half of patch k - 1
-// (the row windows of transform.py:165 are applied here, K3 then only applies the column window).  The lower half
-// waits in shared memory for the next step.  The frames of one (chain, tile) are adjacent CTAs, so the transfer-kernel
-// tile of a step is fetched from HBM once and served to the other frames from L2.
-// Workspace: paired[frame][band][P/2 rows][P/2 bins], band = chain.band0 + k, k = 0 .. length (length + 1 bands).
-struct ChainDesc {
-  int first;    // index of the chain's first patch in the chain-ordered patch list
-  int length;   // patches in the chain
-  int band0;    // first band of the chain in the paired workspace
-  int first_step, n_steps;   // the steps this segment computes; the one before first_step only feeds the carry
-};
-
-template <int P, typename T, bool TILE0>
-__device__ __forceinline__ void k2_chain_steps(const cplx<T>* __restrict__ spec, cplx<T>* __restrict__ paired,
-                                               const cplx<T>* __restrict__ kmain, const cplx<T>* __restrict__ knyq,
-                                               const int* __restrict__ active, const int* __restrict__ patches,
-                                               const ChainDesc ch, const cplx<T>* tw, const T* win, cplx<T>* stage0,
-                                               cplx<T>* carry, int tile, int c, int n1, int slot, int lt, int f,
-                                               int n_active, long long bands_total) {
-  using TL = Tile<P>;
-  constexpr int N1 = TL::N1, N2 = TL::N2, HALF = TL::HALF, C = TL::C, NTILE = TL::NTILE, HN = N2 / 2;
-  constexpr int STAGE = TL::SLOTS * P * C;
-  constexpr int CH = 16 / (int)sizeof(cplx<T>);
-  constexpr int ROW_CHUNKS = C / CH;
-  constexpr int PER_THREAD = (P * ROW_CHUNKS) / TL::SLOT_THREADS;
-  constexpr int ROWS_PER_PASS = TL::SLOT_THREADS / ROW_CHUNKS;
-  const bool special = tile == 0 && c == 0;
-  auto sync = []() { __syncthreads(); };
-  auto nosync = []() {};
-  auto ex = [=](int k2, int nn) { return ((slot * N2 + k2) * N1 + nn) * C + c; };
-  const int row0 = lt / ROW_CHUNKS, part = lt % ROW_CHUNKS;
-  const int dst0 = slot * (P * C) + row0 * C + part * CH;
-  auto issue = [&](int step, cplx<T>* stage) {
-    const int a = __ldg(patches + ch.first + step);
-    const cplx<T>* src = spec + (((long long)f * n_active + a) * P + row0) * HALF + tile * C + part * CH;
-#pragma unroll
-    for (int i = 0; i < PER_THREAD; ++i) cp_async16(stage + dst0 + i * (ROWS_PER_PASS * C), src + (long long)i * (ROWS_PER_PASS * HALF));
-    cp_async_commit();
-  };
-  // the first step of a segment that does not start its chain only produces the carry (its band belongs to the
-  // segment before); a segment's last band is written by the NEXT segment unless the chain ends here
-  const int s_begin = ch.first_step > 0 ? ch.first_step - 1 : 0;
-  const int s_end = ch.first_step + ch.n_steps;
-  // carry: [j / 2][thread][2] so that a thread moves its HN values as 16-byte vectors, conflict-free
-  constexpr int CS = TL::K2_THREADS;
-  static_assert(HN % 2 == 0, "carry is moved in pairs");
-  cplx<T> cr[HN];                                             // the carry of this step, in registers while it is combined
-  static_for<0, HN>([&](auto jj) { cr[decltype(jj)::value] = mk<T>(T(0), T(0)); });
-  auto carry_store = [&]() {
-    static_for<0, HN / 2>([&](auto qq) {
-      constexpr int q = decltype(qq)::value;
-      cplx<T>* dst = carry + ((size_t)q * CS + threadIdx.x) * 2;
-      dst[0] = cr[2 * q]; dst[1] = cr[2 * q + 1];
-    });
-  };
-  auto carry_load = [&]() {
-    static_for<0, HN / 2>([&](auto qq) {
-      constexpr int q = decltype(qq)::value;
-      const cplx<T>* src = carry + ((size_t)q * CS + threadIdx.x) * 2;
-      cr[2 * q] = src[0]; cr[2 * q + 1] = src[1];
-    });
-  };
-  carry_store();
-  int cur = 0;
-  issue(s_begin, stage0);
-  for (int step = s_begin; step < s_end; ++step, cur ^= 1) {
-    cplx<T>* xbuf = stage0 + cur * STAGE;
-    cp_async_wait_all();
-    __syncthreads();          // tile `step` landed for everyone; everyone is done with the stage refilled next
-    if (step + 1 < s_end) issue(step + 1, stage0 + (cur ^ 1) * STAGE);
-    const int a = __ldg(patches + ch.first + step);
-    const int gp = __ldg(active + a);
-    const cplx<T>* kp = kmain + (((long long)gp * NTILE + tile) * N2) * (N1 * C) + n1 * C + c;
-    cplx<T> kv[N2];
-    static_for<0, N2>([&](auto ee) { kv[decltype(ee)::value] = kp[(long long)decltype(ee)::value * (N1 * C)]; });
-    cplx<T> v[N2];
-    static_for<0, N2>([&](auto jj) { v[decltype(jj)::value] = xbuf[ex(decltype(jj)::value, n1)]; });
-    if constexpr (TILE0) coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync);
-    else coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
-    if constexpr (TILE0) {
-      const cplx<T>* kn = knyq + (long long)gp * P + n1;
-      cplx<T>* zs = xbuf + slot * P;
-      if (special) {
-        static_for<0, N2>([&](auto ee) {
-          constexpr int e = decltype(ee)::value;
-          zs[(n1 + N1 * (e / N1)) + N2 * (e % N1)] = v[e];
-        });
-      }
-      __syncthreads();
-      static_for<0, N2>([&](auto ee) {
-        constexpr int e = decltype(ee)::value;
-        const int k = (n1 + N1 * (e / N1)) + N2 * (e % N1);
-        cplx<T> zm = v[e], kny = mk<T>(T(0), T(0));
-        if (special) {
-          const cplx<T> zr = zs[(P - k) & (P - 1)];
-          zm = mk<T>(zr.x, -zr.y);
-          kny = kn[e * N1];
-        }
-        const cplx<T> sum = mk<T>(T(0.5) * (v[e].x + zm.x), T(0.5) * (v[e].y + zm.y));
-        const cplx<T> dif = mk<T>(T(0.5) * (v[e].x - zm.x), T(0.5) * (v[e].y - zm.y));
-        v[e] = cadd(cmul(sum, kv[e]), cmul(dif, kny));
-      });
-      __syncthreads();
-    } else {
-      static_for<0, N2>([&](auto ee) { v[decltype(ee)::value] = cmul(v[decltype(ee)::value], kv[decltype(ee)::value]); });
-    }
-    coop_fft_inverse<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
-    // band `step` = upper half of this patch (row window) + lower half of the previous one; the lower half waits
-    const bool emit = step >= ch.first_step;
-    cplx<T>* out = paired + (((long long)f * bands_total + ch.band0 + step) * HALF + n1) * HALF + tile * C + c;
-    carry_load();
-    const T* wrow = win + n1 * N2;                            // transposed table: [n1][j], upper half then lower half
-    static_for<0, HN>([&](auto jj) {
-      constexpr int j = decltype(jj)::value;
-      const T wu = wrow[j], wl = wrow[HN + j];
-      if (emit) out[(long long)(N1 * j) * HALF] = pfma(v[j], mk<T>(wu, wu), cr[j]);
-      cr[j] = cscale(v[HN + j], wl);
-    });
-    carry_store();
-  }
-  if (s_end == ch.length) {                                   // the chain ends: its last lower half stands alone
-    cplx<T>* out = paired + (((long long)f * bands_total + ch.band0 + ch.length) * HALF + n1) * HALF + tile * C + c;
-    static_for<0, HN>([&](auto jj) { out[(long long)(N1 * decltype(jj)::value) * HALF] = cr[decltype(jj)::value]; });
-  }
-}
-
-template <int P, typename T>
-__global__ void __launch_bounds__(Tile<P>::K2_THREADS, RPSF_K2_MINB)
-k2_chain(const cplx<T>* __restrict__ spec, cplx<T>* __restrict__ paired, const cplx<T>* __restrict__ kmain,
-         const cplx<T>* __restrict__ knyq, const int* __restrict__ active, const ChainDesc* __restrict__ chains,
-         const int* __restrict__ patches, const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, int batch,
-         int n_active, long long bands_total) {
-  using TL = Tile<P>;
-  constexpr int N1 = TL::N1, C = TL::C, NTILE = TL::NTILE, HN = TL::N2 / 2;
-  constexpr int TG = NTILE / TL::SLOTS;                      // tile groups per patch
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
-  T* win = reinterpret_cast<T*>(tw + P);
-  cplx<T>* stage0 = reinterpret_cast<cplx<T>*>(win + P);
-  cplx<T>* carry = stage0 + 2 * TL::SLOTS * P * C;
-  // window table transposed to [n1][j]: thread (c, n1) reads the windows of its rows n1 + N1*j as vectors
-  for (int i = threadIdx.x; i < P; i += blockDim.x) { tw[i] = tw_g[i]; win[(i % N1) * TL::N2 + i / N1] = win_g[i]; }
-  // blockIdx.x = (segment * TG + tile group) * batch + frame: the frames of one (segment, tile) run side by side
-  const int f = blockIdx.x % batch;
-  const int tg = (blockIdx.x / batch) % TG;
-  const ChainDesc ch = chains[blockIdx.x / batch / TG];
-  const int c = threadIdx.x % C;
-  const int n1 = (threadIdx.x / C) % N1;
-  const int slot = threadIdx.x / (C * N1);
-  const int lt = threadIdx.x % TL::SLOT_THREADS;
-  const int tile = tg * TL::SLOTS + slot;
-  (void)HN;
-  if (tg == 0)
-    k2_chain_steps<P, T, true>(spec, paired, kmain, knyq, active, patches, ch, tw, win, stage0, carry, tile, c, n1, slot, lt, f,
-                               n_active, bands_total);
-  else
-    k2_chain_steps<P, T, false>(spec, paired, kmain, knyq, active, patches, ch, tw, win, stage0, carry, tile, c, n1, slot, lt, f,
-                                n_active, bands_total);
-}
-
 // ============================================================================ K3
 // row IFFT + window + overlap-add.  transform.py:164-177 (second IFFT axis, np.real, window,
 // `+=` into the canvas, crop).  Launched once per colour class: patches of one colour never

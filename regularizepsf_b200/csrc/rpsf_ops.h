@@ -4,8 +4,6 @@
 #include <cuda_runtime.h>
 #include "rpsf_kernels.cuh"
 #include "rpsf_stream.cuh"
-#include "rpsf_fused.cuh"
-#include "rpsf_small.cuh"
 
 namespace rpsf {
 
@@ -33,33 +31,8 @@ struct Ops {
   int (*k3s)(int dt, const void* spec, void* out, const StreamTask* tasks, const unsigned* codes, int n_warp_items,
              const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count, const OutMirrors* mirrors,
              cudaStream_t s);
-  // paired column pass (k2_chain): walks chains of patches that share a corner column and writes, per band of P/2
-  // output rows, the windowed sum of the two patches that overlap there; `n_segments` chain segments
-  int (*k2c)(int dt, const void* spec, void* paired, const void* kmain, const void* knyq, const int* active,
-             const ChainDesc* chains, int n_segments, const int* patches, const void* tw, const void* win, int batch,
-             int n_active, long long bands_total, cudaStream_t s);
-  // the streaming overlap-add over that paired workspace (one item per group)
-  int (*k3p)(int dt, const void* paired, void* out, const StreamTask* tasks, const unsigned* codes, int n_warp_items,
-             const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count, const OutMirrors* mirrors,
-             long long bands_total, cudaStream_t s);
-  int (*chain_ok)(int dt);   // 1 if k2c / k3p exist for this patch size and dtype
-  // patches whose half-spectrum fits shared memory (rpsf_small.cuh): the whole per-patch transform in one CTA, then
-  // the overlap-add of the patch planes
-  int (*small_ok)(int dt);
-  int (*small)(int dt, const void* image, void* planes, void* out, const int2* corners, const int* active,
-               const void* kmain, const void* knyq, const void* tw, const void* win, const SmallTile* tiles, int n_tiles,
-               const int* tile_patches, int max_cover, int tile_size, const ApplyGeom& g_in, const ApplyGeom& g_out,
-               int batch, int bulk_ok, cudaStream_t s);
   // teams per warp of the streaming kernels (tasks are laid out in groups of this many)
   int (*stream_tpw)();
-  // the whole apply as one persistent cooperative launch with L2-resident hand-overs (rpsf_fused.cuh).
-  // fused_info: [0] = 1 if this (P, dtype) has a fused path, [1] = K1 warp items per patch (ready1 target),
-  // [2] = K2 units per patch, [3] = warps per CTA x pipeline stages of the row roles (items a K1 CTA holds unpublished)
-  void (*fused_info)(int dt, int info[4]);
-  int (*fused)(int dt, const void* image, void* ring, void* out, const int2* corners, const int* active,
-               const void* kmain, const void* knyq, const StreamTask* tasks, const unsigned* codes, int n_warp_items,
-               const void* tw, const void* win, const ApplyGeom& g_in, const ApplyGeom& g_out, int batch, int bulk_ok,
-               const FusedGeom& fg, cudaStream_t s);
   // shared memory the gather kernel needs for that shape (bytes), to size `teams`
   size_t (*k3g_smem)(int dt, int teams, int seg_w);
   int (*prep)(int dt, int kernel_dt, const void* full, void* kmain, void* knyq, int n_patches, cudaStream_t s);

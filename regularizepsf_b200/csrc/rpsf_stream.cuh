@@ -89,7 +89,7 @@ template <int P, typename T, int STAGES_REQ = RPSF_STREAM_STAGES> struct Stream 
   static constexpr int THREADS = WARPS * 32;
   static constexpr size_t SMEM = RING_OFFSET + (size_t)WARPS * STAGES * STAGE_BYTES;
   static_assert(WARPS >= 2, "stage ring does not fit shared memory");
-  static_assert(WARPS * STAGES * 8 <= 768, "mbarriers overlap the words behind them (rpsf_fused.cuh keeps a watermark at +768)");
+  static_assert(WARPS * STAGES * 8 <= 768, "mbarriers must fit the room reserved between the tables and the ring");
   static_assert(TEAM_BYTES % 16 == 0, "team slots must keep 16-byte alignment for bulk copies");
 
   __device__ static __forceinline__ int ex(int k2, int n1) { return k2 * EX_STRIDE + n1; }
@@ -121,27 +121,13 @@ __device__ __forceinline__ void st_spec(double2* p, double2 v, unsigned long lon
 // ============================================================================ K1, streaming
 // gather + apodize + row FFT (same arithmetic as k1_gather_window_rowfft).  Warp item = ROWS
 // consecutive rows of one patch of one frame; team tm of the warp owns rows (2*tm, 2*tm+1) of it.
-// Where a patch's spectrum lives and who is told when it is complete.  The stand-alone kernels use the plain
-// policies: patch `a` of frame `f` sits at slot f * n_active + a of the workspace and nobody is signalled.  The
-// fused pipeline (rpsf_fused.cuh) substitutes a ring of L2-resident slots with producer / consumer counters.
-struct PlainK1 {
-  // workspace slot (in patches) of patch `a` of frame `f`; may block until the slot may be overwritten
-  __device__ __forceinline__ unsigned slot(int f, int a, int n_active) { return (unsigned)(f * n_active + a); }
-  // Warp item number `item` = (f * n_active + a) * IPP + q, which this warp stored one iteration ago, is complete
-  // (kNone: there is none).  Items are dealt round robin to the warps of the grid, so the WARPS items
-  // [WARPS * k, WARPS * (k + 1)) always belong to one CTA, and (WARPS dividing IPP) to one patch.  Called between the transform and the stores of the NEXT item, so that a policy that
-  // publishes with a memory fence finds those older stores already performed instead of stalling on fresh ones.
-  static constexpr unsigned kNone = 0xffffffffu;
-  __device__ __forceinline__ void publish(unsigned /*item*/, int /*lane*/) {}
-  // the head of the pipeline moved to patch `a`: its slot() follows one iteration later
-  __device__ __forceinline__ void prefetch(int /*a*/) {}
-};
-
-template <int P, typename T, typename ST = Stream<P, T>, typename Pol>
+// Patch `a` of frame `f` sits at slot f * n_active + a of the workspace.  The body stays a function apart from its
+// kernel (as K3's does): written into the kernel, the same source compiles to different instructions.
+template <int P, typename T, typename ST>
 __device__ __forceinline__ void
 k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const int2* __restrict__ corners,
                const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, const ApplyGeom& g, int batch, int bulk_ok,
-               unsigned cta, unsigned n_cta, Pol pol, unsigned char* smem_raw) {
+               unsigned cta, unsigned n_cta, unsigned char* smem_raw) {
   constexpr int N1 = ST::N1, N2 = ST::N2, HALF = ST::HALF, ROWS = ST::ROWS, IPP = ST::IPP;
   constexpr int STAGES = ST::STAGES, WARPS = ST::WARPS;
   constexpr unsigned ROW_BYTES = P * sizeof(T);
@@ -191,7 +177,7 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
     hq += dq; ha += da; hf += df;
     if (hq >= IPP) { hq -= IPP; ++ha; }
     if (ha >= g.n_active) { ha -= g.n_active; ++hf; }
-    if (head < n_items) { hcorner = __ldg(corners + ha); pol.prefetch(ha); }   // consumed one iteration later
+    if (head < n_items) hcorner = __ldg(corners + ha);      // consumed one iteration later
   };
   // first row of the head item in the workspace's (frame, patch, row) order, and its patch row
   auto src_row = [&](int corner_row, int patch_row) { return pad_index(corner_row + patch_row, g.H, g.pad_mode); };
@@ -200,7 +186,7 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
 
   // issue the head item into stage `st`; returns (workspace row index << 2) | kind
   auto issue_head = [&](int st) -> unsigned {
-    const unsigned rowidx = pol.slot(hf, ha, g.n_active) * P + hq * ROWS;
+    const unsigned rowidx = (unsigned)(hf * g.n_active + ha) * P + hq * ROWS;
     unsigned char* stage = my_ring + st * ST::STAGE_BYTES;
     const int x_lo = direct ? hcorner.y : max(hcorner.y, 0);
     const int x_hi = direct ? hcorner.y + P : min(hcorner.y + P, g.W);
@@ -244,7 +230,6 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
   static_for<0, N2>([&](auto jj) { wcol[decltype(jj)::value] = win[t + N1 * decltype(jj)::value]; });
 
   int s = 0;
-  unsigned prev_item = PlainK1::kNone;
   for (unsigned it = first; it < n_items; it += stride) {
     const unsigned cur = pend[0], item = pend_item[0], pf = item / IPP;
 #pragma unroll
@@ -304,8 +289,6 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
     __syncwarp();                                            // samples are in registers: the slot becomes the exchange buffer
     auto sync = []() { __syncwarp(); };
     coop_fft_forward<P, T>(v, t, scr, tw, [](int k2, int n1) { return ST::ex(k2, n1); }, sync);
-    pol.publish(prev_item, lane);                            // the previous item's rows (team barriers above order them)
-    prev_item = item;
 
     // This thread holds Z[k] for k = (t + N1*m) + N2*k1 in v[m*N1 + k1].  Split into the two rows' Hermitian
     // half-spectra: A[k] = (Z[k] + conj Z[P-k]) / 2, B[k] = (Z[k] - conj Z[P-k]) / (2i), scaled by the row
@@ -343,7 +326,6 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
     s = s + 1 == STAGES ? 0 : s + 1;
   }
   __syncwarp();
-  pol.publish(prev_item, lane);                              // the last item
 }
 
 template <int P, typename T>
@@ -351,8 +333,7 @@ __global__ void __launch_bounds__(StreamK1<P, T>::THREADS, 1)
 k1_stream(const T* __restrict__ image, cplx<T>* __restrict__ spec, const int2* __restrict__ corners,
           const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, ApplyGeom g, int batch, int bulk_ok) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  k1_stream_body<P, T, StreamK1<P, T>>(image, spec, corners, tw_g, win_g, g, batch, bulk_ok, blockIdx.x, gridDim.x, PlainK1{},
-                                       smem_raw);
+  k1_stream_body<P, T, StreamK1<P, T>>(image, spec, corners, tw_g, win_g, g, batch, bulk_ok, blockIdx.x, gridDim.x, smem_raw);
 }
 
 // ============================================================================ K3, streaming
@@ -378,7 +359,7 @@ struct StreamTask {
   int item_begin;   // into the item-code list
   int n_steps;      // item codes to walk; 0 = idle team
   int flags;        // TASK_SEAM | TASK_LAST
-  int pad0, pad1, pad2;
+  int pad0, pad1, pad2;   // padding to 32 bytes
 };
 enum : int { TASK_SEAM = 1, TASK_LAST = 2 };
 constexpr unsigned ITEM_LAST_OF_GROUP = 1u << 30;            // item code = (active*P/2 + pair) | flag
@@ -391,42 +372,13 @@ struct OutMirrors {
   long long delta[7];
 };
 
-// Plain policy of the stand-alone kernel: item code = active * P/2 + pair, patch `a` of frame `f` at workspace slot
-// f * n_active + a, no waiting, no signalling.  (The fused pipeline's policy is in rpsf_fused.cuh.)
-template <int P> struct PlainK3 {
-  // row pair inside its patch (for the row windows)
-  __device__ __forceinline__ int pair(unsigned code) const { return int((code & (ITEM_LAST_OF_GROUP - 1)) % (P / 2)); }
-  // element offset of the item's two half-spectrum rows in the workspace
-  __device__ __forceinline__ size_t offset(int f, int n_active, unsigned code, const StreamTask&) const {
-    return ((size_t)f * n_active * (P / 2) + (code & (ITEM_LAST_OF_GROUP - 1))) * P;
-  }
-  // row windows of the item's two rows (transform.py:165)
-  __device__ __forceinline__ void row_windows(const float* win, unsigned code, float& wa, float& wb) const { wa = win[2 * pair(code)]; wb = win[2 * pair(code) + 1]; }
-  __device__ __forceinline__ void row_windows(const double* win, unsigned code, double& wa, double& wb) const { wa = win[2 * pair(code)]; wb = win[2 * pair(code) + 1]; }
-  __device__ __forceinline__ void wait(int /*f*/, const StreamTask&, bool /*live*/) const {}
-  __device__ __forceinline__ void done(int /*f*/, const StreamTask&, bool /*leader*/) const {}
-};
-
-// Policy for the paired workspace of k2_chain (rpsf_kernels.cuh): a group is ONE item — the two patches that overlap
-// on a pair of output rows were summed, row windows included, by the column pass — so item code = band * P/4 + row
-// pair inside the band, every item is the last of its group, and the row windows here are 1.
-template <int P> struct PairedK3 {
-  long long items_per_frame;          // bands * P / 4
-  __device__ __forceinline__ int pair(unsigned code) const { return int((code & (ITEM_LAST_OF_GROUP - 1)) % (P / 4)); }
-  __device__ __forceinline__ size_t offset(int f, int /*n_active*/, unsigned code, const StreamTask&) const {
-    return ((size_t)f * items_per_frame + (code & (ITEM_LAST_OF_GROUP - 1))) * P;
-  }
-  template <typename T> __device__ __forceinline__ void row_windows(const T*, unsigned, T& wa, T& wb) const { wa = T(1); wb = T(1); }
-  __device__ __forceinline__ void wait(int, const StreamTask&, bool) const {}
-  __device__ __forceinline__ void done(int, const StreamTask&, bool) const {}
-};
-
-template <int P, typename T, bool MIRROR, typename Pol>
+// Item code = active * P/2 + pair; patch `a` of frame `f` sits at workspace slot f * n_active + a.
+template <int P, typename T, bool MIRROR>
 __device__ __forceinline__ void
 k3_stream_body(const cplx<T>* __restrict__ spec, T* __restrict__ out, const StreamTask* __restrict__ tasks,
                const unsigned* __restrict__ codes, int n_warp_items, const cplx<T>* __restrict__ tw_g,
                const T* __restrict__ win_g, const ApplyGeom& g, int batch, const OutMirrors& mir, unsigned cta,
-               unsigned n_cta, Pol pol, unsigned char* smem_raw) {
+               unsigned n_cta, unsigned char* smem_raw) {
   auto put = [&](T* p, T val) {
     *p = val;
     if constexpr (MIRROR) {
@@ -474,7 +426,6 @@ k3_stream_body(const cplx<T>* __restrict__ spec, T* __restrict__ out, const Stre
     const bool live = task.n_steps > 0;
     const unsigned live_teams = __popc(__ballot_sync(0xffffffffu, live && t == 0));
     const unsigned* my_codes = codes + task.item_begin;
-    pol.wait(f, task, live);                                 // fused pipeline: the patches this task reads are complete
 
     // issue step k into stage st: every live team's row pair of half-spectra, one bulk copy each
     auto issue = [&](unsigned code, int st) {
@@ -484,7 +435,7 @@ k3_stream_body(const cplx<T>* __restrict__ spec, T* __restrict__ out, const Stre
       }
       __syncwarp();
       if (live && t == 0) {
-        const cplx<T>* src = spec + pol.offset(f, g.n_active, code, task);
+        const cplx<T>* src = spec + ((size_t)f * g.n_active * (P / 2) + (code & (ITEM_LAST_OF_GROUP - 1))) * P;
         bulk_load(my_ring + st * ST::STAGE_BYTES + team_off, src, ITEM_BYTES, bar + st);
       }
     };
@@ -530,8 +481,9 @@ k3_stream_body(const cplx<T>* __restrict__ spec, T* __restrict__ out, const Stre
 
       if (live) {
         // Z[k] += wa*Ua[k] + i*wb*Ub[k] for k <= P/2, Hermitian mirror above; bin 0 packs (DC, Nyquist)
-        T wa_s, wb_s;
-        pol.row_windows(win, code, wa_s, wb_s);
+        // row windows of the item's two rows (transform.py:165)
+        const int pair = int((code & (ITEM_LAST_OF_GROUP - 1)) % (P / 2));
+        const T wa_s = win[2 * pair], wb_s = win[2 * pair + 1];
         const cplx<T> wa = mk<T>(wa_s, wa_s), wb = mk<T>(wb_s, wb_s);
         const cplx<T>* lo = slot + t;                      // Ua[bin] = lo[bin - t], Ub[bin] = lo[P/2 + bin - t]
         const cplx<T>* neg = slot - t;                     // Ua[P - bin] = neg[P - (bin - t)]
@@ -639,7 +591,6 @@ k3_stream_body(const cplx<T>* __restrict__ spec, T* __restrict__ out, const Stre
       }
       s = s + 1 == STAGES ? 0 : s + 1;
     }
-    pol.done(f, task, live && t == 0);                       // every step's copy has landed and been consumed
   }
 }
 
@@ -650,17 +601,7 @@ k3_stream(const cplx<T>* __restrict__ spec, T* __restrict__ out, const StreamTas
           const T* __restrict__ win_g, ApplyGeom g, int batch, OutMirrors mir) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   k3_stream_body<P, T, MIRROR>(spec, out, tasks, codes, n_warp_items, tw_g, win_g, g, batch, mir, blockIdx.x, gridDim.x,
-                               PlainK3<P>{}, smem_raw);
-}
-// the same over the paired workspace of k2_chain (one item per group, row windows already applied)
-template <int P, typename T, bool MIRROR>
-__global__ void __launch_bounds__(Stream<P, T>::THREADS, 1)
-k3_stream_paired(const cplx<T>* __restrict__ paired, T* __restrict__ out, const StreamTask* __restrict__ tasks,
-                 const unsigned* __restrict__ codes, int n_warp_items, const cplx<T>* __restrict__ tw_g,
-                 const T* __restrict__ win_g, ApplyGeom g, int batch, OutMirrors mir, long long items_per_frame) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  k3_stream_body<P, T, MIRROR>(paired, out, tasks, codes, n_warp_items, tw_g, win_g, g, batch, mir, blockIdx.x, gridDim.x,
-                               PairedK3<P>{items_per_frame}, smem_raw);
+                               smem_raw);
 }
 
 }  // namespace rpsf

@@ -132,8 +132,8 @@ class _NativeTransform:
         _native.check(self.lib.rpsf_plan_info(plan, info))
         return {"active_patches": info[0], "colours": info[1], "workspace_bytes": info[2],
                 "rows_read": (info[3], info[4]), "colour0_tiles_band": bool(info[5]),
-                "overlap_add": {2: "streaming chains", 1: "row-pair gather", 0: "colour phases"}[int(info[6]) & 7],
-                "fused_pipeline": bool(int(info[6]) & 8), "gather_teams": info[7]}
+                "overlap_add": {2: "streaming chains", 1: "row-pair gather", 0: "colour phases"}[int(info[6])],
+                "gather_teams": info[7]}
 
 
 class ArrayPSFTransform:

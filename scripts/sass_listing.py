@@ -12,7 +12,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "regularizepsf_b200", "librpsf_b200.so")
 P = sys.argv[1] if len(sys.argv) > 1 else "256"
-WANTED = [rf"k1_streamILi{P}Ef", rf"k2_pipelinedILi{P}Ef", rf"k3_streamILi{P}EfLb0", rf"fused_applyILi{P}Ef"]
+WANTED = [rf"k1_streamILi{P}Ef", rf"k2_pipelinedILi{P}Ef", rf"k3_streamILi{P}EfLb0"]
 MARKERS = ["UBLKCP", "SYNCS", "UTMALDG", "UTMASTG", "LDGSTS", "FFMA2", "FADD2", "FMUL2", "FFMA", "FADD", "FMUL", "LDS", "STS",
            "LDG", "STG", "SHFL", "BAR", "MEMBAR", "ATOMG", "REDG", "HMMA", "UTC", "ACQBULK", "PREEXIT"]
 

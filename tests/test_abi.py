@@ -25,9 +25,9 @@ def test_header_and_binding_agree(native_lib):
         assert hasattr(native_lib, name), name
 
 
-def test_library_is_self_contained(native_lib):
+def test_abi_version_and_supported_patch_sizes(native_lib):
     # static CUDA runtime: the only CUDA dependency is the driver, resolved lazily
-    assert native_lib.rpsf_abi_version() == 1
+    assert native_lib.rpsf_abi_version() == 2
     for p in (16, 32, 64, 128, 256, 512):
         assert native_lib.rpsf_patch_size_supported(p) == 1
     for p in (2, 8, 11, 100, 255, 256 - 1):            # embedded in the next power of two >= 2 P - 1

@@ -165,16 +165,7 @@ def test_forward_unchanged_by_an_adjoint_plan():
     assert torch.equal(t.apply(x), before)
 
 
-@pytest.mark.parametrize("env", ["RPSF_PAIRED", "RPSF_SMALL", "RPSF_FUSED"])
-@pytest.mark.parametrize("name", ["p64", "p256"])
-def test_opt_in_paths_do_not_reach_adjoint_plans(env, name, monkeypatch):
-    monkeypatch.setenv(env, "1")
-    shape, coords, kernel = _setup(name)
-    t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))          # fresh: new plans read the environment
-    _check_against_oracle(t, _frames(shape, 2, seed=12), coords, kernel, "symmetric", "float32")
-
-
-def test_adjoint_plan_rejects_forward_only_settings():
+def test_adjoint_plan_rejects_saturation_mirrors_and_materialised_pad():
     import torch
     shape, coords, kernel = _setup("p256")
     t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))
@@ -183,9 +174,6 @@ def test_adjoint_plan_rejects_forward_only_settings():
     lib = nt.lib
     assert lib.rpsf_plan_set_saturation(plan, 10.0, 1, 7) == _native.E_UNSUPPORTED
     assert lib.rpsf_plan_set_saturation(plan, float("inf"), 1, 7) == 0
-    assert lib.rpsf_plan_set_fused(plan, 2) == _native.E_UNSUPPORTED
-    assert lib.rpsf_plan_set_column_mode(plan, 2) == _native.E_UNSUPPORTED
-    assert lib.rpsf_plan_set_small_mode(plan, 2) == _native.E_UNSUPPORTED
     mirror = torch.empty(1, device="cuda")
     arr = (ctypes.c_void_p * 1)(mirror.data_ptr())
     assert lib.rpsf_plan_set_output_mirrors(plan, 1, arr) == _native.E_UNSUPPORTED

@@ -187,60 +187,6 @@ def test_psf_fft2_returns_without_synchronising_and_reuses_its_tables():
         assert float((out - want).abs().max() / want.abs().max()) <= 2e-6
 
 
-# ------------------------------------------------------------------ fused persistent pipeline (rpsf_fused.cuh, opt-in)
-@pytest.mark.parametrize("shape,batch,rows", [((2048, 2048), 1, None), ((1024, 768), 3, None), ((2048, 1024), 2, (512, 1280)),
-                                              ((512, 512), 5, None)])
-def test_fused_pipeline_is_bit_identical_to_the_three_kernels(shape, batch, rows):
-    """One cooperative launch with L2-resident hand-overs (role K1 -> ring -> role K2 -> role K3, chained by counters)
-    must give the same bits as the three stand-alone kernels: same arithmetic, same per-pixel summation order."""
-    import ctypes
-    import torch
-    from regularizepsf_b200.device import DeviceCube
-    size = 256
-    coords = _covering(shape, size)
-    g = torch.Generator(device="cuda").manual_seed(21)
-    kernel = torch.randn((len(coords), size, size), dtype=torch.complex64, device="cuda", generator=g)
-    t = rp.ArrayPSFTransform(DeviceCube(coords, kernel))
-    frames = torch.rand((batch, *shape), device="cuda", generator=g) * 1000
-    lo, hi = rows if rows else (0, shape[0])
-    nt = t._native_transform("float32")
-    plan = nt.plan(shape[0], shape[1], 0, lo, hi, batch)
-    lib = _native.load()
-    assert not nt.plan_info(plan)["fused_pipeline"]                       # opt-in: the three kernels are the default
-    plain = t._apply_device(frames, "float32", 0, row_range=(lo, hi)).clone()
-    _native.check(lib.rpsf_plan_set_fused(plan, 2))
-    try:
-        assert nt.plan_info(plan)["fused_pipeline"]
-        for _ in range(3):                                                # counters are reset per launch
-            fused = t._apply_device(frames, "float32", 0, row_range=(lo, hi))
-            assert torch.equal(fused, plain)
-        # diagnostics: statistics and the band timeline of one launch
-        stats = (ctypes.c_uint64 * 8)()
-        _native.check(lib.rpsf_plan_fused_stats(plan, 1, None))
-        n_bands = len({c[0] for c in coords if c[0] < hi and c[0] + size > lo})
-        trace = (ctypes.c_uint64 * (3 * batch * n_bands))()
-        _native.check(lib.rpsf_plan_fused_trace(plan, 1, None, 0))
-        assert torch.equal(t._apply_device(frames, "float32", 0, row_range=(lo, hi)), plain)
-        _native.check(lib.rpsf_plan_fused_stats(plan, 0, stats))
-        _native.check(lib.rpsf_plan_fused_trace(plan, 0, trace, len(trace)))
-        assert stats[7] > 0 and all(int(v) > 0 for v in stats[3:6])       # column units ran, every role ran
-        tr = np.array(trace, dtype=np.float64).reshape(3, batch * n_bands)
-        assert np.all(tr > 0) and np.all(tr[0] <= tr[1]) and np.all(tr[1] <= tr[2])   # K1 before K2 before K3, every band
-    finally:
-        _native.check(lib.rpsf_plan_set_fused(plan, 0))
-    assert torch.equal(t._apply_device(frames, "float32", 0, row_range=(lo, hi)), plain)
-
-
-def test_fused_pipeline_refuses_what_it_cannot_do():
-    coords, kernel, image = _small()                                      # 32-px patches: no fused path
-    t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))
-    t.apply(image)
-    nt = t._native_transform("float32")
-    plan = nt.plan(image.shape[0], image.shape[1], 0, 0, image.shape[0], 1)
-    with pytest.raises(NotImplementedError):
-        _native.check(_native.load().rpsf_plan_set_fused(plan, 2))
-
-
 # ------------------------------------------------------------------ real multi-GPU runs (skipped on a one-GPU box)
 def test_frame_and_slab_sharding_across_real_gpus_is_bit_identical():
     """Two ranks over NCCL on two GPUs: config 3 (frames sharded, gathered over NCCL and by peer stores fused into the
@@ -367,16 +313,14 @@ def test_patch_sizes_without_a_native_fft_length(size, shape):
     assert np.max(np.abs(got_nan[ok] - want_nan[ok])) <= TOL["float32"] * scale
 
 
-# ------------------------------------------------------------------ paired column pass (k2_chain + k3_stream_paired)
+# ------------------------------------------------------------------ coverings, row bands and pad modes against the oracle
 @pytest.mark.parametrize("shape,size,dtype,batch,rows", [((2048, 2048), 256, "float32", 1, None), ((2048, 2048), 256, "float32", 3, None),
                                                         ((1024, 768), 128, "float32", 2, None), ((1024, 768), 128, "float64", 1, (256, 640)),
                                                         ((640, 512), 64, "float32", 9, None), ((700, 333), 64, "float64", 2, None),
                                                         ((2048, 1024), 256, "float32", 2, (512, 1408))])
-def test_paired_column_pass_matches_the_classic_one_and_the_oracle(shape, size, dtype, batch, rows):
-    """The column pass that sums overlapping patch rows right after its inverse transform (half the spectrum written and
-    read back) against the classic in-place pass with the sum in the overlap-add kernel: same values to rounding, both
-    within the oracle tolerance; chains cut into segments (small batches) reproduce whole chains bit for bit."""
-    import os
+def test_three_kernels_on_coverings_and_row_bands(shape, size, dtype, batch, rows):
+    """The three kernels on coverings, whole frames and row bands: within the oracle tolerance, bit-stable across fresh
+    plans, and overlap-add chains cut into chunks (RPSF_K3_CHUNKS) reproduce whole chains bit for bit."""
     import torch
     coords = _covering(shape, size)
     rng = np.random.default_rng(17)
@@ -386,39 +330,33 @@ def test_paired_column_pass_matches_the_classic_one_and_the_oracle(shape, size, 
     tdtype = torch.float32 if dtype == "float32" else torch.float64
     dev = torch.from_numpy(frames).to("cuda", tdtype)
     lo, hi = rows if rows else (0, shape[0])
-    lib = _native.load()
 
-    def run(mode, segments=None):
-        if segments is not None:
-            os.environ["RPSF_CHAIN_SEGMENTS"] = str(segments)
+    def run(chunks=None):
+        if chunks is not None:
+            os.environ["RPSF_K3_CHUNKS"] = str(chunks)
         try:
             t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))          # a fresh transform: a fresh plan
             nt = t._native_transform(dtype)
-            plan = nt.plan(shape[0], shape[1], 0, lo, hi, batch)
+            nt.plan(shape[0], shape[1], 0, lo, hi, batch)
         finally:
-            os.environ.pop("RPSF_CHAIN_SEGMENTS", None)
-        if lib.rpsf_plan_set_column_mode(plan, mode) != 0:
-            pytest.skip("no paired column pass for this patch size / dtype")
+            os.environ.pop("RPSF_K3_CHUNKS", None)
         return t._apply_device(dev, dtype, 0, row_range=(lo, hi)).cpu().numpy()
 
-    classic, paired = run(1), run(2)
-    scale = float(frames.max())
-    assert rel_err(paired, classic, scale) <= (2e-6 if dtype == "float32" else 1e-14)
-    assert np.array_equal(run(0), classic)                                 # automatic stays the classic pass
-    for segments in (1, 2, 3):
-        assert np.array_equal(run(2, segments), paired), segments          # seams recompute, they do not approximate
+    three = run()
+    assert np.array_equal(run(), three)
+    for chunks in (1, 2, 3):
+        assert np.array_equal(run(chunks), three), chunks                  # seams recompute, they do not approximate
     if shape[0] * shape[1] <= 1_000_000:
         want = np.stack([oracle.apply_transform(f, coords, kernel) for f in frames])[:, lo:hi]
-        assert rel_err(paired, want, scale) <= TOL[dtype] and rel_err(classic, want, scale) <= TOL[dtype]
+        assert rel_err(three, want, float(frames.max())) <= TOL[dtype]
 
 
-# ------------------------------------------------------------------ small patches: one CTA per patch (rpsf_small.cuh)
 @pytest.mark.parametrize("shape,size,dtype,batch,pad_mode", [((1024, 1024), 128, "float32", 2, "symmetric"), ((300, 260), 64, "float32", 3, "reflect"),
                                                             ((192, 160), 32, "float64", 2, "wrap"), ((96, 80), 16, "float32", 1, "constant"),
                                                             ((512, 384), 64, "float64", 1, "edge"), ((640, 384), 128, "float32", 5, "symmetric")])
-def test_single_cta_patch_path_against_three_kernels_and_oracle(shape, size, dtype, batch, pad_mode):
-    """P <= 128: the per-patch transform inside one CTA + overlap-add of the patch planes in list order, against the
-    three-kernel path and the oracle; row slabs stitch bit-identically; repeated calls are bit-stable."""
+def test_three_kernels_in_every_pad_mode_and_slab_stitching(shape, size, dtype, batch, pad_mode):
+    """P <= 128 in every pad mode: the three kernels against the oracle; row slabs stitch bit-identically; repeated calls
+    are bit-stable."""
     import torch
     coords = _covering(shape, size)
     rng = np.random.default_rng(23)
@@ -427,31 +365,25 @@ def test_single_cta_patch_path_against_three_kernels_and_oracle(shape, size, dty
     frames = np.stack([oracle.starfield(shape, seed=70 + i) for i in range(batch)])
     tdtype = torch.float32 if dtype == "float32" else torch.float64
     dev = torch.from_numpy(frames).to("cuda", tdtype)
-    lib = _native.load()
     code = _native.PAD_MODES[pad_mode]
 
-    def run(mode, rows=None):
+    def run(rows=None):
         t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))
         nt = t._native_transform(dtype)
         lo, hi = rows if rows else (0, shape[0])
-        plan = nt.plan(shape[0], shape[1], code, lo, hi, batch)
-        if lib.rpsf_plan_set_small_mode(plan, mode) != 0:
-            pytest.skip("no single-CTA path for this patch size / dtype")
+        nt.plan(shape[0], shape[1], code, lo, hi, batch)
         return t._apply_device(dev, dtype, code, row_range=(lo, hi)).cpu().numpy()
 
-    three, small = run(1), run(2)
-    scale = float(frames.max())
-    assert rel_err(small, three, scale) <= (3e-6 if dtype == "float32" else 1e-13)
-    assert np.array_equal(small, run(2)) and np.array_equal(three, run(0))      # bit-stable; automatic = the three kernels
+    three = run()
+    assert np.array_equal(three, run())                                    # bit-stable
     want = np.stack([oracle.apply_transform(f, coords, kernel, pad_mode=pad_mode) for f in frames])
-    assert rel_err(small, want, scale) <= TOL[dtype]
+    assert rel_err(three, want, float(frames.max())) <= TOL[dtype]
     from regularizepsf_b200.distributed import slab_bounds
-    parts = [run(2, rows=b) for b in slab_bounds(shape[0], size, 3) if b[1] > b[0]]
-    assert np.array_equal(np.concatenate(parts, axis=1), small)
+    parts = [run(rows=b) for b in slab_bounds(shape[0], size, 3) if b[1] > b[0]]
+    assert np.array_equal(np.concatenate(parts, axis=1), three)
 
 
-def test_single_cta_patch_path_nan_footprint_saturation_and_host_calls(monkeypatch):
-    monkeypatch.setenv("RPSF_SMALL", "1")                                  # new plans take the single-CTA path
+def test_nan_footprint_saturation_and_host_calls_at_64_px():
     coords, kernel, image = _small(shape=(256, 192), size=64, seed=5)
     t = rp.ArrayPSFTransform(rp.IndexedCube(coords, kernel))
     poisoned = image.copy()
