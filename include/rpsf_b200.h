@@ -159,6 +159,19 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int height, int width, 
  * (img_row0 = out_row0 = 0, img_rows = H); rpsf_apply_stages and rpsf_apply_host, a finite saturation threshold and
  * output mirrors are RPSF_E_UNSUPPORTED on it. */
 int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int height, int width, int pad_mode, int max_batch);
+/* Gradient of <apply(image), grad> with respect to the transfer kernel, summed over `batch` frames (no saturation):
+ * kernel_grad[n] = sum_b conj(X_n) G_n / P^2 with X_n = FFT2(w * patch n of the padded image) and G_n = FFT2(w * patch n of
+ * the zero-extended grad), in PyTorch's convention (dL/dRe + i dL/dIm).  `kernel_grad` is a device (n, P, P) complex cube
+ * of the compute dtype in the layout rpsf_transform_set_kernel reads; patches that do not touch the frame get 0.
+ * `adjoint_plan` comes from rpsf_plan_create_adjoint(t, H, W, pad_mode, .), `forward_plan` from rpsf_plan_create(t, H, W,
+ * pad_mode, 0, H, .) with an infinite saturation threshold; both workspaces are reused, nothing is allocated.  Embedded
+ * patch sizes, sharded transforms, a finite saturation threshold, the materialised pad and a partial row band are
+ * RPSF_E_UNSUPPORTED; plans of different transforms, shapes or pad modes and a batch above either plan's capacity are
+ * RPSF_E_INVALID_ARGUMENT.  With rpsf_plan_enable_timing on the forward plan, rpsf_plan_read_timing of that plan
+ * reports K1 of the image, the copy of grad plus K1 of the box, and the zeroing plus the gradient kernel. */
+int rpsf_kernel_gradient(rpsf_plan* adjoint_plan, rpsf_plan* forward_plan, const void* image, int64_t img_pitch,
+                         int64_t img_frame_stride, const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch,
+                         void* kernel_grad, void* stream);
 int rpsf_plan_destroy(rpsf_plan* p);
 /* info[0]=active patches, [1]=colours, [2]=workspace bytes, [3]=first frame row read,
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,

@@ -4,7 +4,9 @@ Same public names as the reference package (regularizepsf/__init__.py:5-16): ``A
 ``ArrayPSFTransform`` (``construct`` / ``apply`` / ``save`` / ``load``), ``IndexedCube``,
 ``calculate_covering``, the functional PSF decorators, ``ArrayPSFBuilder`` (stack averaging on the
 GPU, star finding through the optional ``sep`` dependency as in the reference) and the exception
-types.  Plotting is out of scope (see DESIGN.md).
+types.  ``DeviceCube`` holds a cube as a CUDA tensor: a transform built on one whose tensor requires grad is
+trainable (``ArrayPSFTransform.apply`` differentiates with respect to the transfer kernel).  Plotting is out of scope
+(see DESIGN.md).
 """
 from regularizepsf_b200.exceptions import (
     FunctionParameterMismatchError,
@@ -17,6 +19,7 @@ from regularizepsf_b200.exceptions import (
     RegularizePSFError,
 )
 from regularizepsf_b200.builder import ArrayPSFBuilder
+from regularizepsf_b200.device import DeviceCube
 from regularizepsf_b200.psf import ArrayPSF
 from regularizepsf_b200.functional import (
     SimpleFunctionalPSF,
@@ -30,7 +33,7 @@ from regularizepsf_b200.util import IndexedCube, calculate_covering
 __version__ = "0.1.0"
 
 __all__ = [
-    "ArrayPSF", "ArrayPSFBuilder", "ArrayPSFTransform", "IndexedCube", "calculate_covering", "set_default_dtype",
+    "ArrayPSF", "ArrayPSFBuilder", "ArrayPSFTransform", "DeviceCube", "IndexedCube", "calculate_covering", "set_default_dtype",
     "SimpleFunctionalPSF", "VariedFunctionalPSF", "simple_functional_psf", "varied_functional_psf",
     "RegularizePSFError", "InvalidCoordinateError", "IncorrectShapeError", "InvalidFunctionError",
     "FunctionParameterMismatchError", "PSFBuilderError", "InvalidDataError", "NativeLibraryError",

@@ -47,6 +47,7 @@ SIGNATURES = {
     "rpsf_isolate_cores": (_i, [_vp, _i64, _i, _i, _vp]),
     "rpsf_plan_create": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, _i]),
     "rpsf_plan_create_adjoint": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i]),
+    "rpsf_kernel_gradient": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _i64, _i64, _i, _vp, _vp]),
     "rpsf_plan_destroy": (_i, [_vp]),
     "rpsf_plan_info": (_i, [_vp, ctypes.POINTER(_i64)]),
     "rpsf_plan_set_overlap_mode": (_i, [_vp, _i]),

@@ -339,6 +339,7 @@ struct rpsf_plan {
   int H = 0, W = 0, pad_mode = 0, row_begin = 0, row_end = 0, max_batch = 1;
   int n_active = 0;
   int* active_dev = nullptr;       // active index -> kernel slot of the patch (rpsf_transform::kslot)
+  std::vector<int> active_host;    // active index -> patch index (rpsf_kernel_gradient pairs two plans by it)
   int2* corners_dev = nullptr;     // per active patch
   std::vector<int*> items_dev;     // per colour: active*P/2 + pair
   std::vector<int> n_items;
@@ -388,6 +389,7 @@ struct rpsf_plan {
   // frame (fold_pad_adjoint)
   bool adjoint = false;
   int frame_H = 0, frame_W = 0, box_y0 = 0, box_x0 = 0;
+  int frame_pad_mode = 0;             // the pad mode of the forward map this plan transposes
   long long box_pitch = 0;            // elements, a multiple of 16 bytes (K1's bulk row copies)
   void* box_in = nullptr; void* box_out = nullptr;
   int* fold_rows = nullptr;           // [frame_H + 1 offsets | box row indices], CSR preimages of the row pad map
@@ -937,6 +939,7 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
   if (lo >= hi) { lo = 0; hi = 0; }
   p->img_lo = lo; p->img_hi = hi;
   p->n_active = (int)active.size();
+  p->active_host = active;
   p->colour0_covers = !embedded && colour0_area == (long long)(row_end - row_begin) * W;
   auto destroy_fail = [&](const char* what) {
     rpsf_plan_destroy(p);
@@ -1119,6 +1122,7 @@ int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, i
   DeviceGuard guard(t->device);
   p->adjoint = true;
   p->frame_H = H; p->frame_W = W; p->box_y0 = y0; p->box_x0 = x0;
+  p->frame_pad_mode = pad_mode;
   const size_t rs = real_size(t->dtype), align = 16 / rs;
   p->box_pitch = (long long)((Wb + align - 1) / align * align);
   const size_t box_bytes = (size_t)max_batch * Hb * p->box_pitch * rs;
@@ -1448,6 +1452,25 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   return restore();
 }
 
+// y (whole frames) -> interior of the zero-bordered box of an adjoint plan (the margins stay zero)
+template <typename T>
+int adjoint_copy(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int batch, cudaStream_t s) {
+  const int H = p->frame_H, W = p->frame_W;
+  const long long box_stride = (long long)p->H * p->box_pitch;
+  // the part of the frame inside the box; the rest of y meets no patch
+  const int r0 = std::max(0, p->box_y0), r1 = std::min(H, p->box_y0 + p->H);
+  const int c0 = std::max(0, p->box_x0), c1 = std::min(W, p->box_x0 + p->W);
+  if (r1 > r0 && c1 > c0) {
+    const dim3 grid((unsigned)((c1 - c0 + 255) / 256), (unsigned)std::min(r1 - r0, 1024), (unsigned)batch);
+    adjoint_copy_in<T><<<grid, 256, 0, s>>>((const T*)image + (long long)r0 * img_pitch + c0, img_pitch, img_frame_stride,
+                                            r1 - r0, c1 - c0,
+                                            (T*)p->box_in + (long long)(r0 - p->box_y0) * p->box_pitch + (c0 - p->box_x0),
+                                            p->box_pitch, box_stride);
+    LAUNCH((int)cudaGetLastError());
+  }
+  return RPSF_OK;
+}
+
 // Aᵀ y: y (whole frames) -> interior of the zero-bordered box, the forward kernels on the box with conj(Kh), fold
 template <typename T>
 int apply_adjoint(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
@@ -1464,17 +1487,7 @@ int apply_adjoint(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t im
   DeviceGuard guard(t->device);
   const int H = p->frame_H, W = p->frame_W;
   const long long box_stride = (long long)p->H * p->box_pitch;
-  // the part of the frame inside the box; the rest of y meets no patch
-  const int r0 = std::max(0, p->box_y0), r1 = std::min(H, p->box_y0 + p->H);
-  const int c0 = std::max(0, p->box_x0), c1 = std::min(W, p->box_x0 + p->W);
-  if (r1 > r0 && c1 > c0) {
-    const dim3 grid((unsigned)((c1 - c0 + 255) / 256), (unsigned)std::min(r1 - r0, 1024), (unsigned)batch);
-    adjoint_copy_in<T><<<grid, 256, 0, s>>>((const T*)image + (long long)r0 * img_pitch + c0, img_pitch, img_frame_stride,
-                                            r1 - r0, c1 - c0,
-                                            (T*)p->box_in + (long long)(r0 - p->box_y0) * p->box_pitch + (c0 - p->box_x0),
-                                            p->box_pitch, box_stride);
-    LAUNCH((int)cudaGetLastError());
-  }
+  if (int rc = adjoint_copy<T>(p, image, img_pitch, img_frame_stride, batch, s)) return rc;
   if (int rc = apply_stages(p, p->box_in, p->box_pitch, box_stride, 0, p->H, p->box_out, p->box_pitch, box_stride, 0,
                             batch, 3, s))
     return rc;
@@ -1497,6 +1510,78 @@ int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
   if (p->adjoint) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan runs whole (rpsf_apply)");
   return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
                       out_row0, batch, stages, stream);
+}
+
+int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch, int64_t img_frame_stride,
+                         const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch, void* kernel_grad,
+                         void* stream) {
+  if (!ap || !fp || !image || !grad || !kernel_grad) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (!ap->adjoint || fp->adjoint)
+    return fail(RPSF_E_INVALID_ARGUMENT, "rpsf_kernel_gradient takes an adjoint plan, then a forward plan");
+  rpsf_transform* t = fp->tr;
+  if (ap->tr != t) return fail(RPSF_E_INVALID_ARGUMENT, "the two plans belong to different transforms");
+  if (fp->H != ap->frame_H || fp->W != ap->frame_W)
+    return fail(RPSF_E_INVALID_ARGUMENT, "the plans are for frames of (%d, %d) and (%d, %d)", fp->H, fp->W, ap->frame_H,
+                ap->frame_W);
+  if (t->win_len != t->P)
+    return fail(RPSF_E_UNSUPPORTED, "patch size %d runs embedded in %d; its kernel gradient is not implemented", t->win_len,
+                t->P);
+  if (t->n_kept < t->n) return fail(RPSF_E_UNSUPPORTED, "a sharded transform holds only some patches' kernels");
+  if (fp->sat_threshold < INFINITY)
+    return fail(RPSF_E_UNSUPPORTED, "the kernel gradient has no saturation branch (set an infinite threshold)");
+  if (fp->pad_mode == PAD_NONE) return fail(RPSF_E_UNSUPPORTED, "the materialised pad has no index map");
+  if (fp->row_begin != 0 || fp->row_end != fp->H)
+    return fail(RPSF_E_UNSUPPORTED, "the forward plan owns rows [%d, %d), not the whole frame", fp->row_begin, fp->row_end);
+  if (fp->pad_mode != ap->frame_pad_mode)
+    return fail(RPSF_E_INVALID_ARGUMENT, "the plans use pad modes %d and %d", fp->pad_mode, ap->frame_pad_mode);
+  if (batch < 1 || batch > fp->max_batch || batch > ap->max_batch)
+    return fail(RPSF_E_INVALID_ARGUMENT, "batch %d outside [1, %d]", batch, std::min(fp->max_batch, ap->max_batch));
+  if (img_pitch < fp->W || grad_pitch < fp->W) return fail(RPSF_E_INCORRECT_SHAPE, "row pitch smaller than frame width");
+  // both plans take the patches that touch the frame, sorted by corner: kgrad pairs their workspaces slot by slot
+  if (fp->active_host != ap->active_host)
+    return fail(RPSF_E_INVALID_ARGUMENT, "the forward and adjoint plans list different active patches");
+  DeviceGuard guard(t->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int P = t->P;
+  // per-stage events of the forward plan (bench only): K1(x) | copy + K1(g) | zeroing + kgrad
+  cudaEvent_t* ev = nullptr;
+  if (fp->timing && fp->n_active > 0) {
+    if (fp->events_used + 4 > fp->events.size()) {
+      for (int i = 0; i < 4; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); fp->events.push_back(e); }
+    }
+    ev = &fp->events[fp->events_used];
+    fp->events_used += 4;
+    CU(cudaEventRecord(ev[0], s));
+  }
+  // 1. X: K1 of the forward plan (stages = 1 writes nothing to `out`)
+  if (int rc = apply_stages(fp, image, img_pitch, img_frame_stride, 0, fp->H, kernel_grad, fp->W, 0, 0, batch, 1, s))
+    return rc;
+  if (ev) CU(cudaEventRecord(ev[1], s));
+  // 2-3. G: the gradient into the adjoint plan's zero-bordered box, K1 there
+  const long long box_stride = (long long)ap->H * ap->box_pitch;
+  if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy<float> : adjoint_copy<double>)(ap, grad, grad_pitch, grad_frame_stride,
+                                                                                     batch, s))
+    return rc;
+  if (int rc = apply_stages(ap, ap->box_in, ap->box_pitch, box_stride, 0, ap->H, ap->box_out, ap->box_pitch, box_stride, 0,
+                            batch, 1, s))
+    return rc;
+  if (ev) CU(cudaEventRecord(ev[2], s));
+  // 4. patches that do not touch the frame: an exact zero (neither map reads them)
+  const size_t slot_bytes = (size_t)P * P * 2 * real_size(t->dtype);
+  std::vector<char> touched(t->n, 0);           // the active list is in corner order: zero runs of untouched indices
+  for (int i : fp->active_host) touched[i] = 1;
+  for (int i = 0; i < t->n;) {
+    if (touched[i]) { ++i; continue; }
+    int j = i;
+    while (j < t->n && !touched[j]) ++j;
+    CU(cudaMemsetAsync((char*)kernel_grad + (size_t)i * slot_bytes, 0, (size_t)(j - i) * slot_bytes, s));
+    i = j;
+  }
+  // 5. conj(X) G / P^2, summed over the batch
+  if (fp->n_active > 0)
+    LAUNCH(t->ops->kgrad(t->dtype, fp->workspace, ap->workspace, kernel_grad, fp->active_dev, t->tw, fp->n_active, batch, s));
+  if (ev) CU(cudaEventRecord(ev[3], s));
+  return RPSF_OK;
 }
 
 int rpsf_plan_enable_timing(rpsf_plan* p, int enabled) {

@@ -1,6 +1,7 @@
 // rpsf_inst.cu — instantiates every kernel for one patch size (compile with -DRPSF_P=<P>).
 #include <cstdlib>
 #include "rpsf_ops.h"
+#include "rpsf_kgrad.cuh"
 
 #ifndef RPSF_P
 #error "compile with -DRPSF_P=<patch size>"
@@ -98,6 +99,8 @@ int init() {
   if ((e = set_smem(fft2_rows<P, double, double>, fft2_row_smem<double>()))) return e;
   if ((e = set_smem(fft2_cols<P, float>, col_smem<float>()))) return e;
   if ((e = set_smem(fft2_cols<P, double>, col_smem<double>()))) return e;
+  if ((e = set_smem(kgrad<P, float>, GradTile<P, float>::SMEM))) return e;
+  if ((e = set_smem(kgrad<P, double>, GradTile<P, double>::SMEM))) return e;
   return 0;
 }
 
@@ -279,7 +282,23 @@ int fft2(int dt, int in_dt, const void* values, void* out, const void* tw, long 
   return dt == DT_F32 ? fft2_t<float>(values, out, tw, n, s) : fft2_t<double>(values, out, tw, n, s);
 }
 
-const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2};
+// launched plainly (no programmatic dependent launch): it reads both plans' spectra, written by the kernels before it
+template <typename T>
+int kgrad_t(const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active, int batch,
+            cudaStream_t s) {
+  using GT = GradTile<P, T>;
+  if (n_active == 0) return 0;
+  kgrad<P, T><<<cdiv((long long)n_active * GT::NTILE, GT::SLOTS), GT::THREADS, GT::SMEM, s>>>(
+      (const cplx<T>*)xspec, (const cplx<T>*)gspec, (cplx<T>*)out, active, (const cplx<T>*)tw, n_active, batch);
+  return (int)cudaGetLastError();
+}
+int kgrad_launch(int dt, const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active,
+                 int batch, cudaStream_t s) {
+  return dt == DT_F32 ? kgrad_t<float>(xspec, gspec, out, active, tw, n_active, batch, s)
+                      : kgrad_t<double>(xspec, gspec, out, active, tw, n_active, batch, s);
+}
+
+const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch};
 
 }  // namespace
 

@@ -38,6 +38,10 @@ struct Ops {
   int (*prep)(int dt, int kernel_dt, const void* full, void* kmain, void* knyq, int n_patches, cudaStream_t s);
   int (*fft2)(int dt, int in_dt, const void* values, void* out, const void* tw, long long n_patches,
               cudaStream_t s);
+  // gradient with respect to the transfer kernel (rpsf_kgrad.cuh): conj(X) G / P^2 summed over `batch` frames of the
+  // forward (xspec) and adjoint (gspec) row-spectrum workspaces, into the (n, P, P) cube `out` at slots active[a]
+  int (*kgrad)(int dt, const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active,
+               int batch, cudaStream_t s);
 };
 
 const Ops* ops_for(int P);   // nullptr when P is unsupported

@@ -12,7 +12,9 @@ class DeviceCube(IndexedCube):
 
     ``values`` downloads (once) to a numpy array in the reference layout, so host-side users —
     ``save()``, ``==``, ``cube[coord]`` — see exactly what the reference's cube would hold
-    (regularizepsf/util.py:147-150).
+    (regularizepsf/util.py:147-150).  A tensor that requires grad (a transfer kernel being fitted) is downloaded again
+    after each in-place update (``optimizer.step()``), so ``save()`` and ``==`` see the fitted values; writes through
+    ``tensor.data`` do not bump the tensor's version and are not seen.
     """
 
     def __init__(self, coordinates, tensor) -> None:
@@ -25,6 +27,7 @@ class DeviceCube(IndexedCube):
         self._coordinates = coordinates
         self._tensor = tensor
         self._host = None
+        self._host_version = None
         self._index = {tuple(c): i for i, c in enumerate(coordinates)}
 
     @property
@@ -37,8 +40,14 @@ class DeviceCube(IndexedCube):
 
     @property
     def values(self) -> np.ndarray:
+        t = self._tensor
+        if t.requires_grad:
+            if self._host is None or self._host_version != t._version:
+                self._host = t.detach().cpu().numpy()
+                self._host_version = t._version
+            return self._host
         if self._host is None:
-            self._host = self._tensor.cpu().numpy()
+            self._host = t.cpu().numpy()
         return self._host
 
     @property

@@ -19,6 +19,7 @@ from regularizepsf_b200.exceptions import IncorrectShapeError, InvalidCoordinate
 from regularizepsf_b200.util import IndexedCube
 
 _DTYPES = {"float32": _native.F32, "float64": _native.F64}
+_NATIVE_SIZES = (16, 32, 64, 128, 256, 512)           # patch sizes with an FFT length of their own (no embedding)
 _default_dtype = "float32"
 
 
@@ -68,6 +69,14 @@ class _NativeTransform:
         self._plans: dict[tuple, int] = {}
         self._saturation: dict[int, tuple] = {}          # plan handle -> the saturation settings it was last given
         self._finalizer = weakref.finalize(self, _NativeTransform._cleanup, self.lib, self.handle, self._plans)
+        # a kernel tensor that requires grad may be updated in place (optimizer.step()): the tensor and the version it
+        # had when it was laid out, so that the next call lays it out again (ArrayPSFTransform._native_transform)
+        self.kernel_source = None
+        self.kernel_version = None
+        self.set_kernel(kernel_tensor, stream)
+
+    def set_kernel(self, kernel_tensor, stream: int) -> None:
+        """Lay out ``kernel_tensor`` (contiguous, on this device) for the kernels; stream-ordered on ``stream``."""
         kcode = _native.F32 if str(kernel_tensor.dtype) == "torch.complex64" else _native.F64
         _native.check(self.lib.rpsf_transform_set_kernel(self.handle, kernel_tensor.data_ptr(), kcode, stream))
 
@@ -145,6 +154,8 @@ class ArrayPSFTransform:
 
     def __init__(self, transfer_kernel: IndexedCube) -> None:
         self._transfer_kernel = transfer_kernel
+        # the CUDA tensor of a device-resident kernel: the transform is differentiable in it when it requires grad
+        self._kernel_tensor = transfer_kernel.tensor if isinstance(transfer_kernel, DeviceCube) else None
         self._native: dict[tuple[str, int], _NativeTransform] = {}
         self._coords_i32: np.ndarray | None = None
         # row-slab shard (distributed.shard_transform_rows): coordinates of the COMPLETE transform and which of them
@@ -265,24 +276,42 @@ class ArrayPSFTransform:
             if p0 != p1:
                 # the reference's apodization window only broadcasts for square patches (transform.py:151-155)
                 raise IncorrectShapeError(f"patches must be square, got {(p0, p1)}")
-            kernel = self._transfer_kernel
-            if isinstance(kernel, DeviceCube):
-                kt = kernel.tensor
-                if kt.device.index != device:
-                    kt = kt.to(f"cuda:{device}")
-            else:
-                values = np.ascontiguousarray(kernel.values)
-                if values.dtype not in (np.complex64, np.complex128):
-                    values = values.astype(np.complex128)
-                kt = torch.from_numpy(values).to(f"cuda:{device}")
-            kt = kt.contiguous()
             with torch.cuda.device(device):
                 # set_kernel is stream-ordered on this device's current stream, the stream `kt` was made on, so
                 # the caching allocator cannot hand kt's block to anyone before the layout kernel has read it
+                kt = self._kernel_on(torch, device)
                 nt = _NativeTransform(self._coords(), p0, dtype_name, device, kt, _native.current_stream_ptr(torch),
                                       keep=self._shard_keep)
+            source = self._kernel_tensor
+            if source is not None and source.requires_grad:
+                nt.kernel_source, nt.kernel_version = source, source._version
             self._native[key] = nt
+        elif nt.kernel_source is not None and nt.kernel_source._version != nt.kernel_version:
+            # the kernel tensor was updated in place since it was laid out (optimizer.step()): lay it out again
+            version = nt.kernel_source._version
+            with torch.cuda.device(device):
+                nt.set_kernel(self._kernel_on(torch, device), _native.current_stream_ptr(torch))
+            nt.kernel_version = version
         return nt
+
+    def _kernel_on(self, torch, device: int):
+        """The transfer kernel as a contiguous complex tensor on ``device`` (without autograd history)."""
+        kernel = self._transfer_kernel
+        if isinstance(kernel, DeviceCube):
+            kt = kernel.tensor.detach()
+            if kt.device.index != device:
+                kt = kt.to(f"cuda:{device}")
+        else:
+            values = np.ascontiguousarray(kernel.values)
+            if values.dtype not in (np.complex64, np.complex128):
+                values = values.astype(np.complex128)
+            kt = torch.from_numpy(values).to(f"cuda:{device}")
+        return kt.contiguous()
+
+    def _trainable_kernel(self):
+        """The kernel tensor when the transform is differentiable in it (it requires grad), else None."""
+        kt = self._kernel_tensor
+        return kt if kt is not None and kt.requires_grad else None
 
     # ------------------------------------------------------------------ apply
     def apply(self, image, workers: int | None = None, pad_mode: str = "symmetric",
@@ -299,7 +328,9 @@ class ArrayPSFTransform:
         device-to-host copy, which is what bounds a host-to-host call (DESIGN.md section 5).
         """
         del workers
-        if _is_torch_tensor(image) and image.requires_grad and _native.require_cuda().is_grad_enabled():
+        kt = self._kernel_tensor
+        if (_is_torch_tensor(image) and (image.requires_grad or (kt is not None and kt.requires_grad))
+                and _native.require_cuda().is_grad_enabled()):
             return self._apply_differentiable(image, pad_mode, saturation_threshold, dtype, adjoint=False)
         if (pad_mode == "symmetric" and saturation_threshold == math.inf and dtype is None and out_dtype is None
                 and _is_torch_tensor(image)):
@@ -333,14 +364,16 @@ class ArrayPSFTransform:
         Takes what ``apply`` takes: a numpy array (any real dtype; returns float64) or a CUDA tensor (returns the
         compute dtype ``dtype``, "float32" by default), shaped (H, W) or (B, H, W).  ``pad_mode`` is one of the five
         modes with an index map ("symmetric", "reflect", "edge", "wrap", "constant").  A tensor that requires grad
-        gives a differentiable result whose backward is ``apply``.
+        gives a differentiable result whose backward is ``apply``; so does a transform whose kernel tensor
+        (``DeviceCube``) requires grad, whose kernel gradient is ``transfer_kernel_gradient`` with the roles swapped.
         """
         if pad_mode not in _native.PAD_MODES:
             raise NotImplementedError(f"apply_adjoint supports the pad modes {sorted(_native.PAD_MODES)}, got {pad_mode!r}")
         if self._shard_keep is not None:
             raise NotImplementedError("apply_adjoint needs the kernels of every patch; a sharded transform holds a subset")
         if _is_torch_tensor(image):
-            if image.requires_grad and _native.require_cuda().is_grad_enabled():
+            if ((image.requires_grad or self._trainable_kernel() is not None)
+                    and _native.require_cuda().is_grad_enabled()):
                 return self._apply_differentiable(image, pad_mode, math.inf, dtype, adjoint=True)
             return self._apply_device(image, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
         torch = _native.require_cuda()
@@ -352,7 +385,8 @@ class ArrayPSFTransform:
         return out.cpu().numpy().astype(np.float64, copy=False)
 
     def _apply_differentiable(self, image, pad_mode: str, saturation_threshold: float, dtype, adjoint: bool):
-        """``apply`` / ``apply_adjoint`` of a CUDA tensor that requires grad: a linear map whose backward is the other."""
+        """``apply`` / ``apply_adjoint`` of a CUDA tensor that requires grad, or with a kernel tensor that does: a linear
+        map whose backward is the other, and, for the kernel, ``transfer_kernel_gradient``."""
         if not (saturation_threshold == math.inf or math.isnan(saturation_threshold)):
             raise NotImplementedError("apply is not differentiable with a finite saturation_threshold: the mask and "
                                       "the restored pixels depend on the image")
@@ -361,8 +395,84 @@ class ArrayPSFTransform:
                                       f"{pad_mode!r} is computed by np.pad on the host")
         if self._shard_keep is not None:
             raise NotImplementedError("a sharded transform is not differentiable: its transpose needs every patch's kernel")
-        from regularizepsf_b200._autograd import LinearMap
-        return LinearMap.apply(image, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
+        kernel = self._trainable_kernel()
+        if kernel is None:
+            from regularizepsf_b200._autograd import LinearMap
+            return LinearMap.apply(image, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
+        self._check_kernel_gradient(pad_mode)
+        for nt in self._native.values():
+            if nt.kernel_source is None:       # requires_grad was switched on after the layout: track it from now on
+                nt.kernel_source, nt.kernel_version = kernel, None
+        from regularizepsf_b200._autograd import KernelMap
+        return KernelMap.apply(image, kernel, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
+
+    def _check_kernel_gradient(self, pad_mode: str) -> None:
+        """NotImplementedError for what ``transfer_kernel_gradient`` has no device path for (DESIGN.md section 6)."""
+        if pad_mode not in _native.PAD_MODES:
+            raise NotImplementedError(f"the kernel gradient supports the pad modes {sorted(_native.PAD_MODES)}, got "
+                                      f"{pad_mode!r}")
+        if self._shard_keep is not None:
+            raise NotImplementedError("the kernel gradient of a sharded transform is not implemented")
+        if self.psf_shape[0] not in _NATIVE_SIZES:
+            raise NotImplementedError(f"the kernel gradient is implemented for the patch sizes {_NATIVE_SIZES}; "
+                                      f"{self.psf_shape[0]} runs embedded in a larger FFT")
+
+    def transfer_kernel_gradient(self, image, grad_output, pad_mode: str = "symmetric", *, dtype=None):
+        """The gradient of ``<apply(image), grad_output>`` with respect to the transfer kernel, without saturation: the
+        vector-Jacobian product of ``apply`` in the kernel, for fitting a kernel to calibration pairs.  For patch p,
+        ``conj(X_p) * G_p / P**2`` summed over the frames, with ``X_p`` and ``G_p`` the FFT2 of the apodized patch of
+        the padded image and of the zero-extended ``grad_output``; patches that do not touch the frame get 0.  It uses
+        PyTorch's convention for complex gradients (dL/dRe + i dL/dIm) and is Hermitian per patch.
+
+        ``image`` and ``grad_output`` have the same shape, (H, W) or (B, H, W): numpy arrays (any real dtype; returns an
+        (N, P, P) complex128 array, computed on the device) or CUDA tensors (returns complex64 for the compute dtype
+        "float32", the default, complex128 for "float64").  ``pad_mode`` is one of the five modes with an index map.
+        Embedded patch sizes (not a power of two) and sharded transforms raise NotImplementedError.
+        """
+        self._check_kernel_gradient(pad_mode)
+        dtype_name = _normalize_dtype(dtype)
+        pad_code = _native.PAD_MODES[pad_mode]
+        if _is_torch_tensor(image) or _is_torch_tensor(grad_output):
+            if not (_is_torch_tensor(image) and _is_torch_tensor(grad_output)):
+                raise TypeError("image and grad_output must both be numpy arrays or both CUDA tensors")
+            return self._kernel_gradient_device(image.detach(), grad_output.detach(), dtype_name, pad_code)
+        torch = _native.require_cuda()
+        x, g = np.asarray(image), np.asarray(grad_output)
+        if x.shape != g.shape or x.ndim not in (2, 3):
+            raise IncorrectShapeError(f"image and grad_output must share a shape (H, W) or (B, H, W), got {x.shape} "
+                                      f"and {g.shape}")
+        device = f"cuda:{torch.cuda.current_device()}"
+        xt = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64)).to(device)
+        gt = torch.from_numpy(np.ascontiguousarray(g, dtype=np.float64)).to(device)
+        out = self._kernel_gradient_device(xt, gt, dtype_name, pad_code)
+        return out.cpu().numpy().astype(np.complex128, copy=False)
+
+    def _kernel_gradient_device(self, image, grad, dtype_name: str, pad_code: int = 0):
+        """``transfer_kernel_gradient`` of two CUDA tensors (no autograd history): the (N, P, P) complex tensor."""
+        torch = _native.require_cuda()
+        if not (image.is_cuda and grad.is_cuda) or image.device != grad.device:
+            raise ValueError("image and grad_output must be CUDA tensors on one device")
+        if tuple(image.shape) != tuple(grad.shape) or image.dim() not in (2, 3):
+            raise IncorrectShapeError(f"image and grad_output must share a shape (H, W) or (B, H, W), got "
+                                      f"{tuple(image.shape)} and {tuple(grad.shape)}")
+        want = torch.float32 if dtype_name == "float32" else torch.float64
+        with torch.cuda.device(image.device):
+            nt = self._native_transform(dtype_name, image.device.index)
+            frames = [t.unsqueeze(0) if t.dim() == 2 else t for t in (image, grad)]
+            frames = [t.to(want) if t.dtype != want else t for t in frames]
+            x, g = [t.contiguous() if t.stride(-1) != 1 else t for t in frames]
+            b, h, w = x.shape
+            forward = nt.plan(h, w, pad_code, 0, h, b)
+            adjoint = nt.plan(h, w, pad_code, 0, h, b, adjoint=True)
+            nt.set_saturation(forward, self._NO_SAT)
+            p = self.psf_shape[0]
+            out = torch.empty((len(self), p, p), dtype=torch.complex64 if dtype_name == "float32" else torch.complex128,
+                              device=x.device)
+            _native.check(nt.lib.rpsf_kernel_gradient(
+                adjoint, forward, x.data_ptr(), x.stride(1), x.stride(0) if b > 1 else h * x.stride(1),
+                g.data_ptr(), g.stride(1), g.stride(0) if b > 1 else h * g.stride(1), b, out.data_ptr(),
+                _native.current_stream_ptr(torch, x.device.index)))
+        return out
 
     _NO_SAT = (math.inf, 1, 7)
     _PAD_MATERIALIZED = 5                                  # RPSF_PAD_MATERIALIZED
