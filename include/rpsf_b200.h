@@ -211,6 +211,15 @@ int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_f
                int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
                void* stream);
 
+/* rpsf_apply with the saturation mask decided on `src`: the same `batch` frames before their conversion to the
+ * compute dtype, of src_dtype, row `img_row0 + i` of frame b at src + b*src_frame_stride + i*src_pitch (elements).
+ * The reference compares float64 values with the threshold; a float64 or 32/64-bit integer pixel just above it can
+ * round to it in float32.  Everything but the initial mask (the fill, the correction, the restored pixels) uses
+ * `image`.  Without saturation `src` is not read. */
+int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                      const void* src, int src_dtype, int64_t src_pitch, int64_t src_frame_stride, void* stream);
+
 /* ---- apply, host buffers (the call a reference user makes): H2D + convert + apply + D2H ------
  * image: `batch` contiguous (H, W) frames of image_dtype on the host (pinned or pageable);
  * out: `batch` contiguous (row_end-row_begin, W) frames of out_dtype (RPSF_F32 / RPSF_F64).

@@ -61,6 +61,7 @@ SIGNATURES = {
     "rpsf_upload": (_i, [ctypes.POINTER(_vp), _vp, _i64, _i]),
     "rpsf_device_free": (_i, [_vp, _i]),
     "rpsf_apply": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp]),
+    "rpsf_apply_source": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp, _i, _i64, _i64, _vp]),
     "rpsf_apply_host": (_i, [_vp, _vp, _i, _vp, _i, _i]),
     "rpsf_convert": (_i, [_vp, _i, _i64, _vp, _i, _i64, _i, _i, _i, _vp]),
     "rpsf_plan_workspace": (_i, [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_i64)]),

@@ -18,6 +18,7 @@
 #include <string>
 #include <thread>
 #include <tuple>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/rpsf_b200.h"
@@ -1275,11 +1276,41 @@ int rpsf_plan_set_saturation(rpsf_plan* p, double threshold, int dilation, int n
 }  // extern "C"
 
 namespace {
+// The caller's frames before their conversion to the compute dtype (laid out like the converted ones, with pitches
+// of their own): the saturation mask is decided on these, as the reference decides it on float64 values.
+struct SatSource {
+  const void* ptr;
+  int dtype;
+  long long pitch, frame_stride;
+};
+
+// launch sat_pad_mask with the mask decided on `src` when converting its dtype to T can change a comparison with
+// the threshold (float64 and 32/64-bit integers into float32), else on the converted image itself.  A 64-bit integer
+// rounds to double in the comparison, as it does in the reference's `.astype(float)`.
+template <typename T>
+int launch_sat_pad_mask(rpsf_plan* p, const void* image, const SatSource* src, const SatGeom& sg, int* any_flag,
+                        dim3 grid, cudaStream_t s) {
+  auto go = [&](auto tag, const void* ptr, long long pitch, long long stride) {
+    using TS = decltype(tag);
+    sat_pad_mask<T, TS><<<grid, 256, 0, s>>>((const T*)image, (const TS*)ptr, pitch, stride, (T*)p->sat_pf,
+                                             p->sat_mask[0], any_flag, p->sat_threshold, sg);
+  };
+  const int dt = (src && std::is_same<T, float>::value) ? src->dtype : -1;
+  switch (dt) {
+    case RPSF_F64: go(double(), src->ptr, src->pitch, src->frame_stride); break;
+    case RPSF_I32: go(int32_t(), src->ptr, src->pitch, src->frame_stride); break;
+    case RPSF_U32: go(uint32_t(), src->ptr, src->pitch, src->frame_stride); break;
+    case RPSF_I64: go((long long)0, src->ptr, src->pitch, src->frame_stride); break;
+    default: go(T(), image, sg.img_pitch, sg.img_frame_stride); break;
+  }
+  return (int)cudaGetLastError();
+}
+
 // Saturation pre-fill on the stream: pad + mask, dilate, compact in raster order, ordered fill.
 // On return *filled points at padded pixel (2P, 2P) of frame 0, i.e. at unpadded (0, 0).
 template <typename T>
-int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int batch,
-                cudaStream_t s, SatGeom* sg_out, const void** filled) {
+int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, const SatSource* src,
+                int batch, cudaStream_t s, SatGeom* sg_out, const void** filled) {
   rpsf_transform* t = p->tr;
   const int P = t->P, pad = 2 * P;
   SatGeom sg;
@@ -1301,9 +1332,7 @@ int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_
   int* any_flag = p->sat_flags;
   int* tickets = p->sat_flags + mb;
   const dim3 rows_grid((unsigned)std::min((sg.Wp + 255) / 256, 8), (unsigned)sg.Hp, (unsigned)batch);
-  sat_pad_mask<T><<<rows_grid, 256, 0, s>>>((const T*)image, (T*)p->sat_pf, p->sat_mask[0], any_flag,
-                                            p->sat_threshold, sg);
-  LAUNCH((int)cudaGetLastError());
+  LAUNCH(launch_sat_pad_mask<T>(p, image, src, sg, any_flag, rows_grid, s));
   int cur = 0;
   if (p->sat_dilation < 1) {
     sat_dilate<<<rows_grid, 256, 0, s>>>(p->sat_mask[0], p->sat_mask[1], any_flag, sg.Hp, sg.Wp, 1);
@@ -1341,9 +1370,10 @@ int sat_restore_launch(rpsf_plan* p, const void* image, void* out, int64_t out_p
   return RPSF_OK;
 }
 
+// `src`: the frames before their conversion to the compute dtype, for the saturation mask (nullptr: `image`)
 int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
                  int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
-                 int batch, int stages, void* stream_v) {
+                 int batch, int stages, void* stream_v, const SatSource* src = nullptr) {
   if (p->row_end == p->row_begin && stages >= 3) return RPSF_OK;      // an empty band (more ranks than half-patch rows): nothing to write
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   rpsf_transform* t = p->tr;
@@ -1392,8 +1422,8 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   if (sat) {
     if (img_row0 != 0 || img_rows < p->H)
       return fail(RPSF_E_UNSUPPORTED, "the saturation branch needs the whole frame resident (rows [0,%d))", p->H);
-    int rc = t->dtype == RPSF_F32 ? sat_prefill<float>(p, image, img_pitch, img_frame_stride, batch, s, &sg, &k1_image)
-                                  : sat_prefill<double>(p, image, img_pitch, img_frame_stride, batch, s, &sg, &k1_image);
+    int rc = t->dtype == RPSF_F32 ? sat_prefill<float>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image)
+                                  : sat_prefill<double>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image);
     if (rc) return rc;
     g1.img_row0 = 0; g1.img_rows = sg.Hp; g1.img_pitch = sg.Wp; g1.img_frame_stride = (long long)sg.Hp * sg.Wp;
     g1.pad_mode = PAD_NONE;
@@ -1620,6 +1650,19 @@ int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_f
                            out_frame_stride, out_row0, batch, 3, stream);
 }
 
+int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                      const void* src, int src_dtype, int64_t src_pitch, int64_t src_frame_stride, void* stream) {
+  if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (p->adjoint) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan has no saturation branch (rpsf_apply)");
+  if (!src) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (!elem_size(src_dtype)) return fail(RPSF_E_UNSUPPORTED, "unsupported source dtype code %d", src_dtype);
+  if (src_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "source row pitch smaller than frame width");
+  const SatSource source{src, src_dtype, src_pitch, src_frame_stride};
+  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
+                      out_row0, batch, 3, stream, &source);
+}
+
 
 int rpsf_convert(const void* src, int sdt, int64_t sp, void* dst, int ddt, int64_t dp, int rows, int cols,
                  int device, void* stream) {
@@ -1800,8 +1843,9 @@ int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out,
       if (e) return fail(RPSF_E_UNSUPPORTED, "unsupported image dtype code %d", image_dtype);
       LAUNCH((int)cudaGetLastError());
     }
-    rc = rpsf_apply(p, p->d_in[k], W, (int64_t)frame_px, 0, H, p->d_out[k], W, (int64_t)band_px, p->row_begin, nb,
-                    p->s_comp);
+    const SatSource raw{p->d_in_raw[k], image_dtype, W, (long long)frame_px};
+    rc = apply_stages(p, p->d_in[k], W, (int64_t)frame_px, 0, H, p->d_out[k], W, (int64_t)band_px, p->row_begin, nb, 3,
+                      p->s_comp, conv_in ? &raw : nullptr);
     if (rc) break;
     if (band_px == 0) { CU(cudaEventRecord(p->ev_comp[k], p->s_comp)); continue; }
     if (conv_out) {

@@ -26,21 +26,28 @@ template <typename T> __device__ __forceinline__ T quiet_nan();
 template <> __device__ __forceinline__ float quiet_nan<float>() { return __int_as_float(0x7fc00000); }
 template <> __device__ __forceinline__ double quiet_nan<double>() { return __longlong_as_double(0x7ff8000000000000LL); }
 
-// padded frame + initial mask (+ per-frame "any" flag).  grid (col blocks, Hp, frames).
-template <typename T>
-__global__ void sat_pad_mask(const T* __restrict__ image, T* __restrict__ pf, unsigned char* __restrict__ mask,
+// padded frame + initial mask (+ per-frame "any" flag).  grid (col blocks, Hp, frames).  The mask is decided on
+// `src`, the caller's pixels before their conversion to T (laid out like `image`, with pitches of its own): the
+// reference compares the float64 value, and a float64 or 32/64-bit integer pixel just above the threshold can round
+// to it or below in float32.  Where the conversion is exact, src is the image itself.
+template <typename T, typename TS>
+__global__ void sat_pad_mask(const T* __restrict__ image, const TS* __restrict__ src, long long src_pitch,
+                             long long src_frame_stride, T* __restrict__ pf, unsigned char* __restrict__ mask,
                              int* __restrict__ any_flag, double threshold, SatGeom g) {
   const int i = blockIdx.y, f = blockIdx.z;
   const bool direct = g.pad_mode == PAD_NONE;      // a materialised pad: negative indices address the caller's margin
   const int y = pad_index(i - g.pad, g.H, g.pad_mode);
-  const T* row = (y < 0 && !direct) ? nullptr : image + (long long)f * g.img_frame_stride + (long long)y * g.img_pitch;
+  const bool row_in = y >= 0 || direct;
+  const T* row = row_in ? image + (long long)f * g.img_frame_stride + (long long)y * g.img_pitch : nullptr;
+  const TS* src_row = row_in ? src + (long long)f * src_frame_stride + (long long)y * src_pitch : nullptr;
   const long long base = ((long long)f * g.Hp + i) * g.Wp;
   bool any = false;
   for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < g.Wp; j += gridDim.x * blockDim.x) {
     const int x = pad_index(j - g.pad, g.W, g.pad_mode);
-    const T v = (row && (x >= 0 || direct)) ? row[x] : T(0);
+    const bool in = row && (x >= 0 || direct);
+    const T v = in ? row[x] : T(0);
     pf[base + j] = v;
-    const bool m = double(v) > threshold;
+    const bool m = (in ? double(src_row[x]) : 0.0) > threshold;
     mask[base + j] = m ? 1 : 0;
     any |= m;
   }

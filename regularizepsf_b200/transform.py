@@ -495,10 +495,13 @@ class ArrayPSFTransform:
         want = torch.float32 if dtype_name == "float32" else torch.float64
         device = image.device if is_tensor else torch.device("cuda", torch.cuda.current_device())
         with torch.cuda.device(device):
-            dev = torch.from_numpy(padded).to(device).to(want)
+            dev64 = torch.from_numpy(padded).to(device)
+            dev = dev64.to(want)
             b, h, w = frames.shape
             inner = dev[:, pad:pad + h, pad:pad + w]            # a view: the kernels address the margin through its pitch
-            out = self._apply_device(inner, dtype_name, self._PAD_MATERIALIZED, sat=sat)
+            # the saturation mask is decided on the float64 padded frames, as the reference decides it
+            out = self._apply_device(inner, dtype_name, self._PAD_MATERIALIZED, sat=sat,
+                                     source=dev64[:, pad:pad + h, pad:pad + w])
         if is_tensor:
             return out[0] if squeeze else out
         result = out.cpu().numpy().astype(out_np.type, copy=False)
@@ -529,28 +532,32 @@ class ArrayPSFTransform:
 
     def _apply_device(self, image, dtype_name: str, pad_code: int, row_range: tuple[int, int] | None = None,
                       out=None, sat: tuple = _NO_SAT, mirrors: list[int] | None = None,
-                      frame_rows: tuple[int, int] | None = None, adjoint: bool = False):
+                      frame_rows: tuple[int, int] | None = None, adjoint: bool = False, source=None):
         """``frame_rows = (first, height)``: ``image`` holds only rows [first, first + image.shape[-2]) of frames that
         are ``height`` rows tall (a row slab keeps just the rows its patches read: ``plan_info()["rows_read"]``).
-        ``adjoint``: run the transpose (whole frames, no saturation)."""
+        ``adjoint``: run the transpose (whole frames, no saturation).  ``source``: the frames of ``image`` before a
+        conversion to the compute dtype, laid out alike, on which the saturation mask is decided (by default
+        ``image`` itself, before this call converts it)."""
         torch = _native.require_cuda()
         if not image.is_cuda:
             raise ValueError("apply() takes a numpy array or a CUDA tensor; move the tensor to the GPU first")
         if image.device.index == torch._C._cuda_getDevice():
             return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
-                                         adjoint)
+                                         adjoint, source)
         with torch.cuda.device(image.device):             # plans, streams and launches follow the image's device
             return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
-                                         adjoint)
+                                         adjoint, source)
 
     def _apply_device_on(self, torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows=None,
-                         adjoint=False):
+                         adjoint=False, source=None):
         nt = self._native_transform(dtype_name, image.device.index)
         want = torch.float32 if dtype_name == "float32" else torch.float64
         squeeze = image.dim() == 2
         frames = image.unsqueeze(0) if squeeze else image
         if frames.dim() != 3:
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {tuple(image.shape)}")
+        if source is None and frames.dtype != want and sat[0] != math.inf:
+            source = frames                               # the saturation mask compares the unconverted pixels
         if frames.dtype != want:
             frames = frames.to(want)
         if frames.stride(-1) != 1:
@@ -576,17 +583,34 @@ class ArrayPSFTransform:
             import ctypes
             arr = (ctypes.c_void_p * len(mirrors))(*mirrors)
             _native.check(nt.lib.rpsf_plan_set_output_mirrors(plan, len(mirrors), arr))
+        src_code = None
+        if source is not None and sat[0] != math.inf:
+            source = source.unsqueeze(0) if source.dim() == 2 else source
+            if source.stride(-1) != 1:
+                source = source.contiguous()
+            src_code = _TORCH_CODES.get(str(source.dtype))
         try:
-            rc = nt.lib.rpsf_apply(
-                plan, frames.data_ptr(), frames.stride(1), frames.stride(0) if b > 1 else held * frames.stride(1), first, held,
-                out.data_ptr(), out.stride(1), out.stride(0) if b > 1 else (r1 - r0) * out.stride(1), r0, b,
-                _native.current_stream_ptr(torch, frames.device.index))
+            args = (plan, frames.data_ptr(), frames.stride(1), frames.stride(0) if b > 1 else held * frames.stride(1),
+                    first, held, out.data_ptr(), out.stride(1), out.stride(0) if b > 1 else (r1 - r0) * out.stride(1),
+                    r0, b)
+            stream = _native.current_stream_ptr(torch, frames.device.index)
+            if src_code is None:
+                rc = nt.lib.rpsf_apply(*args, stream)
+            else:
+                rc = nt.lib.rpsf_apply_source(*args, source.data_ptr(), src_code, source.stride(1),
+                                              source.stride(0) if b > 1 else held * source.stride(1), stream)
             if rc:
                 _native.check(rc)
         finally:
             if mirrors:
                 _native.check(nt.lib.rpsf_plan_set_output_mirrors(plan, 0, None))
         return out[0] if squeeze else out
+
+
+# element type codes of the torch dtypes the native code reads (str(dtype) -> code)
+_TORCH_CODES = {"torch.float32": _native.F32, "torch.float64": _native.F64, "torch.uint8": _native.U8,
+                "torch.int16": _native.I16, "torch.uint16": _native.U16, "torch.int32": _native.I32,
+                "torch.int64": _native.I64, "torch.uint32": _native.U32}
 
 
 def _is_torch_tensor(obj) -> bool:

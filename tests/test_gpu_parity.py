@@ -484,9 +484,11 @@ def test_every_kernel_variant_agrees(shape, size, dtype):
     finally:
         nt.lib.rpsf_plan_set_gather_mode(plan, 0)
         nt.lib.rpsf_plan_set_overlap_mode(plan, 0)
+    want_flipped = oracle.apply_transform(image[::-1], coords, kernel)
     scale = max(float(np.max(np.abs(want))), float(np.max(np.abs(image))))
     for key, got in results.items():
         assert rel_err(got[0], want, scale) <= TOL[dtype], key
+        assert rel_err(got[1], want_flipped, scale) <= TOL[dtype], key
 
 
 def test_streaming_overlap_add_chunked_chains_equal_whole_chains():
