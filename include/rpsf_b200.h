@@ -94,10 +94,34 @@ int rpsf_transform_num_colours(const rpsf_transform* t);
 int rpsf_construct_kernel(const void* source_fft, const void* target_fft, void* kernel_out, int64_t count,
                           int dtype, double alpha, double epsilon, int device, void* stream);
 
+/* Vector-Jacobian product of rpsf_construct_kernel (transform.py:78-82), for a gradient that reaches the PSFs, alpha and
+ * epsilon.  kernel_grad is G, the gradient of the loss with respect to K in PyTorch's convention (dL/dRe + i dL/dIm);
+ * with a = |S|, b = |T|, c = epsilon b, D = a^(alpha+1) + c^(alpha+1), f = a^(alpha-1) / D, w = Re(G S conj(T)):
+ *   source_grad = f conj(G) T + w a^(alpha-3) ((alpha-1) c^(alpha+1) - 2 a^(alpha+1)) / D^2 S
+ *   target_grad = f G S - w (alpha+1) epsilon^(alpha+1) a^(alpha-1) b^(alpha-1) / D^2 T
+ *   alpha_epsilon_grad[0] = sum w a^(alpha-1) c^(alpha+1) ln(a/c) / D^2
+ *   alpha_epsilon_grad[1] = -sum w (alpha+1) epsilon^alpha a^(alpha-1) b^(alpha+1) / D^2
+ * A bin with G = 0 contributes exact zeros to all four outputs; where K is finite the 0 * inf products of these forms (at
+ * a = 0, b = 0 or c = 0) take their limit 0; where K is not finite and G != 0 the bin's cube outputs are NaN and so are
+ * both sums.  The four cubes are `count` complex elements on the device, all complex64 (RPSF_F32) or all complex128
+ * (RPSF_F64); source_grad and target_grad may be NULL (not computed).  alpha_epsilon_grad (device, 2 doubles, may be
+ * NULL) is accumulated in double for both dtypes over a fixed partition in a fixed order: bit-stable from run to run.
+ * Stream-ordered (scratch is cudaMallocAsync / cudaFreeAsync on `stream`), no host synchronisation. */
+int rpsf_construct_kernel_backward(const void* source_fft, const void* target_fft, const void* kernel_grad,
+                                   int64_t count, int dtype, double alpha, double epsilon, void* source_grad,
+                                   void* target_grad, double* alpha_epsilon_grad, int device, void* stream);
+
 /* ---- PSF cube FFT: replaces scipy.fft.fft2 in ArrayPSF.__init__ (psf.py:216-219) -----------
  * values: (n, P, P) real on the device; out: (n, P, P) complex, full spectrum, same precision. */
 int rpsf_psf_fft2(const void* values, void* out, int64_t n_patches, int patch_size, int dtype, int device,
                   void* stream);
+/* Vector-Jacobian product of rpsf_psf_fft2 (psf.py:216-219): values_grad = Re(fft2(conj(spectrum_grad))) = P^2
+ * Re(ifft2(spectrum_grad)), the gradient with respect to the real values of a loss whose gradient with respect to the
+ * spectrum is spectrum_grad (PyTorch's convention).  spectrum_grad: (n, P, P) complex on the device; values_grad: (n, P,
+ * P) real, same precision.  Patch sizes 16, 32, ..., 512 only; the others are RPSF_E_UNSUPPORTED.  Stream-ordered
+ * (an (n, P, P) complex scratch cube is cudaMallocAsync / cudaFreeAsync on `stream`). */
+int rpsf_psf_fft2_adjoint(const void* spectrum_grad, void* values_grad, int64_t n_patches, int patch_size, int dtype,
+                          int device, void* stream);
 
 /* ---- builder: per-cell averaging of star cutouts (SURVEY.md section 8f-4) -------------------
  * Replaces regularizepsf/builder.py:45-125 (_average_patches and its mean / percentile helpers):

@@ -5,8 +5,9 @@ Same public names as the reference package (regularizepsf/__init__.py:5-16): ``A
 ``calculate_covering``, the functional PSF decorators, ``ArrayPSFBuilder`` (stack averaging on the
 GPU, star finding through the optional ``sep`` dependency as in the reference) and the exception
 types.  ``DeviceCube`` holds a cube as a CUDA tensor: a transform built on one whose tensor requires grad is
-trainable (``ArrayPSFTransform.apply`` differentiates with respect to the transfer kernel).  Plotting is out of scope
-(see DESIGN.md).
+trainable (``ArrayPSFTransform.apply`` differentiates with respect to the transfer kernel), and an ``ArrayPSF`` whose
+values are a ``DeviceCube`` that requires grad makes ``ArrayPSFTransform.construct`` differentiable in the PSF values,
+as 0-d tensors ``alpha`` and ``epsilon`` do.  Plotting is out of scope (see DESIGN.md).
 """
 from regularizepsf_b200.exceptions import (
     FunctionParameterMismatchError,

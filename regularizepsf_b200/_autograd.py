@@ -3,7 +3,9 @@
 Without saturation, ``apply`` is linear in the image, so the vector-Jacobian product of ``apply`` is ``apply_adjoint``
 of the output gradient and that of ``apply_adjoint`` is ``apply``.  ``LinearMap`` saves nothing for backward, and the
 backward goes through it again, so double backward works too.  ``KernelMap`` is used when the transfer kernel requires
-grad: ``apply`` is linear in the kernel as well, and its kernel gradient is ``transfer_kernel_gradient``.
+grad: ``apply`` is linear in the kernel as well, and its kernel gradient is ``transfer_kernel_gradient``.  ``Construct``
+and ``PsfFFT`` carry that gradient on from the kernel to the PSF values, alpha and epsilon
+(``ArrayPSFTransform.construct``).
 """
 from __future__ import annotations
 
@@ -60,3 +62,75 @@ class KernelMap(torch.autograd.Function):
             grad_kernel = transform._kernel_gradient_device(x.detach(), g.detach(), ctx.dtype_name, ctx.pad_code)
             grad_kernel = grad_kernel.to(device=ctx.kernel_device, dtype=ctx.kernel_dtype)
         return grad_image, grad_kernel, None, None, None, None
+
+
+class PsfFFT(torch.autograd.Function):
+    """``forward(values)``: the FFT cube of a real (N, P, P) CUDA tensor (``rpsf_psf_fft2``, psf.py:216-219), complex64
+    for float32 values and complex128 for float64.  The backward is ``rpsf_psf_fft2_adjoint``, Re(fft2(conj(G))), in the
+    values' dtype; native patch sizes only.  Used by ``ArrayPSFTransform.construct`` for values that require grad, once
+    per call: a graph kept across calls could not be backpropagated twice."""
+
+    @staticmethod
+    def forward(ctx, values):
+        from regularizepsf_b200.psf import _psf_fft2
+        ctx.values_dtype = values.dtype
+        return _psf_fft2(values.detach().contiguous(), torch)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        from regularizepsf_b200 import _native
+        wide = torch.complex64 if ctx.values_dtype == torch.float32 else torch.complex128
+        grad = grad_output.to(wide).contiguous()
+        n, p, _ = grad.shape
+        out = torch.empty(grad.shape, dtype=ctx.values_dtype, device=grad.device)
+        with torch.cuda.device(grad.device):
+            _native.check(_native.load().rpsf_psf_fft2_adjoint(
+                grad.data_ptr(), out.data_ptr(), n, p, _native.F32 if wide == torch.complex64 else _native.F64,
+                grad.device.index, _native.current_stream_ptr(torch)))
+        return out
+
+
+class Construct(torch.autograd.Function):
+    """``forward(source_fft, target_fft, alpha, epsilon, alpha_value, epsilon_value)``: the transfer kernel
+    (``rpsf_construct_kernel``, transform.py:78-82) of two complex cubes of one dtype.  ``alpha`` / ``epsilon`` are the
+    caller's objects (floats or 0-d tensors, which get gradients), ``alpha_value`` / ``epsilon_value`` their values as
+    floats.  The backward is ``rpsf_construct_kernel_backward``: the cube gradients in the cubes' dtype, those of alpha
+    and epsilon accumulated in double and returned in each tensor's dtype and device.  Once-differentiable."""
+
+    @staticmethod
+    def forward(ctx, source_fft, target_fft, alpha, epsilon, alpha_value: float, epsilon_value: float):
+        from regularizepsf_b200 import _native
+        ctx.values = (alpha_value, epsilon_value)
+        ctx.scalars = tuple((x.dtype, x.device) if torch.is_tensor(x) else None for x in (alpha, epsilon))
+        ctx.save_for_backward(source_fft, target_fft)
+        kernel = torch.empty_like(source_fft)
+        code = _native.F32 if source_fft.dtype == torch.complex64 else _native.F64
+        with torch.cuda.device(source_fft.device):
+            _native.check(_native.load().rpsf_construct_kernel(
+                source_fft.data_ptr(), target_fft.data_ptr(), kernel.data_ptr(), source_fft.numel(), code, alpha_value,
+                epsilon_value, source_fft.device.index, _native.current_stream_ptr(torch)))
+        return kernel
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        from regularizepsf_b200 import _native
+        s, t = ctx.saved_tensors
+        grad = grad_output.to(s.dtype).contiguous()
+        need_s, need_t, need_a, need_e = ctx.needs_input_grad[:4]
+        grad_s = torch.empty_like(s) if need_s else None
+        grad_t = torch.empty_like(t) if need_t else None
+        scalars = torch.empty(2, dtype=torch.float64, device=s.device) if need_a or need_e else None
+        code = _native.F32 if s.dtype == torch.complex64 else _native.F64
+        with torch.cuda.device(s.device):
+            _native.check(_native.load().rpsf_construct_kernel_backward(
+                s.data_ptr(), t.data_ptr(), grad.data_ptr(), s.numel(), code, ctx.values[0], ctx.values[1],
+                grad_s.data_ptr() if need_s else None, grad_t.data_ptr() if need_t else None,
+                scalars.data_ptr() if scalars is not None else None, s.device.index, _native.current_stream_ptr(torch)))
+        grad_a = grad_e = None
+        if need_a:
+            grad_a = scalars[0].to(dtype=ctx.scalars[0][0], device=ctx.scalars[0][1])
+        if need_e:
+            grad_e = scalars[1].to(dtype=ctx.scalars[1][0], device=ctx.scalars[1][1])
+        return grad_s, grad_t, grad_a, grad_e, None, None

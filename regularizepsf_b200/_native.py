@@ -40,7 +40,9 @@ SIGNATURES = {
     "rpsf_transform_set_kernel": (_i, [_vp, _vp, _i, _vp]),
     "rpsf_transform_num_colours": (_i, [_vp]),
     "rpsf_construct_kernel": (_i, [_vp, _vp, _vp, _i64, _i, _d, _d, _i, _vp]),
+    "rpsf_construct_kernel_backward": (_i, [_vp, _vp, _vp, _i64, _i, _d, _d, _vp, _vp, _vp, _i, _vp]),
     "rpsf_psf_fft2": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp]),
+    "rpsf_psf_fft2_adjoint": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp]),
     "rpsf_average_patches": (_i, [_vp, _i64, _i, _vp, _vp, _i64, _i, _d, _vp, _i, _vp]),
     "rpsf_plane_background": (_i, [_vp, _i64, _i, _vp, _i, _vp]),
     "rpsf_star_cutouts": (_i, [_vp, _i, _i, _i, _vp, _i64, _i, _d, _d, _d, _vp, _vp, _i, _vp]),

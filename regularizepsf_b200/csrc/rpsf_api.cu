@@ -26,6 +26,7 @@
 #include "rpsf_saturation.cuh"
 #include "rpsf_builder.cuh"
 #include "rpsf_adjoint.cuh"
+#include "rpsf_construct_grad.cuh"
 
 namespace rpsf {
 const Ops* ops_for(int P) {
@@ -573,6 +574,71 @@ int rpsf_construct_kernel(const void* S, const void* Tg, void* K, int64_t count,
     construct_transfer_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>(
         (const double2*)S, (const double2*)Tg, (double2*)K, count, alpha, epsilon);
   LAUNCH((int)cudaGetLastError());
+  return RPSF_OK;
+}
+
+int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G, int64_t count, int dtype, double alpha,
+                                   double epsilon, void* source_grad, void* target_grad, double* alpha_epsilon_grad,
+                                   int device, void* stream) {
+  if (count < 0 || (count > 0 && (!S || !Tg || !G))) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "dtype must be f32 or f64");
+  DeviceGuard guard(device);
+  if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (count == 0) {
+    if (alpha_epsilon_grad) CU(cudaMemsetAsync(alpha_epsilon_grad, 0, 2 * sizeof(double), s));
+    return RPSF_OK;
+  }
+  if (!source_grad && !target_grad && !alpha_epsilon_grad) return RPSF_OK;
+  const int ctas = (int)std::min<long long>((count + CGRAD_THREADS - 1) / CGRAD_THREADS, CGRAD_MAX_CTAS);
+  double2* partial = nullptr;
+  if (alpha_epsilon_grad) {
+    cudaError_t e = cudaMallocAsync((void**)&partial, sizeof(double2) * ctas, s);
+    if (e != cudaSuccess) return fail(RPSF_E_CUDA, "cudaMallocAsync of %d partial sums failed: %s", ctas, cudaGetErrorString(e));
+  }
+  if (dtype == RPSF_F32)
+    construct_transfer_kernel_backward<float><<<ctas, CGRAD_THREADS, 0, s>>>(
+        (const float2*)S, (const float2*)Tg, (const float2*)G, count, (float)alpha, (float)epsilon, (float2*)source_grad,
+        (float2*)target_grad, partial);
+  else
+    construct_transfer_kernel_backward<double><<<ctas, CGRAD_THREADS, 0, s>>>(
+        (const double2*)S, (const double2*)Tg, (const double2*)G, count, alpha, epsilon, (double2*)source_grad,
+        (double2*)target_grad, partial);
+  cudaError_t e = cudaGetLastError();
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  if (e == cudaSuccess && partial) {
+    construct_grad_sum<CGRAD_THREADS><<<1, CGRAD_THREADS, 0, s>>>(partial, ctas, alpha_epsilon_grad);
+    e = cudaGetLastError();
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+  }
+  if (partial) cudaFreeAsync(partial, s);
+  if (e != cudaSuccess) return fail(RPSF_E_CUDA, "construct backward launch failed: %s", cudaGetErrorString(e));
+  return RPSF_OK;
+}
+
+int rpsf_psf_fft2_adjoint(const void* spectrum_grad, void* values_grad, int64_t n, int P, int dtype, int device,
+                          void* stream) {
+  if (n < 0 || (n > 0 && (!spectrum_grad || !values_grad))) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "dtype must be f32 or f64");
+  const Ops* ops = ops_for(P);
+  if (!ops) return fail(RPSF_E_UNSUPPORTED, "the PSF FFT adjoint is implemented for the patch sizes 16, 32, ..., 512, not %d", P);
+  if (n == 0) return RPSF_OK;
+  DeviceGuard guard(device);
+  if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
+  int e = ops->init();
+  if (e) return fail(RPSF_E_CUDA, "kernel attribute setup failed: %s", cudaGetErrorString((cudaError_t)e));
+  void* tw = nullptr; void* win = nullptr;
+  int rc = shared_tables(P, dtype, device, &tw, &win);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  void* scratch = nullptr;                                        // the complex row spectra, (n, P, P)
+  const size_t bytes = 2 * real_size(dtype) * (size_t)n * P * P;
+  cudaError_t ce = cudaMallocAsync(&scratch, bytes, s);
+  if (ce != cudaSuccess) return fail(RPSF_E_CUDA, "cudaMallocAsync of %zu scratch bytes failed: %s", bytes, cudaGetErrorString(ce));
+  e = ops->fft2_adjoint(dtype, spectrum_grad, scratch, values_grad, tw, n, s);
+  g_launches.fetch_add(2, std::memory_order_relaxed);
+  cudaFreeAsync(scratch, s);
+  if (e) return fail(RPSF_E_CUDA, "fft2 adjoint launch failed: %s", cudaGetErrorString((cudaError_t)e));
   return RPSF_OK;
 }
 

@@ -2,6 +2,7 @@
 #include <cstdlib>
 #include "rpsf_ops.h"
 #include "rpsf_kgrad.cuh"
+#include "rpsf_construct_grad.cuh"
 
 #ifndef RPSF_P
 #error "compile with -DRPSF_P=<patch size>"
@@ -101,6 +102,10 @@ int init() {
   if ((e = set_smem(fft2_cols<P, double>, col_smem<double>()))) return e;
   if ((e = set_smem(kgrad<P, float>, GradTile<P, float>::SMEM))) return e;
   if ((e = set_smem(kgrad<P, double>, GradTile<P, double>::SMEM))) return e;
+  if ((e = set_smem(fft2_rows_conj<P, float>, fft2_row_smem<float>()))) return e;
+  if ((e = set_smem(fft2_rows_conj<P, double>, fft2_row_smem<double>()))) return e;
+  if ((e = set_smem(fft2_cols_real<P, float>, col_smem<float>()))) return e;
+  if ((e = set_smem(fft2_cols_real<P, double>, col_smem<double>()))) return e;
   return 0;
 }
 
@@ -282,6 +287,22 @@ int fft2(int dt, int in_dt, const void* values, void* out, const void* tw, long 
   return dt == DT_F32 ? fft2_t<float>(values, out, tw, n, s) : fft2_t<double>(values, out, tw, n, s);
 }
 
+template <typename T>
+int fft2_adjoint_t(const void* grad, void* scratch, void* out, const void* tw, long long n, cudaStream_t s) {
+  if (n == 0) return 0;
+  fft2_rows_conj<P, T><<<cdiv(n * P, TL::TEAMS), TL::ROW_THREADS, fft2_row_smem<T>(), s>>>(
+      (const cplx<T>*)grad, (cplx<T>*)scratch, (const cplx<T>*)tw, n * P);
+  int e = (int)cudaGetLastError();
+  if (e) return e;
+  fft2_cols_real<P, T><<<cdiv(n * (P / TL::C), TL::SLOTS), TL::K2_THREADS, col_smem<T>(), s>>>(
+      (const cplx<T>*)scratch, (T*)out, (const cplx<T>*)tw, n);
+  return (int)cudaGetLastError();
+}
+int fft2_adjoint(int dt, const void* grad, void* scratch, void* out, const void* tw, long long n, cudaStream_t s) {
+  return dt == DT_F32 ? fft2_adjoint_t<float>(grad, scratch, out, tw, n, s)
+                      : fft2_adjoint_t<double>(grad, scratch, out, tw, n, s);
+}
+
 // launched plainly (no programmatic dependent launch): it reads both plans' spectra, written by the kernels before it
 template <typename T>
 int kgrad_t(const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active, int batch,
@@ -298,7 +319,7 @@ int kgrad_launch(int dt, const void* xspec, const void* gspec, void* out, const 
                       : kgrad_t<double>(xspec, gspec, out, active, tw, n_active, batch, s);
 }
 
-const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch};
+const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch, fft2_adjoint};
 
 }  // namespace
 

@@ -42,6 +42,10 @@ struct Ops {
   // forward (xspec) and adjoint (gspec) row-spectrum workspaces, into the (n, P, P) cube `out` at slots active[a]
   int (*kgrad)(int dt, const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active,
                int batch, cudaStream_t s);
+  // adjoint of fft2 (rpsf_construct_grad.cuh): out (n, P, P) real = Re(fft2(conj(grad))), through the complex
+  // (n, P, P) cube `scratch`
+  int (*fft2_adjoint)(int dt, const void* grad, void* scratch, void* out, const void* tw, long long n_patches,
+                      cudaStream_t s);
 };
 
 const Ops* ops_for(int P);   // nullptr when P is unsupported

@@ -9,6 +9,11 @@ The cube is computed the first time something needs it (``fft_evaluations``, ``f
 ``ArrayPSFTransform.construct``, ``save``, ``==``), so building models on a host without a GPU works
 and only the spectrum itself needs the device.  ``save`` / ``load`` keep the reference's h5 and FITS
 layouts (psf.py:262-330).
+
+The values may be a ``DeviceCube``: a real (N, P, P) CUDA tensor of float32 or float64, transformed where it lies.  When
+that tensor requires grad, ``ArrayPSFTransform.construct`` differentiates through the FFT (``_autograd.PsfFFT``), and the
+host accessors see a detached cube that is computed again after each in-place update of the tensor
+(``optimizer.step()``).
 """
 from __future__ import annotations
 
@@ -20,26 +25,45 @@ from regularizepsf_b200.exceptions import IncorrectShapeError, InvalidCoordinate
 from regularizepsf_b200.util import IndexedCube
 
 
-def _device_fft_cube(values_cube: IndexedCube) -> DeviceCube:
-    torch = _native.require_cuda()
-    lib = _native.load()
+def _values_tensor(values_cube: IndexedCube, torch):
+    """The values as a contiguous real CUDA tensor of float32 or float64 (an upload unless they are a ``DeviceCube``),
+    without autograd history."""
+    if isinstance(values_cube, DeviceCube):
+        values = values_cube.tensor.detach()
+        if values.dtype not in (torch.float32, torch.float64):
+            values = values.to(torch.float64)       # scipy.fft promotes the same way
+        return (values if values.is_cuda else values.cuda()).contiguous()
     values = values_cube.values
     if values.dtype not in (np.float32, np.float64):
         values = values.astype(np.float64)          # scipy.fft promotes the same way
+    return torch.from_numpy(np.ascontiguousarray(values)).cuda()
+
+
+def _psf_fft2(values, torch):
+    """``rpsf_psf_fft2`` of a contiguous real (N, P, P) CUDA tensor: the complex spectrum cube, on the same device."""
+    lib = _native.load()
     n, p0, p1 = values.shape
     if p0 != p1:
         raise IncorrectShapeError(f"PSF samples must be square for the device FFT, got {(p0, p1)}")
     if n and not 1 <= p0 <= 512:
         raise NotImplementedError(f"patch size {p0} has no device path (1..512: radix-2 kernels for powers of two "
                                   "16..512, a direct DFT otherwise)")
-    dev_values = torch.from_numpy(np.ascontiguousarray(values)).cuda()
-    cdtype = torch.complex64 if values.dtype == np.float32 else torch.complex128
-    out = torch.empty((n, p0, p1), dtype=cdtype, device=dev_values.device)
+    cdtype = torch.complex64 if values.dtype == torch.float32 else torch.complex128
+    out = torch.empty((n, p0, p1), dtype=cdtype, device=values.device)
     if n:
-        code = _native.F32 if values.dtype == np.float32 else _native.F64
-        _native.check(lib.rpsf_psf_fft2(dev_values.data_ptr(), out.data_ptr(), n, p0, code,
-                                        dev_values.device.index, _native.current_stream_ptr(torch)))
-    return DeviceCube(values_cube.coordinates, out)
+        code = _native.F32 if values.dtype == torch.float32 else _native.F64
+        with torch.cuda.device(values.device):
+            _native.check(lib.rpsf_psf_fft2(values.data_ptr(), out.data_ptr(), n, p0, code, values.device.index,
+                                            _native.current_stream_ptr(torch)))
+    return out
+
+
+def _device_fft_cube(values_cube: IndexedCube) -> DeviceCube:
+    torch = _native.require_cuda()
+    values = _values_tensor(values_cube, torch)
+    if values.dim() != 3:
+        raise IncorrectShapeError(f"PSF values must be (N, P, P), got shape {tuple(values.shape)}")
+    return DeviceCube(values_cube.coordinates, _psf_fft2(values, torch))
 
 
 class ArrayPSF:
@@ -50,6 +74,8 @@ class ArrayPSF:
         self._values_cube = values_cube
         self._workers = workers                      # accepted for API parity; the GPU ignores it
         self._given_fft_cube = fft_cube              # None: computed on the device at first use
+        self._computed_fft_cube = None
+        self._computed_version = None                # values tensor version the computed cube was made from
         if fft_cube is None:
             return                                   # a computed cube matches the values cube by construction
         if fft_cube.sample_shape != self._values_cube.sample_shape:
@@ -65,9 +91,19 @@ class ArrayPSF:
 
     @property
     def _fft_cube(self) -> IndexedCube:
-        if self._given_fft_cube is None:
-            self._given_fft_cube = _device_fft_cube(self._values_cube)
-        return self._given_fft_cube
+        if self._given_fft_cube is not None:
+            return self._given_fft_cube
+        tensor = self._values_device_tensor
+        version = tensor._version if tensor is not None and tensor.requires_grad else None
+        if self._computed_fft_cube is None or version != self._computed_version:
+            self._computed_fft_cube = _device_fft_cube(self._values_cube)
+            self._computed_version = version
+        return self._computed_fft_cube
+
+    @property
+    def _values_device_tensor(self):
+        """The CUDA tensor of the values when they are a ``DeviceCube``, else None."""
+        return self._values_cube.tensor if isinstance(self._values_cube, DeviceCube) else None
 
     @property
     def coordinates(self):

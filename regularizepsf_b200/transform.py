@@ -216,36 +216,91 @@ class ArrayPSFTransform:
 
     # ------------------------------------------------------------------ construct
     @classmethod
-    def construct(cls, source, target, alpha: float, epsilon: float) -> "ArrayPSFTransform":
+    def construct(cls, source, target, alpha, epsilon) -> "ArrayPSFTransform":
         """Build the regularised transfer kernel on the device (transform.py:53-83).
 
         ``K = conj(S) |S|^(alpha-1) / (|S|^(alpha+1) + (epsilon |T|)^(alpha+1)) * T`` elementwise over
         the two FFT cubes, in the cubes' precision, with no zero guard (0/0 bins are NaN, as in
         the reference).
+
+        Differentiable on the device: when grad mode is on and the values of either PSF (an ``ArrayPSF`` built on a
+        ``DeviceCube`` whose tensor requires grad), a given ``DeviceCube`` FFT cube, or ``alpha`` / ``epsilon`` require
+        grad, the result's kernel tensor requires grad, so ``loss(apply(x)).backward()`` reaches them through
+        ``rpsf_construct_kernel_backward`` and ``rpsf_psf_fft2_adjoint`` (DESIGN.md section 6).  ``alpha`` and ``epsilon``
+        are numbers or 0-d real tensors; tensors are read to the host, which synchronises (once for two on one device).  PSF values that
+        require grad need a native patch size (16, 32, ..., 512).  Otherwise the kernel is computed exactly as without
+        autograd.
         """
         if np.any(np.array(source.coordinates) != np.array(target.coordinates)):
             raise InvalidCoordinateError("Source PSF coordinates do not match target PSF coordinates.")
         torch = _native.require_cuda()
-        lib = _native.load()
-        s_cube = source.fft_cube if hasattr(source, "fft_cube") else source._fft_cube
-        t_cube = target.fft_cube if hasattr(target, "fft_cube") else target._fft_cube
-        if s_cube.sample_shape != t_cube.sample_shape:
-            raise IncorrectShapeError(f"source and target sample shapes differ: "
-                                      f"{s_cube.sample_shape} != {t_cube.sample_shape}")
-        s = cube_tensor(s_cube, torch)
-        t = cube_tensor(t_cube, torch)
+        differentiable = torch.is_grad_enabled() and (
+            any(_is_torch_tensor(x) and x.requires_grad for x in (alpha, epsilon))
+            or any(_spectrum_source(psf) is not None for psf in (source, target)))
+        if not differentiable:
+            lib = _native.load()
+            s_cube = source.fft_cube if hasattr(source, "fft_cube") else source._fft_cube
+            t_cube = target.fft_cube if hasattr(target, "fft_cube") else target._fft_cube
+            if s_cube.sample_shape != t_cube.sample_shape:
+                raise IncorrectShapeError(f"source and target sample shapes differ: "
+                                          f"{s_cube.sample_shape} != {t_cube.sample_shape}")
+            s = cube_tensor(s_cube, torch)
+            t = cube_tensor(t_cube, torch)
+            if s.device != t.device:
+                raise ValueError(f"source and target FFT cubes live on different devices: {s.device} and {t.device}")
+            wide = torch.complex128 if torch.complex128 in (s.dtype, t.dtype) else torch.complex64
+            with torch.cuda.device(s.device):                 # the launch stream must belong to the cubes' device
+                s = s.to(wide) if s.dtype != wide else s
+                t = t.to(wide) if t.dtype != wide else t
+                kernel = torch.empty_like(s)
+                code = _native.F32 if wide == torch.complex64 else _native.F64
+                _native.check(lib.rpsf_construct_kernel(s.data_ptr(), t.data_ptr(), kernel.data_ptr(), s.numel(), code,
+                                                        float(alpha), float(epsilon), s.device.index,
+                                                        _native.current_stream_ptr(torch)))
+            return cls(DeviceCube(source.coordinates, kernel))
+        from regularizepsf_b200._autograd import Construct
+        for name, value in (("alpha", alpha), ("epsilon", epsilon)):
+            if _is_torch_tensor(value) and (value.dim() != 0 or value.is_complex()):
+                raise ValueError(f"{name} must be a number or a 0-d real tensor, got shape {tuple(value.shape)} "
+                                 f"{value.dtype}")
+        if _is_torch_tensor(alpha) and _is_torch_tensor(epsilon) and alpha.device == epsilon.device:
+            values = torch.stack([alpha.detach().double(), epsilon.detach().double()]).tolist()   # one synchronisation
+        else:
+            values = [float(x.detach()) if _is_torch_tensor(x) else float(x) for x in (alpha, epsilon)]
+        s, t = _spectrum(source, torch), _spectrum(target, torch)
+        if tuple(s.shape[1:]) != tuple(t.shape[1:]):
+            raise IncorrectShapeError(f"source and target sample shapes differ: {tuple(s.shape[1:])} != "
+                                      f"{tuple(t.shape[1:])}")
         if s.device != t.device:
             raise ValueError(f"source and target FFT cubes live on different devices: {s.device} and {t.device}")
         wide = torch.complex128 if torch.complex128 in (s.dtype, t.dtype) else torch.complex64
-        with torch.cuda.device(s.device):                 # the launch stream must belong to the cubes' device
-            s = s.to(wide) if s.dtype != wide else s
-            t = t.to(wide) if t.dtype != wide else t
-            kernel = torch.empty_like(s)
-            code = _native.F32 if wide == torch.complex64 else _native.F64
-            _native.check(lib.rpsf_construct_kernel(s.data_ptr(), t.data_ptr(), kernel.data_ptr(), s.numel(), code,
-                                                    float(alpha), float(epsilon), s.device.index,
-                                                    _native.current_stream_ptr(torch)))
+        with torch.cuda.device(s.device):
+            s = (s.to(wide) if s.dtype != wide else s).contiguous()
+            t = (t.to(wide) if t.dtype != wide else t).contiguous()
+            kernel = Construct.apply(s, t, alpha, epsilon, *values)
         return cls(DeviceCube(source.coordinates, kernel))
+
+    def reconstruct(self, source, target, alpha, epsilon) -> None:
+        """Replace the transfer kernel by ``construct(source, target, alpha, epsilon)``'s, in place.
+
+        For a fitting loop that builds the kernel from its parameters at every step: the transform keeps its native
+        transforms and plans (with their spectrum workspaces, 75.8 MB per 2048^2 frame at 256 px) and lays the new
+        kernel out at its next call, where a fresh ``construct`` would create them again.  The coordinates and the patch
+        size must be the transform's (InvalidCoordinateError / IncorrectShapeError).  A kernel that requires grad on a
+        sharded transform raises NotImplementedError.
+        """
+        if np.any(np.array(source.coordinates) != np.array(self.coordinates)):
+            raise InvalidCoordinateError("the PSF coordinates do not match the transform's coordinates")
+        new = type(self).construct(source, target, alpha, epsilon)
+        if new.psf_shape != self.psf_shape:
+            raise IncorrectShapeError(f"the PSFs' sample shape {new.psf_shape} is not the transform's {self.psf_shape}")
+        kernel = new._kernel_tensor
+        if kernel.requires_grad and self._shard_keep is not None:
+            raise NotImplementedError("the kernel gradient of a sharded transform is not implemented")
+        self._transfer_kernel = DeviceCube(self.coordinates, kernel)
+        self._kernel_tensor = kernel
+        for nt in self._native.values():
+            nt.kernel_source, nt.kernel_version = kernel, None     # laid out again at the next call
 
     # ------------------------------------------------------------------ native state
     def _coords(self) -> np.ndarray:
@@ -611,6 +666,34 @@ class ArrayPSFTransform:
 _TORCH_CODES = {"torch.float32": _native.F32, "torch.float64": _native.F64, "torch.uint8": _native.U8,
                 "torch.int16": _native.I16, "torch.uint16": _native.U16, "torch.int32": _native.I32,
                 "torch.int64": _native.I64, "torch.uint32": _native.U32}
+
+
+def _spectrum_source(psf):
+    """The tensor through which ``psf``'s FFT cube depends on something that requires grad, or None: a given
+    ``DeviceCube`` FFT cube that requires grad, else a ``DeviceCube`` of values that does."""
+    given = getattr(psf, "_given_fft_cube", None)
+    if given is not None:
+        return given.tensor if isinstance(given, DeviceCube) and given.tensor.requires_grad else None
+    values = getattr(psf, "_values_device_tensor", None)
+    return values if values is not None and values.requires_grad else None
+
+
+def _spectrum(psf, torch):
+    """``psf``'s FFT cube as a CUDA tensor, differentiable in what ``_spectrum_source`` finds: a values tensor goes
+    through ``_autograd.PsfFFT``, afresh at every call."""
+    source = _spectrum_source(psf)
+    if source is None:
+        return cube_tensor(psf.fft_cube if hasattr(psf, "fft_cube") else psf._fft_cube, torch)
+    if psf._given_fft_cube is not None:
+        return source
+    if source.dim() != 3 or source.shape[1] not in _NATIVE_SIZES or source.shape[1] != source.shape[2]:
+        raise NotImplementedError(f"PSF values that require grad need square patches of a native size {_NATIVE_SIZES}; "
+                                  f"got {tuple(source.shape[1:])}, which runs embedded in a larger FFT")
+    if source.is_complex() or not source.is_cuda:
+        raise ValueError(f"PSF values that require grad must be a real CUDA tensor, got {source.dtype} on "
+                         f"{source.device}")
+    from regularizepsf_b200._autograd import PsfFFT
+    return PsfFFT.apply(source if source.dtype in (torch.float32, torch.float64) else source.to(torch.float64))
 
 
 def _is_torch_tensor(obj) -> bool:
