@@ -10,7 +10,11 @@
  * rpsf_last_error() gives the message for the calling thread.  No C++ exceptions cross the
  * ABI.  Device pointers are caller-owned; `stream` is a cudaStream_t passed as void* (NULL =
  * legacy default stream).  Stream-taking calls enqueue work and return without
- * synchronising.  A plan owns one spectrum workspace, so use one plan per concurrent stream.
+ * synchronising.  Calls that touch a transform's device state (its laid-out kernel, its plans'
+ * workspaces and scratch) are ordered by one event per transform: a call on a stream other than
+ * the last one's waits for the last one, so it sees the kernel laid out before it was issued and
+ * never shares a plan's workspace with a call still in flight.  Calls sharing a plan therefore
+ * do not overlap; use one plan per concurrent stream or thread to run them side by side.
  */
 #ifndef RPSF_B200_H
 #define RPSF_B200_H

@@ -315,9 +315,54 @@ struct rpsf_transform {
   // adjoint plan, refreshed by every rpsf_transform_set_kernel after that
   void* kconj_main = nullptr;
   void* kconj_nyq = nullptr;
+  // stream order of the transform's device state (the kernel layouts above, and the workspaces, boxes and scratch of
+  // its plans): recorded after the last launch of every call that touches it, on that call's stream (OrderedCall)
+  std::mutex order_mu;
+  cudaEvent_t order_ev = nullptr;
+  cudaStream_t order_stream = nullptr;   // the stream order_ev was last recorded on
+  bool order_recorded = false;
 };
 
 namespace {
+// Every entry point that reads or writes the transform's device state runs its launches between the two halves of an
+// OrderedCall on its stream.  The first half makes the stream wait for the last call's record when that call ran on
+// another stream (a call on the same stream is already behind it); the second records the event after this call's
+// launches.  So a call sees the kernel laid out by the calls issued before it, and no two calls use one plan's
+// workspace at once, whatever streams they use; a call on the stream of the previous one pays only the record.
+// cudaStreamPerThread names a different stream on every thread, so it always waits.  The mutex keeps the bookkeeping
+// whole for C callers that share a transform across threads.
+struct OrderedCall {
+  rpsf_transform* t;
+  cudaStream_t s;
+  int begin() {
+    std::lock_guard<std::mutex> lock(t->order_mu);
+    if (t->order_recorded && (s != t->order_stream || s == cudaStreamPerThread)) {
+      const cudaError_t e = cudaStreamWaitEvent(s, t->order_ev, 0);
+      if (e != cudaSuccess) return fail(RPSF_E_CUDA, "ordering after the transform's last call failed: %s", cudaGetErrorString(e));
+    }
+    return RPSF_OK;
+  }
+  // `rc`: the status of the launches; the record is made whatever it is, so that what was launched is ordered too
+  int end(int rc) {
+    std::lock_guard<std::mutex> lock(t->order_mu);
+    const cudaError_t e = cudaEventRecord(t->order_ev, s);
+    if (e != cudaSuccess) return rc ? rc : fail(RPSF_E_CUDA, "recording the transform's order event failed: %s", cudaGetErrorString(e));
+    t->order_stream = s;
+    t->order_recorded = true;
+    return rc;
+  }
+};
+
+// body() between the two halves of an OrderedCall on `s`, with the transform's device current
+template <typename F>
+int ordered(rpsf_transform* t, cudaStream_t s, F&& body) {
+  DeviceGuard guard(t->device);
+  if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", t->device);
+  OrderedCall call{t, s};
+  if (int rc = call.begin()) return rc;
+  return call.end(body());
+}
+
 // kconj_* = conj(kmain / knyq), stream-ordered after whatever wrote kmain on `s`
 int refresh_conj_kernel(rpsf_transform* t, cudaStream_t s) {
   if (!t->kconj_main || t->n_kept == 0) return RPSF_OK;
@@ -430,6 +475,11 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
   auto* t = new rpsf_transform;
   t->device = device; t->P = P; t->n = n; t->dtype = dtype; t->ops = ops; t->win_len = win_len;
   t->sm_count = sm_count_of(device);
+  if (cudaEventCreateWithFlags(&t->order_ev, cudaEventDisableTiming) != cudaSuccess) {
+    const cudaError_t ce = cudaGetLastError();
+    delete t;
+    return fail(RPSF_E_CUDA, "cannot create the transform's order event: %s", cudaGetErrorString(ce));
+  }
   t->corners.resize(n);
   for (int i = 0; i < n; ++i) t->corners[i] = make_int2(coords[2 * i], coords[2 * i + 1]);
   // Greedy colouring in list order: same-colour patches are pairwise disjoint.  For
@@ -456,7 +506,7 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
     t->n_colours = (int)members.size();
   }
   int rc = shared_tables(P, dtype, device, &t->tw, &t->win);     // owned by the library, not by the transform
-  if (rc) { delete t; return rc; }
+  if (rc) { rpsf_transform_destroy(t); return rc; }
   if (win_len != P) {
     // the window of the true patch size, zero beyond it (transform.py:151-154 with P = win_len)
     const double pi = 3.14159265358979323846264338327950288;
@@ -464,7 +514,7 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
     for (int i = 0; i < win_len; ++i) w64[i] = std::sin((i + 0.5) * (pi / win_len));
     const size_t rsz = real_size(dtype);
     void* wdev = nullptr;
-    if (cudaMalloc(&wdev, P * rsz) != cudaSuccess) { delete t; return fail(RPSF_E_CUDA, "out of device memory for the window table"); }
+    if (cudaMalloc(&wdev, P * rsz) != cudaSuccess) { rpsf_transform_destroy(t); return fail(RPSF_E_CUDA, "out of device memory for the window table"); }
     cudaError_t ce;
     if (dtype == RPSF_F32) {
       std::vector<float> w32(w64.begin(), w64.end());
@@ -472,7 +522,7 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
     } else {
       ce = cudaMemcpy(wdev, w64.data(), P * rsz, cudaMemcpyHostToDevice);
     }
-    if (ce != cudaSuccess) { cudaFree(wdev); delete t; return fail(RPSF_E_CUDA, "window upload failed: %s", cudaGetErrorString(ce)); }
+    if (ce != cudaSuccess) { cudaFree(wdev); rpsf_transform_destroy(t); return fail(RPSF_E_CUDA, "window upload failed: %s", cudaGetErrorString(ce)); }
     t->win = wdev; t->own_win = true;
   }
   const size_t cs = 2 * real_size(dtype);
@@ -500,18 +550,18 @@ int rpsf_transform_destroy(rpsf_transform* t) {
   cudaFree(t->kmain); cudaFree(t->knyq);
   cudaFree(t->kconj_main); cudaFree(t->kconj_nyq);
   if (t->own_win) cudaFree(t->win);
+  if (t->order_ev) cudaEventDestroy(t->order_ev);
   delete t;
   return RPSF_OK;
 }
 
 int rpsf_transform_num_colours(const rpsf_transform* t) { return t ? t->n_colours : 0; }
 
-int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int kernel_dtype, void* stream) {
-  if (!t || (!kernel_full && t->n_kept > 0)) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (kernel_dtype != RPSF_F32 && kernel_dtype != RPSF_F64)
-    return fail(RPSF_E_UNSUPPORTED, "kernel dtype must be complex64 (RPSF_F32) or complex128 (RPSF_F64)");
-  DeviceGuard guard(t->device);
-  cudaStream_t s = (cudaStream_t)stream;
+}  // extern "C"
+
+namespace {
+// the layout of rpsf_transform_set_kernel, stream-ordered on `s`
+int set_kernel_on(rpsf_transform* t, const void* kernel_full, int kernel_dtype, cudaStream_t s) {
   if (t->n_kept > 0 && t->win_len != t->P) {
     // embedded patch size: K (n, P, P) -> K' (n, M, M) = A K A^T in double (rpsf_kernels.cuh), then the usual layout
     const int P = t->win_len, M = t->P;
@@ -558,6 +608,17 @@ int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int ke
   if (t->n_kept > 0) LAUNCH(t->ops->prep(t->dtype, kernel_dtype, kernel_full, t->kmain, t->knyq, t->n_kept, s));
   t->has_kernel = true;
   return refresh_conj_kernel(t, s);
+}
+}  // namespace
+
+extern "C" {
+
+int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int kernel_dtype, void* stream) {
+  if (!t || (!kernel_full && t->n_kept > 0)) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (kernel_dtype != RPSF_F32 && kernel_dtype != RPSF_F64)
+    return fail(RPSF_E_UNSUPPORTED, "kernel dtype must be complex64 (RPSF_F32) or complex128 (RPSF_F64)");
+  cudaStream_t s = (cudaStream_t)stream;
+  return ordered(t, s, [&]() -> int { return set_kernel_on(t, kernel_full, kernel_dtype, s); });
 }
 
 int rpsf_construct_kernel(const void* S, const void* Tg, void* K, int64_t count, int dtype, double alpha,
@@ -1604,8 +1665,10 @@ int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
                       int batch, int stages, void* stream) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (p->adjoint) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan runs whole (rpsf_apply)");
-  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
-                      out_row0, batch, stages, stream);
+  return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
+    return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
+                        out_row0, batch, stages, stream);
+  });
 }
 
 int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch, int64_t img_frame_stride,
@@ -1636,48 +1699,49 @@ int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_
   // both plans take the patches that touch the frame, sorted by corner: kgrad pairs their workspaces slot by slot
   if (fp->active_host != ap->active_host)
     return fail(RPSF_E_INVALID_ARGUMENT, "the forward and adjoint plans list different active patches");
-  DeviceGuard guard(t->device);
   cudaStream_t s = (cudaStream_t)stream;
-  const int P = t->P;
-  // per-stage events of the forward plan (bench only): K1(x) | copy + K1(g) | zeroing + kgrad
-  cudaEvent_t* ev = nullptr;
-  if (fp->timing && fp->n_active > 0) {
-    if (fp->events_used + 4 > fp->events.size()) {
-      for (int i = 0; i < 4; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); fp->events.push_back(e); }
+  return ordered(t, s, [&]() -> int {
+    const int P = t->P;
+    // per-stage events of the forward plan (bench only): K1(x) | copy + K1(g) | zeroing + kgrad
+    cudaEvent_t* ev = nullptr;
+    if (fp->timing && fp->n_active > 0) {
+      if (fp->events_used + 4 > fp->events.size()) {
+        for (int i = 0; i < 4; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); fp->events.push_back(e); }
+      }
+      ev = &fp->events[fp->events_used];
+      fp->events_used += 4;
+      CU(cudaEventRecord(ev[0], s));
     }
-    ev = &fp->events[fp->events_used];
-    fp->events_used += 4;
-    CU(cudaEventRecord(ev[0], s));
-  }
-  // 1. X: K1 of the forward plan (stages = 1 writes nothing to `out`)
-  if (int rc = apply_stages(fp, image, img_pitch, img_frame_stride, 0, fp->H, kernel_grad, fp->W, 0, 0, batch, 1, s))
-    return rc;
-  if (ev) CU(cudaEventRecord(ev[1], s));
-  // 2-3. G: the gradient into the adjoint plan's zero-bordered box, K1 there
-  const long long box_stride = (long long)ap->H * ap->box_pitch;
-  if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy<float> : adjoint_copy<double>)(ap, grad, grad_pitch, grad_frame_stride,
-                                                                                     batch, s))
-    return rc;
-  if (int rc = apply_stages(ap, ap->box_in, ap->box_pitch, box_stride, 0, ap->H, ap->box_out, ap->box_pitch, box_stride, 0,
-                            batch, 1, s))
-    return rc;
-  if (ev) CU(cudaEventRecord(ev[2], s));
-  // 4. patches that do not touch the frame: an exact zero (neither map reads them)
-  const size_t slot_bytes = (size_t)P * P * 2 * real_size(t->dtype);
-  std::vector<char> touched(t->n, 0);           // the active list is in corner order: zero runs of untouched indices
-  for (int i : fp->active_host) touched[i] = 1;
-  for (int i = 0; i < t->n;) {
-    if (touched[i]) { ++i; continue; }
-    int j = i;
-    while (j < t->n && !touched[j]) ++j;
-    CU(cudaMemsetAsync((char*)kernel_grad + (size_t)i * slot_bytes, 0, (size_t)(j - i) * slot_bytes, s));
-    i = j;
-  }
-  // 5. conj(X) G / P^2, summed over the batch
-  if (fp->n_active > 0)
-    LAUNCH(t->ops->kgrad(t->dtype, fp->workspace, ap->workspace, kernel_grad, fp->active_dev, t->tw, fp->n_active, batch, s));
-  if (ev) CU(cudaEventRecord(ev[3], s));
-  return RPSF_OK;
+    // 1. X: K1 of the forward plan (stages = 1 writes nothing to `out`)
+    if (int rc = apply_stages(fp, image, img_pitch, img_frame_stride, 0, fp->H, kernel_grad, fp->W, 0, 0, batch, 1, s))
+      return rc;
+    if (ev) CU(cudaEventRecord(ev[1], s));
+    // 2-3. G: the gradient into the adjoint plan's zero-bordered box, K1 there
+    const long long box_stride = (long long)ap->H * ap->box_pitch;
+    if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy<float> : adjoint_copy<double>)(ap, grad, grad_pitch, grad_frame_stride,
+                                                                                       batch, s))
+      return rc;
+    if (int rc = apply_stages(ap, ap->box_in, ap->box_pitch, box_stride, 0, ap->H, ap->box_out, ap->box_pitch, box_stride, 0,
+                              batch, 1, s))
+      return rc;
+    if (ev) CU(cudaEventRecord(ev[2], s));
+    // 4. patches that do not touch the frame: an exact zero (neither map reads them)
+    const size_t slot_bytes = (size_t)P * P * 2 * real_size(t->dtype);
+    std::vector<char> touched(t->n, 0);           // the active list is in corner order: zero runs of untouched indices
+    for (int i : fp->active_host) touched[i] = 1;
+    for (int i = 0; i < t->n;) {
+      if (touched[i]) { ++i; continue; }
+      int j = i;
+      while (j < t->n && !touched[j]) ++j;
+      CU(cudaMemsetAsync((char*)kernel_grad + (size_t)i * slot_bytes, 0, (size_t)(j - i) * slot_bytes, s));
+      i = j;
+    }
+    // 5. conj(X) G / P^2, summed over the batch
+    if (fp->n_active > 0)
+      LAUNCH(t->ops->kgrad(t->dtype, fp->workspace, ap->workspace, kernel_grad, fp->active_dev, t->tw, fp->n_active, batch, s));
+    if (ev) CU(cudaEventRecord(ev[3], s));
+    return RPSF_OK;
+  });
 }
 
 int rpsf_plan_enable_timing(rpsf_plan* p, int enabled) {
@@ -1708,12 +1772,14 @@ int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_f
                int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
                void* stream) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  if (p->adjoint)
-    return (p->tr->dtype == RPSF_F32 ? apply_adjoint<float> : apply_adjoint<double>)(
-        p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride, out_row0, batch,
-        (cudaStream_t)stream);
-  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch,
-                           out_frame_stride, out_row0, batch, 3, stream);
+  return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
+    if (p->adjoint)
+      return (p->tr->dtype == RPSF_F32 ? apply_adjoint<float> : apply_adjoint<double>)(
+          p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride, out_row0, batch,
+          (cudaStream_t)stream);
+    return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch,
+                             out_frame_stride, out_row0, batch, 3, stream);
+  });
 }
 
 int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
@@ -1725,8 +1791,10 @@ int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
   if (!elem_size(src_dtype)) return fail(RPSF_E_UNSUPPORTED, "unsupported source dtype code %d", src_dtype);
   if (src_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "source row pitch smaller than frame width");
   const SatSource source{src, src_dtype, src_pitch, src_frame_stride};
-  return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
-                      out_row0, batch, 3, stream, &source);
+  return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
+    return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
+                        out_row0, batch, 3, stream, &source);
+  });
 }
 
 
@@ -1876,7 +1944,10 @@ int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out,
   }
   for (int i = 0; i < slots && stage; ++i)
     if (!p->h_stage[i]) CU(cudaHostAlloc(&p->h_stage[i], p->h_stage_bytes, cudaHostAllocDefault));
-  int rc = RPSF_OK;
+  // the kernels run on s_comp, ordered with the transform's calls on other streams (a kernel layout on the caller's
+  // stream, device calls sharing this plan's workspace)
+  OrderedCall order{t, p->s_comp};
+  int rc = order.begin();
   for (int ci = 0; ci < n_chunks && rc == RPSF_OK; ++ci) {
     const int b0 = ci * mb, nb = std::min(mb, batch - b0), k = ci % R;
     const char* src = (const char*)image + (size_t)b0 * frame_px * isz;
@@ -1928,6 +1999,7 @@ int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out,
                        p->s_out));
     CU(cudaEventRecord(p->ev_out[k], p->s_out));
   }
+  rc = order.end(rc);
   // drain all three streams even on error so no copy is in flight when the caller's buffers go away
   cudaError_t e1 = cudaStreamSynchronize(p->s_in), e2 = cudaStreamSynchronize(p->s_comp),
               e3 = cudaStreamSynchronize(p->s_out);

@@ -378,9 +378,17 @@ class ArrayPSFTransform:
         like the reference) or a CUDA ``torch.Tensor`` (stays on the device; returns a tensor in
         the compute dtype).  A leading batch axis ``(B, H, W)`` is accepted.  ``workers`` is
         accepted for signature parity and ignored.  ``dtype`` picks the arithmetic precision:
-        "float32" (default) or "float64" (validation mode).  ``out_dtype`` (numpy input only) is the
+        "float32" or "float64" (validation mode); ``None`` means ``set_default_dtype``'s choice
+        ("float32" unless changed), for every kind of input.  ``out_dtype`` (numpy input only) is the
         dtype of the returned array: float64 like the reference by default; ``np.float32`` halves the
         device-to-host copy, which is what bounds a host-to-host call (DESIGN.md section 5).
+
+        Streams (INTEGRATION.md): a tensor is read and the result written in order on the current
+        stream, and backward runs on the forward's stream.  The call sees the transfer kernel as it
+        is when the call is issued (after ``reconstruct`` or an in-place update of the kernel tensor
+        too), whatever streams earlier calls used: the library orders its own device state — the
+        laid-out kernel, the plans' workspaces and scratch — across streams, the private streams of a
+        numpy call included.
         """
         del workers
         kt = self._kernel_tensor
@@ -391,7 +399,7 @@ class ArrayPSFTransform:
                 and _is_torch_tensor(image)):
             # the common device-resident call: nothing to normalise (the host side of such a call costs as much as
             # the kernels of a 512^2 frame, scripts/host_cost.py)
-            return self._apply_device(image, "float32", 0)
+            return self._apply_device(image, _default_dtype, 0)
         dtype_name = _normalize_dtype(dtype)
         # (threshold, dilation, neighbourhood width) of the saturation branch, transform.py:125-138;
         # +inf switches it off.  The mask, its dilation, the raster-ordered fill and the final
