@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define RPSF_ABI_VERSION 2
+#define RPSF_ABI_VERSION 3
 
 /* status codes */
 #define RPSF_OK 0
@@ -205,8 +205,9 @@ int rpsf_plan_destroy(rpsf_plan* p);
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,
  * [6]=overlap-add kernel: 2 = streaming chains (registers only), 1 = single-launch row-pair gather
  *      through a shared-memory plane, 0 = one launch per colour class,
- * [7]=teams per CTA of the row-pair gather */
-int rpsf_plan_info(const rpsf_plan* p, int64_t info[8]);
+ * [7]=teams per CTA of the row-pair gather,
+ * [8]=chunks per chain of the streaming chains (from a cost model of max_batch and the SM count), 0 when [6] != 2 */
+int rpsf_plan_info(const rpsf_plan* p, int64_t info[9]);
 /* overlap-add kernel choice: 0 = automatic (streaming chains when every owned row pair is a chain of
  * half-overlapping patch columns — any calculate_covering grid —, else the row-pair gather when patch
  * corner rows share one parity, else colour phases); 1 = force the colour-phase kernel, 2 = force the

@@ -15,8 +15,7 @@ import numpy as np
 from regularizepsf_b200 import exceptions
 from regularizepsf_b200.exceptions import NativeLibraryError
 
-# RPSF_LIB selects a tuning variant built by `python -m regularizepsf_b200.csrc.build --variant ...`
-LIB_PATH = os.environ.get("RPSF_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "librpsf_b200.so")
+LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "librpsf_b200.so")
 
 # element type codes (include/rpsf_b200.h)
 F32, F64, U8, I16, U16, I32, I64, U32 = range(8)

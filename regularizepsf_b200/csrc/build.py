@@ -44,11 +44,8 @@ def _run(cmd: list[str]) -> None:
         raise RuntimeError("command failed: " + " ".join(cmd) + "\n" + proc.stdout + proc.stderr)
 
 
-def build(force: bool = False, verbose: bool = False, extra_defs: tuple[str, ...] = (), suffix: str = "") -> str:
-    """Build the library.  ``extra_defs``/``suffix`` build a tuning variant (e.g. ("-DRPSF_K2_MINB=2",), "_v2")
-    next to the default one; ``RPSF_LIB=<path>`` makes ``_native.load()`` pick it up."""
-    if extra_defs or suffix:
-        return _build_variant(extra_defs, suffix, verbose)
+def build(force: bool = False, verbose: bool = False) -> str:
+    """Build the library."""
     os.makedirs(OBJ, exist_ok=True)
     nvcc = _nvcc()
     deps = [os.path.join(HERE, h) for h in HEADERS] + [os.path.abspath(__file__)]
@@ -73,28 +70,5 @@ def build(force: bool = False, verbose: bool = False, extra_defs: tuple[str, ...
     return LIB
 
 
-def _build_variant(extra_defs, suffix, verbose) -> str:
-    obj_dir = OBJ + suffix
-    os.makedirs(obj_dir, exist_ok=True)
-    nvcc = _nvcc()
-    lib = os.path.join(PKG, f"librpsf_b200{suffix}.so")
-    jobs, objs = [], []
-    for p in SIZES:
-        obj = os.path.join(obj_dir, f"inst_p{p}.o")
-        objs.append(obj)
-        jobs.append([nvcc, *COMMON, *extra_defs, f"-DRPSF_P={p}", "-c", "rpsf_inst.cu", "-o", obj])
-    api = os.path.join(obj_dir, "api.o")
-    objs.append(api)
-    jobs.append([nvcc, *COMMON, *extra_defs, "-c", "rpsf_api.cu", "-o", api])
-    with ThreadPoolExecutor(max_workers=min(len(jobs), os.cpu_count() or 4)) as pool:
-        list(pool.map(_run, jobs))
-    _run([nvcc, "-shared", *ARCH, "-cudart", "static", "-o", lib, *objs])
-    return lib
-
-
 if __name__ == "__main__":
-    if "--variant" in sys.argv:                      # python -m ...build --variant _v2 -DRPSF_K2_MINB=2 ...
-        i = sys.argv.index("--variant")
-        print(build(extra_defs=tuple(sys.argv[i + 2:]), suffix=sys.argv[i + 1], verbose=True))
-        sys.exit(0)
     print(build(force="--force" in sys.argv, verbose=True))

@@ -8,7 +8,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
-#include <chrono>
 #if defined(__SSE2__)
 #include <emmintrin.h>
 #endif
@@ -200,6 +199,7 @@ struct StreamTables {
   std::vector<StreamTask> tasks;
   std::vector<unsigned> codes;
   int n_warp_items = 0;
+  int chunks = 0;              // chunks per chain
   bool ok = false;
 };
 
@@ -248,9 +248,7 @@ StreamTables build_stream_tables(const std::vector<int2>& corners, const std::ve
   // that minimises the product (small launches want many short tasks, large ones whole chains).
   long long chunks = 1;
   const long long whole = (long long)n_rp * std::max(max_batch, 1);
-  if (const char* v = getenv("RPSF_K3_CHUNKS")) {
-    chunks = std::max(1, std::min(atoi(v), (int)min_groups));
-  } else if (team_slots > 0) {
+  if (team_slots > 0) {
     long long best = LLONG_MAX;
     for (long long c = 1; c <= (long long)min_groups; ++c) {
       const long long per_task = ((long long)min_groups + c - 1) / c + (c > 1 ? 1 : 0);
@@ -288,6 +286,7 @@ StreamTables build_stream_tables(const std::vector<int2>& corners, const std::ve
   }
   while (st.tasks.size() % tpw) st.tasks.push_back(StreamTask{});
   st.n_warp_items = (int)(st.tasks.size() / tpw);
+  st.chunks = (int)chunks;
   st.ok = st.n_warp_items > 0;
   return st;
 }
@@ -381,6 +380,10 @@ int refresh_conj_kernel(rpsf_transform* t, cudaStream_t s) {
 }
 }  // namespace
 
+// The row pass (K1) and overlap-add (K3) kernels of a plan.  The overlap-add values are what rpsf_plan_info reports.
+enum class K1Kernel { plain, bulk };
+enum class Overlap { phases = 0, gather = 1, stream = 2 };
+
 struct rpsf_plan {
   rpsf_transform* tr = nullptr;
   int H = 0, W = 0, pad_mode = 0, row_begin = 0, row_end = 0, max_batch = 1;
@@ -398,15 +401,15 @@ struct rpsf_plan {
   RowGroup* groups_dev = nullptr;
   int* gitems_dev = nullptr;
   int n_tiles = 0, teams = 0, seg_w = 0;
-  bool force_phases = false;   // test hook: run the colour-phase kernel even when gather is possible
-  // kernel variants (test / A-B hooks; default = the persistent bulk-async kernels of rpsf_stream.cuh)
-  bool k1_stream = true;
-  bool k3_stream = true;       // allowed (RPSF_K3=old disables); used when stream_ok
-  bool force_gather = false;   // test hook: the shared-memory row-pair gather even when chains exist
   bool stream_ok = false;      // every owned row pair is a chain of half-overlapping groups covering [0, W)
   StreamTask* stasks_dev = nullptr;
   unsigned* scodes_dev = nullptr;
   int n_warp_items = 0;
+  int stream_chunks = 0;       // chunks per chain of the streaming tables
+  // the kernels apply runs: chosen by plan_build from the geometry (rpsf_plan_set_overlap_mode and
+  // rpsf_plan_set_gather_mode let tests pick the others)
+  K1Kernel k1 = K1Kernel::bulk;
+  Overlap overlap = Overlap::phases;
   void* workspace = nullptr;       // allocated at the first apply
   size_t workspace_bytes = 0;
   int img_lo = 0, img_hi = 0;      // resident frame rows needed: [img_lo, img_hi)
@@ -981,6 +984,14 @@ int check_corners(const rpsf_transform* t, int H, int W) {
   return RPSF_OK;
 }
 
+// The overlap-add kernel of a plan: streaming chains where every owned row pair forms one, else the row-pair gather
+// where its tables exist, else colour phases.  Embedded patch sizes only have colour phases, the one overlap-add kernel
+// that honours ApplyGeom::win_len.
+Overlap default_overlap(const rpsf_plan* p) {
+  if (p->tr->win_len != p->tr->P) return Overlap::phases;
+  return p->stream_ok ? Overlap::stream : p->gather ? Overlap::gather : Overlap::phases;
+}
+
 // Where the plan of a transpose sits: the frame coordinates of box pixel (0, 0) and the frame shape.
 struct AdjointBox { int y0, x0, frame_H, frame_W; };
 
@@ -989,15 +1000,6 @@ struct AdjointBox { int y0, x0, frame_H, frame_W; };
 // only the default three-kernel path is prepared — the opt-in paths do not read the conjugated kernel.
 int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int row_begin, int row_end,
                int max_batch, const AdjointBox* box) {
-  // RPSF_PLAN_TIMING=1 prints where the planning time goes (host-side work lists and their uploads)
-  const bool plan_timing = getenv("RPSF_PLAN_TIMING") != nullptr;
-  auto plan_t0 = std::chrono::steady_clock::now();
-  auto tick = [&](const char* what) {
-    if (!plan_timing) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[rpsf plan] %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - plan_t0).count());
-    plan_t0 = now;
-  };
   if (!out || !t) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (H <= 0 || W <= 0) return fail(RPSF_E_INCORRECT_SHAPE, "frame shape must be positive, got (%d, %d)", H, W);
   if (pad_mode < 0 || pad_mode > RPSF_PAD_MATERIALIZED) return fail(RPSF_E_UNSUPPORTED, "unknown pad mode %d", pad_mode);
@@ -1019,10 +1021,7 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
   auto* p = new rpsf_plan;
   p->tr = t; p->H = H; p->W = W; p->pad_mode = pad_mode; p->row_begin = row_begin; p->row_end = row_end;
   p->max_batch = max_batch;
-  if (const char* v = getenv("RPSF_K1")) p->k1_stream = strcmp(v, "old") != 0;
-  if (const char* v = getenv("RPSF_K3")) p->k3_stream = strcmp(v, "old") != 0;
   const bool embedded = t->win_len != t->P;
-  if (embedded) { p->k1_stream = false; p->force_phases = true; }      // the two kernels that honour ApplyGeom::win_len
   std::vector<int> active;
   std::vector<int2> corners;
   std::vector<std::vector<int>> items(std::max(t->n_colours, 1));
@@ -1094,7 +1093,6 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
     if (cudaMalloc(&p->items_dev[c], sizeof(int) * items[c].size()) != cudaSuccess) return destroy_fail("work list");
     if (cudaMemcpy(p->items_dev[c], items[c].data(), sizeof(int) * items[c].size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
   }
-  tick("active list and colour items");
   // ---- row-pair gather tables: tiles -> groups (same corner column, summed in registers in colour
   // order) -> at most two layers of disjoint groups (one shared-memory plane each)
   {
@@ -1180,7 +1178,6 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
       }
     }
   }
-  tick("row-pair gather tables");
   // ---- streaming overlap-add tables
   if (p->n_active > 0 && (long long)p->n_active * (P / 2) < (1LL << 30)) {
     std::vector<int> colours(active.size());
@@ -1194,10 +1191,12 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
       if (cudaMalloc(&p->scodes_dev, sizeof(unsigned) * stt.codes.size()) != cudaSuccess) return destroy_fail("stream item codes");
       if (cudaMemcpy(p->scodes_dev, stt.codes.data(), sizeof(unsigned) * stt.codes.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
       p->n_warp_items = stt.n_warp_items;
+      p->stream_chunks = stt.chunks;
       p->stream_ok = true;
     }
   }
-  tick("streaming overlap-add tables");
+  p->k1 = embedded ? K1Kernel::plain : K1Kernel::bulk;       // the plain K1 honours ApplyGeom::win_len
+  p->overlap = default_overlap(p);
   p->workspace_bytes = (size_t)max_batch * p->n_active * P * (P / 2) * 2 * real_size(t->dtype);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { rpsf_plan_destroy(p); return fail(RPSF_E_CUDA, "plan upload failed: %s", cudaGetErrorString(e)); }
@@ -1314,24 +1313,25 @@ int rpsf_plan_destroy(rpsf_plan* p) {
 int rpsf_plan_set_overlap_mode(rpsf_plan* p, int mode) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (p->tr->win_len != p->tr->P) return RPSF_OK;             // embedded patch sizes only have the colour-phase kernel
-  p->force_phases = mode == 1;
-  p->force_gather = mode == 2;
+  if (mode == 1) p->overlap = Overlap::phases;
+  else if (mode == 2) p->overlap = p->gather ? Overlap::gather : Overlap::phases;
+  else p->overlap = default_overlap(p);
   return RPSF_OK;
 }
 
 int rpsf_plan_set_gather_mode(rpsf_plan* p, int mode) {
   if (!p) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (p->tr->win_len != p->tr->P) return RPSF_OK;             // embedded patch sizes only have the plain gather kernel
-  p->k1_stream = mode != 1;
+  p->k1 = mode == 1 ? K1Kernel::plain : K1Kernel::bulk;
   return RPSF_OK;
 }
 
-int rpsf_plan_info(const rpsf_plan* p, int64_t info[8]) {
+int rpsf_plan_info(const rpsf_plan* p, int64_t info[9]) {
   if (!p || !info) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
-  const bool stream = p->stream_ok && p->k3_stream && !p->force_phases && !p->force_gather;
-  info[6] = stream ? 2 : (p->gather && !p->force_phases) ? 1 : 0; info[7] = p->teams;
   info[0] = p->n_active; info[1] = p->tr->n_colours; info[2] = (int64_t)p->workspace_bytes;
   info[3] = p->img_lo; info[4] = p->img_hi; info[5] = p->colour0_covers ? 1 : 0;
+  info[6] = (int64_t)p->overlap; info[7] = p->teams;
+  info[8] = p->overlap == Overlap::stream ? p->stream_chunks : 0;
   return RPSF_OK;
 }
 
@@ -1523,8 +1523,8 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   g.win_len = t->win_len;
   const size_t rs = real_size(t->dtype);
   const int band = p->row_end - p->row_begin;
-  const bool use_stream = p->stream_ok && p->k3_stream && !p->force_phases && !p->force_gather;
-  const bool use_gather = p->gather && !p->force_phases && !use_stream;
+  const bool use_stream = p->overlap == Overlap::stream;
+  const bool use_gather = p->overlap == Overlap::gather;
   const bool need_zero = !((p->colour0_covers || use_gather || use_stream) && stages >= 3);
   cudaEvent_t* ev = nullptr;
   if (p->timing && stages >= 3 && p->n_active > 0) {
@@ -1563,7 +1563,7 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   };
   if (p->n_active == 0) return restore();
   if (int rc = ensure_workspace(p)) return rc;
-  if (p->k1_stream && (long long)batch * p->n_active * (t->P / 2) < (1LL << 30)) {
+  if (p->k1 == K1Kernel::bulk && (long long)batch * p->n_active * (t->P / 2) < (1LL << 30)) {
     // bulk (1-D TMA) row copies need 16-byte aligned rows; the kernel still checks each patch's column offset
     const size_t rsz = real_size(t->dtype);
     const int bulk_ok = ((reinterpret_cast<uintptr_t>(k1_image) & 15) == 0 && ((size_t)g1.img_pitch * rsz) % 16 == 0 &&
@@ -1824,8 +1824,7 @@ bool is_pageable_host(const void* ptr) {
   return attr.type == cudaMemoryTypeUnregistered;
 }
 int host_copy_threads() {
-  if (const char* v = getenv("RPSF_HOST_COPY_THREADS")) { const int n = atoi(v); if (n >= 1) return std::min(n, 64); }
-  // measured on a 16-core host (scripts/pageable_probe.py): 4 threads 8.5 ms per 8 frames, 8 threads 9.2, 16 threads 10.1 —
+  // measured on a 16-core host: 4 threads 8.5 ms per 8 frames, 8 threads 9.2, 16 threads 10.1 —
   // the copy competes with the DMA for the host memory system, more threads only add contention
   const unsigned hw = std::thread::hardware_concurrency();
   return (int)std::max(1u, std::min(4u, hw / 2));
@@ -1858,19 +1857,11 @@ void stream_copy(char* dst, const char* src, size_t bytes) {
 #endif
 }
 // A call that fits one chunk has no earlier chunk to hide its staging behind: it is staged in pieces, the DMA of a
-// piece under the staging of the next.  Measured (scripts/pageable_probe.py, one 2048^2 frame): float32 1.58 ms through
-// the driver's own pageable path, 1.37 staged whole, 1.26 in 4 MB pieces (2 MB: slower); uint16 1.20 / 1.11 / 1.05.
-// Several chunks are staged whole (6.7 ms per 8 frames; in 4 MB pieces 7.3).  RPSF_STAGE_SINGLE=0 keeps the
-// driver's path for single chunks, RPSF_STAGE_PIECE_MB overrides the piece size.
-size_t stage_piece_bytes(bool single_chunk) {
-  static const size_t env = [] { const char* e = getenv("RPSF_STAGE_PIECE_MB"); const int mb = e ? atoi(e) : 0; return (size_t)(mb > 0 ? mb : 0) << 20; }();
-  if (env) return env;
-  return single_chunk ? (size_t)4 << 20 : ~(size_t)0;
-}
-bool stage_single_chunk(size_t chunk_bytes) {
-  static const bool off = [] { const char* e = getenv("RPSF_STAGE_SINGLE"); return e && e[0] == '0'; }();
-  return !off && chunk_bytes >= ((size_t)4 << 20);
-}
+// piece under the staging of the next.  Measured (one 2048^2 frame): float32 1.58 ms through the driver's own pageable
+// path, 1.37 staged whole, 1.26 in 4 MB pieces (2 MB: slower); uint16 1.20 / 1.11 / 1.05.  Several chunks are staged
+// whole (6.7 ms per 8 frames; in 4 MB pieces 7.3).  A single chunk below 4 MB keeps the driver's path.
+size_t stage_piece_bytes(bool single_chunk) { return single_chunk ? (size_t)4 << 20 : ~(size_t)0; }
+bool stage_single_chunk(size_t chunk_bytes) { return chunk_bytes >= ((size_t)4 << 20); }
 void parallel_copy(void* dst, const void* src, size_t bytes, int threads) {
   const size_t grain = (size_t)1 << 20;
   const int n = (int)std::min<size_t>((size_t)threads, std::max<size_t>(bytes / grain, 1));

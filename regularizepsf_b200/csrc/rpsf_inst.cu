@@ -1,5 +1,4 @@
 // rpsf_inst.cu — instantiates every kernel for one patch size (compile with -DRPSF_P=<P>).
-#include <cstdlib>
 #include "rpsf_ops.h"
 #include "rpsf_kgrad.cuh"
 #include "rpsf_construct_grad.cuh"
@@ -21,9 +20,9 @@ template <typename T> constexpr size_t col_smem() {
   return sizeof(cplx<T>) * P + sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
 }
 template <typename T> constexpr size_t col_pipe_smem() {
-  return sizeof(cplx<T>) * P + RPSF_K2_STAGES * sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
+  return sizeof(cplx<T>) * P + K2_STAGES * sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
 }
-// the pipelined column kernel needs RPSF_K2_STAGES tile stages per CTA; use it while a stage is at most
+// the pipelined column kernel needs K2_STAGES tile stages per CTA; use it while a stage is at most
 // 32 KB (two or three CTAs then fit an SM)
 template <typename T> constexpr bool use_col_pipe() {
   return sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C <= 32 * 1024 + 4096;
@@ -34,15 +33,12 @@ template <typename T> constexpr size_t fft2_row_smem() {
 
 // Launch one of the chained kernels (k1_stream -> k2_pipelined -> k3_stream -> the next call's k1_stream) so that its
 // CTAs may start while the kernel before it in the stream drains (programmatic dependent launch; the kernels wait in
-// grid_dependency_wait() before they touch anything a predecessor wrote).  RPSF_PDL=0 launches them the plain way.
-// RPSF_PDL is a mask: 1 = k1_stream, 2 = k2_pipelined, 4 = k3_stream may start early.  Measured (scripts/chain_ab.py):
-// all three at P <= 128 (one 1024^2 frame: 41.1 -> 34.1 us at 128 px, 39.4 -> 31.8 at 64 px); at P >= 256 an early
-// column pass costs 1 % (its first wave of CTAs is placed on the SMs the row pass leaves first), so only the row
-// kernels start early there (2048^2 / 256 px: 97.0 -> 95.2 us for one frame, 64.4 -> 63.5 per frame at 8).
-inline int pdl_mask() {
-  static const int mask = [] { const char* v = getenv("RPSF_PDL"); return v ? atoi(v) : (P <= 128 ? 7 : 5); }();
-  return mask;
-}
+// grid_dependency_wait() before they touch anything a predecessor wrote).  `which`: 1 = k1_stream, 2 = k2_pipelined,
+// 4 = k3_stream.  Measured: all three start early at P <= 128 (one 1024^2 frame: 41.1 -> 34.1 us at 128 px,
+// 39.4 -> 31.8 at 64 px); at P >= 256 an early column pass costs 1 % (its first wave of CTAs is placed on the SMs the
+// row pass leaves first), so only the row kernels start early there (2048^2 / 256 px: 97.0 -> 95.2 us for one frame,
+// 64.4 -> 63.5 per frame at 8).
+constexpr int PDL_MASK = P <= 128 ? 7 : 5;
 template <typename... KArgs, typename... Args>
 int launch_chain(int which, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg{};
@@ -54,7 +50,7 @@ int launch_chain(int which, void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl_mask() & which) ? 1 : 0;
+  cfg.numAttrs = (PDL_MASK & which) ? 1 : 0;
   return (int)cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
@@ -88,10 +84,6 @@ int init() {
     if ((e = set_smem(k2_pipelined<P, float, 2>, col_pipe_smem<float>()))) return e;
   if constexpr (use_col_pipe<double>() && TL::SLOTS == 1 && TL::NTILE % 2 == 0)
     if ((e = set_smem(k2_pipelined<P, double, 2>, col_pipe_smem<double>()))) return e;
-  if constexpr (use_col_pipe<float>() && TL::SLOTS == 1 && TL::NTILE % 4 == 0)
-    if ((e = set_smem(k2_pipelined<P, float, 4>, col_pipe_smem<float>()))) return e;
-  if constexpr (use_col_pipe<double>() && TL::SLOTS == 1 && TL::NTILE % 4 == 0)
-    if ((e = set_smem(k2_pipelined<P, double, 4>, col_pipe_smem<double>()))) return e;
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, float>, row_smem<float>()))) return e;
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, double>, row_smem<double>()))) return e;
   if ((e = set_smem(k3_rowpair_gather<P, float>, K3G_SMEM_MAX))) return e;
@@ -163,21 +155,13 @@ int k2_t(void* spec, const void* kmain, const void* knyq, const int* active, con
   }
   if constexpr (use_col_pipe<T>() && TL::SLOTS == 1 && TL::NTILE % 2 == 0) {
     // few frames per CTA: walk two adjacent tiles per CTA so that the stage ring and the transfer-kernel loads have
-    // something to overlap with (RPSF_K2_TPC=1 switches it off).  Only for one-slot CTAs (P >= 256): with two slots
-    // per CTA (P = 128) the same change was measured 2 % (1024^2) to 8 % (2048^2) slower, at P = 64 1 % faster.
-    static const int tpc_env = [] { const char* v = getenv("RPSF_K2_TPC"); return v ? atoi(v) : 0; }();
-    const int tpc = tpc_env ? tpc_env : (fpc <= 1 ? 2 : 1);
-    if (tpc == 2) {
+    // something to overlap with.  Only for one-slot CTAs (P >= 256): with two slots per CTA (P = 128) the same change
+    // was measured 2 % (1024^2) to 8 % (2048^2) slower, at P = 64 1 % faster.  Four tiles per CTA (2048^2 / 256 px:
+    // 89.9 vs 87.3 us) and two tiles at 8 frames per call (4 % slower) lost.
+    if (fpc <= 1) {
       grid.x = (unsigned)cdiv(ctas, 2);
       return launch_chain(2, k2_pipelined<P, T, 2>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, (cplx<T>*)spec,
                           (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
-    }
-    if constexpr (TL::NTILE % 4 == 0) {
-      if (tpc == 4) {
-        grid.x = (unsigned)cdiv(ctas, 4);
-        return launch_chain(2, k2_pipelined<P, T, 4>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, (cplx<T>*)spec,
-                            (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
-      }
     }
   }
   if constexpr (use_col_pipe<T>())

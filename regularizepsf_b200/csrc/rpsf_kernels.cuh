@@ -74,20 +74,14 @@ struct ApplyGeom {
   int win_len;
 };
 
-#ifndef RPSF_K2_C            // columns per column-FFT tile (tuning switch; 16 = a full 128-byte line per row)
-#define RPSF_K2_C 16
-#endif
-#ifndef RPSF_K2_CTA          // threads per column-FFT CTA: tiles are packed into slots up to this size
-#define RPSF_K2_CTA 256
-#endif
-
 template <int P> struct Tile {
   static constexpr int N1 = Split<P>::N1, N2 = Split<P>::N2;
   static constexpr int HALF = P / 2;
-  static constexpr int C = HALF < RPSF_K2_C ? HALF : RPSF_K2_C;   // columns per column-FFT tile
+  static constexpr int C = HALF < 16 ? HALF : 16;           // columns per column-FFT tile (16 = a full 128-byte line per row)
   static constexpr int NTILE = HALF / C;
   static constexpr int SLOT_THREADS = C * N1;
-  static constexpr int SLOTS = SLOT_THREADS >= RPSF_K2_CTA ? 1 : RPSF_K2_CTA / SLOT_THREADS;
+  static constexpr int CTA_THREADS = 256;                   // per column-FFT CTA: tiles are packed into slots up to this size
+  static constexpr int SLOTS = SLOT_THREADS >= CTA_THREADS ? 1 : CTA_THREADS / SLOT_THREADS;
   static constexpr int K2_THREADS = SLOTS * SLOT_THREADS;
   // row kernels: teams of N1 threads inside a warp
   static constexpr int TEAMS = 256 / N1;
@@ -322,21 +316,9 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait_pending() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-#ifndef RPSF_K2_MINB
-#define RPSF_K2_MINB 2
-#endif
-#ifndef RPSF_K2_PREFETCH
-#define RPSF_K2_PREFETCH 1
-#endif
-#ifndef RPSF_K2_REVERSE     // 1: a CTA walks its frames from the last to the first (see k2_frames)
-#define RPSF_K2_REVERSE 0
-#endif
-#ifndef RPSF_K2_STAGES      // shared-memory tile stages per CTA: tiles f+1 .. f+STAGES-1 are in flight while tile f is transformed
-#define RPSF_K2_STAGES 2
-#endif
-#ifndef RPSF_K2_FWD_TAIL_SYNC   // 1 = keep the barrier after the forward exchange reads (not needed: see k2_frames)
-#define RPSF_K2_FWD_TAIL_SYNC 0
-#endif
+// shared-memory tile stages per CTA: tiles f+1 .. f+K2_STAGES-1 are in flight while tile f is transformed.  Three
+// stages were measured slower than two (32.4 vs 31.2 us per frame at B=8): the tile always lands in time.
+constexpr int K2_STAGES = 2;
 
 // The frame loop of one CTA.  TILE0: some slot of this CTA holds tile 0, whose column 0 packs the DC
 // and Nyquist columns (z = a + i*b, both real sequences over rows):
@@ -363,7 +345,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
   constexpr int PER_THREAD = (P * ROW_CHUNKS) / TL::SLOT_THREADS;
   constexpr int ROWS_PER_PASS = TL::SLOT_THREADS / ROW_CHUNKS;
   static_assert(C % CH == 0 && (P * ROW_CHUNKS) % TL::SLOT_THREADS == 0, "tile does not split into 16-byte chunks");
-  constexpr bool PREFETCH = RPSF_K2_PREFETCH && sizeof(cplx<T>) * N2 <= 128;
+  constexpr bool PREFETCH = sizeof(cplx<T>) * N2 <= 128;
 
   // the transfer-kernel tile is loaded once and reused for every frame this CTA walks
   cplx<T> kv[PREFETCH ? N2 : 1];
@@ -389,15 +371,12 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
   const int live_rows = (g.win_len + 1) & ~1;               // PRUNED: rows the gather wrote / the overlap-add reads
   const cplx<T>* src0 = tile_base0 + (long long)row0 * HALF + part * CH;
   const int dst0 = slot * (P * C) + row0 * C + part * CH;
-  // K1 writes the batch frame by frame, so the last frame is the one still in L2 (its stores carry an
-  // evict_last hint): walk the frames from the last to the first
-  auto fr = [=](int i) { return RPSF_K2_REVERSE ? f_end - 1 - (i - f_begin) : i; };
   const int nf = f_end - f_begin;
   const int n_it = TPC * nf;                                // iteration it = unit (it / nf), frame f_begin + it % nf
   auto issue = [&](int it, cplx<T>* stage) {
     if (valid) {
       const int u = TPC == 1 ? 0 : it / nf;
-      const int f = fr(f_begin + (TPC == 1 ? it : it - u * nf));
+      const int f = f_begin + (TPC == 1 ? it : it - u * nf);
       const cplx<T>* src = src0 + u * C + f * frame_stride;
 #pragma unroll
       for (int i = 0; i < PER_THREAD; ++i) {
@@ -413,7 +392,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
 
   // One commit group per tile slot, empty past the end, so "at most NS-2 groups pending" always
   // means "tile f has landed".
-  constexpr int NS = RPSF_K2_STAGES;
+  constexpr int NS = K2_STAGES;
   static_assert(NS >= 2 && NS <= 4, "2..4 tile stages");
   int cur = 0;
   grid_dependency_wait();         // the transfer-kernel tile above is already in flight; the spectrum is K1's
@@ -442,20 +421,10 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
       v[j] = xbuf[ex(j, n1)];                               // row n1 + N1*j, column c: the slot pass A writes back to
     });
 
-#ifdef RPSF_K2_COPYONLY   // memory-pattern ceiling probe: same loads and stores, no transform
-    if (valid) {
-      cplx<T>* base = const_cast<cplx<T>*>(tile_base) + fr(f) * frame_stride + c;
-      static_for<0, N2>([&](auto jj) {
-        constexpr int j = decltype(jj)::value;
-        base[(long long)(n1 + N1 * j) * HALF] = cmul(v[j], kval(jj));
-      });
-    }
-    continue;
-#endif
     // The exchange slots a thread reads in the forward pass B are exactly the ones it writes in the
     // inverse pass B, so no barrier is needed between the two unless the buffer is reused in
     // between (the DC/Nyquist column of tile 0 does that).
-    if constexpr (TILE0 || RPSF_K2_FWD_TAIL_SYNC) coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync);
+    if constexpr (TILE0) coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync);
     else coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
 
     if constexpr (TILE0) {
@@ -503,7 +472,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
     // before anything is copied into this stage again
     coop_fft_inverse<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
     if (valid) {
-      cplx<T>* base = const_cast<cplx<T>*>(tile_base) + fr(f) * frame_stride + c;
+      cplx<T>* base = const_cast<cplx<T>*>(tile_base) + f * frame_stride + c;
       static_for<0, N2>([&](auto jj) {
         constexpr int j = decltype(jj)::value;
         if (!PRUNED || n1 + N1 * j < live_rows) base[(long long)(n1 + N1 * j) * HALF] = v[j];
@@ -512,8 +481,10 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
   }
 }
 
+// Two CTAs per SM keep the transfer-kernel tile in registers; three (78 registers, the tile re-read from L2) were
+// measured slower (35.3 vs 32.2 us per frame).
 template <int P, typename T, int TPC = 1, bool PRUNED = false>
-__global__ void __launch_bounds__(Tile<P>::K2_THREADS, RPSF_K2_MINB)
+__global__ void __launch_bounds__(Tile<P>::K2_THREADS, 2)
 k2_pipelined(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kmain, const cplx<T>* __restrict__ knyq,
              const int* __restrict__ active, const cplx<T>* __restrict__ tw_g, int batch, int frames_per_cta,
              ApplyGeom g) {
@@ -644,12 +615,9 @@ k3_rowifft_window_overlap_add(const cplx<T>* __restrict__ spec, T* __restrict__ 
 struct RowTile { int group_begin, group_count, y, x0; };              // output rows y, y+1; columns [x0, x0+seg)
 struct RowGroup { int item_begin, item_count, cx, layer, clipped; };  // items: active*HALF + pair, colour order
 constexpr int K3G_SMEM_MAX = 200 * 1024;                              // dynamic shared memory the kernel may ask for
-#ifndef RPSF_K3_MINB
-#define RPSF_K3_MINB 3
-#endif
 
 template <int P, typename T>
-__global__ void __launch_bounds__(288, RPSF_K3_MINB)
+__global__ void __launch_bounds__(288, 3)
 k3_rowpair_gather(const cplx<T>* __restrict__ spec, T* __restrict__ out, const RowTile* __restrict__ tiles,
                   const RowGroup* __restrict__ groups, const int* __restrict__ items,
                   const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, int seg_w, ApplyGeom g) {

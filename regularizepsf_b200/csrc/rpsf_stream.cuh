@@ -53,18 +53,11 @@ __device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, 
 // orders this thread's earlier generic-proxy shared-memory accesses before later async-proxy ones
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-#ifndef RPSF_STREAM_SMEM_KB
-#define RPSF_STREAM_SMEM_KB 224
-#endif
-constexpr int STREAM_SMEM_BUDGET = RPSF_STREAM_SMEM_KB * 1024;
-#ifndef RPSF_STREAM_MAX_WARPS
-#define RPSF_STREAM_MAX_WARPS 16
-#endif
-#ifndef RPSF_STREAM_STAGES
-#define RPSF_STREAM_STAGES 3
-#endif
+constexpr int STREAM_SMEM_BUDGET = 224 * 1024;
+constexpr int STREAM_MAX_WARPS = 16;
+constexpr int STREAM_STAGES = 3;
 
-template <int P, typename T, int STAGES_REQ = RPSF_STREAM_STAGES> struct Stream {
+template <int P, typename T, int STAGES_REQ = STREAM_STAGES> struct Stream {
   static constexpr int N1 = Split<P>::N1, N2 = Split<P>::N2, HALF = P / 2;
   static constexpr int TPW = 32 / N1;                                      // teams per warp
   static constexpr int ROWS = 2 * TPW;                                     // patch rows per warp item
@@ -85,7 +78,7 @@ template <int P, typename T, int STAGES_REQ = RPSF_STREAM_STAGES> struct Stream 
   static constexpr int WS = AVAIL / (STAGES_REQ * STAGE_BYTES);
   static constexpr int STAGES = WS >= 8 ? STAGES_REQ : 2;
   static constexpr int WFIT = AVAIL / (STAGES * STAGE_BYTES);
-  static constexpr int WARPS = WFIT > RPSF_STREAM_MAX_WARPS ? RPSF_STREAM_MAX_WARPS : WFIT;
+  static constexpr int WARPS = WFIT > STREAM_MAX_WARPS ? STREAM_MAX_WARPS : WFIT;
   static constexpr int THREADS = WARPS * 32;
   static constexpr size_t SMEM = RING_OFFSET + (size_t)WARPS * STAGES * STAGE_BYTES;
   static_assert(WARPS >= 2, "stage ring does not fit shared memory");
@@ -99,22 +92,17 @@ template <int P, typename T, int STAGES_REQ = RPSF_STREAM_STAGES> struct Stream 
 // items are short enough that two stages and 16 warps are faster (single 1024^2 frame: 17.0 -> 15.1 us, 8 frames: 7.0
 // -> 6.8 us per frame), while the overlap-add kernel keeps three (6.2 vs 6.5 us).
 template <int P, typename T>
-using StreamK1 = Stream<P, T, (P == 128 && sizeof(T) == 4) ? 2 : RPSF_STREAM_STAGES>;
+using StreamK1 = Stream<P, T, (P == 128 && sizeof(T) == 4) ? 2 : STREAM_STAGES>;
 
-#ifndef RPSF_K1_EVICT_LAST   // 1: K1's spectrum stores carry an L2 evict_last hint (K2 reads them next)
-#define RPSF_K1_EVICT_LAST 1
-#endif
+// K1's spectrum stores carry an L2 evict_last hint: K2 reads them next, and the tail of K1's output then survives in L2
+// (K2 -0.5 us per frame at B=8, -2.6 us on a single frame)
 __device__ __forceinline__ unsigned long long l2_policy_evict_last() {
   unsigned long long pol;
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
 __device__ __forceinline__ void st_spec(float2* p, float2 v, unsigned long long pol) {
-#if RPSF_K1_EVICT_LAST
   asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1, %2}, %3;" ::"l"(p), "f"(v.x), "f"(v.y), "l"(pol) : "memory");
-#else
-  (void)pol; *p = v;
-#endif
 }
 __device__ __forceinline__ void st_spec(double2* p, double2 v, unsigned long long) { *p = v; }
 
@@ -150,7 +138,7 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
   grid_launch_dependents();
 
   unsigned char* my_ring = ring + (size_t)warp * STAGES * ST::STAGE_BYTES;
-  const unsigned long long l2_keep = RPSF_K1_EVICT_LAST ? l2_policy_evict_last() : 0ull;
+  const unsigned long long l2_keep = l2_policy_evict_last();
   const unsigned n_items = (unsigned)batch * (unsigned)g.n_active * IPP;       // host guarantees < 2^30
   const unsigned stride = n_cta * WARPS;
   const unsigned first = cta * WARPS + warp;

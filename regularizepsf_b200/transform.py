@@ -137,12 +137,12 @@ class _NativeTransform:
             self._saturation[plan] = sat
 
     def plan_info(self, plan: int) -> dict:
-        info = (ctypes.c_int64 * 8)()
+        info = (ctypes.c_int64 * 9)()
         _native.check(self.lib.rpsf_plan_info(plan, info))
         return {"active_patches": info[0], "colours": info[1], "workspace_bytes": info[2],
                 "rows_read": (info[3], info[4]), "colour0_tiles_band": bool(info[5]),
                 "overlap_add": {2: "streaming chains", 1: "row-pair gather", 0: "colour phases"}[int(info[6])],
-                "gather_teams": info[7]}
+                "gather_teams": info[7], "overlap_chunks": info[8]}
 
 
 class ArrayPSFTransform:

@@ -1,4 +1,4 @@
-"""Per-stage device times of apply() on config 2 (device-resident), for quick A/B runs of library variants."""
+"""Per-stage device times of apply() on config 2 (device-resident)."""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -33,6 +33,5 @@ ms = (ctypes.c_double * 3)(); calls = ctypes.c_int()
 lib.rpsf_plan_read_timing(plan, ms, ctypes.byref(calls))
 per = [1e3 * ms[i] / calls.value / B for i in range(3)]
 tot = 1e3 * e0.elapsed_time(e1) / steps / B
-name = os.path.basename(os.environ.get("RPSF_LIB", "default"))
-print(f"{name:>28s} B={B} P={P} HW={HW}: us/frame total {tot:.1f}  k1 {per[0]:.1f}  k2 {per[1]:.1f}  k3 {per[2]:.1f}  "
+print(f"B={B} P={P} HW={HW}: us/frame total {tot:.1f}  k1 {per[0]:.1f}  k2 {per[1]:.1f}  k3 {per[2]:.1f}  "
       f"-> {HW * HW / tot:.0f} Mpix/s")

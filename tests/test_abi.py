@@ -25,9 +25,10 @@ def test_header_and_binding_agree(native_lib):
         assert hasattr(native_lib, name), name
 
 
-def test_abi_version_and_supported_patch_sizes(native_lib):
-    # static CUDA runtime: the only CUDA dependency is the driver, resolved lazily
-    assert native_lib.rpsf_abi_version() == 2
+def test_abi_version_3_and_supported_patch_sizes(native_lib):
+    # static CUDA runtime: the only CUDA dependency is the driver, resolved lazily.  Version 3: rpsf_plan_info fills
+    # nine entries (info[8] = overlap-add chunks per chain), so a caller built for version 2 must not pass its array.
+    assert native_lib.rpsf_abi_version() == 3
     for p in (16, 32, 64, 128, 256, 512):
         assert native_lib.rpsf_patch_size_supported(p) == 1
     for p in (2, 8, 11, 100, 255, 256 - 1):            # embedded in the next power of two >= 2 P - 1
