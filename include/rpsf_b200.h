@@ -60,6 +60,23 @@ extern "C" {
 typedef struct rpsf_transform rpsf_transform;
 typedef struct rpsf_plan rpsf_plan;
 
+/* CUDA graphs.  A stream capture may contain, once their plans exist and each has run once outside the capture:
+ * rpsf_apply (forward and adjoint plans), rpsf_apply_source, rpsf_kernel_gradient, rpsf_transform_set_kernel,
+ * rpsf_construct_kernel(_dev), rpsf_construct_kernel_backward(_dev), rpsf_psf_fft2 and rpsf_psf_fft2_adjoint (native
+ * patch sizes).  These neither cudaMalloc nor synchronise then; their scratch is cudaMallocAsync on the stream, which
+ * the capture turns into allocation nodes.  On a capturing stream a call that touches a transform's device state makes
+ * the transform's order event an external dependency of the graph (cudaEventWaitExternal at its start,
+ * cudaEventRecordExternal at its end), so each replay is ordered after the calls issued before its launch and before
+ * those issued after it; from then on every eager call on that transform waits for the event.  What would allocate
+ * or synchronise (a plan's first call, the first saturation branch, plan creation, the host path, upload / free, IPC,
+ * the builder) returns RPSF_E_UNSUPPORTED while a capture is open, before any CUDA call that would invalidate it.
+ * Entry points without a stream argument see a capture once a call of this library has run on the capturing stream:
+ * the library remembers such streams, on every thread, until it finds their capture ended (at a stream-less call, or
+ * at an eager call on the same stream).  While any of them captures, plan creation, upload / free, IPC and the host
+ * path are refused on every thread, which is stricter than a relaxed capture mode needs.  A stream the library has
+ * seen capturing must not be destroyed before its capture has ended and a later call of the library has run.
+ * The caller keeps the transforms and plans a graph uses alive as long as the graph. */
+
 int rpsf_abi_version(void);
 const char* rpsf_last_error(void);
 /* 1: patch size P runs natively (powers of two 16..512); 2: it runs embedded in the next power of two M >= 2 P - 1
@@ -91,12 +108,21 @@ int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int ke
 /* number of colour classes of the overlap graph (4 for calculate_covering inputs, util.py:10-53) */
 int rpsf_transform_num_colours(const rpsf_transform* t);
 
+/* A fence in the transform's stream order, with no launches: `stream` waits for the transform's previous calls (eager
+ * calls and graph replays) and the calls issued after this one wait for what `stream` has queued up to here.  For a
+ * caller that writes, on `stream`, a buffer that captured calls of the transform read. */
+int rpsf_transform_order(rpsf_transform* t, void* stream);
+
 /* ---- construct: replaces the arithmetic of ArrayPSFTransform.construct (transform.py:78-82) -
  * source_fft / target_fft / kernel_out: `count` complex elements on the device, all complex64
  * (dtype RPSF_F32) or all complex128 (RPSF_F64).  The coordinate check (transform.py:74-76)
  * stays on the host. */
 int rpsf_construct_kernel(const void* source_fft, const void* target_fft, void* kernel_out, int64_t count,
                           int dtype, double alpha, double epsilon, int device, void* stream);
+/* The same with alpha and epsilon read on the device from alpha_epsilon (2 doubles, [alpha, epsilon]), so that a caller
+ * holding them in device memory need not synchronise; bit-identical to rpsf_construct_kernel given the same values. */
+int rpsf_construct_kernel_dev(const void* source_fft, const void* target_fft, void* kernel_out, int64_t count,
+                              int dtype, const double* alpha_epsilon, int device, void* stream);
 
 /* Vector-Jacobian product of rpsf_construct_kernel (transform.py:78-82), for a gradient that reaches the PSFs, alpha and
  * epsilon.  kernel_grad is G, the gradient of the loss with respect to K in PyTorch's convention (dL/dRe + i dL/dIm);
@@ -114,6 +140,11 @@ int rpsf_construct_kernel(const void* source_fft, const void* target_fft, void* 
 int rpsf_construct_kernel_backward(const void* source_fft, const void* target_fft, const void* kernel_grad,
                                    int64_t count, int dtype, double alpha, double epsilon, void* source_grad,
                                    void* target_grad, double* alpha_epsilon_grad, int device, void* stream);
+/* The same with alpha and epsilon read on the device from alpha_epsilon (2 doubles; not the output alpha_epsilon_grad);
+ * bit-identical to rpsf_construct_kernel_backward given the same values. */
+int rpsf_construct_kernel_backward_dev(const void* source_fft, const void* target_fft, const void* kernel_grad,
+                                       int64_t count, int dtype, const double* alpha_epsilon, void* source_grad,
+                                       void* target_grad, double* alpha_epsilon_grad, int device, void* stream);
 
 /* ---- PSF cube FFT: replaces scipy.fft.fft2 in ArrayPSF.__init__ (psf.py:216-219) -----------
  * values: (n, P, P) real on the device; out: (n, P, P) complex, full spectrum, same precision. */

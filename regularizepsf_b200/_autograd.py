@@ -92,45 +92,64 @@ class PsfFFT(torch.autograd.Function):
 
 
 class Construct(torch.autograd.Function):
-    """``forward(source_fft, target_fft, alpha, epsilon, alpha_value, epsilon_value)``: the transfer kernel
+    """``forward(source_fft, target_fft, alpha, epsilon, alpha_value, epsilon_value, values)``: the transfer kernel
     (``rpsf_construct_kernel``, transform.py:78-82) of two complex cubes of one dtype.  ``alpha`` / ``epsilon`` are the
-    caller's objects (floats or 0-d tensors, which get gradients), ``alpha_value`` / ``epsilon_value`` their values as
-    floats.  The backward is ``rpsf_construct_kernel_backward``: the cube gradients in the cubes' dtype, those of alpha
-    and epsilon accumulated in double and returned in each tensor's dtype and device.  Once-differentiable."""
+    caller's objects (floats or 0-d tensors, which get gradients).  Their values are either ``alpha_value`` /
+    ``epsilon_value`` as floats (``values`` None), or ``values``, a float64 CUDA tensor [alpha, epsilon] on the cubes'
+    device, read there by ``rpsf_construct_kernel_dev`` (no host synchronisation; used whenever alpha or epsilon is a
+    tensor).  The backward is ``rpsf_construct_kernel_backward`` (``_dev``): the cube gradients in the cubes' dtype,
+    those of alpha and epsilon accumulated in double and returned in each tensor's dtype and device.
+    Once-differentiable."""
 
     @staticmethod
-    def forward(ctx, source_fft, target_fft, alpha, epsilon, alpha_value: float, epsilon_value: float):
+    def forward(ctx, source_fft, target_fft, alpha, epsilon, alpha_value, epsilon_value, values=None):
         from regularizepsf_b200 import _native
         ctx.values = (alpha_value, epsilon_value)
+        ctx.on_device = values is not None
         ctx.scalars = tuple((x.dtype, x.device) if torch.is_tensor(x) else None for x in (alpha, epsilon))
-        ctx.save_for_backward(source_fft, target_fft)
+        ctx.save_for_backward(source_fft, target_fft, values)
         kernel = torch.empty_like(source_fft)
         code = _native.F32 if source_fft.dtype == torch.complex64 else _native.F64
+        lib = _native.load()
         with torch.cuda.device(source_fft.device):
-            _native.check(_native.load().rpsf_construct_kernel(
-                source_fft.data_ptr(), target_fft.data_ptr(), kernel.data_ptr(), source_fft.numel(), code, alpha_value,
-                epsilon_value, source_fft.device.index, _native.current_stream_ptr(torch)))
+            stream = _native.current_stream_ptr(torch)
+            if values is not None:
+                _native.check(lib.rpsf_construct_kernel_dev(
+                    source_fft.data_ptr(), target_fft.data_ptr(), kernel.data_ptr(), source_fft.numel(), code,
+                    values.data_ptr(), source_fft.device.index, stream))
+            else:
+                _native.check(lib.rpsf_construct_kernel(
+                    source_fft.data_ptr(), target_fft.data_ptr(), kernel.data_ptr(), source_fft.numel(), code,
+                    alpha_value, epsilon_value, source_fft.device.index, stream))
         return kernel
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_output):
         from regularizepsf_b200 import _native
-        s, t = ctx.saved_tensors
+        s, t, values = ctx.saved_tensors
         grad = grad_output.to(s.dtype).contiguous()
         need_s, need_t, need_a, need_e = ctx.needs_input_grad[:4]
         grad_s = torch.empty_like(s) if need_s else None
         grad_t = torch.empty_like(t) if need_t else None
         scalars = torch.empty(2, dtype=torch.float64, device=s.device) if need_a or need_e else None
         code = _native.F32 if s.dtype == torch.complex64 else _native.F64
+        outputs = (grad_s.data_ptr() if need_s else None, grad_t.data_ptr() if need_t else None,
+                   scalars.data_ptr() if scalars is not None else None)
+        lib = _native.load()
         with torch.cuda.device(s.device):
-            _native.check(_native.load().rpsf_construct_kernel_backward(
-                s.data_ptr(), t.data_ptr(), grad.data_ptr(), s.numel(), code, ctx.values[0], ctx.values[1],
-                grad_s.data_ptr() if need_s else None, grad_t.data_ptr() if need_t else None,
-                scalars.data_ptr() if scalars is not None else None, s.device.index, _native.current_stream_ptr(torch)))
+            stream = _native.current_stream_ptr(torch)
+            if ctx.on_device:
+                _native.check(lib.rpsf_construct_kernel_backward_dev(
+                    s.data_ptr(), t.data_ptr(), grad.data_ptr(), s.numel(), code, values.data_ptr(), *outputs,
+                    s.device.index, stream))
+            else:
+                _native.check(lib.rpsf_construct_kernel_backward(
+                    s.data_ptr(), t.data_ptr(), grad.data_ptr(), s.numel(), code, ctx.values[0], ctx.values[1], *outputs,
+                    s.device.index, stream))
         grad_a = grad_e = None
         if need_a:
             grad_a = scalars[0].to(dtype=ctx.scalars[0][0], device=ctx.scalars[0][1])
         if need_e:
             grad_e = scalars[1].to(dtype=ctx.scalars[1][0], device=ctx.scalars[1][1])
-        return grad_s, grad_t, grad_a, grad_e, None, None
+        return grad_s, grad_t, grad_a, grad_e, None, None, None

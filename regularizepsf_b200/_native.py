@@ -38,8 +38,11 @@ SIGNATURES = {
     "rpsf_transform_destroy": (_i, [_vp]),
     "rpsf_transform_set_kernel": (_i, [_vp, _vp, _i, _vp]),
     "rpsf_transform_num_colours": (_i, [_vp]),
+    "rpsf_transform_order": (_i, [_vp, _vp]),
     "rpsf_construct_kernel": (_i, [_vp, _vp, _vp, _i64, _i, _d, _d, _i, _vp]),
     "rpsf_construct_kernel_backward": (_i, [_vp, _vp, _vp, _i64, _i, _d, _d, _vp, _vp, _vp, _i, _vp]),
+    "rpsf_construct_kernel_dev": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _i, _vp]),
+    "rpsf_construct_kernel_backward_dev": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp, _i, _vp]),
     "rpsf_psf_fft2": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp]),
     "rpsf_psf_fft2_adjoint": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp]),
     "rpsf_average_patches": (_i, [_vp, _i64, _i, _vp, _vp, _i64, _i, _d, _vp, _i, _vp]),
@@ -107,11 +110,18 @@ def last_error() -> str:
     return msg.decode("utf-8", "replace") if msg else ""
 
 
+#: what the library's refusals on a capturing stream say (rpsf_api.cu, refuse_capture)
+CAPTURE_REFUSAL = "while a CUDA graph is being captured"
+
+
 def check(rc: int) -> None:
-    """Translate a status code into the reference's exception types."""
+    """Translate a status code into the reference's exception types (a refusal during graph capture: RuntimeError)."""
     if rc == 0:
         return
-    raise exceptions.for_status(rc)(last_error())
+    msg = last_error()
+    if rc == E_UNSUPPORTED and CAPTURE_REFUSAL in msg:
+        raise RuntimeError(msg)
+    raise exceptions.for_status(rc)(msg)
 
 
 def dtype_code(dtype) -> int | None:
@@ -141,6 +151,18 @@ def current_stream_ptr(torch, device: int | None = None) -> int:
     if raw is not None:
         return int(raw(torch._C._cuda_getDevice() if device is None else device))
     return int(torch.cuda.current_stream(device).cuda_stream)
+
+
+def capturing(torch) -> bool:
+    """Whether torch's current stream is capturing a CUDA graph (one C call)."""
+    return torch.cuda.is_current_stream_capturing()
+
+
+def refuse_in_capture(torch, what: str) -> None:
+    """RuntimeError when the current stream is capturing: ``what`` allocates, synchronises or runs on the host."""
+    if capturing(torch):
+        raise RuntimeError(f"{what} cannot run while a CUDA graph is being captured; call it outside the capture "
+                           "(INTEGRATION.md, \"CUDA graphs\")")
 
 
 def launch_count() -> int:

@@ -94,6 +94,69 @@ struct DeviceGuard {
   ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
+// ---- CUDA graph capture (DESIGN.md section 5) ---------------------------------------------------------------------
+// Streams this library has seen capturing: the entry points that take no stream (plan creation, upload, IPC, the host
+// path) look here to refuse while a capture that went through the library is still open.
+std::mutex g_capture_mu;
+std::vector<cudaStream_t> g_capture_streams;
+std::atomic<int> g_capture_count{0};      // g_capture_streams.size(), read without the mutex by eager calls
+
+// 1 when `s` is capturing, 0 when not.  The legacy stream cannot be asked while another stream captures
+// (cudaErrorStreamCaptureImplicit): that counts as capturing, since work on it would invalidate the capture.
+int stream_capturing(cudaStream_t s, unsigned long long* id = nullptr) {
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  unsigned long long cid = 0;
+  const cudaError_t e = cudaStreamGetCaptureInfo(s, &st, &cid);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return e == cudaErrorStreamCaptureImplicit ? 1 : 0;
+  }
+  if (id) *id = cid;
+  return st != cudaStreamCaptureStatusNone ? 1 : 0;
+}
+
+void note_capture(cudaStream_t s) {
+  std::lock_guard<std::mutex> lock(g_capture_mu);
+  if (std::find(g_capture_streams.begin(), g_capture_streams.end(), s) == g_capture_streams.end()) {
+    g_capture_streams.push_back(s);
+    g_capture_count.store((int)g_capture_streams.size());
+  }
+}
+
+// an eager call on `s`: a capture on it has ended, so it leaves the list (cheap when the list is empty)
+void forget_capture(cudaStream_t s) {
+  if (g_capture_count.load() == 0) return;
+  std::lock_guard<std::mutex> lock(g_capture_mu);
+  auto it = std::find(g_capture_streams.begin(), g_capture_streams.end(), s);
+  if (it != g_capture_streams.end()) g_capture_streams.erase(it);
+  g_capture_count.store((int)g_capture_streams.size());
+}
+
+// whether a capture the library has taken part in is still open (finished ones are forgotten)
+bool capture_open() {
+  std::lock_guard<std::mutex> lock(g_capture_mu);
+  bool open = false;
+  for (size_t i = 0; i < g_capture_streams.size();) {
+    if (stream_capturing(g_capture_streams[i])) { open = true; ++i; }
+    else g_capture_streams.erase(g_capture_streams.begin() + (long)i);
+  }
+  g_capture_count.store((int)g_capture_streams.size());
+  return open;
+}
+
+int refuse_capture(const char* what) {
+  return fail(RPSF_E_UNSUPPORTED, "%s cannot run while a CUDA graph is being captured (it allocates or synchronises): "
+              "run the call once before capturing so that its plans, workspaces and kernel layout exist", what);
+}
+
+// refuse a stream-less entry point while a capture is open
+#define REFUSE_IN_CAPTURE(what) do { if (capture_open()) return refuse_capture(what); } while (0)
+// refuse an entry point that would allocate or synchronise on `s` while `s` captures
+#define REFUSE_ON_CAPTURING(s, what) do { if (stream_capturing(s) || capture_open()) return refuse_capture(what); } while (0)
+
+// the calls on this thread between the halves of an OrderedCall on a capturing stream (lazy allocations refuse)
+thread_local bool t_capturing = false;
+
 // FFT length for a patch size without a native one: the next power of two >= 2 P - 1 (0 if none fits 16..512)
 int embedded_length(int P) {
   if (P < 2) return 0;
@@ -146,21 +209,28 @@ int upload_tables(int P, void** tw_out, void** win_out) {
 // Twiddle / window tables are a pure function of (P, dtype): one copy per device for the life of the
 // library (3 KB at P = 256), shared by every transform and by rpsf_psf_fft2 — nothing to free, no
 // synchronisation when a call returns.
+struct TableEntry { void* tw; void* win; };
+std::mutex g_tables_mu;
+std::map<std::tuple<int, int, int>, TableEntry> g_tables;
+
 int shared_tables(int P, int dtype, int device, void** tw, void** win) {
-  struct Entry { void* tw; void* win; };
-  static std::mutex mu;
-  static std::map<std::tuple<int, int, int>, Entry> cache;
-  std::lock_guard<std::mutex> lock(mu);
+  std::lock_guard<std::mutex> lock(g_tables_mu);
   const auto key = std::make_tuple(P, dtype, device);
-  auto it = cache.find(key);
-  if (it == cache.end()) {
-    Entry e{nullptr, nullptr};
+  auto it = g_tables.find(key);
+  if (it == g_tables.end()) {
+    TableEntry e{nullptr, nullptr};
     int rc = dtype == RPSF_F32 ? upload_tables<float>(P, &e.tw, &e.win) : upload_tables<double>(P, &e.tw, &e.win);
     if (rc) { cudaFree(e.tw); cudaFree(e.win); return rc; }
-    it = cache.emplace(key, e).first;
+    it = g_tables.emplace(key, e).first;
   }
   *tw = it->second.tw; *win = it->second.win;
   return 0;
+}
+
+// whether the tables of (P, dtype, device) exist already, so that a call can take them while a graph is captured
+bool tables_ready(int P, int dtype, int device) {
+  std::lock_guard<std::mutex> lock(g_tables_mu);
+  return g_tables.count(std::make_tuple(P, dtype, device)) != 0;
 }
 
 }  // namespace
@@ -320,6 +390,14 @@ struct rpsf_transform {
   cudaEvent_t order_ev = nullptr;
   cudaStream_t order_stream = nullptr;   // the stream order_ev was last recorded on
   bool order_recorded = false;
+  // CUDA graphs: a capture makes order_ev an external dependency of the graph, so replays record it without the host
+  // knowing; once captured, every eager call waits for it.  capture_ev orders the calls inside one capture (capture_id).
+  bool captured = false;
+  cudaEvent_t capture_ev = nullptr;
+  unsigned long long capture_id = 0;
+  bool capture_recorded = false;
+  // embedded patch sizes: the (M, P) embedding matrix of set_kernel_on, uploaded at the first layout
+  void* embed_A = nullptr;
 };
 
 namespace {
@@ -330,12 +408,31 @@ namespace {
 // workspace at once, whatever streams they use; a call on the stream of the previous one pays only the record.
 // cudaStreamPerThread names a different stream on every thread, so it always waits.  The mutex keeps the bookkeeping
 // whole for C callers that share a transform across threads.
+//
+// On a capturing stream the event becomes an external dependency of the graph: an external wait at the start (each
+// replay waits for the calls issued before its launch) and an external record at the end (calls issued after the launch
+// are ordered behind the replay).  A replay runs no library code, so the host cannot know which stream recorded the
+// event last: once a transform has been captured, every eager call waits for it.  Calls inside one capture are also
+// ordered among themselves through capture_ev, an ordinary record / wait pair that becomes a graph edge.
 struct OrderedCall {
   rpsf_transform* t;
   cudaStream_t s;
+  bool capturing = false;
+  unsigned long long capture_id = 0;
   int begin() {
+    capturing = stream_capturing(s, &capture_id) != 0;
     std::lock_guard<std::mutex> lock(t->order_mu);
-    if (t->order_recorded && (s != t->order_stream || s == cudaStreamPerThread)) {
+    if (capturing) {
+      note_capture(s);
+      cudaError_t e = cudaStreamWaitEvent(s, t->order_ev, cudaEventWaitExternal);
+      if (e == cudaSuccess && t->capture_recorded && t->capture_id == capture_id) e = cudaStreamWaitEvent(s, t->capture_ev, 0);
+      if (e != cudaSuccess) return fail(RPSF_E_CUDA, "ordering a captured call after the transform's last call failed: %s", cudaGetErrorString(e));
+      t->captured = true;
+      t_capturing = true;
+      return RPSF_OK;
+    }
+    forget_capture(s);
+    if (t->order_recorded && (t->captured || s != t->order_stream || s == cudaStreamPerThread)) {
       const cudaError_t e = cudaStreamWaitEvent(s, t->order_ev, 0);
       if (e != cudaSuccess) return fail(RPSF_E_CUDA, "ordering after the transform's last call failed: %s", cudaGetErrorString(e));
     }
@@ -344,6 +441,16 @@ struct OrderedCall {
   // `rc`: the status of the launches; the record is made whatever it is, so that what was launched is ordered too
   int end(int rc) {
     std::lock_guard<std::mutex> lock(t->order_mu);
+    if (capturing) {
+      t_capturing = false;
+      cudaError_t e = cudaEventRecordWithFlags(t->order_ev, s, cudaEventRecordExternal);
+      if (e == cudaSuccess) e = cudaEventRecord(t->capture_ev, s);
+      if (e != cudaSuccess) return rc ? rc : fail(RPSF_E_CUDA, "recording the transform's order event in a capture failed: %s", cudaGetErrorString(e));
+      t->capture_id = capture_id;
+      t->capture_recorded = true;
+      t->order_recorded = true;           // replays record it: eager calls after them must wait
+      return rc;
+    }
     const cudaError_t e = cudaEventRecord(t->order_ev, s);
     if (e != cudaSuccess) return rc ? rc : fail(RPSF_E_CUDA, "recording the transform's order event failed: %s", cudaGetErrorString(e));
     t->order_stream = s;
@@ -462,6 +569,7 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
                                  const uint8_t* keep) {
   if (!out || (!coords && n > 0) || n < 0) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "compute dtype must be f32 or f64");
+  REFUSE_IN_CAPTURE("rpsf_transform_create");
   const int win_len = P;
   const Ops* ops = ops_for(P);
   if (!ops) {
@@ -478,8 +586,10 @@ int rpsf_transform_create_subset(rpsf_transform** out, const int32_t* coords, in
   auto* t = new rpsf_transform;
   t->device = device; t->P = P; t->n = n; t->dtype = dtype; t->ops = ops; t->win_len = win_len;
   t->sm_count = sm_count_of(device);
-  if (cudaEventCreateWithFlags(&t->order_ev, cudaEventDisableTiming) != cudaSuccess) {
+  if (cudaEventCreateWithFlags(&t->order_ev, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&t->capture_ev, cudaEventDisableTiming) != cudaSuccess) {
     const cudaError_t ce = cudaGetLastError();
+    if (t->order_ev) cudaEventDestroy(t->order_ev);
     delete t;
     return fail(RPSF_E_CUDA, "cannot create the transform's order event: %s", cudaGetErrorString(ce));
   }
@@ -553,48 +663,72 @@ int rpsf_transform_destroy(rpsf_transform* t) {
   cudaFree(t->kmain); cudaFree(t->knyq);
   cudaFree(t->kconj_main); cudaFree(t->kconj_nyq);
   if (t->own_win) cudaFree(t->win);
+  cudaFree(t->embed_A);
   if (t->order_ev) cudaEventDestroy(t->order_ev);
+  if (t->capture_ev) cudaEventDestroy(t->capture_ev);
   delete t;
   return RPSF_OK;
 }
 
 int rpsf_transform_num_colours(const rpsf_transform* t) { return t ? t->n_colours : 0; }
 
+int rpsf_transform_order(rpsf_transform* t, void* stream) {
+  if (!t) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  return ordered(t, (cudaStream_t)stream, []() -> int { return RPSF_OK; });
+}
+
 }  // extern "C"
 
 namespace {
-// the layout of rpsf_transform_set_kernel, stream-ordered on `s`
+// the (M, P) embedding matrix of an embedded patch size, uploaded once per transform (at its first kernel layout, which
+// is never captured): A[u][p] = (1/P) sum_{i=-(P-1)}^{P-1} exp(2 pi i (p/P - u/M) i), stored complex with a zero
+// imaginary part
+int upload_embed_matrix(rpsf_transform* t) {
+  if (t->embed_A) return RPSF_OK;
+  const int P = t->win_len, M = t->P;
+  std::vector<double> A(2 * (size_t)M * P);
+  const double two_pi = 6.283185307179586476925286766559;
+  for (int u = 0; u < M; ++u)
+    for (int p = 0; p < P; ++p) {
+      // the phase reduced exactly: (p M - u P) i mod (P M) = sin((2P-1) theta/2) / sin(theta/2) / P with theta/2 = pi r /
+      // (P M), r = (p M - u P) mod (P M); real, because the terms i and -i are conjugates
+      const long long den = (long long)P * M;
+      long long r = ((long long)p * M - (long long)u * P) % den; if (r < 0) r += den;
+      double re = double(2 * P - 1);
+      if (r != 0) {
+        const long long rn = ((2LL * P - 1) * r) % (2 * den);         // numerator angle, reduced mod 2 pi
+        re = std::sin(0.5 * two_pi * double(rn) / double(den)) / std::sin(0.5 * two_pi * double(r) / double(den));
+      }
+      A[2 * ((size_t)u * P + p)] = re / P; A[2 * ((size_t)u * P + p) + 1] = 0.0;
+    }
+  void* dA = nullptr;
+  if (cudaMalloc(&dA, sizeof(double2) * M * P) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(RPSF_E_CUDA, "out of device memory for the embedding matrix (%d x %d)", M, P);
+  }
+  const cudaError_t e = cudaMemcpy(dA, A.data(), sizeof(double2) * M * P, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { cudaFree(dA); return fail(RPSF_E_CUDA, "embedding matrix upload failed: %s", cudaGetErrorString(e)); }
+  t->embed_A = dA;
+  return RPSF_OK;
+}
+
+// the layout of rpsf_transform_set_kernel, stream-ordered on `s`; on a capturing stream it allocates only with
+// cudaMallocAsync (allocation nodes of the graph)
 int set_kernel_on(rpsf_transform* t, const void* kernel_full, int kernel_dtype, cudaStream_t s) {
   if (t->n_kept > 0 && t->win_len != t->P) {
     // embedded patch size: K (n, P, P) -> K' (n, M, M) = A K A^T in double (rpsf_kernels.cuh), then the usual layout
     const int P = t->win_len, M = t->P;
-    std::vector<double> A(2 * (size_t)M * P);
-    const double two_pi = 6.283185307179586476925286766559;
-    for (int u = 0; u < M; ++u)
-      for (int p = 0; p < P; ++p) {
-        // (1/P) sum_{i=-(P-1)}^{P-1} exp(2 pi i (p/P - u/M) i), the phase reduced exactly: (p M - u P) i mod (P M)
-        // = sin((2P-1) theta/2) / sin(theta/2) / P with theta/2 = pi r / (P M), r = (p M - u P) mod (P M); real, because the
-        // terms i and -i are conjugates
-        const long long den = (long long)P * M;
-        long long r = ((long long)p * M - (long long)u * P) % den; if (r < 0) r += den;
-        double re = double(2 * P - 1);
-        if (r != 0) {
-          const long long rn = ((2LL * P - 1) * r) % (2 * den);         // numerator angle, reduced mod 2 pi
-          re = std::sin(0.5 * two_pi * double(rn) / double(den)) / std::sin(0.5 * two_pi * double(r) / double(den));
-        }
-        A[2 * ((size_t)u * P + p)] = re / P; A[2 * ((size_t)u * P + p) + 1] = 0.0;
-      }
-    double2 *dA = nullptr, *dT = nullptr, *dK = nullptr;
-    auto release = [&]() { for (void* q : {(void*)dA, (void*)dT, (void*)dK}) if (q) cudaFreeAsync(q, s); };
+    if (!t->embed_A && t_capturing) return refuse_capture("the first kernel layout of an embedded patch size");
+    if (int rc = upload_embed_matrix(t)) return rc;
+    const double2* dA = (const double2*)t->embed_A;
+    double2 *dT = nullptr, *dK = nullptr;
+    auto release = [&]() { for (void* q : {(void*)dT, (void*)dK}) if (q) cudaFreeAsync(q, s); };
     const size_t n = (size_t)t->n_kept;
-    if (cudaMallocAsync((void**)&dA, sizeof(double2) * M * P, s) != cudaSuccess ||
-        cudaMallocAsync((void**)&dT, sizeof(double2) * n * M * P, s) != cudaSuccess ||
+    if (cudaMallocAsync((void**)&dT, sizeof(double2) * n * M * P, s) != cudaSuccess ||
         cudaMallocAsync((void**)&dK, sizeof(double2) * n * M * M, s) != cudaSuccess) {
       release(); cudaGetLastError();
       return fail(RPSF_E_CUDA, "out of device memory embedding %zu kernels of %d in %d", n, P, M);
     }
-    // the host matrix is read by the copy before this function returns (pageable source: staged synchronously)
-    CU(cudaMemcpyAsync(dA, A.data(), sizeof(double2) * M * P, cudaMemcpyHostToDevice, s));
     const unsigned blocks = (unsigned)t->sm_count * 16;
     if (kernel_dtype == RPSF_F32) embed_pass1<float2><<<blocks, 256, 0, s>>>((const float2*)kernel_full, dA, dT, (int)n, P, M);
     else embed_pass1<double2><<<blocks, 256, 0, s>>>((const double2*)kernel_full, dA, dT, (int)n, P, M);
@@ -624,26 +758,38 @@ int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int ke
   return ordered(t, s, [&]() -> int { return set_kernel_on(t, kernel_full, kernel_dtype, s); });
 }
 
-int rpsf_construct_kernel(const void* S, const void* Tg, void* K, int64_t count, int dtype, double alpha,
-                          double epsilon, int device, void* stream) {
+}  // extern "C"
+
+namespace {
+// rpsf_construct_kernel (ae == nullptr: the host scalars alpha, epsilon) and rpsf_construct_kernel_dev (ae: two device
+// doubles); launches only, so a capture may hold it
+int construct_kernel(const void* S, const void* Tg, void* K, int64_t count, int dtype, double alpha, double epsilon,
+                     const double* ae, int device, void* stream) {
   if (count < 0 || (count > 0 && (!S || !Tg || !K))) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "dtype must be f32 or f64");
   if (count == 0) return RPSF_OK;
   DeviceGuard guard(device);
   const unsigned blocks = (unsigned)std::min<long long>((count + 255) / 256, (long long)sm_count_of(device) * 16);
-  if (dtype == RPSF_F32)
-    construct_transfer_kernel<float><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-        (const float2*)S, (const float2*)Tg, (float2*)K, count, (float)alpha, (float)epsilon);
-  else
-    construct_transfer_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-        (const double2*)S, (const double2*)Tg, (double2*)K, count, alpha, epsilon);
+  const cudaStream_t s = (cudaStream_t)stream;
+  if (dtype == RPSF_F32) {
+    if (ae) construct_transfer_kernel<float, true><<<blocks, 256, 0, s>>>((const float2*)S, (const float2*)Tg, (float2*)K,
+                                                                        count, 0.f, 0.f, ae);
+    else construct_transfer_kernel<float><<<blocks, 256, 0, s>>>((const float2*)S, (const float2*)Tg, (float2*)K, count,
+                                                                 (float)alpha, (float)epsilon);
+  } else {
+    if (ae) construct_transfer_kernel<double, true><<<blocks, 256, 0, s>>>((const double2*)S, (const double2*)Tg,
+                                                                         (double2*)K, count, 0.0, 0.0, ae);
+    else construct_transfer_kernel<double><<<blocks, 256, 0, s>>>((const double2*)S, (const double2*)Tg, (double2*)K,
+                                                                  count, alpha, epsilon);
+  }
   LAUNCH((int)cudaGetLastError());
   return RPSF_OK;
 }
 
-int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G, int64_t count, int dtype, double alpha,
-                                   double epsilon, void* source_grad, void* target_grad, double* alpha_epsilon_grad,
-                                   int device, void* stream) {
+// rpsf_construct_kernel_backward and its _dev form (ae: alpha and epsilon as two device doubles)
+int construct_kernel_backward(const void* S, const void* Tg, const void* G, int64_t count, int dtype, double alpha,
+                              double epsilon, const double* ae, void* source_grad, void* target_grad,
+                              double* alpha_epsilon_grad, int device, void* stream) {
   if (count < 0 || (count > 0 && (!S || !Tg || !G))) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "dtype must be f32 or f64");
   DeviceGuard guard(device);
@@ -660,14 +806,25 @@ int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G,
     cudaError_t e = cudaMallocAsync((void**)&partial, sizeof(double2) * ctas, s);
     if (e != cudaSuccess) return fail(RPSF_E_CUDA, "cudaMallocAsync of %d partial sums failed: %s", ctas, cudaGetErrorString(e));
   }
-  if (dtype == RPSF_F32)
-    construct_transfer_kernel_backward<float><<<ctas, CGRAD_THREADS, 0, s>>>(
-        (const float2*)S, (const float2*)Tg, (const float2*)G, count, (float)alpha, (float)epsilon, (float2*)source_grad,
-        (float2*)target_grad, partial);
-  else
-    construct_transfer_kernel_backward<double><<<ctas, CGRAD_THREADS, 0, s>>>(
-        (const double2*)S, (const double2*)Tg, (const double2*)G, count, alpha, epsilon, (double2*)source_grad,
-        (double2*)target_grad, partial);
+  if (dtype == RPSF_F32) {
+    if (ae)
+      construct_transfer_kernel_backward<float, true><<<ctas, CGRAD_THREADS, 0, s>>>(
+          (const float2*)S, (const float2*)Tg, (const float2*)G, count, 0.f, 0.f, (float2*)source_grad,
+          (float2*)target_grad, partial, ae);
+    else
+      construct_transfer_kernel_backward<float><<<ctas, CGRAD_THREADS, 0, s>>>(
+          (const float2*)S, (const float2*)Tg, (const float2*)G, count, (float)alpha, (float)epsilon, (float2*)source_grad,
+          (float2*)target_grad, partial);
+  } else {
+    if (ae)
+      construct_transfer_kernel_backward<double, true><<<ctas, CGRAD_THREADS, 0, s>>>(
+          (const double2*)S, (const double2*)Tg, (const double2*)G, count, 0.0, 0.0, (double2*)source_grad,
+          (double2*)target_grad, partial, ae);
+    else
+      construct_transfer_kernel_backward<double><<<ctas, CGRAD_THREADS, 0, s>>>(
+          (const double2*)S, (const double2*)Tg, (const double2*)G, count, alpha, epsilon, (double2*)source_grad,
+          (double2*)target_grad, partial);
+  }
   cudaError_t e = cudaGetLastError();
   g_launches.fetch_add(1, std::memory_order_relaxed);
   if (e == cudaSuccess && partial) {
@@ -679,6 +836,35 @@ int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G,
   if (e != cudaSuccess) return fail(RPSF_E_CUDA, "construct backward launch failed: %s", cudaGetErrorString(e));
   return RPSF_OK;
 }
+}  // namespace
+
+extern "C" {
+
+int rpsf_construct_kernel(const void* S, const void* Tg, void* K, int64_t count, int dtype, double alpha,
+                          double epsilon, int device, void* stream) {
+  return construct_kernel(S, Tg, K, count, dtype, alpha, epsilon, nullptr, device, stream);
+}
+
+int rpsf_construct_kernel_dev(const void* S, const void* Tg, void* K, int64_t count, int dtype,
+                              const double* alpha_epsilon, int device, void* stream) {
+  if (!alpha_epsilon) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  return construct_kernel(S, Tg, K, count, dtype, 0.0, 0.0, alpha_epsilon, device, stream);
+}
+
+int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G, int64_t count, int dtype, double alpha,
+                                   double epsilon, void* source_grad, void* target_grad, double* alpha_epsilon_grad,
+                                   int device, void* stream) {
+  return construct_kernel_backward(S, Tg, G, count, dtype, alpha, epsilon, nullptr, source_grad, target_grad,
+                                   alpha_epsilon_grad, device, stream);
+}
+
+int rpsf_construct_kernel_backward_dev(const void* S, const void* Tg, const void* G, int64_t count, int dtype,
+                                       const double* alpha_epsilon, void* source_grad, void* target_grad,
+                                       double* alpha_epsilon_grad, int device, void* stream) {
+  if (!alpha_epsilon) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  return construct_kernel_backward(S, Tg, G, count, dtype, 0.0, 0.0, alpha_epsilon, source_grad, target_grad,
+                                   alpha_epsilon_grad, device, stream);
+}
 
 int rpsf_psf_fft2_adjoint(const void* spectrum_grad, void* values_grad, int64_t n, int P, int dtype, int device,
                           void* stream) {
@@ -689,12 +875,13 @@ int rpsf_psf_fft2_adjoint(const void* spectrum_grad, void* values_grad, int64_t 
   if (n == 0) return RPSF_OK;
   DeviceGuard guard(device);
   if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!tables_ready(P, dtype, device) && stream_capturing(s)) return refuse_capture("the first rpsf_psf_fft2_adjoint of a patch size");
   int e = ops->init();
   if (e) return fail(RPSF_E_CUDA, "kernel attribute setup failed: %s", cudaGetErrorString((cudaError_t)e));
   void* tw = nullptr; void* win = nullptr;
   int rc = shared_tables(P, dtype, device, &tw, &win);
   if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
   void* scratch = nullptr;                                        // the complex row spectra, (n, P, P)
   const size_t bytes = 2 * real_size(dtype) * (size_t)n * P * P;
   cudaError_t ce = cudaMallocAsync(&scratch, bytes, s);
@@ -713,6 +900,8 @@ int rpsf_psf_fft2(const void* values, void* out, int64_t n, int P, int dtype, in
   if (!ops && (P < 1 || P > 512)) return fail(RPSF_E_UNSUPPORTED, "patch size %d has no device path", P);
   if (n == 0) return RPSF_OK;
   DeviceGuard guard(device);
+  if ((!ops || !tables_ready(P, dtype, device)) && stream_capturing((cudaStream_t)stream))
+    return refuse_capture(ops ? "the first rpsf_psf_fft2 of a patch size" : "rpsf_psf_fft2 of a patch size without a native FFT length");
   if (!ops) {
     // no native FFT length: separable direct DFT in double (setup cost only, O(P^3) per patch)
     cudaStream_t s = (cudaStream_t)stream;
@@ -754,6 +943,7 @@ int rpsf_average_patches(const double* cutouts, int64_t n_cutouts, int P, const 
   if (P <= 0 || n_cutouts < 0 || n_cells < 0) return fail(RPSF_E_INVALID_ARGUMENT, "negative size");
   if (n_cells == 0) return RPSF_OK;
   if (!cell_offsets || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_ON_CAPTURING((cudaStream_t)stream, "rpsf_average_patches");
   if (method != RPSF_AVG_MEAN && method != RPSF_AVG_MEDIAN && method != RPSF_AVG_PERCENTILE)
     return fail(RPSF_E_UNSUPPORTED, "unknown averaging method %d", method);
   if (method == RPSF_AVG_PERCENTILE && !(percentile >= 0.0 && percentile <= 100.0))
@@ -862,6 +1052,7 @@ int patch_stage(const double* in, double* out, int64_t n, int P, int device, voi
   if (n == 0) return RPSF_OK;
   if (!out || (!isolate && !in)) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (n > INT_MAX || (long long)P * P > INT_MAX / 2) return fail(RPSF_E_UNSUPPORTED, "too many patches or patch too large");
+  REFUSE_ON_CAPTURING((cudaStream_t)stream, isolate ? "rpsf_isolate_cores" : "rpsf_plane_background");
   DeviceGuard guard(device);
   if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
   cudaStream_t s = (cudaStream_t)stream;
@@ -887,6 +1078,7 @@ int rpsf_star_cutouts(const void* frame, int frame_dtype, int H, int W, const do
   if (!frame || !corners || !out || !accepted) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (frame_dtype != RPSF_F32 && frame_dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "frames must be float32 or float64");
   if (n_stars > INT_MAX || (long long)width * width > INT_MAX / 2) return fail(RPSF_E_UNSUPPORTED, "too many stars or cutout too large");
+  REFUSE_ON_CAPTURING((cudaStream_t)stream, "rpsf_star_cutouts");
   for (int64_t i = 0; i < 2 * n_stars; ++i)
     if (!(std::fabs(corners[i]) < 1e9)) return fail(RPSF_E_INVALID_COORDINATE, "star corner %lld is not a finite pixel position", (long long)(i / 2));
   DeviceGuard guard(device);
@@ -938,6 +1130,7 @@ int rpsf_plan_set_output_mirrors(rpsf_plan* p, int n, void* const* ptrs) {
 int rpsf_ipc_alloc(void** ptr, int64_t bytes, int device, unsigned char handle[64]) {
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
   if (!ptr || !handle || bytes <= 0) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_ipc_alloc");
   DeviceGuard guard(device);
   if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
   CU(cudaMalloc(ptr, (size_t)bytes));
@@ -950,6 +1143,7 @@ int rpsf_ipc_alloc(void** ptr, int64_t bytes, int device, unsigned char handle[6
 
 int rpsf_ipc_open(void** ptr, const unsigned char handle[64], int device) {
   if (!ptr || !handle) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_ipc_open");
   DeviceGuard guard(device);
   if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
   cudaIpcMemHandle_t h;
@@ -960,6 +1154,7 @@ int rpsf_ipc_open(void** ptr, const unsigned char handle[64], int device) {
 
 int rpsf_ipc_close(void* ptr, int device) {
   if (!ptr) return RPSF_OK;
+  REFUSE_IN_CAPTURE("rpsf_ipc_close");
   DeviceGuard guard(device);
   if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
   CU(cudaDeviceSynchronize());
@@ -1223,6 +1418,7 @@ extern "C" {
 
 int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int row_begin, int row_end,
                      int max_batch) {
+  if (out && t) REFUSE_IN_CAPTURE("rpsf_plan_create");
   return plan_build(out, t, H, W, pad_mode, row_begin, row_end, max_batch, nullptr);
 }
 
@@ -1232,6 +1428,7 @@ int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, i
   if (pad_mode < 0 || pad_mode >= RPSF_PAD_MATERIALIZED)
     return fail(RPSF_E_UNSUPPORTED, "the transpose needs a pad mode with an index map (0..4), got %d", pad_mode);
   if (max_batch < 1) return fail(RPSF_E_INVALID_ARGUMENT, "max_batch must be >= 1");
+  REFUSE_IN_CAPTURE("rpsf_plan_create_adjoint");
   if (int rc = check_corners(t, H, W)) return rc;
   // the box: bounding box of the footprints of the patches that touch the frame (a 1 x 1 box when none does)
   const int L = t->win_len;
@@ -1337,6 +1534,7 @@ int rpsf_plan_info(const rpsf_plan* p, int64_t info[9]) {
 
 static int ensure_workspace(rpsf_plan* p) {
   if (p->workspace || p->workspace_bytes == 0) return RPSF_OK;
+  if (t_capturing) return refuse_capture("the first call of a plan (its spectrum workspace)");
   DeviceGuard guard(p->tr->device);
   if (cudaMalloc(&p->workspace, p->workspace_bytes) != cudaSuccess) {
     cudaGetLastError();
@@ -1360,6 +1558,7 @@ int rpsf_plan_column_info(const rpsf_plan* p, int64_t info[2]) {
 
 int rpsf_upload(void** device_ptr, const void* src_host, int64_t bytes, int device) {
   if (!device_ptr || bytes < 0 || (bytes > 0 && !src_host)) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_upload");
   DeviceGuard guard(device);
   *device_ptr = nullptr;
   if (bytes == 0) return RPSF_OK;
@@ -1374,6 +1573,7 @@ int rpsf_upload(void** device_ptr, const void* src_host, int64_t bytes, int devi
 
 int rpsf_device_free(void* device_ptr, int device) {
   if (!device_ptr) return RPSF_OK;
+  REFUSE_IN_CAPTURE("rpsf_device_free");
   DeviceGuard guard(device);
   CU(cudaDeviceSynchronize());
   CU(cudaFree(device_ptr));
@@ -1382,6 +1582,7 @@ int rpsf_device_free(void* device_ptr, int device) {
 
 int rpsf_copy_to_host(void* dst, const void* src, int64_t bytes, int device) {
   if (bytes < 0 || (bytes > 0 && (!dst || !src))) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_copy_to_host");
   DeviceGuard guard(device);
   CU(cudaDeviceSynchronize());
   CU(cudaMemcpy(dst, src, (size_t)bytes, cudaMemcpyDeviceToHost));
@@ -1448,6 +1649,7 @@ int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_
   const size_t px = (size_t)sg.Hp * sg.Wp, mb = (size_t)p->max_batch;
   if ((long long)px > 0x7fffffffLL) return fail(RPSF_E_UNSUPPORTED, "padded frame too large for the saturation branch");
   if (!p->sat_pf) {
+    if (t_capturing) return refuse_capture("the first saturation branch of a plan (its scratch)");
     CU(cudaMalloc(&p->sat_pf, px * sizeof(T) * mb));
     CU(cudaMalloc((void**)&p->sat_mask[0], px * mb));
     CU(cudaMalloc((void**)&p->sat_mask[1], px * mb));
@@ -1528,6 +1730,7 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   const bool need_zero = !((p->colour0_covers || use_gather || use_stream) && stages >= 3);
   cudaEvent_t* ev = nullptr;
   if (p->timing && stages >= 3 && p->n_active > 0) {
+    if (t_capturing) return refuse_capture("a plan with stage timing");
     if (p->events_used + 4 > p->events.size()) {
       for (int i = 0; i < 4; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); p->events.push_back(e); }
     }
@@ -1705,6 +1908,7 @@ int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_
     // per-stage events of the forward plan (bench only): K1(x) | copy + K1(g) | zeroing + kgrad
     cudaEvent_t* ev = nullptr;
     if (fp->timing && fp->n_active > 0) {
+      if (t_capturing) return refuse_capture("a plan with stage timing");
       if (fp->events_used + 4 > fp->events.size()) {
         for (int i = 0; i < 4; ++i) { cudaEvent_t e; CU(cudaEventCreate(&e)); fp->events.push_back(e); }
       }
@@ -1752,6 +1956,7 @@ int rpsf_plan_enable_timing(rpsf_plan* p, int enabled) {
 
 int rpsf_plan_read_timing(rpsf_plan* p, double ms[3], int* calls) {
   if (!p || !ms || !calls) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_plan_read_timing");
   DeviceGuard guard(p->tr->device);
   ms[0] = ms[1] = ms[2] = 0.0;
   *calls = 0;
@@ -1886,6 +2091,7 @@ int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out,
   if (p->row_end == p->row_begin) return RPSF_OK;                      // empty band: no bytes to produce
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (out_dtype != RPSF_F32 && out_dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "output dtype must be f32 or f64");
+  REFUSE_IN_CAPTURE("rpsf_apply_host");
   const size_t isz = elem_size(image_dtype);
   if (!isz) return fail(RPSF_E_UNSUPPORTED, "unsupported image dtype code %d", image_dtype);
   rpsf_transform* t = p->tr;

@@ -27,11 +27,20 @@ constexpr int CGRAD_MAX_CTAS = 148 * 8;
 
 // Elementwise over `count` bins.  gS / gT may be null (not computed, not written).  partial (nullable): one
 // (grad_alpha, grad_eps) pair per CTA, summed in double in a fixed order (grid-stride per thread, then a fixed tree).
-template <typename T>
+// DEV: alpha and epsilon come from two device doubles (`ae`), loaded once per CTA (construct_transfer_kernel's DEV).
+template <typename T, bool DEV = false>
 __global__ void __launch_bounds__(CGRAD_THREADS)
 construct_transfer_kernel_backward(const cplx<T>* __restrict__ S, const cplx<T>* __restrict__ Tg,
                                    const cplx<T>* __restrict__ G, long long count, T alpha, T epsilon,
-                                   cplx<T>* __restrict__ gS, cplx<T>* __restrict__ gT, double2* __restrict__ partial) {
+                                   cplx<T>* __restrict__ gS, cplx<T>* __restrict__ gT, double2* __restrict__ partial,
+                                   const double* __restrict__ ae = nullptr) {
+  if constexpr (DEV) {
+    __shared__ T scalars[2];
+    if (threadIdx.x == 0) { scalars[0] = T(ae[0]); scalars[1] = T(ae[1]); }
+    __syncthreads();
+    alpha = scalars[0];
+    epsilon = scalars[1];
+  }
   double acc_alpha = 0.0, acc_eps = 0.0;
   const T nan = T(NAN);
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count;

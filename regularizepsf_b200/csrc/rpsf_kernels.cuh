@@ -790,9 +790,19 @@ template <typename T> __device__ __forceinline__ T pow_like_numpy(T x, T p) {
   if (p == T(-1)) return T(1) / x;
   return pow(x, p);
 }
-template <typename T>
+// DEV: alpha and epsilon are read from two device doubles (`ae`), once per CTA, and converted to T as the host-scalar
+// entry point converts its arguments, so the same bins take the same arithmetic (rpsf_construct_kernel_dev).
+template <typename T, bool DEV = false>
 __global__ void construct_transfer_kernel(const cplx<T>* __restrict__ S, const cplx<T>* __restrict__ Tg,
-                                          cplx<T>* __restrict__ K, long long count, T alpha, T epsilon) {
+                                          cplx<T>* __restrict__ K, long long count, T alpha, T epsilon,
+                                          const double* __restrict__ ae = nullptr) {
+  if constexpr (DEV) {
+    __shared__ T scalars[2];
+    if (threadIdx.x == 0) { scalars[0] = T(ae[0]); scalars[1] = T(ae[1]); }
+    __syncthreads();
+    alpha = scalars[0];
+    epsilon = scalars[1];
+  }
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count;
        i += (long long)gridDim.x * blockDim.x) {
     const cplx<T> s = S[i], tg = Tg[i];

@@ -76,6 +76,8 @@ class ArrayPSF:
         self._given_fft_cube = fft_cube              # None: computed on the device at first use
         self._computed_fft_cube = None
         self._computed_version = None                # values tensor version the computed cube was made from
+        self._uploaded_fft = None                    # the last upload of a host FFT cube given here (_device_spectrum)
+        self._captured_uploads = []                  # uploads CUDA graphs read: never freed before the PSF
         if fft_cube is None:
             return                                   # a computed cube matches the values cube by construction
         if fft_cube.sample_shape != self._values_cube.sample_shape:
@@ -99,6 +101,24 @@ class ArrayPSF:
             self._computed_fft_cube = _device_fft_cube(self._values_cube)
             self._computed_version = version
         return self._computed_fft_cube
+
+    def _device_spectrum(self, torch):
+        """The FFT cube as a CUDA tensor.  A host cube given to the constructor is uploaded at every eager call; the last
+        upload serves calls captured in a CUDA graph, which cannot copy from the host (RuntimeError when no eager call
+        has made one), and an upload a capture has used is kept with the PSF, since its graphs read it at every
+        replay."""
+        cube = self._fft_cube
+        if isinstance(cube, DeviceCube):
+            return cube.tensor.contiguous()
+        if _native.capturing(torch):
+            if self._uploaded_fft is None:
+                raise RuntimeError("this PSF's FFT cube is on the host, and uploading it cannot be captured in a CUDA "
+                                   "graph: run the same call once before capturing")
+            if not any(u is self._uploaded_fft for u in self._captured_uploads):
+                self._captured_uploads.append(self._uploaded_fft)
+            return self._uploaded_fft
+        self._uploaded_fft = torch.from_numpy(np.ascontiguousarray(cube.values)).cuda()
+        return self._uploaded_fft
 
     @property
     def _values_device_tensor(self):

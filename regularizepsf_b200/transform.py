@@ -73,6 +73,9 @@ class _NativeTransform:
         # had when it was laid out, so that the next call lays it out again (ArrayPSFTransform._native_transform)
         self.kernel_source = None
         self.kernel_version = None
+        self.captured = False           # a CUDA graph holds calls of this transform (reconstruct lays out at once)
+        # the kernel tensors captured layouts read, kept alive with the transform: [(tensor, made by construct)]
+        self.graph_sources: list = []
         self.set_kernel(kernel_tensor, stream)
 
     def set_kernel(self, kernel_tensor, stream: int) -> None:
@@ -87,12 +90,15 @@ class _NativeTransform:
         plans.clear()
         _destroy(lib, "transform", handle)
 
+    #: keys of plans a CUDA graph has captured: never evicted, freed with the transform (a replay uses their workspaces)
+    _pinned: frozenset = frozenset()
+
     #: at most this many plans stay alive per transform and compute dtype; each owns max_batch spectrum
     #: workspaces (75.8 MB per 2048^2 / 256-px frame), so an unbounded cache is an HBM leak
     MAX_PLANS = 6
 
     def plan(self, height: int, width: int, pad_mode: int, row_begin: int, row_end: int, max_batch: int,
-             adjoint: bool = False) -> int:
+             adjoint: bool = False, capturing: bool = False) -> int:
         """Plan for this geometry able to take ``max_batch`` frames per call (``adjoint``: the transpose of the
         whole-frame plan, ``rpsf_plan_create_adjoint``; it has workspaces of its own).
 
@@ -100,12 +106,18 @@ class _NativeTransform:
         (``rpsf_apply`` accepts any batch up to the plan's; the factor keeps a single-frame call off a plan
         whose work lists were cut for large batches).  Plans are evicted least-recently-used beyond
         ``MAX_PLANS``; eviction calls ``rpsf_plan_destroy`` (its ``cudaFree`` waits for work in flight).
+
+        ``capturing``: the call is being captured in a CUDA graph.  The plan must exist (creating one allocates and
+        synchronises: RuntimeError), and it is pinned: never evicted, freed with the transform, since every replay of
+        the graph uses its workspaces.
         """
         geometry = (height, width, pad_mode, row_begin, row_end, adjoint)
         exact = geometry + (max_batch,)
         if exact in self._plans:
             if next(reversed(self._plans)) != exact:
                 self._plans[exact] = self._plans.pop(exact)
+            if capturing:
+                self._pinned = self._pinned | {exact}
             return self._plans[exact]
         best = None
         for key in self._plans:
@@ -114,7 +126,13 @@ class _NativeTransform:
         if best is not None:
             plan = self._plans.pop(best)
             self._plans[best] = plan                      # most recently used last
+            if capturing:
+                self._pinned = self._pinned | {best}
             return plan
+        if capturing:
+            raise RuntimeError(f"no plan for {'adjoint ' if adjoint else ''}frames of {height} x {width} (pad mode "
+                               f"{pad_mode}, rows [{row_begin}, {row_end}), {max_batch} frames) exists, and creating one "
+                               "cannot be captured in a CUDA graph: run the same call once before capturing")
         out = ctypes.c_void_p()
         if adjoint:
             _native.check(self.lib.rpsf_plan_create_adjoint(ctypes.byref(out), self.handle, height, width, pad_mode,
@@ -123,8 +141,8 @@ class _NativeTransform:
             _native.check(self.lib.rpsf_plan_create(ctypes.byref(out), self.handle, height, width, pad_mode,
                                                     row_begin, row_end, max_batch))
         self._plans[geometry + (max_batch,)] = out.value
-        while len(self._plans) > self.MAX_PLANS:
-            oldest = next(iter(self._plans))
+        while len(self._plans) - len(self._pinned) > self.MAX_PLANS:
+            oldest = next(key for key in self._plans if key not in self._pinned)
             handle = self._plans.pop(oldest)
             self._saturation.pop(handle, None)
             _destroy(self.lib, "plan", handle)
@@ -227,9 +245,10 @@ class ArrayPSFTransform:
         ``DeviceCube`` whose tensor requires grad), a given ``DeviceCube`` FFT cube, or ``alpha`` / ``epsilon`` require
         grad, the result's kernel tensor requires grad, so ``loss(apply(x)).backward()`` reaches them through
         ``rpsf_construct_kernel_backward`` and ``rpsf_psf_fft2_adjoint`` (DESIGN.md section 6).  ``alpha`` and ``epsilon``
-        are numbers or 0-d real tensors; tensors are read to the host, which synchronises (once for two on one device).  PSF values that
-        require grad need a native patch size (16, 32, ..., 512).  Otherwise the kernel is computed exactly as without
-        autograd.
+        are numbers or 0-d real tensors.  A tensor is never read to the host: the kernels take both values from device
+        memory (``rpsf_construct_kernel_dev``, bit-identical to passing them as numbers), so the call does not
+        synchronise and can be captured in a CUDA graph.  PSF values that require grad need a native patch size (16, 32,
+        ..., 512).  Otherwise the kernel is computed exactly as without autograd.
         """
         if np.any(np.array(source.coordinates) != np.array(target.coordinates)):
             raise InvalidCoordinateError("Source PSF coordinates do not match target PSF coordinates.")
@@ -244,8 +263,7 @@ class ArrayPSFTransform:
             if s_cube.sample_shape != t_cube.sample_shape:
                 raise IncorrectShapeError(f"source and target sample shapes differ: "
                                           f"{s_cube.sample_shape} != {t_cube.sample_shape}")
-            s = cube_tensor(s_cube, torch)
-            t = cube_tensor(t_cube, torch)
+            s, t = _plain_spectrum(source, s_cube, torch), _plain_spectrum(target, t_cube, torch)
             if s.device != t.device:
                 raise ValueError(f"source and target FFT cubes live on different devices: {s.device} and {t.device}")
             wide = torch.complex128 if torch.complex128 in (s.dtype, t.dtype) else torch.complex64
@@ -254,19 +272,20 @@ class ArrayPSFTransform:
                 t = t.to(wide) if t.dtype != wide else t
                 kernel = torch.empty_like(s)
                 code = _native.F32 if wide == torch.complex64 else _native.F64
-                _native.check(lib.rpsf_construct_kernel(s.data_ptr(), t.data_ptr(), kernel.data_ptr(), s.numel(), code,
-                                                        float(alpha), float(epsilon), s.device.index,
-                                                        _native.current_stream_ptr(torch)))
-            return cls(DeviceCube(source.coordinates, kernel))
+                stream = _native.current_stream_ptr(torch)
+                if _is_torch_tensor(alpha) or _is_torch_tensor(epsilon):
+                    values = _device_scalars(torch, alpha, epsilon, s.device)
+                    _native.check(lib.rpsf_construct_kernel_dev(s.data_ptr(), t.data_ptr(), kernel.data_ptr(), s.numel(),
+                                                                code, values.data_ptr(), s.device.index, stream))
+                else:
+                    _native.check(lib.rpsf_construct_kernel(s.data_ptr(), t.data_ptr(), kernel.data_ptr(), s.numel(),
+                                                            code, float(alpha), float(epsilon), s.device.index, stream))
+            return cls._constructed(source.coordinates, kernel)
         from regularizepsf_b200._autograd import Construct
         for name, value in (("alpha", alpha), ("epsilon", epsilon)):
             if _is_torch_tensor(value) and (value.dim() != 0 or value.is_complex()):
                 raise ValueError(f"{name} must be a number or a 0-d real tensor, got shape {tuple(value.shape)} "
                                  f"{value.dtype}")
-        if _is_torch_tensor(alpha) and _is_torch_tensor(epsilon) and alpha.device == epsilon.device:
-            values = torch.stack([alpha.detach().double(), epsilon.detach().double()]).tolist()   # one synchronisation
-        else:
-            values = [float(x.detach()) if _is_torch_tensor(x) else float(x) for x in (alpha, epsilon)]
         s, t = _spectrum(source, torch), _spectrum(target, torch)
         if tuple(s.shape[1:]) != tuple(t.shape[1:]):
             raise IncorrectShapeError(f"source and target sample shapes differ: {tuple(s.shape[1:])} != "
@@ -277,30 +296,85 @@ class ArrayPSFTransform:
         with torch.cuda.device(s.device):
             s = (s.to(wide) if s.dtype != wide else s).contiguous()
             t = (t.to(wide) if t.dtype != wide else t).contiguous()
-            kernel = Construct.apply(s, t, alpha, epsilon, *values)
-        return cls(DeviceCube(source.coordinates, kernel))
+            if _is_torch_tensor(alpha) or _is_torch_tensor(epsilon):
+                kernel = Construct.apply(s, t, alpha, epsilon, None, None, _device_scalars(torch, alpha, epsilon, s.device))
+            else:
+                kernel = Construct.apply(s, t, alpha, epsilon, float(alpha), float(epsilon))
+        return cls._constructed(source.coordinates, kernel)
+
+    #: the kernel tensor was made by construct / reconstruct, not given by the caller (reconstruct may write into it)
+    _kernel_owned = False
+
+    @classmethod
+    def _constructed(cls, coordinates, kernel) -> "ArrayPSFTransform":
+        obj = cls(DeviceCube(coordinates, kernel))
+        obj._kernel_owned = True
+        return obj
 
     def reconstruct(self, source, target, alpha, epsilon) -> None:
         """Replace the transfer kernel by ``construct(source, target, alpha, epsilon)``'s, in place.
 
         For a fitting loop that builds the kernel from its parameters at every step: the transform keeps its native
         transforms and plans (with their spectrum workspaces, 75.8 MB per 2048^2 frame at 256 px) and lays the new
-        kernel out at its next call, where a fresh ``construct`` would create them again.  The coordinates and the patch
+        kernel out at its next call, where a fresh ``construct`` would create them again.  A transform whose calls a CUDA
+        graph has captured lays it out in this call instead, so that replays launched after it read the new kernel; a
+        graph that lays the kernel out itself reads the kernel tensor it was captured with, so the new kernel is copied
+        into that tensor too (RuntimeError if that tensor is one the caller gave, not one ``construct`` made).  If the
+        new kernel cannot be built, the transform is left as it was (inside a capture: with the previous kernel
+        detached from its autograd graph, which a captured call lets go of before it builds the next).  The coordinates and the patch
         size must be the transform's (InvalidCoordinateError / IncorrectShapeError).  A kernel that requires grad on a
         sharded transform raises NotImplementedError.
         """
         if np.any(np.array(source.coordinates) != np.array(self.coordinates)):
             raise InvalidCoordinateError("the PSF coordinates do not match the transform's coordinates")
-        new = type(self).construct(source, target, alpha, epsilon)
-        if new.psf_shape != self.psf_shape:
-            raise IncorrectShapeError(f"the PSFs' sample shape {new.psf_shape} is not the transform's {self.psf_shape}")
-        kernel = new._kernel_tensor
-        if kernel.requires_grad and self._shard_keep is not None:
-            raise NotImplementedError("the kernel gradient of a sharded transform is not implemented")
+        torch = _native.require_cuda()
+        capturing = _native.capturing(torch)
+        if not capturing and any(not owned for nt in self._native.values() for _, owned in nt.graph_sources):
+            raise RuntimeError("CUDA graphs of this transform lay out the kernel tensor it was given, and reconstruct "
+                               "would leave them reading that tensor: update the tensor in place instead, or capture "
+                               "the graphs again on a fresh transform")
+        old = self._kernel_tensor
+        if capturing and old is not None and old.grad_fn is not None:
+            # let go of the previous kernel's autograd graph before building the next: otherwise the new graph reuses
+            # the PSF values' gradient accumulators it holds, which belong to the stream of the eager call that made
+            # them, and the captured backward would accumulate on a stream outside the capture
+            old = old.detach()
+            self._kernel_tensor, self._transfer_kernel = old, DeviceCube(self.coordinates, old)
+            for nt in self._native.values():
+                if nt.kernel_source is not None:
+                    nt.kernel_source = old
+        saved = (self._kernel_tensor, self._transfer_kernel, [(nt, nt.kernel_source) for nt in self._native.values()])
+        try:
+            new = type(self).construct(source, target, alpha, epsilon)
+            if new.psf_shape != self.psf_shape:
+                raise IncorrectShapeError(f"the PSFs' sample shape {new.psf_shape} is not the transform's "
+                                          f"{self.psf_shape}")
+            kernel = new._kernel_tensor
+            if kernel.requires_grad and self._shard_keep is not None:
+                raise NotImplementedError("the kernel gradient of a sharded transform is not implemented")
+        except BaseException:
+            self._kernel_tensor, self._transfer_kernel, sources = saved     # the transform is as it was
+            for nt, source_tensor in sources:
+                nt.kernel_source = source_tensor
+            raise
         self._transfer_kernel = DeviceCube(self.coordinates, kernel)
         self._kernel_tensor = kernel
-        for nt in self._native.values():
+        self._kernel_owned = True
+        for (_, device), nt in self._native.items():
             nt.kernel_source, nt.kernel_version = kernel, None     # laid out again at the next call
+            if nt.captured and not capturing:
+                # a replay runs no Python: lay the kernel out now, stream-ordered, so that replays launched after this
+                # call read it (inside a capture, the next captured call lays it out).  Captured layouts read the
+                # kernel tensors they were captured with: the new kernel is copied into them, after every call issued
+                # so far (rpsf_transform_order) and before every call issued after this one (the layout records).
+                with torch.cuda.device(device):
+                    stream = _native.current_stream_ptr(torch)
+                    if nt.graph_sources:
+                        _native.check(nt.lib.rpsf_transform_order(nt.handle, stream))
+                        for tensor, _ in nt.graph_sources:
+                            tensor.copy_(kernel.detach())
+                    nt.set_kernel(self._kernel_on(torch, device), stream)
+                nt.kernel_version = kernel._version if kernel.requires_grad else None
 
     # ------------------------------------------------------------------ native state
     def _coords(self) -> np.ndarray:
@@ -318,14 +392,39 @@ class ArrayPSFTransform:
             self._coords_i32 = np.ascontiguousarray(as_int, dtype=np.int32)
         return self._coords_i32
 
-    def _native_transform(self, dtype_name: str, device: int | None = None) -> _NativeTransform:
+    def _native_transform(self, dtype_name: str, device: int | None = None, capturing: bool = False,
+                          reads_kernel: bool = True) -> _NativeTransform:
         """The native transform for (compute dtype, device); ``device`` defaults to the current CUDA device.
-        Call with that device current (``_apply_device`` / ``_apply_host`` do)."""
+        Call with that device current (``_apply_device`` / ``_apply_host`` do).
+
+        ``capturing``: the call is being captured in a CUDA graph.  The native transform must exist (RuntimeError
+        otherwise: creating it and the first kernel layout allocate and synchronise).  A kernel tensor that requires
+        grad, or one not laid out yet (``reconstruct``), is laid out again inside the graph at every captured call, so
+        that each replay reads the tensor as it is then (``optimizer.step()`` between replays updates it in place, where
+        no Python runs to see the new version); the transform keeps that tensor alive (``graph_sources``).
+        ``reads_kernel=False`` (the kernel gradient, which reads no kernel) skips that layout."""
         torch = _native.require_cuda()
         if device is None:
             device = torch.cuda.current_device()
         key = (dtype_name, device)
         nt = self._native.get(key)
+        if capturing:
+            if nt is not None:
+                nt.captured = True
+            if nt is None:
+                raise RuntimeError(f"this transform has no native state for {dtype_name} on cuda:{device} yet, and "
+                                   "creating it (with the first kernel layout) cannot be captured in a CUDA graph: run "
+                                   "the same call once before capturing")
+            if (nt.kernel_source is not None and reads_kernel
+                    and (nt.kernel_source.requires_grad or nt.kernel_version is None)):
+                # the graph reads the kernel tensor by address at every replay: keep it alive with the transform
+                source = self._transfer_kernel.tensor.detach()
+                if not any(t.data_ptr() == source.data_ptr() for t, _ in nt.graph_sources):
+                    nt.graph_sources.append((source, self._kernel_owned))
+                with torch.cuda.device(device):
+                    nt.set_kernel(self._kernel_on(torch, device), _native.current_stream_ptr(torch))
+                nt.kernel_version = None       # the layout happens at replays: the next eager call lays it out again
+            return nt
         if nt is None:
             p0, p1 = self.psf_shape
             if p0 != p1:
@@ -388,7 +487,8 @@ class ArrayPSFTransform:
         is when the call is issued (after ``reconstruct`` or an in-place update of the kernel tensor
         too), whatever streams earlier calls used: the library orders its own device state — the
         laid-out kernel, the plans' workspaces and scratch — across streams, the private streams of a
-        numpy call included.
+        numpy call included.  A tensor call does not synchronise with the host, and once warmed up it can be
+        captured in a CUDA graph (INTEGRATION.md, "CUDA graphs"); a numpy call synchronises and cannot.
         """
         del workers
         kt = self._kernel_tensor
@@ -414,6 +514,7 @@ class ArrayPSFTransform:
             return self._apply_materialized_pad(image, dtype_name, pad_mode, out_np, sat)
         if _is_torch_tensor(image):
             return self._apply_device(image, dtype_name, _native.PAD_MODES[pad_mode], sat=sat)
+        _native.refuse_in_capture(_native.require_cuda(), "apply() of a numpy array (a host-to-host call)")
         image = np.asarray(image)
         if image.ndim not in (2, 3):
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {image.shape}")
@@ -440,6 +541,7 @@ class ArrayPSFTransform:
                 return self._apply_differentiable(image, pad_mode, math.inf, dtype, adjoint=True)
             return self._apply_device(image, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
         torch = _native.require_cuda()
+        _native.refuse_in_capture(torch, "apply_adjoint() of a numpy array (a host-to-host call)")
         host = np.asarray(image)
         if host.ndim not in (2, 3):
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {host.shape}")
@@ -500,6 +602,7 @@ class ArrayPSFTransform:
                 raise TypeError("image and grad_output must both be numpy arrays or both CUDA tensors")
             return self._kernel_gradient_device(image.detach(), grad_output.detach(), dtype_name, pad_code)
         torch = _native.require_cuda()
+        _native.refuse_in_capture(torch, "transfer_kernel_gradient() of numpy arrays (a host-to-host call)")
         x, g = np.asarray(image), np.asarray(grad_output)
         if x.shape != g.shape or x.ndim not in (2, 3):
             raise IncorrectShapeError(f"image and grad_output must share a shape (H, W) or (B, H, W), got {x.shape} "
@@ -520,13 +623,14 @@ class ArrayPSFTransform:
                                       f"{tuple(image.shape)} and {tuple(grad.shape)}")
         want = torch.float32 if dtype_name == "float32" else torch.float64
         with torch.cuda.device(image.device):
-            nt = self._native_transform(dtype_name, image.device.index)
+            capturing = _native.capturing(torch)
+            nt = self._native_transform(dtype_name, image.device.index, capturing, reads_kernel=False)
             frames = [t.unsqueeze(0) if t.dim() == 2 else t for t in (image, grad)]
             frames = [t.to(want) if t.dtype != want else t for t in frames]
             x, g = [t.contiguous() if t.stride(-1) != 1 else t for t in frames]
             b, h, w = x.shape
-            forward = nt.plan(h, w, pad_code, 0, h, b)
-            adjoint = nt.plan(h, w, pad_code, 0, h, b, adjoint=True)
+            forward = nt.plan(h, w, pad_code, 0, h, b, capturing=capturing)
+            adjoint = nt.plan(h, w, pad_code, 0, h, b, adjoint=True, capturing=capturing)
             nt.set_saturation(forward, self._NO_SAT)
             p = self.psf_shape[0]
             out = torch.empty((len(self), p, p), dtype=torch.complex64 if dtype_name == "float32" else torch.complex128,
@@ -547,6 +651,7 @@ class ArrayPSFTransform:
         the width); the padded frames are uploaded and the kernels read the margin in place.  Slower than the five
         index-map modes (4.5 x the upload at 2048^2 / 256 px) — those stay the fast path."""
         torch = _native.require_cuda()
+        _native.refuse_in_capture(torch, f"apply() with pad_mode={pad_mode!r} (np.pad on the host)")
         is_tensor = _is_torch_tensor(image)
         host = image.detach().cpu().numpy() if is_tensor else np.asarray(image)
         if host.ndim not in (2, 3):
@@ -613,7 +718,8 @@ class ArrayPSFTransform:
 
     def _apply_device_on(self, torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows=None,
                          adjoint=False, source=None):
-        nt = self._native_transform(dtype_name, image.device.index)
+        capturing = _native.capturing(torch)
+        nt = self._native_transform(dtype_name, image.device.index, capturing)
         want = torch.float32 if dtype_name == "float32" else torch.float64
         squeeze = image.dim() == 2
         frames = image.unsqueeze(0) if squeeze else image
@@ -640,7 +746,7 @@ class ArrayPSFTransform:
                                           f"stride, got {out.dtype} {tuple(out.shape)}")
         if r1 <= r0:                                       # an empty band: nothing to compute, no native call
             return out[0] if squeeze else out
-        plan = nt.plan(h, w, pad_code, r0, r1, b, adjoint=adjoint)
+        plan = nt.plan(h, w, pad_code, r0, r1, b, adjoint=adjoint, capturing=capturing)
         nt.set_saturation(plan, sat)
         if mirrors:        # device pointers of peer buffers laid out like `out` (distributed.PeerFrames)
             import ctypes
@@ -686,11 +792,21 @@ def _spectrum_source(psf):
     return values if values is not None and values.requires_grad else None
 
 
+def _plain_spectrum(psf, cube, torch):
+    """The FFT cube ``cube`` of ``psf`` as a CUDA tensor without autograd history (``ArrayPSF._device_spectrum`` for an
+    ``ArrayPSF``, so that a host cube is not copied inside a CUDA graph capture)."""
+    if hasattr(psf, "_device_spectrum"):
+        return psf._device_spectrum(torch)
+    return cube_tensor(cube, torch)
+
+
 def _spectrum(psf, torch):
     """``psf``'s FFT cube as a CUDA tensor, differentiable in what ``_spectrum_source`` finds: a values tensor goes
     through ``_autograd.PsfFFT``, afresh at every call."""
     source = _spectrum_source(psf)
     if source is None:
+        if hasattr(psf, "_device_spectrum"):
+            return psf._device_spectrum(torch)
         return cube_tensor(psf.fft_cube if hasattr(psf, "fft_cube") else psf._fft_cube, torch)
     if psf._given_fft_cube is not None:
         return source
@@ -702,6 +818,18 @@ def _spectrum(psf, torch):
                          f"{source.device}")
     from regularizepsf_b200._autograd import PsfFFT
     return PsfFFT.apply(source if source.dtype in (torch.float32, torch.float64) else source.to(torch.float64))
+
+
+def _device_scalars(torch, alpha, epsilon, device):
+    """[alpha, epsilon] as a float64 tensor on ``device``, without a host synchronisation: a CUDA tensor is copied on the
+    device, a number (or a CPU tensor, whose value the host has) is filled in."""
+    values = torch.empty(2, dtype=torch.float64, device=device)
+    for i, x in enumerate((alpha, epsilon)):
+        if _is_torch_tensor(x) and x.is_cuda:
+            values[i].copy_(x.detach().reshape(()))
+        else:
+            values[i].fill_(float(x.detach()) if _is_torch_tensor(x) else float(x))
+    return values
 
 
 def _is_torch_tensor(obj) -> bool:
