@@ -61,7 +61,7 @@ typedef struct rpsf_transform rpsf_transform;
 typedef struct rpsf_plan rpsf_plan;
 
 /* CUDA graphs.  A stream capture may contain, once their plans exist and each has run once outside the capture:
- * rpsf_apply (forward and adjoint plans), rpsf_apply_source, rpsf_kernel_gradient, rpsf_transform_set_kernel,
+ * rpsf_apply (forward and adjoint plans), rpsf_apply_source, rpsf_apply_masked, rpsf_kernel_gradient(_masked), rpsf_transform_set_kernel,
  * rpsf_construct_kernel(_dev), rpsf_construct_kernel_backward(_dev), rpsf_psf_fft2 and rpsf_psf_fft2_adjoint (native
  * patch sizes).  These neither cudaMalloc nor synchronise then; their scratch is cudaMallocAsync on the stream, which
  * the capture turns into allocation nodes.  On a capturing stream a call that touches a transform's device state makes
@@ -231,6 +231,15 @@ int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int height, int
 int rpsf_kernel_gradient(rpsf_plan* adjoint_plan, rpsf_plan* forward_plan, const void* image, int64_t img_pitch,
                          int64_t img_frame_stride, const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch,
                          void* kernel_grad, void* stream);
+/* rpsf_kernel_gradient of apply with a caller-given bad-pixel mask (rpsf_apply_masked): X is K1 of the padded frame
+ * filled under the mask (the forward plan's rpsf_plan_set_saturation gives the neighbourhood width; its threshold must be
+ * infinite), G that of (1 - M) grad.  mask: uint8, nonzero = masked, pixel (y, x) of frame b at mask +
+ * b*mask_frame_stride + y*mask_pitch + x; mask_frame_stride 0 shares one mask across the frames.  The first call of a
+ * forward plan allocates its fill scratch (as the saturation branch does) and cannot be captured. */
+int rpsf_kernel_gradient_masked(rpsf_plan* adjoint_plan, rpsf_plan* forward_plan, const void* image, int64_t img_pitch,
+                                int64_t img_frame_stride, const void* grad, int64_t grad_pitch, int64_t grad_frame_stride,
+                                int batch, void* kernel_grad, const void* mask, int64_t mask_pitch,
+                                int64_t mask_frame_stride, void* stream);
 int rpsf_plan_destroy(rpsf_plan* p);
 /* info[0]=active patches, [1]=colours, [2]=workspace bytes, [3]=first frame row read,
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,
@@ -279,6 +288,21 @@ int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_f
 int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
                       int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
                       const void* src, int src_dtype, int64_t src_pitch, int64_t src_frame_stride, void* stream);
+
+/* rpsf_apply with a caller-given bad-pixel mask M (uint8, nonzero = masked, laid out as for
+ * rpsf_kernel_gradient_masked; mask_frame_stride 0 shares one mask across the frames).  On a forward plan: the pixels of
+ * pad(M) (padded with the plan's index map; the margin of constant mode is unmasked), ORed into the dilated saturation
+ * mask (only pad(M) with an infinite threshold), are filled in raster order with the nanmean of their neighbourhood as
+ * saturated pixels are, and get their raw values back after the correction.  `src` (may be null) is rpsf_apply_source's.
+ * On an adjoint plan (src null, infinite threshold, rpsf_plan_set_saturation giving the neighbourhood width): the
+ * transpose of that map, which with an infinite threshold is linear in the image, with the fill's contributors decided
+ * by the mask alone (finite-input semantics; a structural NaN, a masked pixel whose window holds no contributor,
+ * passes nothing back).  Needs a pad mode with an index map and whole frames resident.  The first call of a plan
+ * allocates its padded-size scratch and cannot be captured in a CUDA graph; later ones can. */
+int rpsf_apply_masked(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                      const void* src, int src_dtype, int64_t src_pitch, int64_t src_frame_stride, const void* mask,
+                      int64_t mask_pitch, int64_t mask_frame_stride, void* stream);
 
 /* ---- apply, host buffers (the call a reference user makes): H2D + convert + apply + D2H ------
  * image: `batch` contiguous (H, W) frames of image_dtype on the host (pinned or pageable);

@@ -52,6 +52,7 @@ SIGNATURES = {
     "rpsf_plan_create": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, _i]),
     "rpsf_plan_create_adjoint": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i]),
     "rpsf_kernel_gradient": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _i64, _i64, _i, _vp, _vp]),
+    "rpsf_kernel_gradient_masked": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _i64, _i64, _i, _vp, _vp, _i64, _i64, _vp]),
     "rpsf_plan_destroy": (_i, [_vp]),
     "rpsf_plan_info": (_i, [_vp, ctypes.POINTER(_i64)]),
     "rpsf_plan_set_overlap_mode": (_i, [_vp, _i]),
@@ -66,6 +67,8 @@ SIGNATURES = {
     "rpsf_device_free": (_i, [_vp, _i]),
     "rpsf_apply": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp]),
     "rpsf_apply_source": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp, _i, _i64, _i64, _vp]),
+    "rpsf_apply_masked": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp, _i, _i64, _i64, _vp, _i64, _i64,
+                               _vp]),
     "rpsf_apply_host": (_i, [_vp, _vp, _i, _vp, _i, _i]),
     "rpsf_convert": (_i, [_vp, _i, _i64, _vp, _i, _i64, _i, _i, _i, _vp]),
     "rpsf_plan_workspace": (_i, [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_i64)]),

@@ -551,6 +551,13 @@ struct rpsf_plan {
   void* box_in = nullptr; void* box_out = nullptr;
   int* fold_rows = nullptr;           // [frame_H + 1 offsets | box row indices], CSR preimages of the row pad map
   int* fold_cols = nullptr;           // the same for columns
+  // masked transpose (rpsf_apply_masked on an adjoint plan): the same preimages over the whole padded frame (the fill
+  // carries gradient out of the box), and, allocated at the first masked call, the padded-size buffers: v / shares in
+  // sat_pf, the combined gradient in mask_out, contributor counts in mask_count (state, list, rows and tickets: sat_*)
+  int* fold_prows = nullptr;
+  int* fold_pcols = nullptr;
+  void* mask_out = nullptr;
+  int* mask_count = nullptr;
   // per-stage timing (bench only)
   bool timing = false;
   std::vector<cudaEvent_t> events;   // 4 per recorded apply call
@@ -1451,6 +1458,8 @@ int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, i
   p->box_pitch = (long long)((Wb + align - 1) / align * align);
   const size_t box_bytes = (size_t)max_batch * Hb * p->box_pitch * rs;
   const std::vector<int> rows = fold_table(H, y0, Hb, pad_mode), cols = fold_table(W, x0, Wb, pad_mode);
+  const int pad = 2 * t->P;
+  const std::vector<int> prows = fold_table(H, -pad, H + 2 * pad, pad_mode), pcols = fold_table(W, -pad, W + 2 * pad, pad_mode);
   auto bail = [&](const char* what) {
     const cudaError_t e = cudaGetLastError();
     rpsf_plan_destroy(p);
@@ -1465,6 +1474,12 @@ int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, i
   if (cudaMemcpy(p->fold_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemcpy(p->fold_cols, cols.data(), sizeof(int) * cols.size(), cudaMemcpyHostToDevice) != cudaSuccess)
     return bail("fold table upload");
+  if (cudaMalloc(&p->fold_prows, sizeof(int) * prows.size()) != cudaSuccess ||
+      cudaMalloc(&p->fold_pcols, sizeof(int) * pcols.size()) != cudaSuccess)
+    return bail("padded fold tables");
+  if (cudaMemcpy(p->fold_prows, prows.data(), sizeof(int) * prows.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(p->fold_pcols, pcols.data(), sizeof(int) * pcols.size(), cudaMemcpyHostToDevice) != cudaSuccess)
+    return bail("padded fold table upload");
   if (!t->kconj_main && t->n_kept > 0) {
     const size_t cs = 2 * rs;
     if (cudaMalloc(&t->kconj_main, (size_t)t->n_kept * t->P * (t->P / 2) * cs) != cudaSuccess ||
@@ -1501,6 +1516,7 @@ int rpsf_plan_destroy(rpsf_plan* p) {
   cudaFree(p->sat_pf); cudaFree(p->sat_mask[0]); cudaFree(p->sat_mask[1]); cudaFree(p->sat_list);
   cudaFree(p->sat_rows); cudaFree(p->sat_flags);
   cudaFree(p->box_in); cudaFree(p->box_out); cudaFree(p->fold_rows); cudaFree(p->fold_cols);
+  cudaFree(p->fold_prows); cudaFree(p->fold_pcols); cudaFree(p->mask_out); cudaFree(p->mask_count);
   for (int* d : p->items_dev) cudaFree(d);
   for (cudaEvent_t e : p->events) cudaEventDestroy(e);
   delete p;
@@ -1612,6 +1628,38 @@ struct SatSource {
   long long pitch, frame_stride;
 };
 
+// A caller-given bad-pixel mask (rpsf_apply_masked): uint8, nonzero = masked, pixel (y, x) of frame b at
+// ptr + b*frame_stride + y*pitch + x; frame_stride 0 shares one mask across the frames.
+struct MaskArg {
+  const unsigned char* ptr;
+  long long pitch, frame_stride;
+};
+
+SatGeom mask_geom(const rpsf_plan* p, int H, int W, int pad_mode) {
+  SatGeom sg{};
+  const int pad = 2 * p->tr->P;
+  sg.H = H; sg.W = W; sg.pad = pad; sg.Hp = H + 2 * pad; sg.Wp = W + 2 * pad;
+  sg.half = p->sat_width / 2; sg.row_begin = 0; sg.row_end = H; sg.pad_mode = pad_mode;
+  return sg;
+}
+
+void launch_mask_ingest(const MaskArg& m, unsigned char* state, const SatGeom& sg, int batch, cudaStream_t s) {
+  const dim3 rows_grid((unsigned)std::min((sg.Wp + 255) / 256, 8), (unsigned)sg.Hp, (unsigned)batch);
+  mask_ingest<<<rows_grid, 256, 0, s>>>(m.ptr, m.pitch, m.frame_stride, state, sg);
+}
+
+// raster-ordered list of the masked pixels of `state`: per-row counts, scan, ordered scatter
+int mask_compact(rpsf_plan* p, const unsigned char* state, const SatGeom& sg, int batch, cudaStream_t s) {
+  const dim3 warp_rows((unsigned)((sg.Hp + 7) / 8), (unsigned)batch);
+  sat_row_count<<<warp_rows, 256, 0, s>>>(state, p->sat_rows, sg.Hp, sg.Wp);
+  LAUNCH((int)cudaGetLastError());
+  sat_row_scan<<<batch, 1024, 0, s>>>(p->sat_rows, sg.Hp);
+  LAUNCH((int)cudaGetLastError());
+  sat_row_scatter<<<warp_rows, 256, 0, s>>>(state, p->sat_rows, p->sat_list, sg.Hp, sg.Wp);
+  LAUNCH((int)cudaGetLastError());
+  return RPSF_OK;
+}
+
 // launch sat_pad_mask with the mask decided on `src` when converting its dtype to T can change a comparison with
 // the threshold (float64 and 32/64-bit integers into float32), else on the converted image itself.  A 64-bit integer
 // rounds to double in the comparison, as it does in the reference's `.astype(float)`.
@@ -1634,11 +1682,12 @@ int launch_sat_pad_mask(rpsf_plan* p, const void* image, const SatSource* src, c
   return (int)cudaGetLastError();
 }
 
-// Saturation pre-fill on the stream: pad + mask, dilate, compact in raster order, ordered fill.
+// Saturation pre-fill on the stream: pad + mask, dilate, OR the caller's mask (`mask`, may be null), compact in raster
+// order, ordered fill.  With an infinite threshold the threshold mask is empty and only the caller's mask is used.
 // On return *filled points at padded pixel (2P, 2P) of frame 0, i.e. at unpadded (0, 0).
 template <typename T>
 int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, const SatSource* src,
-                int batch, cudaStream_t s, SatGeom* sg_out, const void** filled) {
+                int batch, cudaStream_t s, SatGeom* sg_out, const void** filled, const MaskArg* mask = nullptr) {
   rpsf_transform* t = p->tr;
   const int P = t->P, pad = 2 * P;
   SatGeom sg;
@@ -1663,7 +1712,9 @@ int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_
   const dim3 rows_grid((unsigned)std::min((sg.Wp + 255) / 256, 8), (unsigned)sg.Hp, (unsigned)batch);
   LAUNCH(launch_sat_pad_mask<T>(p, image, src, sg, any_flag, rows_grid, s));
   int cur = 0;
-  if (p->sat_dilation < 1) {
+  if (mask && p->sat_threshold == INFINITY) {
+    // nothing is above the threshold: no dilation
+  } else if (p->sat_dilation < 1) {
     sat_dilate<<<rows_grid, 256, 0, s>>>(p->sat_mask[0], p->sat_mask[1], any_flag, sg.Hp, sg.Wp, 1);
     LAUNCH((int)cudaGetLastError());
     cur = 1;
@@ -1675,13 +1726,11 @@ int sat_prefill(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_
     }
   }
   unsigned char* state = p->sat_mask[cur];
-  const dim3 warp_rows((unsigned)((sg.Hp + 7) / 8), (unsigned)batch);
-  sat_row_count<<<warp_rows, 256, 0, s>>>(state, p->sat_rows, sg.Hp, sg.Wp);
-  LAUNCH((int)cudaGetLastError());
-  sat_row_scan<<<batch, 1024, 0, s>>>(p->sat_rows, sg.Hp);
-  LAUNCH((int)cudaGetLastError());
-  sat_row_scatter<<<warp_rows, 256, 0, s>>>(state, p->sat_rows, p->sat_list, sg.Hp, sg.Wp);
-  LAUNCH((int)cudaGetLastError());
+  if (mask) {
+    launch_mask_ingest(*mask, state, sg, batch, s);
+    LAUNCH((int)cudaGetLastError());
+  }
+  if (int rc = mask_compact(p, state, sg, batch, s)) return rc;
   // every CTA of the fill must be resident at once only for speed, not for correctness (tickets)
   sat_fill<T><<<dim3((unsigned)t->sm_count * 2, (unsigned)batch), 256, 0, s>>>((T*)p->sat_pf, state, p->sat_list, p->sat_rows, tickets, sg);
   LAUNCH((int)cudaGetLastError());
@@ -1702,7 +1751,7 @@ int sat_restore_launch(rpsf_plan* p, const void* image, void* out, int64_t out_p
 // `src`: the frames before their conversion to the compute dtype, for the saturation mask (nullptr: `image`)
 int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
                  int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
-                 int batch, int stages, void* stream_v, const SatSource* src = nullptr) {
+                 int batch, int stages, void* stream_v, const SatSource* src = nullptr, const MaskArg* mask = nullptr) {
   if (p->row_end == p->row_begin && stages >= 3) return RPSF_OK;      // an empty band (more ranks than half-patch rows): nothing to write
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   rpsf_transform* t = p->tr;
@@ -1744,7 +1793,8 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
       CU(cudaMemset2DAsync(dst, (size_t)out_pitch * rs, 0, (size_t)p->W * rs, band, s));
     }
   }
-  const bool sat = p->sat_threshold < INFINITY && stages >= 3;
+  // a caller's mask fills the frame before K1 at every stage count (the kernel gradient's X is K1 of the filled frame)
+  const bool sat = (p->sat_threshold < INFINITY && stages >= 3) || mask;
   if (p->n_active == 0 && !sat) return RPSF_OK;
   SatGeom sg;
   const void* k1_image = image;
@@ -1752,14 +1802,14 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   if (sat) {
     if (img_row0 != 0 || img_rows < p->H)
       return fail(RPSF_E_UNSUPPORTED, "the saturation branch needs the whole frame resident (rows [0,%d))", p->H);
-    int rc = t->dtype == RPSF_F32 ? sat_prefill<float>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image)
-                                  : sat_prefill<double>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image);
+    int rc = t->dtype == RPSF_F32 ? sat_prefill<float>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image, mask)
+                                  : sat_prefill<double>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image, mask);
     if (rc) return rc;
     g1.img_row0 = 0; g1.img_rows = sg.Hp; g1.img_pitch = sg.Wp; g1.img_frame_stride = (long long)sg.Hp * sg.Wp;
     g1.pad_mode = PAD_NONE;
   }
   auto restore = [&]() -> int {
-    if (!sat) return RPSF_OK;
+    if (!sat || stages < 3) return RPSF_OK;
     return t->dtype == RPSF_F32
                ? sat_restore_launch<float>(p, image, out, out_pitch, out_frame_stride, out_row0, batch, s, sg)
                : sat_restore_launch<double>(p, image, out, out_pitch, out_frame_stride, out_row0, batch, s, sg);
@@ -1859,6 +1909,89 @@ int apply_adjoint(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t im
   LAUNCH((int)cudaGetLastError());
   return RPSF_OK;
 }
+
+// (1 - M) y (whole frames) -> interior of the zero-bordered box of an adjoint plan
+template <typename T>
+int adjoint_copy_masked(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, const MaskArg& m,
+                        int batch, cudaStream_t s) {
+  const int H = p->frame_H, W = p->frame_W;
+  const long long box_stride = (long long)p->H * p->box_pitch;
+  const int r0 = std::max(0, p->box_y0), r1 = std::min(H, p->box_y0 + p->H);
+  const int c0 = std::max(0, p->box_x0), c1 = std::min(W, p->box_x0 + p->W);
+  if (r1 > r0 && c1 > c0) {
+    const dim3 grid((unsigned)((c1 - c0 + 255) / 256), (unsigned)std::min(r1 - r0, 1024), (unsigned)batch);
+    mask_copy_in<T><<<grid, 256, 0, s>>>((const T*)image + (long long)r0 * img_pitch + c0, img_pitch, img_frame_stride,
+                                         m.ptr + (long long)r0 * m.pitch + c0, m.pitch, m.frame_stride, r1 - r0, c1 - c0,
+                                         (T*)p->box_in + (long long)(r0 - p->box_y0) * p->box_pitch + (c0 - p->box_x0),
+                                         p->box_pitch, box_stride);
+    LAUNCH((int)cudaGetLastError());
+  }
+  return RPSF_OK;
+}
+
+// L_Mᵀ y = padᵀ(pad(M) g_ext + (1 - pad(M)) Fᵀ v), v = the patch path's transpose of (1 - M) y on the padded frame:
+// masked copy into the box, the three kernels with conj(Kh), the box onto the padded frame, the fill's structure from
+// the mask alone (ingest, raster list, counts), the transposed fill, the gather and combine, the fold over the padded frame
+template <typename T>
+int apply_adjoint_masked(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                         int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                         const MaskArg& m, cudaStream_t s) {
+  rpsf_transform* t = p->tr;
+  if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (!t->has_kernel) return fail(RPSF_E_NO_KERNEL, "transfer kernel not loaded (call rpsf_transform_set_kernel)");
+  if (batch < 1 || batch > p->max_batch)
+    return fail(RPSF_E_INVALID_ARGUMENT, "batch %d outside [1, max_batch=%d]", batch, p->max_batch);
+  if (img_row0 != 0 || img_rows != p->frame_H || out_row0 != 0)
+    return fail(RPSF_E_INVALID_ARGUMENT, "an adjoint plan takes and writes whole frames (row0 = 0, rows = %d)", p->frame_H);
+  if (img_pitch < p->frame_W || out_pitch < p->frame_W) return fail(RPSF_E_INCORRECT_SHAPE, "row pitch smaller than frame width");
+  DeviceGuard guard(t->device);
+  const int H = p->frame_H, W = p->frame_W;
+  const SatGeom sg = mask_geom(p, H, W, p->frame_pad_mode);
+  const size_t px = (size_t)sg.Hp * sg.Wp, mb = (size_t)p->max_batch;
+  if ((long long)px > 0x7fffffffLL) return fail(RPSF_E_UNSUPPORTED, "padded frame too large for the masked transpose");
+  if (p->box_y0 < -sg.pad || p->box_x0 < -sg.pad || p->box_y0 + p->H > H + sg.pad || p->box_x0 + p->W > W + sg.pad)
+    return fail(RPSF_E_UNSUPPORTED, "the patch footprints reach past the padded frame");
+  if (!p->mask_count) {
+    if (t_capturing) return refuse_capture("the first masked transpose of a plan (its scratch)");
+    CU(cudaMalloc(&p->sat_pf, px * sizeof(T) * mb));
+    CU(cudaMalloc(&p->mask_out, px * sizeof(T) * mb));
+    CU(cudaMalloc((void**)&p->sat_mask[0], px * mb));
+    CU(cudaMalloc((void**)&p->sat_list, px * sizeof(int) * mb));
+    CU(cudaMalloc((void**)&p->sat_rows, (size_t)(sg.Hp + 1) * sizeof(int) * mb));
+    CU(cudaMalloc((void**)&p->sat_flags, 2 * sizeof(int) * mb));
+    CU(cudaMalloc((void**)&p->mask_count, px * sizeof(int) * mb));
+  }
+  const long long box_stride = (long long)p->H * p->box_pitch;
+  if (int rc = adjoint_copy_masked<T>(p, image, img_pitch, img_frame_stride, m, batch, s)) return rc;
+  if (int rc = apply_stages(p, p->box_in, p->box_pitch, box_stride, 0, p->H, p->box_out, p->box_pitch, box_stride, 0,
+                            batch, 3, s))
+    return rc;
+  const dim3 rows_grid((unsigned)std::min((sg.Wp + 255) / 256, 8), (unsigned)sg.Hp, (unsigned)batch);
+  T* u = (T*)p->sat_pf;
+  unsigned char* state = p->sat_mask[0];
+  box_to_padded<T><<<rows_grid, 256, 0, s>>>((const T*)p->box_out, p->box_pitch, box_stride, p->box_y0, p->box_x0, p->H,
+                                             p->W, u, sg);
+  LAUNCH((int)cudaGetLastError());
+  CU(cudaMemsetAsync(state, 0, px * batch, s));
+  CU(cudaMemsetAsync(p->sat_flags, 0, 2 * sizeof(int) * mb, s));
+  launch_mask_ingest(m, state, sg, batch, s);
+  LAUNCH((int)cudaGetLastError());
+  if (int rc = mask_compact(p, state, sg, batch, s)) return rc;
+  const dim3 fill_grid((unsigned)t->sm_count * 2, (unsigned)batch);
+  sat_fill_count<<<fill_grid, 256, 0, s>>>(state, p->sat_list, p->sat_rows, p->sat_flags, p->mask_count, sg);
+  LAUNCH((int)cudaGetLastError());
+  sat_fill_adjoint<T><<<fill_grid, 256, 0, s>>>(u, state, p->sat_list, p->sat_rows, p->sat_flags + mb, p->mask_count, sg);
+  LAUNCH((int)cudaGetLastError());
+  mask_gather_adjoint<T><<<rows_grid, 256, 0, s>>>(u, state, (const T*)image, img_pitch, img_frame_stride,
+                                                   (T*)p->mask_out, sg);
+  LAUNCH((int)cudaGetLastError());
+  const dim3 grid((unsigned)((W + 255) / 256), (unsigned)std::min(H, 1024), (unsigned)batch);
+  fold_pad_adjoint<T><<<grid, 256, 0, s>>>((const T*)p->mask_out, sg.Wp, (long long)px, p->fold_prows,
+                                           p->fold_prows + H + 1, p->fold_pcols, p->fold_pcols + W + 1, (T*)out,
+                                           out_pitch, out_frame_stride, H, W);
+  LAUNCH((int)cudaGetLastError());
+  return RPSF_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1874,9 +2007,10 @@ int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
   });
 }
 
-int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch, int64_t img_frame_stride,
-                         const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch, void* kernel_grad,
-                         void* stream) {
+// `mask` (may be null): X is K1 of the frame filled under the caller's mask, G that of (1 - M) grad
+static int kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch, int64_t img_frame_stride,
+                           const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch, void* kernel_grad,
+                           void* stream, const MaskArg* mask) {
   if (!ap || !fp || !image || !grad || !kernel_grad) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (!ap->adjoint || fp->adjoint)
     return fail(RPSF_E_INVALID_ARGUMENT, "rpsf_kernel_gradient takes an adjoint plan, then a forward plan");
@@ -1917,14 +2051,20 @@ int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_
       CU(cudaEventRecord(ev[0], s));
     }
     // 1. X: K1 of the forward plan (stages = 1 writes nothing to `out`)
-    if (int rc = apply_stages(fp, image, img_pitch, img_frame_stride, 0, fp->H, kernel_grad, fp->W, 0, 0, batch, 1, s))
+    if (int rc = apply_stages(fp, image, img_pitch, img_frame_stride, 0, fp->H, kernel_grad, fp->W, 0, 0, batch, 1, s,
+                              nullptr, mask))
       return rc;
     if (ev) CU(cudaEventRecord(ev[1], s));
     // 2-3. G: the gradient into the adjoint plan's zero-bordered box, K1 there
     const long long box_stride = (long long)ap->H * ap->box_pitch;
-    if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy<float> : adjoint_copy<double>)(ap, grad, grad_pitch, grad_frame_stride,
-                                                                                       batch, s))
+    if (mask) {
+      if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy_masked<float> : adjoint_copy_masked<double>)(
+              ap, grad, grad_pitch, grad_frame_stride, *mask, batch, s))
+        return rc;
+    } else if (int rc = (t->dtype == RPSF_F32 ? adjoint_copy<float> : adjoint_copy<double>)(ap, grad, grad_pitch,
+                                                                                              grad_frame_stride, batch, s)) {
       return rc;
+    }
     if (int rc = apply_stages(ap, ap->box_in, ap->box_pitch, box_stride, 0, ap->H, ap->box_out, ap->box_pitch, box_stride, 0,
                               batch, 1, s))
       return rc;
@@ -1946,6 +2086,24 @@ int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_
     if (ev) CU(cudaEventRecord(ev[3], s));
     return RPSF_OK;
   });
+}
+
+int rpsf_kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch, int64_t img_frame_stride,
+                         const void* grad, int64_t grad_pitch, int64_t grad_frame_stride, int batch, void* kernel_grad,
+                         void* stream) {
+  return kernel_gradient(ap, fp, image, img_pitch, img_frame_stride, grad, grad_pitch, grad_frame_stride, batch, kernel_grad,
+                         stream, nullptr);
+}
+
+int rpsf_kernel_gradient_masked(rpsf_plan* ap, rpsf_plan* fp, const void* image, int64_t img_pitch,
+                                int64_t img_frame_stride, const void* grad, int64_t grad_pitch, int64_t grad_frame_stride,
+                                int batch, void* kernel_grad, const void* mask, int64_t mask_pitch,
+                                int64_t mask_frame_stride, void* stream) {
+  if (!mask) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (fp && mask_pitch < fp->W) return fail(RPSF_E_INCORRECT_SHAPE, "mask row pitch smaller than frame width");
+  const MaskArg m{(const unsigned char*)mask, mask_pitch, mask_frame_stride};
+  return kernel_gradient(ap, fp, image, img_pitch, img_frame_stride, grad, grad_pitch, grad_frame_stride, batch, kernel_grad,
+                         stream, &m);
 }
 
 int rpsf_plan_enable_timing(rpsf_plan* p, int enabled) {
@@ -1984,6 +2142,31 @@ int rpsf_apply(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_f
           (cudaStream_t)stream);
     return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch,
                              out_frame_stride, out_row0, batch, 3, stream);
+  });
+}
+
+int rpsf_apply_masked(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
+                      int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0, int batch,
+                      const void* src, int src_dtype, int64_t src_pitch, int64_t src_frame_stride, const void* mask,
+                      int64_t mask_pitch, int64_t mask_frame_stride, void* stream) {
+  if (!p || !mask) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  const int W = p->adjoint ? p->frame_W : p->W;
+  if (mask_pitch < W) return fail(RPSF_E_INCORRECT_SHAPE, "mask row pitch smaller than frame width");
+  if (p->pad_mode == PAD_NONE) return fail(RPSF_E_UNSUPPORTED, "a mask needs a pad mode with an index map (0..4)");
+  if (p->adjoint && src) return fail(RPSF_E_UNSUPPORTED, "an adjoint plan has no saturation branch (src)");
+  if (src && !elem_size(src_dtype)) return fail(RPSF_E_UNSUPPORTED, "unsupported source dtype code %d", src_dtype);
+  if (src && src_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "source row pitch smaller than frame width");
+  const MaskArg m{(const unsigned char*)mask, mask_pitch, mask_frame_stride};
+  const SatSource source{src, src_dtype, src_pitch, src_frame_stride};
+  return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
+    if (p->adjoint)
+      return (p->tr->dtype == RPSF_F32 ? apply_adjoint_masked<float> : apply_adjoint_masked<double>)(
+          p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride, out_row0, batch, m,
+          (cudaStream_t)stream);
+    if (img_row0 != 0 || img_rows < p->H)
+      return fail(RPSF_E_UNSUPPORTED, "a mask needs the whole frame resident (rows [0,%d))", p->H);
+    return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
+                        out_row0, batch, 3, stream, src ? &source : nullptr, &m);
   });
 }
 

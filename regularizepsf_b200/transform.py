@@ -470,7 +470,7 @@ class ArrayPSFTransform:
     # ------------------------------------------------------------------ apply
     def apply(self, image, workers: int | None = None, pad_mode: str = "symmetric",
               saturation_threshold: float = math.inf, saturation_dilation: int = 1,
-              neighborhood_width: int = 7, *, dtype=None, out_dtype=None):
+              neighborhood_width: int = 7, *, dtype=None, out_dtype=None, mask=None):
         """Apply the transform to an image (transform.py:85-177).
 
         ``image`` may be a numpy array (any real dtype; returns a fresh float64 numpy array exactly
@@ -489,8 +489,22 @@ class ArrayPSFTransform:
         laid-out kernel, the plans' workspaces and scratch — across streams, the private streams of a
         numpy call included.  A tensor call does not synchronise with the host, and once warmed up it can be
         captured in a CUDA graph (INTEGRATION.md, "CUDA graphs"); a numpy call synchronises and cannot.
+
+        ``mask``: a caller-given bad-pixel mask, boolean (or uint8 0/1) of shape (H, W), shared by every frame, or
+        (B, H, W): a numpy array with numpy input, a CUDA tensor on the image's device with tensor input.  A pixel marked
+        True is treated exactly like a saturated pixel after dilation: the image and the mask are padded alike (with
+        "constant" the margin is unmasked), the padded mask is ORed into the dilated saturation mask (it alone with an
+        infinite threshold), the masked pixels are filled in raster order with the nanmean of their neighbourhood, and
+        they get their raw values back after the correction.  So a NaN or a defect under the mask stays at its own pixel
+        instead of poisoning every patch that holds it.  With an infinite threshold the map is linear in the image and
+        differentiable (``apply_adjoint(mask=)``, ``transfer_kernel_gradient(mask=)``).  A numpy image with a mask is
+        uploaded and corrected on the device path and returned as float64 (or ``out_dtype``).  Pad modes without an
+        index map and sharded transforms raise NotImplementedError (DESIGN.md section 6).
         """
         del workers
+        if mask is not None:
+            return self._apply_masked(image, pad_mode, saturation_threshold, saturation_dilation, neighborhood_width,
+                                      mask, dtype, out_dtype)
         kt = self._kernel_tensor
         if (_is_torch_tensor(image) and (image.requires_grad or (kt is not None and kt.requires_grad))
                 and _native.require_cuda().is_grad_enabled()):
@@ -520,7 +534,7 @@ class ArrayPSFTransform:
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {image.shape}")
         return self._apply_host(image, dtype_name, _native.PAD_MODES[pad_mode], out_dtype=out_np.type, sat=sat)
 
-    def apply_adjoint(self, image, pad_mode: str = "symmetric", *, dtype=None):
+    def apply_adjoint(self, image, pad_mode: str = "symmetric", *, dtype=None, mask=None, neighborhood_width: int = 7):
         """The transpose of ``apply`` without saturation, a linear map of the image: ``<apply(x), y> = <x,
         apply_adjoint(y)>``.  For forward modelling and iterative solvers (Landweber, CG on the normal equations), and
         the backward of ``apply`` under autograd.
@@ -530,15 +544,23 @@ class ArrayPSFTransform:
         modes with an index map ("symmetric", "reflect", "edge", "wrap", "constant").  A tensor that requires grad
         gives a differentiable result whose backward is ``apply``; so does a transform whose kernel tensor
         (``DeviceCube``) requires grad, whose kernel gradient is ``transfer_kernel_gradient`` with the roles swapped.
+
+        ``mask`` (as in ``apply``) with ``neighborhood_width``: the transpose of ``apply(x, mask=mask,
+        neighborhood_width=neighborhood_width)`` with an infinite threshold, in which the pixels that contribute to a
+        fill are decided by the mask alone (as if the image were finite outside it).
         """
         if pad_mode not in _native.PAD_MODES:
             raise NotImplementedError(f"apply_adjoint supports the pad modes {sorted(_native.PAD_MODES)}, got {pad_mode!r}")
         if self._shard_keep is not None:
             raise NotImplementedError("apply_adjoint needs the kernels of every patch; a sharded transform holds a subset")
+        sat = (math.inf, 1, int(neighborhood_width))
         if _is_torch_tensor(image):
             if ((image.requires_grad or self._trainable_kernel() is not None)
                     and _native.require_cuda().is_grad_enabled()):
-                return self._apply_differentiable(image, pad_mode, math.inf, dtype, adjoint=True)
+                return self._apply_differentiable(image, pad_mode, math.inf, dtype, adjoint=True, mask=mask, width=sat[2])
+            if mask is not None:
+                return self._apply_device(image, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True,
+                                          sat=sat, mask=mask)
             return self._apply_device(image, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
         torch = _native.require_cuda()
         _native.refuse_in_capture(torch, "apply_adjoint() of a numpy array (a host-to-host call)")
@@ -546,12 +568,48 @@ class ArrayPSFTransform:
         if host.ndim not in (2, 3):
             raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {host.shape}")
         dev = torch.from_numpy(np.ascontiguousarray(host, dtype=np.float64)).to(f"cuda:{torch.cuda.current_device()}")
+        if mask is not None:
+            out = self._apply_device(dev, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True, sat=sat,
+                                     mask=_upload_mask(torch, mask, host.shape, dev.device))
+            return out.cpu().numpy().astype(np.float64, copy=False)
         out = self._apply_device(dev, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint=True)
         return out.cpu().numpy().astype(np.float64, copy=False)
 
-    def _apply_differentiable(self, image, pad_mode: str, saturation_threshold: float, dtype, adjoint: bool):
+    def _apply_masked(self, image, pad_mode: str, threshold, dilation, width, mask, dtype, out_dtype):
+        """``apply(mask=...)``: the saturation branch with the caller's mask ORed into its own, on the device path."""
+        if pad_mode not in _native.PAD_MODES:
+            raise NotImplementedError(f"a mask needs one of the pad modes {sorted(_native.PAD_MODES)}; {pad_mode!r} is "
+                                      "computed by np.pad on the host")
+        if self._shard_keep is not None:
+            raise NotImplementedError("a mask needs the whole frame: a sharded transform holds a subset of the patches")
+        torch = _native.require_cuda()
+        threshold = float(threshold)
+        if math.isnan(threshold):
+            threshold = math.inf                           # `padded > nan` is all False in the reference
+        sat = (threshold, int(dilation), int(width))
+        dtype_name = _normalize_dtype(dtype)
+        pad_code = _native.PAD_MODES[pad_mode]
+        if _is_torch_tensor(image):
+            kt = self._kernel_tensor
+            if (image.requires_grad or (kt is not None and kt.requires_grad)) and torch.is_grad_enabled():
+                return self._apply_differentiable(image, pad_mode, threshold, dtype, adjoint=False, mask=mask, width=sat[2])
+            return self._apply_device(image, dtype_name, pad_code, sat=sat, mask=mask)
+        _native.refuse_in_capture(torch, "apply() of a numpy array (a host-to-host call)")
+        out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
+        if out_np not in (np.dtype(np.float32), np.dtype(np.float64)):
+            raise NotImplementedError(f"out_dtype must be float32 or float64, got {out_np}")
+        host = np.asarray(image)
+        if host.ndim not in (2, 3):
+            raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {host.shape}")
+        dev = torch.from_numpy(np.ascontiguousarray(host, dtype=np.float64)).to(f"cuda:{torch.cuda.current_device()}")
+        out = self._apply_device(dev, dtype_name, pad_code, sat=sat, mask=_upload_mask(torch, mask, host.shape, dev.device))
+        return out.cpu().numpy().astype(out_np.type, copy=False)
+
+    def _apply_differentiable(self, image, pad_mode: str, saturation_threshold: float, dtype, adjoint: bool, mask=None,
+                              width: int = 7):
         """``apply`` / ``apply_adjoint`` of a CUDA tensor that requires grad, or with a kernel tensor that does: a linear
-        map whose backward is the other, and, for the kernel, ``transfer_kernel_gradient``."""
+        map whose backward is the other, and, for the kernel, ``transfer_kernel_gradient`` (``mask`` and the
+        neighbourhood ``width`` carried along)."""
         if not (saturation_threshold == math.inf or math.isnan(saturation_threshold)):
             raise NotImplementedError("apply is not differentiable with a finite saturation_threshold: the mask and "
                                       "the restored pixels depend on the image")
@@ -563,13 +621,15 @@ class ArrayPSFTransform:
         kernel = self._trainable_kernel()
         if kernel is None:
             from regularizepsf_b200._autograd import LinearMap
-            return LinearMap.apply(image, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
+            return LinearMap.apply(image, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint, mask,
+                                   width)
         self._check_kernel_gradient(pad_mode)
         for nt in self._native.values():
             if nt.kernel_source is None:       # requires_grad was switched on after the layout: track it from now on
                 nt.kernel_source, nt.kernel_version = kernel, None
         from regularizepsf_b200._autograd import KernelMap
-        return KernelMap.apply(image, kernel, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint)
+        return KernelMap.apply(image, kernel, self, _normalize_dtype(dtype), _native.PAD_MODES[pad_mode], adjoint, mask,
+                               width)
 
     def _check_kernel_gradient(self, pad_mode: str) -> None:
         """NotImplementedError for what ``transfer_kernel_gradient`` has no device path for (DESIGN.md section 6)."""
@@ -582,7 +642,8 @@ class ArrayPSFTransform:
             raise NotImplementedError(f"the kernel gradient is implemented for the patch sizes {_NATIVE_SIZES}; "
                                       f"{self.psf_shape[0]} runs embedded in a larger FFT")
 
-    def transfer_kernel_gradient(self, image, grad_output, pad_mode: str = "symmetric", *, dtype=None):
+    def transfer_kernel_gradient(self, image, grad_output, pad_mode: str = "symmetric", *, dtype=None, mask=None,
+                                 neighborhood_width: int = 7):
         """The gradient of ``<apply(image), grad_output>`` with respect to the transfer kernel, without saturation: the
         vector-Jacobian product of ``apply`` in the kernel, for fitting a kernel to calibration pairs.  For patch p,
         ``conj(X_p) * G_p / P**2`` summed over the frames, with ``X_p`` and ``G_p`` the FFT2 of the apodized patch of
@@ -593,6 +654,10 @@ class ArrayPSFTransform:
         (N, P, P) complex128 array, computed on the device) or CUDA tensors (returns complex64 for the compute dtype
         "float32", the default, complex128 for "float64").  ``pad_mode`` is one of the five modes with an index map.
         Embedded patch sizes (not a power of two) and sharded transforms raise NotImplementedError.
+
+        ``mask`` (as in ``apply``) with ``neighborhood_width``: the gradient of ``<apply(image, mask=mask), grad_output>``
+        with an infinite threshold; ``X_p`` is then taken from the padded image filled under the mask, and ``G_p`` from
+        ``grad_output`` with the masked pixels set to 0.
         """
         self._check_kernel_gradient(pad_mode)
         dtype_name = _normalize_dtype(dtype)
@@ -600,7 +665,8 @@ class ArrayPSFTransform:
         if _is_torch_tensor(image) or _is_torch_tensor(grad_output):
             if not (_is_torch_tensor(image) and _is_torch_tensor(grad_output)):
                 raise TypeError("image and grad_output must both be numpy arrays or both CUDA tensors")
-            return self._kernel_gradient_device(image.detach(), grad_output.detach(), dtype_name, pad_code)
+            return self._kernel_gradient_device(image.detach(), grad_output.detach(), dtype_name, pad_code, mask=mask,
+                                                width=int(neighborhood_width))
         torch = _native.require_cuda()
         _native.refuse_in_capture(torch, "transfer_kernel_gradient() of numpy arrays (a host-to-host call)")
         x, g = np.asarray(image), np.asarray(grad_output)
@@ -610,10 +676,12 @@ class ArrayPSFTransform:
         device = f"cuda:{torch.cuda.current_device()}"
         xt = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64)).to(device)
         gt = torch.from_numpy(np.ascontiguousarray(g, dtype=np.float64)).to(device)
-        out = self._kernel_gradient_device(xt, gt, dtype_name, pad_code)
+        if mask is not None:
+            mask = _upload_mask(torch, mask, x.shape, xt.device)
+        out = self._kernel_gradient_device(xt, gt, dtype_name, pad_code, mask=mask, width=int(neighborhood_width))
         return out.cpu().numpy().astype(np.complex128, copy=False)
 
-    def _kernel_gradient_device(self, image, grad, dtype_name: str, pad_code: int = 0):
+    def _kernel_gradient_device(self, image, grad, dtype_name: str, pad_code: int = 0, mask=None, width: int = 7):
         """``transfer_kernel_gradient`` of two CUDA tensors (no autograd history): the (N, P, P) complex tensor."""
         torch = _native.require_cuda()
         if not (image.is_cuda and grad.is_cuda) or image.device != grad.device:
@@ -622,6 +690,8 @@ class ArrayPSFTransform:
             raise IncorrectShapeError(f"image and grad_output must share a shape (H, W) or (B, H, W), got "
                                       f"{tuple(image.shape)} and {tuple(grad.shape)}")
         want = torch.float32 if dtype_name == "float32" else torch.float64
+        if mask is not None:
+            mask, mask_pitch, mask_stride = _mask_view(torch, mask, tuple(image.shape), image.device)
         with torch.cuda.device(image.device):
             capturing = _native.capturing(torch)
             nt = self._native_transform(dtype_name, image.device.index, capturing, reads_kernel=False)
@@ -631,10 +701,16 @@ class ArrayPSFTransform:
             b, h, w = x.shape
             forward = nt.plan(h, w, pad_code, 0, h, b, capturing=capturing)
             adjoint = nt.plan(h, w, pad_code, 0, h, b, adjoint=True, capturing=capturing)
-            nt.set_saturation(forward, self._NO_SAT)
+            nt.set_saturation(forward, self._NO_SAT if mask is None else (math.inf, 1, width))
             p = self.psf_shape[0]
             out = torch.empty((len(self), p, p), dtype=torch.complex64 if dtype_name == "float32" else torch.complex128,
                               device=x.device)
+            if mask is not None:
+                _native.check(nt.lib.rpsf_kernel_gradient_masked(
+                    adjoint, forward, x.data_ptr(), x.stride(1), x.stride(0) if b > 1 else h * x.stride(1),
+                    g.data_ptr(), g.stride(1), g.stride(0) if b > 1 else h * g.stride(1), b, out.data_ptr(),
+                    mask.data_ptr(), mask_pitch, mask_stride, _native.current_stream_ptr(torch, x.device.index)))
+                return out
             _native.check(nt.lib.rpsf_kernel_gradient(
                 adjoint, forward, x.data_ptr(), x.stride(1), x.stride(0) if b > 1 else h * x.stride(1),
                 g.data_ptr(), g.stride(1), g.stride(0) if b > 1 else h * g.stride(1), b, out.data_ptr(),
@@ -700,24 +776,29 @@ class ArrayPSFTransform:
 
     def _apply_device(self, image, dtype_name: str, pad_code: int, row_range: tuple[int, int] | None = None,
                       out=None, sat: tuple = _NO_SAT, mirrors: list[int] | None = None,
-                      frame_rows: tuple[int, int] | None = None, adjoint: bool = False, source=None):
+                      frame_rows: tuple[int, int] | None = None, adjoint: bool = False, source=None, mask=None):
         """``frame_rows = (first, height)``: ``image`` holds only rows [first, first + image.shape[-2]) of frames that
         are ``height`` rows tall (a row slab keeps just the rows its patches read: ``plan_info()["rows_read"]``).
         ``adjoint``: run the transpose (whole frames, no saturation).  ``source``: the frames of ``image`` before a
         conversion to the compute dtype, laid out alike, on which the saturation mask is decided (by default
-        ``image`` itself, before this call converts it)."""
+        ``image`` itself, before this call converts it).  ``mask``: the caller's bad-pixel mask (``apply(mask=)``), a CUDA
+        tensor; with ``adjoint`` the transpose of the masked map."""
         torch = _native.require_cuda()
         if not image.is_cuda:
             raise ValueError("apply() takes a numpy array or a CUDA tensor; move the tensor to the GPU first")
         if image.device.index == torch._C._cuda_getDevice():
             return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
-                                         adjoint, source)
+                                         adjoint, source, mask)
         with torch.cuda.device(image.device):             # plans, streams and launches follow the image's device
             return self._apply_device_on(torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows,
-                                         adjoint, source)
+                                         adjoint, source, mask)
 
     def _apply_device_on(self, torch, image, dtype_name, pad_code, row_range, out, sat, mirrors, frame_rows=None,
-                         adjoint=False, source=None):
+                         adjoint=False, source=None, mask=None):
+        if mask is not None:
+            if image.dim() not in (2, 3):
+                raise IncorrectShapeError(f"image must be (H, W) or (B, H, W), got shape {tuple(image.shape)}")
+            mask, mask_pitch, mask_stride = _mask_view(torch, mask, tuple(image.shape), image.device)
         capturing = _native.capturing(torch)
         nt = self._native_transform(dtype_name, image.device.index, capturing)
         want = torch.float32 if dtype_name == "float32" else torch.float64
@@ -763,7 +844,11 @@ class ArrayPSFTransform:
                     first, held, out.data_ptr(), out.stride(1), out.stride(0) if b > 1 else (r1 - r0) * out.stride(1),
                     r0, b)
             stream = _native.current_stream_ptr(torch, frames.device.index)
-            if src_code is None:
+            if mask is not None:
+                src_args = (None, 0, 0, 0) if src_code is None else (
+                    source.data_ptr(), src_code, source.stride(1), source.stride(0) if b > 1 else held * source.stride(1))
+                rc = nt.lib.rpsf_apply_masked(*args, *src_args, mask.data_ptr(), mask_pitch, mask_stride, stream)
+            elif src_code is None:
                 rc = nt.lib.rpsf_apply(*args, stream)
             else:
                 rc = nt.lib.rpsf_apply_source(*args, source.data_ptr(), src_code, source.stride(1),
@@ -780,6 +865,39 @@ class ArrayPSFTransform:
 _TORCH_CODES = {"torch.float32": _native.F32, "torch.float64": _native.F64, "torch.uint8": _native.U8,
                 "torch.int16": _native.I16, "torch.uint16": _native.U16, "torch.int32": _native.I32,
                 "torch.int64": _native.I64, "torch.uint32": _native.U32}
+
+
+def _mask_view(torch, mask, image_shape: tuple, device):
+    """The caller's mask for an image of ``image_shape`` on CUDA ``device``: a uint8 tensor with unit column stride (a
+    view of a bool or uint8 tensor when it has one), its row pitch, and its frame stride (0: one mask for every frame).
+    IncorrectShapeError for a shape other than (H, W) or the image's (B, H, W), ValueError for a mask that is not a
+    CUDA tensor on ``device``, TypeError for a dtype other than bool or uint8."""
+    if not _is_torch_tensor(mask) or mask.device != device:
+        where = mask.device if _is_torch_tensor(mask) else type(mask).__name__
+        raise ValueError(f"with a CUDA tensor image, mask must be a CUDA tensor on {device}, got {where}")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise TypeError(f"mask must be bool or uint8, got {mask.dtype}")
+    shape = tuple(mask.shape)
+    if shape != tuple(image_shape[-2:]) and not (len(image_shape) == 3 and shape == tuple(image_shape)):
+        raise IncorrectShapeError(f"mask must be (H, W) or the image's (B, H, W) for an image of shape "
+                                  f"{tuple(image_shape)}, got {shape}")
+    view = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+    if view.stride(-1) != 1:
+        view = view.contiguous()
+    return view, view.stride(-2), (view.stride(0) if view.dim() == 3 and view.shape[0] > 1 else 0)
+
+
+def _upload_mask(torch, mask, image_shape: tuple, device):
+    """A numpy mask for a numpy image of ``image_shape``, checked and copied to ``device`` (a tensor: ValueError)."""
+    if _is_torch_tensor(mask):
+        raise ValueError("with a numpy image, mask must be a numpy array, got a tensor")
+    host = np.asarray(mask)
+    if host.dtype not in (np.dtype(np.bool_), np.dtype(np.uint8)):
+        raise TypeError(f"mask must be bool or uint8, got {host.dtype}")
+    if host.shape != tuple(image_shape[-2:]) and not (len(image_shape) == 3 and host.shape == tuple(image_shape)):
+        raise IncorrectShapeError(f"mask must be (H, W) or the image's (B, H, W) for an image of shape "
+                                  f"{tuple(image_shape)}, got {host.shape}")
+    return torch.from_numpy(np.ascontiguousarray(host).view(np.uint8)).to(device)
 
 
 def _spectrum_source(psf):
