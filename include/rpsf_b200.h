@@ -241,7 +241,8 @@ int rpsf_kernel_gradient_masked(rpsf_plan* adjoint_plan, rpsf_plan* forward_plan
                                 int batch, void* kernel_grad, const void* mask, int64_t mask_pitch,
                                 int64_t mask_frame_stride, void* stream);
 int rpsf_plan_destroy(rpsf_plan* p);
-/* info[0]=active patches, [1]=colours, [2]=workspace bytes, [3]=first frame row read,
+/* info[0]=active patches, [1]=colours, [2]=workspace bytes (patch spectra and row bands, see rpsf_plan_workspace),
+ * [3]=first frame row read,
  * [4]=one past the last frame row read, [5]=1 if colour 0 tiles the band exactly,
  * [6]=overlap-add kernel: 2 = streaming chains (registers only), 1 = single-launch row-pair gather
  *      through a shared-memory plane, 0 = one launch per colour class,
@@ -257,7 +258,7 @@ int rpsf_plan_set_overlap_mode(rpsf_plan* p, int mode);
  * one-row-pair-per-team kernel with direct loads (test hook; same arithmetic up to rounding) */
 int rpsf_plan_set_gather_mode(rpsf_plan* p, int mode);
 
-/* column pass: info[0] = 0 (the in-place column pass over the spectrum workspace, the only one there is) and
+/* column pass: info[0] = 0 (the column pass from the row bands into the spectrum workspace, the only one there is) and
  * info[1] = 0 (bytes per frame of a column-pass workspace of its own: none).  Kept so that callers that report
  * the column pass keep working. */
 int rpsf_plan_column_info(const rpsf_plan* p, int64_t info[2]);
@@ -314,7 +315,11 @@ int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out,
 /* 2-D dtype conversion on the device (the `.astype(float)` of transform.py:117) */
 int rpsf_convert(const void* src, int src_dtype, int64_t src_pitch, void* dst, int dst_dtype, int64_t dst_pitch,
                  int rows, int cols, int device, void* stream);
-/* stage outputs for tests: copy the plan's spectrum workspace pointer / size */
+/* stage outputs for tests: the plan's workspace pointer / size.  It holds the patch spectra
+ * [max_batch][active patch][P][P/2] complex at offset 0, then the row bands: the row pass transforms each frame row
+ * once per corner column (and corner-row parity) and stores it there without the row window, and the column pass
+ * applies the window as it reads a patch's rows.  After rpsf_apply_stages(..., 2) the first bytes are the patch
+ * spectra exactly as with a spectrum of its own per patch; after stages = 1 the patch part holds nothing defined. */
 int rpsf_plan_workspace(const rpsf_plan* p, void** ptr, int64_t* bytes);
 /* run only the first `stages` kernels of apply (1 = K1, 2 = K1+K2, 3 = all); test hook */
 int rpsf_apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,

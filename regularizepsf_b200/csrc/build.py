@@ -21,7 +21,7 @@ LIB = os.path.join(PKG, "librpsf_b200.so")
 SIZES = (16, 32, 64, 128, 256, 512)
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-std=c++17", "-O3", "-lineinfo", "-Xcompiler", "-fPIC"] + ARCH
-HEADERS = ["rpsf_fft.cuh", "rpsf_kernels.cuh", "rpsf_saturation.cuh", "rpsf_stream.cuh", "rpsf_builder.cuh", "rpsf_adjoint.cuh", "rpsf_kgrad.cuh", "rpsf_construct_grad.cuh", "rpsf_ops.h", os.path.join("..", "..", "include", "rpsf_b200.h")]
+HEADERS = ["rpsf_fft.cuh", "rpsf_bands.cuh", "rpsf_kernels.cuh", "rpsf_saturation.cuh", "rpsf_stream.cuh", "rpsf_builder.cuh", "rpsf_adjoint.cuh", "rpsf_kgrad.cuh", "rpsf_construct_grad.cuh", "rpsf_ops.h", os.path.join("..", "..", "include", "rpsf_b200.h")]
 
 
 def _nvcc() -> str:

@@ -517,8 +517,14 @@ struct rpsf_plan {
   // rpsf_plan_set_gather_mode let tests pick the others)
   K1Kernel k1 = K1Kernel::bulk;
   Overlap overlap = Overlap::phases;
-  void* workspace = nullptr;       // allocated at the first apply
-  size_t workspace_bytes = 0;
+  // workspace, allocated at the first apply: the spectrum of every active patch ([frame][active][P][P/2], what the
+  // column pass writes and the overlap-add reads) at offset 0, then the band buffer the row pass writes
+  // (rpsf_bands.cuh) at band_offset
+  void* workspace = nullptr;
+  size_t workspace_bytes = 0, band_offset = 0;
+  BandItem* band_items_dev = nullptr;
+  int* patch_row_dev = nullptr;
+  int n_band_items = 0, band_frame_rows = 0;
   int img_lo = 0, img_hi = 0;      // resident frame rows needed: [img_lo, img_hi)
   // host path: a ring of HOST_SLOTS chunk buffers so the upload of chunk i+1, the kernels of
   // chunk i and the download of chunk i-1 run concurrently on three streams (two copy engines)
@@ -1397,9 +1403,21 @@ int plan_build(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, i
       p->stream_ok = true;
     }
   }
+  // ---- row bands: each frame row is transformed once per band and shared by the band's patches
+  if (p->n_active > 0) {
+    const BandLayout bl = build_row_bands(corners, t->win_len, 2 * t->ops->stream_tpw());
+    p->n_band_items = (int)bl.items.size();
+    p->band_frame_rows = bl.frame_rows;
+    if (cudaMalloc(&p->band_items_dev, sizeof(BandItem) * bl.items.size()) != cudaSuccess) return destroy_fail("band items");
+    if (cudaMemcpy(p->band_items_dev, bl.items.data(), sizeof(BandItem) * bl.items.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
+    if (cudaMalloc(&p->patch_row_dev, sizeof(int) * bl.patch_row.size()) != cudaSuccess) return destroy_fail("band rows of the patches");
+    if (cudaMemcpy(p->patch_row_dev, bl.patch_row.data(), sizeof(int) * bl.patch_row.size(), cudaMemcpyHostToDevice) != cudaSuccess) return upload_fail();
+  }
   p->k1 = embedded ? K1Kernel::plain : K1Kernel::bulk;       // the plain K1 honours ApplyGeom::win_len
   p->overlap = default_overlap(p);
-  p->workspace_bytes = (size_t)max_batch * p->n_active * P * (P / 2) * 2 * real_size(t->dtype);
+  const size_t cs = 2 * real_size(t->dtype);
+  p->band_offset = (size_t)max_batch * p->n_active * P * (P / 2) * cs;
+  p->workspace_bytes = p->band_offset + (size_t)max_batch * p->band_frame_rows * (P / 2) * cs;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { rpsf_plan_destroy(p); return fail(RPSF_E_CUDA, "plan upload failed: %s", cudaGetErrorString(e)); }
   *out = p;
@@ -1511,6 +1529,7 @@ int rpsf_plan_destroy(rpsf_plan* p) {
     if (p->h_stage[i]) cudaFreeHost(p->h_stage[i]);
   }
   cudaFree(p->active_dev); cudaFree(p->corners_dev); cudaFree(p->workspace);
+  cudaFree(p->band_items_dev); cudaFree(p->patch_row_dev);
   cudaFree(p->tiles_dev); cudaFree(p->groups_dev); cudaFree(p->gitems_dev);
   cudaFree(p->stasks_dev); cudaFree(p->scodes_dev);
   cudaFree(p->sat_pf); cudaFree(p->sat_mask[0]); cudaFree(p->sat_mask[1]); cudaFree(p->sat_list);
@@ -1547,6 +1566,11 @@ int rpsf_plan_info(const rpsf_plan* p, int64_t info[9]) {
   info[8] = p->overlap == Overlap::stream ? p->stream_chunks : 0;
   return RPSF_OK;
 }
+
+static RowBands row_bands(const rpsf_plan* p) {
+  return RowBands{p->band_items_dev, p->patch_row_dev, p->n_band_items, p->band_frame_rows};
+}
+static void* band_buffer(const rpsf_plan* p) { return (char*)p->workspace + p->band_offset; }
 
 static int ensure_workspace(rpsf_plan* p) {
   if (p->workspace || p->workspace_bytes == 0) return RPSF_OK;
@@ -1816,20 +1840,21 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
   };
   if (p->n_active == 0) return restore();
   if (int rc = ensure_workspace(p)) return rc;
-  if (p->k1 == K1Kernel::bulk && (long long)batch * p->n_active * (t->P / 2) < (1LL << 30)) {
-    // bulk (1-D TMA) row copies need 16-byte aligned rows; the kernel still checks each patch's column offset
+  const RowBands rb = row_bands(p);
+  // the streaming K1 packs a band-buffer row index and a 2-bit kind into 32 bits
+  if (p->k1 == K1Kernel::bulk && (long long)batch * p->band_frame_rows < (1LL << 30)) {
+    // bulk (1-D TMA) row copies need 16-byte aligned rows; the kernel still checks each band's column offset
     const size_t rsz = real_size(t->dtype);
     const int bulk_ok = ((reinterpret_cast<uintptr_t>(k1_image) & 15) == 0 && ((size_t)g1.img_pitch * rsz) % 16 == 0 &&
                          ((size_t)g1.img_frame_stride * rsz) % 16 == 0) ? 1 : 0;
-    LAUNCH(t->ops->k1s(t->dtype, k1_image, p->workspace, p->corners_dev, t->tw, t->win, g1, batch, bulk_ok,
-                       t->sm_count, s));
+    LAUNCH(t->ops->k1s(t->dtype, k1_image, band_buffer(p), rb, t->tw, t->win, g1, batch, bulk_ok, t->sm_count, s));
   } else {
-    LAUNCH(t->ops->k1(t->dtype, k1_image, p->workspace, p->corners_dev, t->tw, t->win, g1, batch, s));
+    LAUNCH(t->ops->k1(t->dtype, k1_image, band_buffer(p), rb, t->tw, t->win, g1, batch, s));
   }
   if (ev) CU(cudaEventRecord(ev[1], s));
   if (stages < 2) return RPSF_OK;
-  LAUNCH(t->ops->k2(t->dtype, p->workspace, p->adjoint ? t->kconj_main : t->kmain, p->adjoint ? t->kconj_nyq : t->knyq,
-                    p->active_dev, t->tw, g, batch, t->sm_count, s));
+  LAUNCH(t->ops->k2(t->dtype, band_buffer(p), rb, p->workspace, p->adjoint ? t->kconj_main : t->kmain,
+                    p->adjoint ? t->kconj_nyq : t->knyq, p->active_dev, t->tw, t->win, g, batch, t->sm_count, s));
   if (ev) CU(cudaEventRecord(ev[2], s));
   if (stages < 3) return RPSF_OK;
   if (!p->mirrors.empty() && (!use_stream || sat))
@@ -2082,7 +2107,8 @@ static int kernel_gradient(rpsf_plan* ap, rpsf_plan* fp, const void* image, int6
     }
     // 5. conj(X) G / P^2, summed over the batch
     if (fp->n_active > 0)
-      LAUNCH(t->ops->kgrad(t->dtype, fp->workspace, ap->workspace, kernel_grad, fp->active_dev, t->tw, fp->n_active, batch, s));
+      LAUNCH(t->ops->kgrad(t->dtype, band_buffer(fp), row_bands(fp), band_buffer(ap), row_bands(ap), kernel_grad,
+                           fp->active_dev, t->tw, t->win, fp->n_active, batch, s));
     if (ev) CU(cudaEventRecord(ev[3], s));
     return RPSF_OK;
   });

@@ -55,6 +55,11 @@ template <typename C> __device__ __forceinline__ C cmulc(C a, C b) {
 }
 // a * s for a real scalar s
 template <typename C, typename T> __device__ __forceinline__ C cscale(C a, T s) { C b; b.x = s; b.y = s; return pmul(a, b); }
+// a * s rounded on its own, never contracted with the add that consumes it (the row window the readers of the band
+// buffer apply must round exactly as the product stored by the row pass once did).  Scalar __fmul_rn: ptxas was seen
+// to fuse the packed __fmul2_rn into the FFMA2 of the first butterfly.
+__device__ __forceinline__ float2 cscale_rn(float2 a, float s) { return make_float2(__fmul_rn(a.x, s), __fmul_rn(a.y, s)); }
+__device__ __forceinline__ double2 cscale_rn(double2 a, double s) { return make_double2(__dmul_rn(a.x, s), __dmul_rn(a.y, s)); }
 
 // ---- compile-time twiddles: cos(2*pi*m/64), m = 0..16, correctly rounded doubles ----------
 __host__ __device__ constexpr double cos64_table(int m) {

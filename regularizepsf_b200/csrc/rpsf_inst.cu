@@ -19,8 +19,10 @@ template <typename T> constexpr size_t row_smem() {
 template <typename T> constexpr size_t col_smem() {
   return sizeof(cplx<T>) * P + sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
 }
+// the column pass keeps the row window (P reals) beside the twiddles
+template <typename T> constexpr size_t col_k2_smem() { return col_smem<T>() + sizeof(T) * P; }
 template <typename T> constexpr size_t col_pipe_smem() {
-  return sizeof(cplx<T>) * P + K2_STAGES * sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
+  return sizeof(cplx<T>) * P + sizeof(T) * P + K2_STAGES * sizeof(cplx<T>) * size_t(TL::SLOTS) * P * TL::C;
 }
 // the pipelined column kernel needs K2_STAGES tile stages per CTA; use it while a stage is at most
 // 32 KB (two or three CTAs then fit an SM)
@@ -68,10 +70,10 @@ int init() {
   if ((e = set_smem(k3_stream<P, double, false>, Stream<P, double>::SMEM))) return e;
   if ((e = set_smem(k3_stream<P, float, true>, Stream<P, float>::SMEM))) return e;
   if ((e = set_smem(k3_stream<P, double, true>, Stream<P, double>::SMEM))) return e;
-  if ((e = set_smem(k2_colfft_mul_colifft<P, float>, col_smem<float>()))) return e;
-  if ((e = set_smem(k2_colfft_mul_colifft<P, double>, col_smem<double>()))) return e;
-  if ((e = set_smem(k2_colfft_mul_colifft<P, float, true>, col_smem<float>()))) return e;
-  if ((e = set_smem(k2_colfft_mul_colifft<P, double, true>, col_smem<double>()))) return e;
+  if ((e = set_smem(k2_colfft_mul_colifft<P, float>, col_k2_smem<float>()))) return e;
+  if ((e = set_smem(k2_colfft_mul_colifft<P, double>, col_k2_smem<double>()))) return e;
+  if ((e = set_smem(k2_colfft_mul_colifft<P, float, true>, col_k2_smem<float>()))) return e;
+  if ((e = set_smem(k2_colfft_mul_colifft<P, double, true>, col_k2_smem<double>()))) return e;
   if constexpr (use_col_pipe<float>())
     if ((e = set_smem(k2_pipelined<P, float, 1, true>, col_pipe_smem<float>()))) return e;
   if constexpr (use_col_pipe<double>())
@@ -104,53 +106,57 @@ int init() {
 inline unsigned cdiv(long long a, long long b) { return (unsigned)((a + b - 1) / b); }
 
 template <typename T>
-int k1_t(const void* image, void* spec, const int2* corners, const void* tw, const void* win,
-         const ApplyGeom& g, int batch, cudaStream_t s) {
-  dim3 grid(cdiv((long long)g.n_active * TL::HALF, TL::TEAMS), batch);
+int k1_t(const void* image, void* bands, const RowBands& rb, const void* tw, const void* win, const ApplyGeom& g, int batch,
+         cudaStream_t s) {
+  if (rb.n_items == 0) return 0;
+  dim3 grid(cdiv((long long)rb.n_items * (band_quantum<P>() / 2), TL::TEAMS), batch);
   k1_gather_window_rowfft<P, T><<<grid, TL::ROW_THREADS, row_smem<T>(), s>>>(
-      (const T*)image, (cplx<T>*)spec, corners, (const cplx<T>*)tw, (const T*)win, g);
+      (const T*)image, (cplx<T>*)bands, rb, (const cplx<T>*)tw, (const T*)win, g);
   return (int)cudaGetLastError();
 }
-int k1(int dt, const void* image, void* spec, const int2* corners, const void* tw, const void* win,
-       const ApplyGeom& g, int batch, cudaStream_t s) {
-  return dt == DT_F32 ? k1_t<float>(image, spec, corners, tw, win, g, batch, s)
-                      : k1_t<double>(image, spec, corners, tw, win, g, batch, s);
+int k1(int dt, const void* image, void* bands, const RowBands& rb, const void* tw, const void* win, const ApplyGeom& g,
+       int batch, cudaStream_t s) {
+  return dt == DT_F32 ? k1_t<float>(image, bands, rb, tw, win, g, batch, s)
+                      : k1_t<double>(image, bands, rb, tw, win, g, batch, s);
 }
 
 template <typename T>
-int k1s_t(const void* image, void* spec, const int2* corners, const void* tw, const void* win,
-          const ApplyGeom& g, int batch, int bulk_ok, int sm_count, cudaStream_t s) {
+int k1s_t(const void* image, void* bands, const RowBands& rb, const void* tw, const void* win, const ApplyGeom& g,
+          int batch, int bulk_ok, int sm_count, cudaStream_t s) {
   using ST = StreamK1<P, T>;
-  const long long items = (long long)batch * g.n_active * ST::IPP;
+  const long long items = (long long)batch * rb.n_items;
   if (items == 0) return 0;
   const long long ctas = (items + ST::WARPS - 1) / ST::WARPS;
   const unsigned grid = (unsigned)(ctas < sm_count ? ctas : sm_count);
-  return launch_chain(1, k1_stream<P, T>, dim3(grid), dim3(ST::THREADS), ST::SMEM, s, (const T*)image, (cplx<T>*)spec, corners,
+  return launch_chain(1, k1_stream<P, T>, dim3(grid), dim3(ST::THREADS), ST::SMEM, s, (const T*)image, (cplx<T>*)bands, rb,
                       (const cplx<T>*)tw, (const T*)win, g, batch, bulk_ok);
 }
-int k1s(int dt, const void* image, void* spec, const int2* corners, const void* tw, const void* win,
-        const ApplyGeom& g, int batch, int bulk_ok, int sm_count, cudaStream_t s) {
-  return dt == DT_F32 ? k1s_t<float>(image, spec, corners, tw, win, g, batch, bulk_ok, sm_count, s)
-                      : k1s_t<double>(image, spec, corners, tw, win, g, batch, bulk_ok, sm_count, s);
+int k1s(int dt, const void* image, void* bands, const RowBands& rb, const void* tw, const void* win, const ApplyGeom& g,
+        int batch, int bulk_ok, int sm_count, cudaStream_t s) {
+  return dt == DT_F32 ? k1s_t<float>(image, bands, rb, tw, win, g, batch, bulk_ok, sm_count, s)
+                      : k1s_t<double>(image, bands, rb, tw, win, g, batch, bulk_ok, sm_count, s);
 }
 
 template <typename T>
-int k2_t(void* spec, const void* kmain, const void* knyq, const int* active, const void* tw,
-         const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
+int k2_t(const void* bands, const RowBands& rb, void* spec, const void* kmain, const void* knyq, const int* active,
+         const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
   // Walk several frames per CTA so the transfer-kernel tile is read once per batch, but keep
   // at least ~4 waves of CTAs in flight (SMs x 3 resident CTAs).
   const long long ctas = cdiv((long long)g.n_active * TL::NTILE, TL::SLOTS);
   int fpc = batch;
   while (fpc > 1 && ctas * cdiv(batch, fpc) < (long long)sm_count * 3 * 4) fpc = (fpc + 1) / 2;
   dim3 grid((unsigned)ctas, cdiv(batch, fpc));
+  const cplx<T>* bnd = (const cplx<T>*)bands;
   if (g.win_len < P) {
-    // embedded patch size: only the first win_len rows of a patch's spectrum carry data (rpsf_kernels.cuh: PRUNED)
+    // embedded patch size: only the first win_len rows of a patch carry data (rpsf_kernels.cuh: PRUNED)
     if constexpr (use_col_pipe<T>())
-      return launch_chain(2, k2_pipelined<P, T, 1, true>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, (cplx<T>*)spec,
-                          (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
+      return launch_chain(2, k2_pipelined<P, T, 1, true>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, bnd, rb,
+                          (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw,
+                          (const T*)win, batch, fpc, g);
     else
-      k2_colfft_mul_colifft<P, T, true><<<grid, TL::K2_THREADS, col_smem<T>(), s>>>(
-          (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
+      k2_colfft_mul_colifft<P, T, true><<<grid, TL::K2_THREADS, col_k2_smem<T>(), s>>>(
+          bnd, rb, (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, (const T*)win,
+          batch, fpc, g);
     return (int)cudaGetLastError();
   }
   if constexpr (use_col_pipe<T>() && TL::SLOTS == 1 && TL::NTILE % 2 == 0) {
@@ -160,22 +166,25 @@ int k2_t(void* spec, const void* kmain, const void* knyq, const int* active, con
     // 89.9 vs 87.3 us) and two tiles at 8 frames per call (4 % slower) lost.
     if (fpc <= 1) {
       grid.x = (unsigned)cdiv(ctas, 2);
-      return launch_chain(2, k2_pipelined<P, T, 2>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, (cplx<T>*)spec,
-                          (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
+      return launch_chain(2, k2_pipelined<P, T, 2>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, bnd, rb,
+                          (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw,
+                          (const T*)win, batch, fpc, g);
     }
   }
   if constexpr (use_col_pipe<T>())
-    return launch_chain(2, k2_pipelined<P, T>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, (cplx<T>*)spec,
-                        (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
+    return launch_chain(2, k2_pipelined<P, T>, grid, dim3(TL::K2_THREADS), col_pipe_smem<T>(), s, bnd, rb, (cplx<T>*)spec,
+                        (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, (const T*)win, batch, fpc,
+                        g);
   else
-    k2_colfft_mul_colifft<P, T><<<grid, TL::K2_THREADS, col_smem<T>(), s>>>(
-        (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, batch, fpc, g);
+    k2_colfft_mul_colifft<P, T><<<grid, TL::K2_THREADS, col_k2_smem<T>(), s>>>(
+        bnd, rb, (cplx<T>*)spec, (const cplx<T>*)kmain, (const cplx<T>*)knyq, active, (const cplx<T>*)tw, (const T*)win,
+        batch, fpc, g);
   return (int)cudaGetLastError();
 }
-int k2(int dt, void* spec, const void* kmain, const void* knyq, const int* active, const void* tw,
-       const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
-  return dt == DT_F32 ? k2_t<float>(spec, kmain, knyq, active, tw, g, batch, sm_count, s)
-                      : k2_t<double>(spec, kmain, knyq, active, tw, g, batch, sm_count, s);
+int k2(int dt, const void* bands, const RowBands& rb, void* spec, const void* kmain, const void* knyq, const int* active,
+       const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
+  return dt == DT_F32 ? k2_t<float>(bands, rb, spec, kmain, knyq, active, tw, win, g, batch, sm_count, s)
+                      : k2_t<double>(bands, rb, spec, kmain, knyq, active, tw, win, g, batch, sm_count, s);
 }
 
 template <typename T>
@@ -289,18 +298,19 @@ int fft2_adjoint(int dt, const void* grad, void* scratch, void* out, const void*
 
 // launched plainly (no programmatic dependent launch): it reads both plans' spectra, written by the kernels before it
 template <typename T>
-int kgrad_t(const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active, int batch,
-            cudaStream_t s) {
+int kgrad_t(const void* xspec, const RowBands& xb, const void* gspec, const RowBands& gb, void* out, const int* active,
+            const void* tw, const void* win, int n_active, int batch, cudaStream_t s) {
   using GT = GradTile<P, T>;
   if (n_active == 0) return 0;
   kgrad<P, T><<<cdiv((long long)n_active * GT::NTILE, GT::SLOTS), GT::THREADS, GT::SMEM, s>>>(
-      (const cplx<T>*)xspec, (const cplx<T>*)gspec, (cplx<T>*)out, active, (const cplx<T>*)tw, n_active, batch);
+      (const cplx<T>*)xspec, xb, (const cplx<T>*)gspec, gb, (cplx<T>*)out, active, (const cplx<T>*)tw, (const T*)win,
+      n_active, batch);
   return (int)cudaGetLastError();
 }
-int kgrad_launch(int dt, const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active,
-                 int batch, cudaStream_t s) {
-  return dt == DT_F32 ? kgrad_t<float>(xspec, gspec, out, active, tw, n_active, batch, s)
-                      : kgrad_t<double>(xspec, gspec, out, active, tw, n_active, batch, s);
+int kgrad_launch(int dt, const void* xspec, const RowBands& xb, const void* gspec, const RowBands& gb, void* out,
+                 const int* active, const void* tw, const void* win, int n_active, int batch, cudaStream_t s) {
+  return dt == DT_F32 ? kgrad_t<float>(xspec, xb, gspec, gb, out, active, tw, win, n_active, batch, s)
+                      : kgrad_t<double>(xspec, xb, gspec, gb, out, active, tw, win, n_active, batch, s);
 }
 
 const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch, fft2_adjoint};

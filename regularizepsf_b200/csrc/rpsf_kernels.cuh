@@ -16,6 +16,7 @@
 #pragma once
 #include <cstdint>
 #include "rpsf_fft.cuh"
+#include "rpsf_bands.cuh"
 
 // Programmatic dependent launch (sm_90+).  K1 -> K2 -> K3 -> next K1 are launched with
 // cudaLaunchAttributeProgrammaticStreamSerialization (rpsf_inst.cu: launch_chain): a kernel's CTAs may become resident
@@ -99,15 +100,14 @@ __device__ __forceinline__ unsigned team_mask(int n1) {
 
 // ============================================================================ K1
 // gather + apodize + row FFT.  transform.py:141-163 (slice, stack, window, first FFT axis).
-// One team per pair of patch rows: z = (row_a + i*row_b) * w_col, complex FFT-P, split into the
-// two Hermitian half-spectra, scaled by the row window, stored packed.
+// One team per pair of band rows (rpsf_bands.cuh): z = (row_a + i*row_b) * w_col, complex FFT-P, split into the
+// two Hermitian half-spectra, stored packed without the row window.
 template <int P, typename T>
 __global__ void __launch_bounds__(Tile<P>::ROW_THREADS)
-k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
-                        const int2* __restrict__ corners,      // per active patch (row, col)
+k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec, const RowBands rb,
                         const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, ApplyGeom g) {
   using TL = Tile<P>;
-  constexpr int N1 = TL::N1, N2 = TL::N2, HALF = TL::HALF;
+  constexpr int N1 = TL::N1, N2 = TL::N2, HALF = TL::HALF, PAIRS = band_quantum<P>() / 2;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
   T* win = reinterpret_cast<T*>(tw + P);
@@ -117,40 +117,40 @@ k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
 
   const int team = threadIdx.x / N1, t = threadIdx.x % N1;
   cplx<T>* scr = scratch_all + team * TL::SCR;
-  const long long item = (long long)blockIdx.x * TL::TEAMS + team;   // (active patch, row pair)
-  const int a = int(item / HALF), pair = int(item % HALF);
-  if (a >= g.n_active) return;
+  const long long item = (long long)blockIdx.x * TL::TEAMS + team;   // (band item, row pair)
+  const int bi = int(item / PAIRS), pair = int(item % PAIRS);
+  if (bi >= rb.n_items) return;
   const unsigned mask = team_mask(N1);
   auto ex = [](int k2, int n1) { return k2 * TL::EX_STRIDE + n1; };
   auto sync = [mask]() { __syncwarp(mask); };
 
-  const int2 corner = corners[a];
-  const int ra = 2 * pair, rb = ra + 1;
-  // embedded patch sizes: rows past the window are zero and nobody reads their spectra (the pruned column pass
-  // below treats them as zero without loading them) — the whole team leaves
-  if (ra >= g.win_len) return;
-  const int ya = pad_index(corner.x + ra, g.H, g.pad_mode);
-  const int yb = pad_index(corner.x + rb, g.H, g.pad_mode);
+  const BandItem it = rb.items[bi];
+  const int ra = 2 * pair, rb_ = ra + 1;
+  const bool live_a = (it.live >> ra) & 1u, live_b = (it.live >> rb_) & 1u;
+  // neither row is in a patch window: nobody reads this pair — the whole team leaves
+  if (!live_a && !live_b) return;
+  const int ya = pad_index(it.row + ra, g.H, g.pad_mode);
+  const int yb = pad_index(it.row + rb_, g.H, g.pad_mode);
   const T* img = image + (long long)blockIdx.y * g.img_frame_stride;
   const bool direct = g.pad_mode == PAD_NONE;
-  // rows / columns past the window (embedded patch sizes) are exact zeros, not 0 * pixel: a NaN outside the patch
-  // must not leak in
-  const T* rowa = ((ya < 0 && !direct) || ra >= g.win_len) ? nullptr : img + (long long)(ya - g.img_row0) * g.img_pitch;
-  const T* rowb = ((yb < 0 && !direct) || rb >= g.win_len) ? nullptr : img + (long long)(yb - g.img_row0) * g.img_pitch;
+  // zero rows of the band and columns past the window (embedded patch sizes) are exact zeros, not 0 * pixel: a NaN
+  // outside the patch must not leak in
+  const T* rowa = ((ya < 0 && !direct) || !live_a) ? nullptr : img + (long long)(ya - g.img_row0) * g.img_pitch;
+  const T* rowb = ((yb < 0 && !direct) || !live_b) ? nullptr : img + (long long)(yb - g.img_row0) * g.img_pitch;
 
   cplx<T> v[N2];
-  const bool interior = (direct || (corner.y >= 0 && corner.y + P <= g.W)) && g.win_len >= P;
+  const bool interior = (direct || (it.cx >= 0 && it.cx + P <= g.W)) && g.win_len >= P;
   if (interior && rowa && rowb) {
     static_for<0, N2>([&](auto jj) {
       constexpr int j = decltype(jj)::value;
       const int n = t + N1 * j;
-      v[j] = cscale(mk<T>(rowa[corner.y + n], rowb[corner.y + n]), win[n]);
+      v[j] = cscale(mk<T>(rowa[it.cx + n], rowb[it.cx + n]), win[n]);
     });
   } else {
     static_for<0, N2>([&](auto jj) {
       constexpr int j = decltype(jj)::value;
       const int n = t + N1 * j;
-      const int x = pad_index(corner.y + n, g.W, g.pad_mode);
+      const int x = pad_index(it.cx + n, g.W, g.pad_mode);
       const bool inside = (x >= 0 || direct) && n < g.win_len;
       const T pa = (rowa && inside) ? rowa[x] : T(0);
       const T pb = (rowb && inside) ? rowb[x] : T(0);
@@ -167,9 +167,9 @@ k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
     scr[(t + N1 * m) + N2 * k1] = v[e];
   });
   sync();
-  // A[k] = (Z[k] + conj Z[P-k]) / 2,  B[k] = (Z[k] - conj Z[P-k]) / (2i); scaled by row window
-  const T wa = T(0.5) * win[ra], wb = T(0.5) * win[rb];
-  cplx<T>* outa = spec + (((long long)blockIdx.y * g.n_active + a) * P + ra) * HALF;
+  // A[k] = Z[k] + conj Z[P-k],  B[k] = -i (Z[k] - conj Z[P-k]): twice the half-spectra; the reader applies 1/2 and the
+  // row window
+  cplx<T>* outa = spec + ((long long)blockIdx.y * rb.frame_rows + it.buf_row + ra) * HALF;
   cplx<T>* outb = outa + HALF;
 #pragma unroll
   for (int i = 0; i < HALF / N1; ++i) {
@@ -177,12 +177,12 @@ k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
     const cplx<T> z1 = scr[k];
     const cplx<T> z2 = scr[(P - k) & (P - 1)];
     const cplx<T> D = padd(z1, mk<T>(-z2.x, z2.y));                 // z1 - conj z2
-    cplx<T> A = cscale(padd(z1, mk<T>(z2.x, -z2.y)), wa);           // (z1 + conj z2) wa
-    cplx<T> B = cscale(mk<T>(D.y, -D.x), wb);                       // -i (z1 - conj z2) wb
+    cplx<T> A = padd(z1, mk<T>(z2.x, -z2.y));                       // z1 + conj z2
+    cplx<T> B = mk<T>(D.y, -D.x);                                   // -i (z1 - conj z2)
     if (k == 0) {                       // pack (DC, Nyquist): both real
       const cplx<T> zn = scr[HALF];
-      A = mk<T>(T(2) * wa * z1.x, T(2) * wa * zn.x);
-      B = mk<T>(T(2) * wb * z1.y, T(2) * wb * zn.y);
+      A = mk<T>(T(2) * z1.x, T(2) * zn.x);
+      B = mk<T>(T(2) * z1.y, T(2) * zn.y);
     }
     outa[k] = A;
     outb[k] = B;
@@ -190,7 +190,8 @@ k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
 }
 
 // ============================================================================ K2
-// column FFT x transfer kernel x column IFFT, in place on the spectrum workspace.
+// column FFT x transfer kernel x column IFFT: from a patch's rows of the band buffer (rpsf_bands.cuh), scaled by the
+// row window on load, to the patch's slot of the spectrum workspace.
 // transform.py:163-164 (second FFT axis, `patches * kernel`, first IFFT axis).
 // A CTA owns SLOTS tiles of [P rows] x [C bins]; thread (c, n1) of a slot owns P/N1 = N2
 // elements of column c.  c is the fastest thread index, so every global access is a
@@ -200,15 +201,18 @@ k1_gather_window_rowfft(const T* __restrict__ image, cplx<T>* __restrict__ spec,
 // (win_len rounded up to a whole row pair): the pass moves win_len / P of the bytes.
 template <int P, typename T, bool PRUNED = false>
 __global__ void __launch_bounds__(Tile<P>::K2_THREADS, (Tile<P>::N2 * sizeof(T) <= 64) ? 3 : (Tile<P>::N2 * sizeof(T) <= 128) ? 2 : 1)
-k2_colfft_mul_colifft(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kmain,
-                      const cplx<T>* __restrict__ knyq, const int* __restrict__ active,
-                      const cplx<T>* __restrict__ tw_g, int batch, int frames_per_cta, ApplyGeom g) {
+k2_colfft_mul_colifft(const cplx<T>* __restrict__ bands, const RowBands rb, cplx<T>* __restrict__ spec,
+                      const cplx<T>* __restrict__ kmain, const cplx<T>* __restrict__ knyq, const int* __restrict__ active,
+                      const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, int batch, int frames_per_cta,
+                      ApplyGeom g) {
   using TL = Tile<P>;
   constexpr int N1 = TL::N1, N2 = TL::N2, HALF = TL::HALF, C = TL::C, NTILE = TL::NTILE;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
   cplx<T>* xbuf = tw + P;                                   // SLOTS * P * C complex
-  for (int i = threadIdx.x; i < P; i += blockDim.x) tw[i] = tw_g[i];
+  T* wy = reinterpret_cast<T*>(xbuf + TL::SLOTS * P * C);   // row window as the row pass applied it: 0.5 * win
+  for (int i = threadIdx.x; i < P; i += blockDim.x) { tw[i] = tw_g[i]; wy[i] = T(0.5) * win_g[i]; }
+  __syncthreads();
 
   const int c = threadIdx.x % C;
   const int n1 = (threadIdx.x / C) % N1;
@@ -248,15 +252,18 @@ k2_colfft_mul_colifft(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ km
   const int f_begin = blockIdx.y * frames_per_cta;
   const int f_end = min(batch, f_begin + frames_per_cta);
   const int live_rows = (g.win_len + 1) & ~1;               // the overlap-add reads whole row pairs
+  const int prow = valid ? rb.patch_row[a] : 0;
   for (int f = f_begin; f < f_end; ++f) {
     cplx<T>* base = spec + (((long long)f * g.n_active + a) * P) * HALF + tile * C + c;
+    const cplx<T>* src = bands + ((long long)f * rb.frame_rows + prow) * HALF + tile * C + c;
     cplx<T> v[N2];
     static_for<0, N2>([&](auto jj) {
       constexpr int j = decltype(jj)::value;
-      const bool live = !PRUNED || n1 + N1 * j < live_rows;
-      v[j] = (valid && live) ? base[(long long)(n1 + N1 * j) * HALF] : mk<T>(T(0), T(0));
+      const int r = n1 + N1 * j;
+      const bool live = !PRUNED || r < live_rows;
+      v[j] = (valid && live) ? cscale_rn(src[(long long)r * HALF], wy[r]) : mk<T>(T(0), T(0));
     });
-    __syncthreads();                                        // twiddle table visible (first pass)
+    __syncthreads();                                        // the previous frame's exchange reads are done
 
     coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync);
 
@@ -331,10 +338,10 @@ constexpr int K2_STAGES = 2;
 // loaded while the inverse transform of this one runs (a single-frame call otherwise exposes a full memory latency
 // per CTA).
 template <int P, typename T, bool TILE0, int TPC = 1, bool PRUNED = false>
-__device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kp,
-                                          const cplx<T>* __restrict__ kn, const cplx<T>* tw, cplx<T>* stage0,
-                                          bool valid_in, bool special_in, int a, int tile, int c, int n1, int slot, int lt,
-                                          int f_begin, int f_end, const ApplyGeom& g) {
+__device__ __forceinline__ void k2_frames(const cplx<T>* __restrict__ bands, const RowBands& rb, cplx<T>* __restrict__ spec,
+                                          const cplx<T>* __restrict__ kp, const cplx<T>* __restrict__ kn, const cplx<T>* tw,
+                                          const T* wy, cplx<T>* stage0, bool valid_in, bool special_in, int a, int tile,
+                                          int c, int n1, int slot, int lt, int f_begin, int f_end, const ApplyGeom& g) {
   using TL = Tile<P>;
   static_assert(TPC == 1 || TL::SLOTS == 1, "several tiles per CTA need one slot per CTA");
   const bool valid = TL::SLOTS == 1 ? true : valid_in;      // one slot per CTA: the grid is exact
@@ -366,10 +373,12 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
 
   // cp.async addressing, hoisted: chunk i of this thread is row (lt / ROW_CHUNKS) + i*ROWS_PER_PASS
   const long long frame_stride = (long long)g.n_active * P * HALF;
-  const cplx<T>* tile_base0 = spec + ((long long)a * P) * HALF + tile * C;      // frame 0, first tile of this CTA
+  const long long band_frame_stride = (long long)rb.frame_rows * HALF;
+  cplx<T>* tile_base0 = spec + ((long long)a * P) * HALF + tile * C;            // frame 0, first tile of this CTA
   const int row0 = lt / ROW_CHUNKS, part = lt % ROW_CHUNKS;
-  const int live_rows = (g.win_len + 1) & ~1;               // PRUNED: rows the gather wrote / the overlap-add reads
-  const cplx<T>* src0 = tile_base0 + (long long)row0 * HALF + part * CH;
+  const int live_rows = (g.win_len + 1) & ~1;               // PRUNED: rows the overlap-add reads
+  const cplx<T>* src0 =
+      bands + ((long long)(valid ? rb.patch_row[a] : 0) + row0) * HALF + tile * C + part * CH;   // the patch's band rows
   const int dst0 = slot * (P * C) + row0 * C + part * CH;
   const int nf = f_end - f_begin;
   const int n_it = TPC * nf;                                // iteration it = unit (it / nf), frame f_begin + it % nf
@@ -377,7 +386,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
     if (valid) {
       const int u = TPC == 1 ? 0 : it / nf;
       const int f = f_begin + (TPC == 1 ? it : it - u * nf);
-      const cplx<T>* src = src0 + u * C + f * frame_stride;
+      const cplx<T>* src = src0 + u * C + f * band_frame_stride;
 #pragma unroll
       for (int i = 0; i < PER_THREAD; ++i) {
         if (!PRUNED || row0 + i * ROWS_PER_PASS < live_rows)
@@ -406,7 +415,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
     const int u = TPC == 1 ? 0 : it / nf;
     const int f = f_begin + (TPC == 1 ? it : it - u * nf);
     const bool special = special_in && (TPC == 1 || u == 0);
-    const cplx<T>* tile_base = tile_base0 + u * C;
+    cplx<T>* tile_base = tile_base0 + u * C;
     cplx<T>* xbuf = stage0 + cur * STAGE;
     cp_async_wait_pending<NS - 2>();
     __syncthreads();          // tile `it` landed for everyone; everyone is done with the stage refilled next
@@ -418,7 +427,8 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
     cplx<T> v[N2];
     static_for<0, N2>([&](auto jj) {
       constexpr int j = decltype(jj)::value;
-      v[j] = xbuf[ex(j, n1)];                               // row n1 + N1*j, column c: the slot pass A writes back to
+      // row n1 + N1*j, column c (the slot pass A writes back to), times the row window
+      v[j] = cscale_rn(xbuf[ex(j, n1)], wy[n1 + N1 * j]);
     });
 
     // The exchange slots a thread reads in the forward pass B are exactly the ones it writes in the
@@ -472,7 +482,7 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
     // before anything is copied into this stage again
     coop_fft_inverse<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
     if (valid) {
-      cplx<T>* base = const_cast<cplx<T>*>(tile_base) + f * frame_stride + c;
+      cplx<T>* base = tile_base + f * frame_stride + c;
       static_for<0, N2>([&](auto jj) {
         constexpr int j = decltype(jj)::value;
         if (!PRUNED || n1 + N1 * j < live_rows) base[(long long)(n1 + N1 * j) * HALF] = v[j];
@@ -485,16 +495,17 @@ __device__ __forceinline__ void k2_frames(cplx<T>* __restrict__ spec, const cplx
 // measured slower (35.3 vs 32.2 us per frame).
 template <int P, typename T, int TPC = 1, bool PRUNED = false>
 __global__ void __launch_bounds__(Tile<P>::K2_THREADS, 2)
-k2_pipelined(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kmain, const cplx<T>* __restrict__ knyq,
-             const int* __restrict__ active, const cplx<T>* __restrict__ tw_g, int batch, int frames_per_cta,
-             ApplyGeom g) {
+k2_pipelined(const cplx<T>* __restrict__ bands, const RowBands rb, cplx<T>* __restrict__ spec,
+             const cplx<T>* __restrict__ kmain, const cplx<T>* __restrict__ knyq, const int* __restrict__ active,
+             const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, int batch, int frames_per_cta, ApplyGeom g) {
   using TL = Tile<P>;
   constexpr int N1 = TL::N1, N2 = TL::N2, C = TL::C, NTILE = TL::NTILE;
   static_assert(TPC == 1 || (TL::SLOTS == 1 && NTILE % TPC == 0), "tiles per CTA must divide the tiles of a patch");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
-  cplx<T>* stage0 = tw + P;
-  for (int i = threadIdx.x; i < P; i += blockDim.x) tw[i] = tw_g[i];
+  T* wy = reinterpret_cast<T*>(tw + P);                     // row window as the row pass applied it: 0.5 * win
+  cplx<T>* stage0 = reinterpret_cast<cplx<T>*>(wy + P);
+  for (int i = threadIdx.x; i < P; i += blockDim.x) { tw[i] = tw_g[i]; wy[i] = T(0.5) * win_g[i]; }
 
   const int c = threadIdx.x % C;
   const int n1 = (threadIdx.x / C) % N1;
@@ -517,9 +528,11 @@ k2_pipelined(cplx<T>* __restrict__ spec, const cplx<T>* __restrict__ kmain, cons
   const int f_begin = blockIdx.y * frames_per_cta;
   const int f_end = min(batch, f_begin + frames_per_cta);
   if (any_tile0)
-    k2_frames<P, T, true, TPC, PRUNED>(spec, kp, kn, tw, stage0, valid, special, a, tile, c, n1, slot, lt, f_begin, f_end, g);
+    k2_frames<P, T, true, TPC, PRUNED>(bands, rb, spec, kp, kn, tw, wy, stage0, valid, special, a, tile, c, n1, slot, lt,
+                                       f_begin, f_end, g);
   else
-    k2_frames<P, T, false, TPC, PRUNED>(spec, kp, kn, tw, stage0, valid, special, a, tile, c, n1, slot, lt, f_begin, f_end, g);
+    k2_frames<P, T, false, TPC, PRUNED>(bands, rb, spec, kp, kn, tw, wy, stage0, valid, special, a, tile, c, n1, slot, lt,
+                                        f_begin, f_end, g);
 }
 
 // ============================================================================ K3

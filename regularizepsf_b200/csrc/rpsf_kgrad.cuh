@@ -38,13 +38,15 @@ template <int P, typename T> struct GradTile {
   static_assert(SMEM <= 227 * 1024, "kgrad tile does not fit shared memory");
 };
 
-// xspec / gspec: the spectrum workspaces of the forward and adjoint plans after K1 (same active patches, same order).
+// xspec / gspec: the band buffers of the forward and adjoint plans after K1 (rpsf_bands.cuh), each read through its own
+// plan's bands and scaled by the row window on load (same active patches, same order).
 // out: (n, P, P) complex, reference layout; the slot of active patch a is active[a].  Slots of patches that are not
 // active are not touched (the caller zeroes them).
 template <int P, typename T>
 __global__ void __launch_bounds__(GradTile<P, T>::THREADS)
-kgrad(const cplx<T>* __restrict__ xspec, const cplx<T>* __restrict__ gspec, cplx<T>* __restrict__ out,
-      const int* __restrict__ active, const cplx<T>* __restrict__ tw_g, int n_active, int batch) {
+kgrad(const cplx<T>* __restrict__ xspec, const RowBands xb, const cplx<T>* __restrict__ gspec, const RowBands gb,
+      cplx<T>* __restrict__ out, const int* __restrict__ active, const cplx<T>* __restrict__ tw_g,
+      const T* __restrict__ win_g, int n_active, int batch) {
   using GT = GradTile<P, T>;
   constexpr int N1 = GT::N1, N2 = GT::N2, HALF = GT::HALF, C = GT::C, NTILE = GT::NTILE, SLOTS = GT::SLOTS;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -84,15 +86,15 @@ kgrad(const cplx<T>* __restrict__ xspec, const cplx<T>* __restrict__ gspec, cplx
   });
   __syncthreads();                                          // twiddle table visible
 
-  const long long frame_stride = (long long)n_active * P * HALF;
-  const long long column = (long long)a * P * HALF + tile * C + c;
+  const long long column = tile * C + c;
   // the column spectrum of one frame's tile in v (for the packed column: the DC column).  The Nyquist column of the
   // packed column goes to nyq_x (X), or is multiplied by conj(nyq_x) into nyq_acc (G).
-  auto column_fft = [&](const cplx<T>* __restrict__ spec, int f, cplx<T>(&v)[N2], bool is_g) {
-    const cplx<T>* base = spec + f * frame_stride + column;
+  auto column_fft = [&](const cplx<T>* __restrict__ spec, const RowBands& rb, int f, cplx<T>(&v)[N2], bool is_g) {
+    const cplx<T>* base = spec + ((long long)f * rb.frame_rows + (valid ? rb.patch_row[a] : 0)) * HALF + column;
     static_for<0, N2>([&](auto jj) {
       constexpr int j = decltype(jj)::value;
-      v[j] = valid ? base[(long long)(n1 + N1 * j) * HALF] : mk<T>(T(0), T(0));
+      const int r = n1 + N1 * j;
+      v[j] = valid ? cscale_rn(base[(long long)r * HALF], T(0.5) * __ldg(win_g + r)) : mk<T>(T(0), T(0));
     });
     coop_fft_forward<P, T>(v, n1, xbuf, tw, ex, sync);
     if (any_tile0) {
@@ -124,9 +126,9 @@ kgrad(const cplx<T>* __restrict__ xspec, const cplx<T>* __restrict__ gspec, cplx
 
   for (int f = 0; f < batch; ++f) {
     cplx<T> v[N2];
-    column_fft(xspec, f, v, false);
+    column_fft(xspec, xb, f, v, false);
     static_for<0, N2>([&](auto ee) { xs[ex(decltype(ee)::value, n1)] = v[decltype(ee)::value]; });
-    column_fft(gspec, f, v, true);
+    column_fft(gspec, gb, f, v, true);
     static_for<0, N2>([&](auto ee) {
       constexpr int e = decltype(ee)::value;
       const cplx<T> prod = cmulc(v[e], xs[ex(e, n1)]);                         // G conj(X)

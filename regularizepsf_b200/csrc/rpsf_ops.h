@@ -13,13 +13,16 @@ struct Ops {
   int P;
   // set shared-memory attributes for the current device; returns a cudaError_t
   int (*init)();
-  int (*k1)(int dt, const void* image, void* spec, const int2* corners, const void* tw, const void* win,
+  // the row passes write the band buffer `bands` (rpsf_bands.cuh)
+  int (*k1)(int dt, const void* image, void* bands, const RowBands& rb, const void* tw, const void* win,
             const ApplyGeom& g, int batch, cudaStream_t s);
   // persistent bulk-async K1 (rpsf_stream.cuh); `bulk_ok`: frame base, pitch and frame stride are 16-byte aligned
-  int (*k1s)(int dt, const void* image, void* spec, const int2* corners, const void* tw, const void* win,
+  int (*k1s)(int dt, const void* image, void* bands, const RowBands& rb, const void* tw, const void* win,
              const ApplyGeom& g, int batch, int bulk_ok, int sm_count, cudaStream_t s);
-  int (*k2)(int dt, void* spec, const void* kmain, const void* knyq, const int* active, const void* tw,
-            const ApplyGeom& g, int batch, int sm_count, cudaStream_t s);
+  // the column pass reads the band buffer and writes the spectrum workspace `spec`
+  int (*k2)(int dt, const void* bands, const RowBands& rb, void* spec, const void* kmain, const void* knyq,
+            const int* active, const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count,
+            cudaStream_t s);
   int (*k3)(int dt, const void* spec, void* out, const int2* corners, const int* items, int n_items,
             const void* tw, const void* win, int store_only, const ApplyGeom& g, int batch, cudaStream_t s);
   // single-launch overlap-add: `teams` teams per CTA, `seg_w` output columns per CTA
@@ -39,9 +42,9 @@ struct Ops {
   int (*fft2)(int dt, int in_dt, const void* values, void* out, const void* tw, long long n_patches,
               cudaStream_t s);
   // gradient with respect to the transfer kernel (rpsf_kgrad.cuh): conj(X) G / P^2 summed over `batch` frames of the
-  // forward (xspec) and adjoint (gspec) row-spectrum workspaces, into the (n, P, P) cube `out` at slots active[a]
-  int (*kgrad)(int dt, const void* xspec, const void* gspec, void* out, const int* active, const void* tw, int n_active,
-               int batch, cudaStream_t s);
+  // forward (xspec) and adjoint (gspec) band buffers, into the (n, P, P) cube `out` at slots active[a]
+  int (*kgrad)(int dt, const void* xspec, const RowBands& xb, const void* gspec, const RowBands& gb, void* out,
+               const int* active, const void* tw, const void* win, int n_active, int batch, cudaStream_t s);
   // adjoint of fft2 (rpsf_construct_grad.cuh): out (n, P, P) real = Re(fft2(conj(grad))), through the complex
   // (n, P, P) cube `scratch`
   int (*fft2_adjoint)(int dt, const void* grad, void* scratch, void* out, const void* tw, long long n_patches,

@@ -19,6 +19,7 @@
 #pragma once
 #include <cstdint>
 #include "rpsf_kernels.cuh"
+#include "rpsf_bands.cuh"
 
 namespace rpsf {
 
@@ -107,18 +108,20 @@ __device__ __forceinline__ void st_spec(float2* p, float2 v, unsigned long long 
 __device__ __forceinline__ void st_spec(double2* p, double2 v, unsigned long long) { *p = v; }
 
 // ============================================================================ K1, streaming
-// gather + apodize + row FFT (same arithmetic as k1_gather_window_rowfft).  Warp item = ROWS
-// consecutive rows of one patch of one frame; team tm of the warp owns rows (2*tm, 2*tm+1) of it.
-// Patch `a` of frame `f` sits at slot f * n_active + a of the workspace.  The body stays a function apart from its
-// kernel (as K3's does): written into the kernel, the same source compiles to different instructions.
+// gather + apodize + row FFT (same arithmetic as k1_gather_window_rowfft).  Warp item = one BandItem (ROWS consecutive
+// rows of one band) of one frame; team tm of the warp owns rows (2*tm, 2*tm+1) of it.  The rows are stored to the band
+// buffer without the row window (rpsf_bands.cuh).  The body stays a function apart from its kernel (as K3's does):
+// written into the kernel, the same source compiles to different instructions.
 template <int P, typename T, typename ST>
 __device__ __forceinline__ void
-k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const int2* __restrict__ corners,
+k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const RowBands rb,
                const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, const ApplyGeom& g, int batch, int bulk_ok,
                unsigned cta, unsigned n_cta, unsigned char* smem_raw) {
-  constexpr int N1 = ST::N1, N2 = ST::N2, HALF = ST::HALF, ROWS = ST::ROWS, IPP = ST::IPP;
+  constexpr int N1 = ST::N1, N2 = ST::N2, HALF = ST::HALF, ROWS = ST::ROWS;
   constexpr int STAGES = ST::STAGES, WARPS = ST::WARPS;
   constexpr unsigned ROW_BYTES = P * sizeof(T);
+  constexpr unsigned ALL_LIVE = (1u << ROWS) - 1u;
+  static_assert(ROWS == band_quantum<P>(), "a band item is one warp item");
   cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
   T* win = reinterpret_cast<T*>(tw + P);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + ST::TABLE_BYTES);            // [WARPS][STAGES]
@@ -139,52 +142,53 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
 
   unsigned char* my_ring = ring + (size_t)warp * STAGES * ST::STAGE_BYTES;
   const unsigned long long l2_keep = l2_policy_evict_last();
-  const unsigned n_items = (unsigned)batch * (unsigned)g.n_active * IPP;       // host guarantees < 2^30
+  const unsigned n_items = (unsigned)batch * (unsigned)rb.n_items;           // host guarantees batch * frame_rows < 2^30
   const unsigned stride = n_cta * WARPS;
   const unsigned first = cta * WARPS + warp;
   const bool direct = g.pad_mode == PAD_NONE;
 
   // How an item's rows reach its stage:
   //   BULK    every column lies inside the frame: one bulk copy per row
-  //   PARTIAL the patch hangs over the left/right frame edge: bulk copy of the in-frame span, then the
+  //   PARTIAL the band hangs over the left/right frame edge: bulk copy of the in-frame span, then the
   //           overhanging columns are filled from their pad_index() sources (mirrored columns are
   //           read back from the stage itself when the source lies in the copied span)
-  //   MANUAL  unaligned corners, `constant` rows above/below the frame: the warp gathers every sample
+  //   MANUAL  unaligned corners, `constant` rows above/below the frame, zero rows of the band: the warp gathers every
+  //           sample
   enum : unsigned { BULK = 0, PARTIAL = 1, MANUAL = 2 };
 
   // ---- the head of the pipeline: the next item to be issued, decoded incrementally ----------
-  // item = (f * n_active + a) * IPP + q; one step adds `stride` = (df, da, dq) with carries
+  // item = f * n_items + i; one step adds `stride` = (df, di) with a carry
   unsigned head = first;
-  int hq = int(first % IPP), ha = int((first / IPP) % (unsigned)g.n_active), hf = int((first / IPP) / (unsigned)g.n_active);
-  const int dq = int(stride % IPP), da = int((stride / IPP) % (unsigned)g.n_active),
-            df = int((stride / IPP) / (unsigned)g.n_active);
-  int2 hcorner = make_int2(0, 0);
-  if (head < n_items) hcorner = __ldg(corners + ha);
+  int hi = int(first % (unsigned)rb.n_items), hf = int(first / (unsigned)rb.n_items);
+  const int di = int(stride % (unsigned)rb.n_items), df = int(stride / (unsigned)rb.n_items);
+  BandItem hitem{0, 0, 0, 0};
+  auto load_item = [&](int i) {
+    const int4 v = __ldg(reinterpret_cast<const int4*>(rb.items) + i);
+    return BandItem{v.x, v.y, v.z, (unsigned)v.w};
+  };
+  if (head < n_items) hitem = load_item(hi);
   auto advance_head = [&]() {
     head += stride;
-    hq += dq; ha += da; hf += df;
-    if (hq >= IPP) { hq -= IPP; ++ha; }
-    if (ha >= g.n_active) { ha -= g.n_active; ++hf; }
-    if (head < n_items) hcorner = __ldg(corners + ha);      // consumed one iteration later
+    hi += di; hf += df;
+    if (hi >= rb.n_items) { hi -= rb.n_items; ++hf; }
+    if (head < n_items) hitem = load_item(hi);      // consumed one iteration later
   };
-  // first row of the head item in the workspace's (frame, patch, row) order, and its patch row
-  auto src_row = [&](int corner_row, int patch_row) { return pad_index(corner_row + patch_row, g.H, g.pad_mode); };
 
   unsigned phase = 0;      // bit s: parity the next wait on stage s must see
 
-  // issue the head item into stage `st`; returns (workspace row index << 2) | kind
+  // issue the head item into stage `st`; returns (band-buffer row index << 2) | kind
   auto issue_head = [&](int st) -> unsigned {
-    const unsigned rowidx = (unsigned)(hf * g.n_active + ha) * P + hq * ROWS;
+    const unsigned rowidx = (unsigned)hf * (unsigned)rb.frame_rows + (unsigned)hitem.buf_row;
     unsigned char* stage = my_ring + st * ST::STAGE_BYTES;
-    const int x_lo = direct ? hcorner.y : max(hcorner.y, 0);
-    const int x_hi = direct ? hcorner.y + P : min(hcorner.y + P, g.W);
+    const int x_lo = direct ? hitem.cx : max(hitem.cx, 0);
+    const int x_hi = direct ? hitem.cx + P : min(hitem.cx + P, g.W);
     // source span AND its landing offset inside the stage row must keep the 16-byte granularity of bulk copies
-    // (a patch overhanging both frame edges can have aligned ends but a misaligned offset x_lo - corner.y)
+    // (a band overhanging both frame edges can have aligned ends but a misaligned offset x_lo - cx)
     const bool aligned = bulk_ok && x_hi > x_lo && ((x_lo * (int)sizeof(T)) & 15) == 0 && ((x_hi * (int)sizeof(T)) & 15) == 0 &&
-                         (((x_lo - hcorner.y) * (int)sizeof(T)) & 15) == 0;
+                         (((x_lo - hitem.cx) * (int)sizeof(T)) & 15) == 0;
     int y = 0;
-    if (lane < ROWS) y = src_row(hcorner.x, hq * ROWS + lane);
-    const bool rows_ok = __all_sync(0xffffffffu, direct || y >= 0);
+    if (lane < ROWS) y = pad_index(hitem.row + lane, g.H, g.pad_mode);
+    const bool rows_ok = __all_sync(0xffffffffu, direct || y >= 0) && hitem.live == ALL_LIVE;
     const unsigned kind = !(aligned && rows_ok) ? MANUAL : (x_hi - x_lo == P ? BULK : PARTIAL);
     if (kind != MANUAL) {
       const unsigned bytes = (unsigned)(x_hi - x_lo) * (unsigned)sizeof(T);
@@ -198,14 +202,14 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
       __syncwarp();
       if (lane < ROWS) {
         const T* src = image + (long long)hf * g.img_frame_stride + (long long)(y - g.img_row0) * g.img_pitch + x_lo;
-        bulk_load(stage + (lane >> 1) * ST::TEAM_BYTES + (lane & 1) * ROW_BYTES + (x_lo - hcorner.y) * (int)sizeof(T), src, bytes,
+        bulk_load(stage + (lane >> 1) * ST::TEAM_BYTES + (lane & 1) * ROW_BYTES + (x_lo - hitem.cx) * (int)sizeof(T), src, bytes,
                   bar + st);
       }
     }
     return (rowidx << 2) | kind;
   };
 
-  unsigned pend[STAGES - 1], pend_item[STAGES - 1];    // (workspace row << 2) | kind, and the item's number
+  unsigned pend[STAGES - 1], pend_item[STAGES - 1];    // (band-buffer row << 2) | kind, and the item's number
 #pragma unroll
   for (int k = 0; k < STAGES - 1; ++k) {
     pend[k] = 0; pend_item[k] = 0;
@@ -219,7 +223,7 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
 
   int s = 0;
   for (unsigned it = first; it < n_items; it += stride) {
-    const unsigned cur = pend[0], item = pend_item[0], pf = item / IPP;
+    const unsigned cur = pend[0], item = pend_item[0];
 #pragma unroll
     for (int k = 0; k + 1 < STAGES - 1; ++k) { pend[k] = pend[k + 1]; pend_item[k] = pend_item[k + 1]; }
     // the stage the previous iteration released receives the head item
@@ -235,19 +239,18 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
       phase ^= 1u << s;
     }
     if (kind >= PARTIAL) {
-      // rare path: recover the item's coordinates from its patch-frame and workspace row index
-      const int q_rows = int(rowidx & (P - 1));
-      const int a = int(pf % (unsigned)g.n_active), f = int(pf / (unsigned)g.n_active);
-      const int2 corner = __ldg(corners + a);
+      // rare path: recover the item from its number
+      const int f = int(item / (unsigned)rb.n_items);
+      const BandItem bi = load_item(int(item - (unsigned)f * (unsigned)rb.n_items));
       const T* img = image + (long long)f * g.img_frame_stride;
-      const int lo_c = kind == PARTIAL ? max(-corner.y, 0) : 0;                   // bulk-copied columns [lo_c, hi_c)
-      const int hi_c = kind == PARTIAL ? min(g.W - corner.y, P) : 0;
+      const int lo_c = kind == PARTIAL ? max(-bi.cx, 0) : 0;                      // bulk-copied columns [lo_c, hi_c)
+      const int hi_c = kind == PARTIAL ? min(g.W - bi.cx, P) : 0;
       const int n_fill = lo_c + (P - hi_c);                                       // columns outside [lo_c, hi_c)
 #pragma unroll 1
       for (int ci = lane; ci < n_fill; ci += 32) {
         const int c = ci < lo_c ? ci : ci - lo_c + hi_c;
-        const int x = pad_index(corner.y + c, g.W, g.pad_mode);
-        const int cs = x - corner.y;                                              // source column inside the stage?
+        const int x = pad_index(bi.cx + c, g.W, g.pad_mode);
+        const int cs = x - bi.cx;                                                 // source column inside the stage?
         const bool in_stage = !direct && x >= 0 && cs >= lo_c && cs < hi_c;
 #pragma unroll 1
         for (int r = 0; r < ROWS; ++r) {
@@ -255,8 +258,8 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
           T val = T(0);
           if (in_stage) {
             val = dst[cs];
-          } else {
-            const int y = src_row(corner.x, q_rows + r);
+          } else if ((bi.live >> r) & 1u) {
+            const int y = pad_index(bi.row + r, g.H, g.pad_mode);
             if (direct || (x >= 0 && y >= 0)) val = img[(long long)(y - g.img_row0) * g.img_pitch + x];
           }
           dst[c] = val;
@@ -279,11 +282,10 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
     coop_fft_forward<P, T>(v, t, scr, tw, [](int k2, int n1) { return ST::ex(k2, n1); }, sync);
 
     // This thread holds Z[k] for k = (t + N1*m) + N2*k1 in v[m*N1 + k1].  Split into the two rows' Hermitian
-    // half-spectra: A[k] = (Z[k] + conj Z[P-k]) / 2, B[k] = (Z[k] - conj Z[P-k]) / (2i), scaled by the row
-    // window.  Z[P-k] for k = t + N1*i sits in lane N1-t of the team at a compile-time register, so it comes by
-    // shuffle — no second pass through shared memory (the data pipe is this kernel's bound).
-    const int ra = int(rowidx & (P - 1)) + 2 * tm;
-    const T wa = T(0.5) * win[ra], wb = T(0.5) * win[ra + 1];
+    // half-spectra times two: A[k] = Z[k] + conj Z[P-k], B[k] = -i (Z[k] - conj Z[P-k]); the factor 1/2 and the row
+    // window are applied by the reader (rpsf_bands.cuh).  Z[P-k] for k = t + N1*i sits in lane N1-t of the team at a
+    // compile-time register, so it comes by shuffle — no second pass through shared memory (the data pipe is this
+    // kernel's bound).
     cplx<T>* outa = spec + ((size_t)rowidx + 2 * tm) * HALF + t;
     constexpr int R = N2 / N1;
     auto reg_of = [](int i) constexpr { return (i % R) * N1 + i / R; };   // register holding bin (lane) + N1*i
@@ -298,13 +300,13 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
       z2.y = __shfl_sync(0xffffffffu, theirs.y, partner, N1);
       if (t == 0) z2 = mine;
       const cplx<T> D = padd(z1, mk<T>(-z2.x, z2.y));
-      cplx<T> A = cscale(padd(z1, mk<T>(z2.x, -z2.y)), wa);
-      cplx<T> B = cscale(mk<T>(D.y, -D.x), wb);
+      cplx<T> A = padd(z1, mk<T>(z2.x, -z2.y));
+      cplx<T> B = mk<T>(D.y, -D.x);
       if constexpr (i == 0) {
         if (t == 0) {                                        // pack (DC, Nyquist): both real
           const cplx<T> zn = v[reg_of(N2 / 2)];
-          A = mk<T>(T(2) * wa * z1.x, T(2) * wa * zn.x);
-          B = mk<T>(T(2) * wb * z1.y, T(2) * wb * zn.y);
+          A = mk<T>(T(2) * z1.x, T(2) * zn.x);
+          B = mk<T>(T(2) * z1.y, T(2) * zn.y);
         }
       }
       st_spec(outa + N1 * i, A, l2_keep);
@@ -318,10 +320,10 @@ k1_stream_body(const T* __restrict__ image, cplx<T>* __restrict__ spec, const in
 
 template <int P, typename T>
 __global__ void __launch_bounds__(StreamK1<P, T>::THREADS, 1)
-k1_stream(const T* __restrict__ image, cplx<T>* __restrict__ spec, const int2* __restrict__ corners,
-          const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g, ApplyGeom g, int batch, int bulk_ok) {
+k1_stream(const T* __restrict__ image, cplx<T>* __restrict__ spec, RowBands rb, const cplx<T>* __restrict__ tw_g,
+          const T* __restrict__ win_g, ApplyGeom g, int batch, int bulk_ok) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  k1_stream_body<P, T, StreamK1<P, T>>(image, spec, corners, tw_g, win_g, g, batch, bulk_ok, blockIdx.x, gridDim.x, smem_raw);
+  k1_stream_body<P, T, StreamK1<P, T>>(image, spec, rb, tw_g, win_g, g, batch, bulk_ok, blockIdx.x, gridDim.x, smem_raw);
 }
 
 // ============================================================================ K3, streaming
