@@ -63,7 +63,7 @@ typedef struct rpsf_plan rpsf_plan;
 /* CUDA graphs.  A stream capture may contain, once their plans exist and each has run once outside the capture:
  * rpsf_apply (forward and adjoint plans), rpsf_apply_source, rpsf_apply_masked, rpsf_kernel_gradient(_masked), rpsf_transform_set_kernel,
  * rpsf_construct_kernel(_dev), rpsf_construct_kernel_backward(_dev), rpsf_psf_fft2 and rpsf_psf_fft2_adjoint (native
- * patch sizes).  These neither cudaMalloc nor synchronise then; their scratch is cudaMallocAsync on the stream, which
+ * patch sizes), rpsf_apply_stack, rpsf_stack_set_kernel and rpsf_construct_kernels(_dev).  These neither cudaMalloc nor synchronise then; their scratch is cudaMallocAsync on the stream, which
  * the capture turns into allocation nodes.  On a capturing stream a call that touches a transform's device state makes
  * the transform's order event an external dependency of the graph (cudaEventWaitExternal at its start,
  * cudaEventRecordExternal at its end), so each replay is ordered after the calls issued before its launch and before
@@ -310,6 +310,51 @@ int rpsf_apply_masked(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
  * out: `batch` contiguous (row_end-row_begin, W) frames of out_dtype (RPSF_F32 / RPSF_F64).
  * Synchronous on return. */
 int rpsf_apply_host(rpsf_plan* p, const void* image, int image_dtype, void* out, int out_dtype, int batch);
+
+/* ---- transform stacks: M transfer kernels on one set of patch corners and one patch size ------
+ * For a sweep of (alpha, epsilon): one call applies every kernel to the same frames, and the work that does not depend
+ * on the kernel (the saturation / mask fill, the row pass) runs once per frame instead of once per kernel. */
+typedef struct rpsf_stack rpsf_stack;
+
+/* rpsf_construct_kernel for n_kernels (alpha, epsilon) pairs in one pass over S and T: kernel m, bit-identical to
+ * rpsf_construct_kernel(..., alpha_epsilon[2m], alpha_epsilon[2m + 1], ...), is written to kernel_out + m * count
+ * (complex elements).  alpha_epsilon: HOST array of 2 * n_kernels doubles.  Launches only (one per 64 kernels). */
+int rpsf_construct_kernels(const void* source_fft, const void* target_fft, void* kernel_out, int64_t count, int dtype,
+                           const double* alpha_epsilon, int n_kernels, int device, void* stream);
+/* The same with alpha_epsilon in device memory (2 * n_kernels doubles); bit-identical to rpsf_construct_kernel_dev. */
+int rpsf_construct_kernels_dev(const void* source_fft, const void* target_fft, void* kernel_out, int64_t count,
+                               int dtype, const double* alpha_epsilon, int n_kernels, int device, void* stream);
+
+/* A stack of n_kernels >= 1 transfer kernels on the coordinates of rpsf_transform_create (same arguments, same errors).
+ * Each kernel is loaded with rpsf_stack_set_kernel(index, ...), which takes what rpsf_transform_set_kernel takes.
+ * rpsf_stack_destroy frees the stack; destroy its plans first. */
+int rpsf_stack_create(rpsf_stack** out, const int32_t* coords, int n_patches, int patch_size, int compute_dtype,
+                      int device, int n_kernels);
+int rpsf_stack_set_kernel(rpsf_stack* stack, int index, const void* kernel_full, int kernel_dtype, void* stream);
+int rpsf_stack_destroy(rpsf_stack* stack);
+/* A whole-frame plan (rows [0, height)) of a stack for up to max_batch frames per call; n_kernels * max_batch <= 65535.
+ * Its workspace holds the patch spectra of n_kernels * max_batch frames and the row bands of max_batch frames (the
+ * spectra are 75.8 MB per frame and kernel at 2048^2 / 256 px, float32).  It runs through rpsf_apply_stack only (the
+ * other apply entry points return RPSF_E_INVALID_ARGUMENT); free it with rpsf_plan_destroy, and set its saturation
+ * with rpsf_plan_set_saturation.  RPSF_PAD_MATERIALIZED is RPSF_E_UNSUPPORTED. */
+int rpsf_plan_create_stack(rpsf_plan** out, rpsf_stack* stack, int height, int width, int pad_mode, int max_batch);
+/* Every kernel of the stack applied to `batch` whole frames: output frame m * batch + b (at out + (m * batch + b) *
+ * out_frame_stride) is bit-identical to rpsf_apply_masked (mask non-null), rpsf_apply_source (src non-null) or rpsf_apply
+ * with kernel m alone on frame b.  n_kernels must be the stack's.  The saturation / mask fill and the row pass run once
+ * per frame; the column pass runs once per kernel from the shared row spectra; one overlap-add covers every output
+ * frame.  The first call of a plan allocates its workspace (and, with saturation or a mask, its fill scratch) and
+ * cannot be captured in a CUDA graph; later ones can. */
+/* Column pass of a stack plan: mode 0 (the default) runs k2_stack, which transforms each tile of the row spectra once
+ * per frame and then multiplies and inverse-transforms it per kernel, for stacks of two kernels or more where it exists (native patch sizes whose
+ * column-pass stage ring fits a 36 KB stage: float32 up to 256 px, float64 up to 64 px); mode 1 forces the per-kernel column pass (the existing
+ * one, once per kernel on the shared row spectra), which embedded patch sizes always run.  Both give the same bits
+ * (test and benchmark hook).  rpsf_plan_stack_info sets *fused to 1 when the plan runs k2_stack. */
+int rpsf_plan_set_stack_mode(rpsf_plan* p, int mode);
+int rpsf_plan_stack_info(const rpsf_plan* p, int* fused);
+int rpsf_apply_stack(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, void* out,
+                     int64_t out_pitch, int64_t out_frame_stride, int n_kernels, int batch, const void* src, int src_dtype,
+                     int64_t src_pitch, int64_t src_frame_stride, const void* mask, int64_t mask_pitch,
+                     int64_t mask_frame_stride, void* stream);
 
 /* ---- helpers -------------------------------------------------------------------------------- */
 /* 2-D dtype conversion on the device (the `.astype(float)` of transform.py:117) */

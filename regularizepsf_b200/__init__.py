@@ -7,7 +7,8 @@ GPU, star finding through the optional ``sep`` dependency as in the reference) a
 types.  ``DeviceCube`` holds a cube as a CUDA tensor: a transform built on one whose tensor requires grad is
 trainable (``ArrayPSFTransform.apply`` differentiates with respect to the transfer kernel), and an ``ArrayPSF`` whose
 values are a ``DeviceCube`` that requires grad makes ``ArrayPSFTransform.construct`` differentiable in the PSF values,
-as 0-d tensors ``alpha`` and ``epsilon`` do.  Plotting is out of scope (see DESIGN.md).
+as 0-d tensors ``alpha`` and ``epsilon`` do.  ``TransformStack`` applies many transfer kernels (an alpha / epsilon
+sweep) to the same frames in one call.  Plotting is out of scope (see DESIGN.md).
 """
 from regularizepsf_b200.exceptions import (
     FunctionParameterMismatchError,
@@ -29,12 +30,13 @@ from regularizepsf_b200.functional import (
     varied_functional_psf,
 )
 from regularizepsf_b200.transform import ArrayPSFTransform, set_default_dtype
+from regularizepsf_b200.stack import TransformStack
 from regularizepsf_b200.util import IndexedCube, calculate_covering
 
 __version__ = "0.1.0"
 
 __all__ = [
-    "ArrayPSF", "ArrayPSFBuilder", "ArrayPSFTransform", "DeviceCube", "IndexedCube", "calculate_covering", "set_default_dtype",
+    "ArrayPSF", "ArrayPSFBuilder", "ArrayPSFTransform", "TransformStack", "DeviceCube", "IndexedCube", "calculate_covering", "set_default_dtype",
     "SimpleFunctionalPSF", "VariedFunctionalPSF", "simple_functional_psf", "varied_functional_psf",
     "RegularizePSFError", "InvalidCoordinateError", "IncorrectShapeError", "InvalidFunctionError",
     "FunctionParameterMismatchError", "PSFBuilderError", "InvalidDataError", "NativeLibraryError",

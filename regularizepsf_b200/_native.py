@@ -70,6 +70,15 @@ SIGNATURES = {
     "rpsf_apply_masked": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _vp, _i, _i64, _i64, _vp, _i64, _i64,
                                _vp]),
     "rpsf_apply_host": (_i, [_vp, _vp, _i, _vp, _i, _i]),
+    "rpsf_construct_kernels": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _i, _i, _vp]),
+    "rpsf_construct_kernels_dev": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _i, _i, _vp]),
+    "rpsf_stack_create": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i]),
+    "rpsf_stack_set_kernel": (_i, [_vp, _i, _vp, _i, _vp]),
+    "rpsf_stack_destroy": (_i, [_vp]),
+    "rpsf_plan_create_stack": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i]),
+    "rpsf_plan_set_stack_mode": (_i, [_vp, _i]),
+    "rpsf_plan_stack_info": (_i, [_vp, ctypes.POINTER(_i)]),
+    "rpsf_apply_stack": (_i, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i, _i, _vp, _i, _i64, _i64, _vp, _i64, _i64, _vp]),
     "rpsf_convert": (_i, [_vp, _i, _i64, _vp, _i, _i64, _i, _i, _i, _vp]),
     "rpsf_plan_workspace": (_i, [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_i64)]),
     "rpsf_apply_stages": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _i64, _i, _i, _i, _vp]),

@@ -568,6 +568,21 @@ struct rpsf_plan {
   bool timing = false;
   std::vector<cudaEvent_t> events;   // 4 per recorded apply call
   size_t events_used = 0;
+  // the transform stack of a plan made by rpsf_plan_create_stack (null otherwise): the workspace holds the spectra of
+  // stack->m * max_batch frames ([kernel][frame]) and the row bands of max_batch frames; only rpsf_apply_stack runs it
+  rpsf_stack* stack = nullptr;
+  // its column pass: 0 = k2_stack where it exists (native patch sizes whose stage ring fits), 1 = the per-kernel K2
+  // (rpsf_plan_set_stack_mode, a test and benchmark hook)
+  int stack_mode = 0;
+};
+
+// M transfer kernels on one set of patch corners: `t` holds the geometry, and its kmain / knyq hold kernel m's layout at
+// slot m (n_kept patches each).  `t` is never exposed, so only stack calls touch it.
+struct rpsf_stack {
+  rpsf_transform* t = nullptr;
+  int m = 0;
+  std::vector<char> loaded;          // kernel m has been laid out
+  size_t main_bytes = 0, nyq_bytes = 0;   // bytes of one kernel's kmain / knyq
 };
 
 extern "C" {
@@ -725,9 +740,9 @@ int upload_embed_matrix(rpsf_transform* t) {
   return RPSF_OK;
 }
 
-// the layout of rpsf_transform_set_kernel, stream-ordered on `s`; on a capturing stream it allocates only with
-// cudaMallocAsync (allocation nodes of the graph)
-int set_kernel_on(rpsf_transform* t, const void* kernel_full, int kernel_dtype, cudaStream_t s) {
+// the layout of rpsf_transform_set_kernel into `kmain` / `knyq` (the transform's own, or a stack's slot), stream-ordered
+// on `s`; on a capturing stream it allocates only with cudaMallocAsync (allocation nodes of the graph)
+int layout_kernel(rpsf_transform* t, const void* kernel_full, int kernel_dtype, void* kmain, void* knyq, cudaStream_t s) {
   if (t->n_kept > 0 && t->win_len != t->P) {
     // embedded patch size: K (n, P, P) -> K' (n, M, M) = A K A^T in double (rpsf_kernels.cuh), then the usual layout
     const int P = t->win_len, M = t->P;
@@ -748,14 +763,18 @@ int set_kernel_on(rpsf_transform* t, const void* kernel_full, int kernel_dtype, 
     LAUNCH((int)cudaGetLastError());
     embed_pass2<double2><<<blocks, 256, 0, s>>>(dT, dA, dK, (int)n, P, M);
     LAUNCH((int)cudaGetLastError());
-    int e = t->ops->prep(t->dtype, RPSF_F64, dK, t->kmain, t->knyq, t->n_kept, s);
+    int e = t->ops->prep(t->dtype, RPSF_F64, dK, kmain, knyq, t->n_kept, s);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     release();
     if (e) return fail(RPSF_E_CUDA, "kernel layout launch failed: %s", cudaGetErrorString((cudaError_t)e));
-    t->has_kernel = true;
-    return refresh_conj_kernel(t, s);
+    return RPSF_OK;
   }
-  if (t->n_kept > 0) LAUNCH(t->ops->prep(t->dtype, kernel_dtype, kernel_full, t->kmain, t->knyq, t->n_kept, s));
+  if (t->n_kept > 0) LAUNCH(t->ops->prep(t->dtype, kernel_dtype, kernel_full, kmain, knyq, t->n_kept, s));
+  return RPSF_OK;
+}
+
+int set_kernel_on(rpsf_transform* t, const void* kernel_full, int kernel_dtype, cudaStream_t s) {
+  if (int rc = layout_kernel(t, kernel_full, kernel_dtype, t->kmain, t->knyq, s)) return rc;
   t->has_kernel = true;
   return refresh_conj_kernel(t, s);
 }
@@ -769,6 +788,55 @@ int rpsf_transform_set_kernel(rpsf_transform* t, const void* kernel_full, int ke
     return fail(RPSF_E_UNSUPPORTED, "kernel dtype must be complex64 (RPSF_F32) or complex128 (RPSF_F64)");
   cudaStream_t s = (cudaStream_t)stream;
   return ordered(t, s, [&]() -> int { return set_kernel_on(t, kernel_full, kernel_dtype, s); });
+}
+
+int rpsf_stack_create(rpsf_stack** out, const int32_t* coords, int n, int P, int dtype, int device, int n_kernels) {
+  if (!out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (n_kernels < 1) return fail(RPSF_E_INVALID_ARGUMENT, "a stack needs at least one kernel, got %d", n_kernels);
+  rpsf_transform* t = nullptr;
+  if (int rc = rpsf_transform_create(&t, coords, n, P, dtype, device)) return rc;
+  auto* st = new rpsf_stack;
+  st->t = t; st->m = n_kernels;
+  st->loaded.assign(n_kernels, 0);
+  const size_t cs = 2 * real_size(dtype);
+  st->main_bytes = (size_t)t->n_kept * t->P * (t->P / 2) * cs;
+  st->nyq_bytes = (size_t)t->n_kept * t->P * cs;
+  if (n_kernels > 1 && t->n_kept > 0) {
+    DeviceGuard guard(device);
+    cudaFree(t->kmain); cudaFree(t->knyq);
+    t->kmain = t->knyq = nullptr;
+    if (cudaMalloc(&t->kmain, st->main_bytes * n_kernels) != cudaSuccess ||
+        cudaMalloc(&t->knyq, st->nyq_bytes * n_kernels) != cudaSuccess) {
+      cudaGetLastError();
+      rpsf_stack_destroy(st);
+      return fail(RPSF_E_CUDA, "out of device memory for %d transfer kernels (%d patches of %d)", n_kernels, n, P);
+    }
+  }
+  *out = st;
+  return RPSF_OK;
+}
+
+int rpsf_stack_set_kernel(rpsf_stack* st, int index, const void* kernel_full, int kernel_dtype, void* stream) {
+  if (!st || (!kernel_full && st->t->n_kept > 0)) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (index < 0 || index >= st->m) return fail(RPSF_E_INVALID_ARGUMENT, "kernel %d outside [0, %d)", index, st->m);
+  if (kernel_dtype != RPSF_F32 && kernel_dtype != RPSF_F64)
+    return fail(RPSF_E_UNSUPPORTED, "kernel dtype must be complex64 (RPSF_F32) or complex128 (RPSF_F64)");
+  rpsf_transform* t = st->t;
+  cudaStream_t s = (cudaStream_t)stream;
+  return ordered(t, s, [&]() -> int {
+    void* kmain = t->kmain ? (char*)t->kmain + st->main_bytes * index : nullptr;
+    void* knyq = t->knyq ? (char*)t->knyq + st->nyq_bytes * index : nullptr;
+    if (int rc = layout_kernel(t, kernel_full, kernel_dtype, kmain, knyq, s)) return rc;
+    st->loaded[index] = 1;
+    return RPSF_OK;
+  });
+}
+
+int rpsf_stack_destroy(rpsf_stack* st) {
+  if (!st) return RPSF_OK;
+  rpsf_transform_destroy(st->t);
+  delete st;
+  return RPSF_OK;
 }
 
 }  // extern "C"
@@ -849,6 +917,41 @@ int construct_kernel_backward(const void* S, const void* Tg, const void* G, int6
   if (e != cudaSuccess) return fail(RPSF_E_CUDA, "construct backward launch failed: %s", cudaGetErrorString(e));
   return RPSF_OK;
 }
+
+// rpsf_construct_kernels (host pairs `hp`) and rpsf_construct_kernels_dev (device pairs `dp`): CONSTRUCT_BATCH kernels
+// per launch, each launch reading S and T once
+int construct_kernels(const void* S, const void* Tg, void* K, int64_t count, int dtype, const double* hp,
+                      const double* dp, int n_kernels, int device, void* stream) {
+  if (count < 0 || n_kernels < 0 || (count > 0 && n_kernels > 0 && (!S || !Tg || !K || !(hp || dp))))
+    return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (dtype != RPSF_F32 && dtype != RPSF_F64) return fail(RPSF_E_UNSUPPORTED, "dtype must be f32 or f64");
+  if (count == 0 || n_kernels == 0) return RPSF_OK;
+  DeviceGuard guard(device);
+  if (!guard.ok) return fail(RPSF_E_CUDA, "cannot select CUDA device %d", device);
+  const unsigned blocks = (unsigned)std::min<long long>((count + 255) / 256, (long long)sm_count_of(device) * 16);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const size_t cs = dtype == RPSF_F32 ? sizeof(float2) : sizeof(double2);
+  for (int m0 = 0; m0 < n_kernels; m0 += CONSTRUCT_BATCH) {
+    const int mb = std::min(CONSTRUCT_BATCH, n_kernels - m0);
+    ConstructPairs pairs{};
+    if (hp) std::copy(hp + 2 * (size_t)m0, hp + 2 * (size_t)(m0 + mb), pairs.v);
+    const double* dpm = dp ? dp + 2 * (size_t)m0 : nullptr;
+    void* Km = (char*)K + (size_t)m0 * (size_t)count * cs;
+    if (dtype == RPSF_F32) {
+      if (dp) construct_transfer_kernels<float, true><<<blocks, 256, 0, s>>>((const float2*)S, (const float2*)Tg, (float2*)Km,
+                                                                           count, mb, pairs, dpm);
+      else construct_transfer_kernels<float><<<blocks, 256, 0, s>>>((const float2*)S, (const float2*)Tg, (float2*)Km, count,
+                                                                    mb, pairs, nullptr);
+    } else {
+      if (dp) construct_transfer_kernels<double, true><<<blocks, 256, 0, s>>>((const double2*)S, (const double2*)Tg,
+                                                                            (double2*)Km, count, mb, pairs, dpm);
+      else construct_transfer_kernels<double><<<blocks, 256, 0, s>>>((const double2*)S, (const double2*)Tg, (double2*)Km,
+                                                                     count, mb, pairs, nullptr);
+    }
+    LAUNCH((int)cudaGetLastError());
+  }
+  return RPSF_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -862,6 +965,18 @@ int rpsf_construct_kernel_dev(const void* S, const void* Tg, void* K, int64_t co
                               const double* alpha_epsilon, int device, void* stream) {
   if (!alpha_epsilon) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   return construct_kernel(S, Tg, K, count, dtype, 0.0, 0.0, alpha_epsilon, device, stream);
+}
+
+int rpsf_construct_kernels(const void* S, const void* Tg, void* K, int64_t count, int dtype, const double* alpha_epsilon,
+                           int n_kernels, int device, void* stream) {
+  if (!alpha_epsilon && n_kernels > 0) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  return construct_kernels(S, Tg, K, count, dtype, alpha_epsilon, nullptr, n_kernels, device, stream);
+}
+
+int rpsf_construct_kernels_dev(const void* S, const void* Tg, void* K, int64_t count, int dtype,
+                               const double* alpha_epsilon, int n_kernels, int device, void* stream) {
+  if (!alpha_epsilon && n_kernels > 0) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  return construct_kernels(S, Tg, K, count, dtype, nullptr, alpha_epsilon, n_kernels, device, stream);
 }
 
 int rpsf_construct_kernel_backward(const void* S, const void* Tg, const void* G, int64_t count, int dtype, double alpha,
@@ -1447,6 +1562,26 @@ int rpsf_plan_create(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_m
   return plan_build(out, t, H, W, pad_mode, row_begin, row_end, max_batch, nullptr);
 }
 
+int rpsf_plan_create_stack(rpsf_plan** out, rpsf_stack* st, int H, int W, int pad_mode, int max_batch) {
+  if (!out || !st) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  REFUSE_IN_CAPTURE("rpsf_plan_create_stack");
+  if (pad_mode == RPSF_PAD_MATERIALIZED) return fail(RPSF_E_UNSUPPORTED, "a stack plan needs a pad mode with an index map");
+  if (max_batch < 1) return fail(RPSF_E_INVALID_ARGUMENT, "max_batch must be >= 1");
+  // the overlap-add runs once over n_kernels * batch spectra: a grid dimension
+  if ((long long)max_batch * st->m > 65535)
+    return fail(RPSF_E_INVALID_ARGUMENT, "kernels x max_batch = %lld exceeds 65535", (long long)max_batch * st->m);
+  // built for n_kernels * max_batch frames, so that the overlap-add's work split fits the batch it runs
+  if (int rc = plan_build(out, st->t, H, W, pad_mode, 0, H, max_batch * st->m, nullptr)) return rc;
+  rpsf_plan* p = *out;
+  rpsf_transform* t = st->t;
+  const size_t cs = 2 * real_size(t->dtype);
+  p->max_batch = max_batch;            // frames per call: the row bands and the saturation scratch
+  p->stack = st;
+  p->band_offset = (size_t)st->m * max_batch * p->n_active * t->P * (t->P / 2) * cs;
+  p->workspace_bytes = p->band_offset + (size_t)max_batch * p->band_frame_rows * (t->P / 2) * cs;
+  return RPSF_OK;
+}
+
 int rpsf_plan_create_adjoint(rpsf_plan** out, rpsf_transform* t, int H, int W, int pad_mode, int max_batch) {
   if (!out || !t) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   if (H <= 0 || W <= 0) return fail(RPSF_E_INCORRECT_SHAPE, "frame shape must be positive, got (%d, %d)", H, W);
@@ -1776,6 +1911,7 @@ int sat_restore_launch(rpsf_plan* p, const void* image, void* out, int64_t out_p
 int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, int img_row0,
                  int img_rows, void* out, int64_t out_pitch, int64_t out_frame_stride, int out_row0,
                  int batch, int stages, void* stream_v, const SatSource* src = nullptr, const MaskArg* mask = nullptr) {
+  if (p->stack) return fail(RPSF_E_INVALID_ARGUMENT, "a plan of a transform stack runs through rpsf_apply_stack only");
   if (p->row_end == p->row_begin && stages >= 3) return RPSF_OK;      // an empty band (more ranks than half-patch rows): nothing to write
   if (!image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
   rpsf_transform* t = p->tr;
@@ -1884,6 +2020,105 @@ int apply_stages(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img
                       store_only, g, batch, s));
   }
   if (ev) CU(cudaEventRecord(ev[3], s));
+  return restore();
+}
+
+// whether a stack plan runs k2_stack: from two kernels on (with one it has no forward transform to share, and was
+// measured 9 % slower than K2 in float32), not at embedded patch sizes (their pruned column pass), nor where the stage
+// ring of the pipelined column pass does not fit (ops->k2s_ok), nor when rpsf_plan_set_stack_mode forced the per-kernel K2
+bool stack_fused(const rpsf_plan* p) {
+  const rpsf_transform* t = p->tr;
+  return p->stack_mode == 0 && p->stack->m >= 2 && t->win_len == t->P && t->ops->k2s_ok(t->dtype);
+}
+
+// rpsf_apply_stack: the saturation / mask fill and K1 once for the `batch` frames, K2 once per kernel from the shared row
+// bands into that kernel's spectra, and one overlap-add over all n_kernels * batch spectra.  Each kernel's output is
+// what apply_stages computes for it alone: the same kernels run on the same data, and none of them depends on where
+// its frame sits in the batch.
+int apply_stack(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, void* out,
+                int64_t out_pitch, int64_t out_frame_stride, int batch, cudaStream_t s, const SatSource* src,
+                const MaskArg* mask) {
+  rpsf_transform* t = p->tr;
+  const rpsf_stack* st = p->stack;
+  const int M = st->m;
+  for (int m = 0; m < M; ++m)
+    if (!st->loaded[m]) return fail(RPSF_E_NO_KERNEL, "transfer kernel %d of the stack not loaded (call rpsf_stack_set_kernel)", m);
+  if (batch < 1 || batch > p->max_batch)
+    return fail(RPSF_E_INVALID_ARGUMENT, "batch %d outside [1, max_batch=%d]", batch, p->max_batch);
+  if (img_pitch < p->W || out_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "row pitch smaller than frame width");
+  DeviceGuard guard(t->device);
+  ApplyGeom g;
+  g.H = p->H; g.W = p->W; g.img_row0 = 0; g.img_rows = p->H; g.img_pitch = img_pitch;
+  g.img_frame_stride = img_frame_stride; g.out_row0 = 0; g.row_begin = 0; g.row_end = p->H;
+  g.out_pitch = out_pitch; g.out_frame_stride = out_frame_stride; g.n_active = p->n_active; g.pad_mode = p->pad_mode;
+  g.win_len = t->win_len;
+  const size_t rs = real_size(t->dtype), cs = 2 * rs;
+  const int frames = M * batch;                 // output frame m * batch + b is kernel m applied to frame b
+  const bool use_stream = p->overlap == Overlap::stream;
+  const bool use_gather = p->overlap == Overlap::gather;
+  if (!(p->colour0_covers || use_gather || use_stream))
+    for (int j = 0; j < frames; ++j)
+      CU(cudaMemset2DAsync((char*)out + (size_t)j * out_frame_stride * rs, (size_t)out_pitch * rs, 0, (size_t)p->W * rs,
+                           p->H, s));
+  const bool sat = p->sat_threshold < INFINITY || mask;
+  if (p->n_active == 0 && !sat) return RPSF_OK;
+  SatGeom sg;
+  const void* k1_image = image;
+  ApplyGeom g1 = g;
+  if (sat) {
+    int rc = t->dtype == RPSF_F32 ? sat_prefill<float>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image, mask)
+                                  : sat_prefill<double>(p, image, img_pitch, img_frame_stride, src, batch, s, &sg, &k1_image, mask);
+    if (rc) return rc;
+    g1.img_row0 = 0; g1.img_rows = sg.Hp; g1.img_pitch = sg.Wp; g1.img_frame_stride = (long long)sg.Hp * sg.Wp;
+    g1.pad_mode = PAD_NONE;
+  }
+  auto restore = [&]() -> int {
+    if (!sat) return RPSF_OK;
+    for (int m = 0; m < M; ++m) {
+      void* om = (char*)out + (size_t)m * batch * out_frame_stride * rs;
+      int rc = t->dtype == RPSF_F32 ? sat_restore_launch<float>(p, image, om, out_pitch, out_frame_stride, 0, batch, s, sg)
+                                    : sat_restore_launch<double>(p, image, om, out_pitch, out_frame_stride, 0, batch, s, sg);
+      if (rc) return rc;
+    }
+    return RPSF_OK;
+  };
+  if (p->n_active == 0) return restore();
+  if (int rc = ensure_workspace(p)) return rc;
+  const RowBands rb = row_bands(p);
+  if (p->k1 == K1Kernel::bulk && (long long)batch * p->band_frame_rows < (1LL << 30)) {
+    const int bulk_ok = ((reinterpret_cast<uintptr_t>(k1_image) & 15) == 0 && ((size_t)g1.img_pitch * rs) % 16 == 0 &&
+                         ((size_t)g1.img_frame_stride * rs) % 16 == 0) ? 1 : 0;
+    LAUNCH(t->ops->k1s(t->dtype, k1_image, band_buffer(p), rb, t->tw, t->win, g1, batch, bulk_ok, t->sm_count, s));
+  } else {
+    LAUNCH(t->ops->k1(t->dtype, k1_image, band_buffer(p), rb, t->tw, t->win, g1, batch, s));
+  }
+  const size_t spec_frame = (size_t)p->n_active * t->P * (t->P / 2) * cs;
+  if (stack_fused(p)) {
+    // one forward column FFT per tile and frame, then the multiply and inverse FFT of every kernel (k2_stack)
+    LAUNCH(t->ops->k2s(t->dtype, band_buffer(p), rb, p->workspace, (long long)((size_t)batch * spec_frame / cs), t->kmain,
+                       (long long)(st->main_bytes / cs), t->knyq, (long long)(st->nyq_bytes / cs), M, p->active_dev, t->tw,
+                       t->win, g, batch, t->sm_count, s));
+  } else {
+    // per-kernel column pass: the existing K2 once per kernel, on the shared row bands
+    for (int m = 0; m < M; ++m)
+      LAUNCH(t->ops->k2(t->dtype, band_buffer(p), rb, (char*)p->workspace + (size_t)m * batch * spec_frame,
+                        (char*)t->kmain + st->main_bytes * m, (char*)t->knyq + st->nyq_bytes * m, p->active_dev, t->tw,
+                        t->win, g, batch, t->sm_count, s));
+  }
+  if (use_stream) {
+    LAUNCH(t->ops->k3s(t->dtype, p->workspace, out, p->stasks_dev, p->scodes_dev, p->n_warp_items, t->tw, t->win, g,
+                       frames, t->sm_count, nullptr, s));
+  } else if (use_gather) {
+    LAUNCH(t->ops->k3g(t->dtype, p->workspace, out, p->tiles_dev, p->n_tiles, p->groups_dev, p->gitems_dev, t->tw,
+                       t->win, p->teams, p->seg_w, g, frames, s));
+  } else {
+    for (size_t c = 0; c < p->items_dev.size(); ++c) {
+      if (p->n_items[c] == 0) continue;
+      const int store_only = (c == 0 && p->colour0_covers) ? 1 : 0;
+      LAUNCH(t->ops->k3(t->dtype, p->workspace, out, p->corners_dev, p->items_dev[c], p->n_items[c], t->tw, t->win,
+                        store_only, g, frames, s));
+    }
+  }
   return restore();
 }
 
@@ -2208,6 +2443,38 @@ int rpsf_apply_source(rpsf_plan* p, const void* image, int64_t img_pitch, int64_
   return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
     return apply_stages(p, image, img_pitch, img_frame_stride, img_row0, img_rows, out, out_pitch, out_frame_stride,
                         out_row0, batch, 3, stream, &source);
+  });
+}
+
+int rpsf_plan_set_stack_mode(rpsf_plan* p, int mode) {
+  if (!p || !p->stack) return fail(RPSF_E_INVALID_ARGUMENT, "not a plan of a transform stack");
+  if (mode != 0 && mode != 1) return fail(RPSF_E_INVALID_ARGUMENT, "stack mode must be 0 or 1, got %d", mode);
+  p->stack_mode = mode;
+  return RPSF_OK;
+}
+
+int rpsf_plan_stack_info(const rpsf_plan* p, int* fused) {
+  if (!p || !p->stack || !fused) return fail(RPSF_E_INVALID_ARGUMENT, "null argument or not a plan of a transform stack");
+  *fused = stack_fused(p) ? 1 : 0;
+  return RPSF_OK;
+}
+
+int rpsf_apply_stack(rpsf_plan* p, const void* image, int64_t img_pitch, int64_t img_frame_stride, void* out,
+                     int64_t out_pitch, int64_t out_frame_stride, int n_kernels, int batch, const void* src, int src_dtype,
+                     int64_t src_pitch, int64_t src_frame_stride, const void* mask, int64_t mask_pitch,
+                     int64_t mask_frame_stride, void* stream) {
+  if (!p || !image || !out) return fail(RPSF_E_INVALID_ARGUMENT, "null argument");
+  if (!p->stack) return fail(RPSF_E_INVALID_ARGUMENT, "not a plan of a transform stack (rpsf_plan_create_stack)");
+  if (n_kernels != p->stack->m)
+    return fail(RPSF_E_INVALID_ARGUMENT, "%d kernels given, the plan's stack has %d", n_kernels, p->stack->m);
+  if (mask && mask_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "mask row pitch smaller than frame width");
+  if (src && !elem_size(src_dtype)) return fail(RPSF_E_UNSUPPORTED, "unsupported source dtype code %d", src_dtype);
+  if (src && src_pitch < p->W) return fail(RPSF_E_INCORRECT_SHAPE, "source row pitch smaller than frame width");
+  const MaskArg m{(const unsigned char*)mask, mask_pitch, mask_frame_stride};
+  const SatSource source{src, src_dtype, src_pitch, src_frame_stride};
+  return ordered(p->tr, (cudaStream_t)stream, [&]() -> int {
+    return apply_stack(p, image, img_pitch, img_frame_stride, out, out_pitch, out_frame_stride, batch,
+                       (cudaStream_t)stream, src ? &source : nullptr, mask ? &m : nullptr);
   });
 }
 

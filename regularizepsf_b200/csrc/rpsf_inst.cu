@@ -86,6 +86,10 @@ int init() {
     if ((e = set_smem(k2_pipelined<P, float, 2>, col_pipe_smem<float>()))) return e;
   if constexpr (use_col_pipe<double>() && TL::SLOTS == 1 && TL::NTILE % 2 == 0)
     if ((e = set_smem(k2_pipelined<P, double, 2>, col_pipe_smem<double>()))) return e;
+  if constexpr (use_col_pipe<float>())
+    if ((e = set_smem(k2_stack<P, float>, col_pipe_smem<float>()))) return e;
+  if constexpr (use_col_pipe<double>())
+    if ((e = set_smem(k2_stack<P, double>, col_pipe_smem<double>()))) return e;
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, float>, row_smem<float>()))) return e;
   if ((e = set_smem(k3_rowifft_window_overlap_add<P, double>, row_smem<double>()))) return e;
   if ((e = set_smem(k3_rowpair_gather<P, float>, K3G_SMEM_MAX))) return e;
@@ -186,6 +190,33 @@ int k2(int dt, const void* bands, const RowBands& rb, void* spec, const void* km
   return dt == DT_F32 ? k2_t<float>(bands, rb, spec, kmain, knyq, active, tw, win, g, batch, sm_count, s)
                       : k2_t<double>(bands, rb, spec, kmain, knyq, active, tw, win, g, batch, sm_count, s);
 }
+
+template <typename T>
+int k2s_t(const void* bands, const RowBands& rb, void* spec, long long kspec_stride, const void* kmain,
+          long long kmain_stride, const void* knyq, long long knyq_stride, int n_kernels, const int* active, const void* tw,
+          const void* win, const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
+  if constexpr (use_col_pipe<T>()) {
+    // k2_t's grid: several frames per CTA while at least ~4 waves of CTAs stay in flight
+    const long long ctas = cdiv((long long)g.n_active * TL::NTILE, TL::SLOTS);
+    int fpc = batch;
+    while (fpc > 1 && ctas * cdiv(batch, fpc) < (long long)sm_count * 3 * 4) fpc = (fpc + 1) / 2;
+    return launch_chain(2, k2_stack<P, T>, dim3((unsigned)ctas, cdiv(batch, fpc)), dim3(TL::K2_THREADS), col_pipe_smem<T>(),
+                        s, (const cplx<T>*)bands, rb, (cplx<T>*)spec, kspec_stride, (const cplx<T>*)kmain, kmain_stride,
+                        (const cplx<T>*)knyq, knyq_stride, n_kernels, active, (const cplx<T>*)tw, (const T*)win, batch, fpc,
+                        g);
+  } else {
+    return (int)cudaErrorNotSupported;
+  }
+}
+int k2s(int dt, const void* bands, const RowBands& rb, void* spec, long long kspec_stride, const void* kmain,
+        long long kmain_stride, const void* knyq, long long knyq_stride, int n_kernels, const int* active, const void* tw,
+        const void* win, const ApplyGeom& g, int batch, int sm_count, cudaStream_t s) {
+  return dt == DT_F32 ? k2s_t<float>(bands, rb, spec, kspec_stride, kmain, kmain_stride, knyq, knyq_stride, n_kernels, active,
+                                     tw, win, g, batch, sm_count, s)
+                      : k2s_t<double>(bands, rb, spec, kspec_stride, kmain, kmain_stride, knyq, knyq_stride, n_kernels,
+                                      active, tw, win, g, batch, sm_count, s);
+}
+int k2s_ok(int dt) { return dt == DT_F32 ? use_col_pipe<float>() : use_col_pipe<double>(); }
 
 template <typename T>
 int k3_t(const void* spec, void* out, const int2* corners, const int* items, int n_items, const void* tw,
@@ -313,7 +344,7 @@ int kgrad_launch(int dt, const void* xspec, const RowBands& xb, const void* gspe
                       : kgrad_t<double>(xspec, xb, gspec, gb, out, active, tw, win, n_active, batch, s);
 }
 
-const Ops kOps = {P, init, k1, k1s, k2, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch, fft2_adjoint};
+const Ops kOps = {P, init, k1, k1s, k2, k2s, k2s_ok, k3, k3g, k3s, stream_tpw, k3g_smem, prep, fft2, kgrad_launch, fft2_adjoint};
 
 }  // namespace
 

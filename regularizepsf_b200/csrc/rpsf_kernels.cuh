@@ -535,6 +535,174 @@ k2_pipelined(const cplx<T>* __restrict__ bands, const RowBands rb, cplx<T>* __re
                                         f_begin, f_end, g);
 }
 
+// ---------------------------------------------------------------------------- K2 of a transform stack
+// k2_pipelined's frame loop for M transfer kernels: per frame, the tile streams in through the same cp.async stage
+// ring and the forward column FFT runs once; then, per kernel m, the multiply by kernel m's tile and the inverse FFT,
+// stored to spectrum slot (m, f) at spec + m * kspec_stride.  The forward spectrum stays in registers (vf, and for the
+// tile-0 instantiation zm, the conjugate mirror of the packed DC/Nyquist column) across the M inverse transforms.
+// Kernel m's tile is re-read from L2 per frame (M tiles do not fit the registers).  The arithmetic of every element is
+// k2_frames' (same device functions, same operand order), so each slot equals what k2_pipelined writes for kernel m.
+template <int P, typename T, bool TILE0>
+__device__ __forceinline__ void k2_stack_frames(const cplx<T>* __restrict__ bands, const RowBands& rb, cplx<T>* __restrict__ spec,
+                                                long long kspec_stride, const cplx<T>* __restrict__ kp,
+                                                long long kmain_stride, const cplx<T>* __restrict__ kn, long long knyq_stride,
+                                                int n_kernels, const cplx<T>* tw, const T* wy, cplx<T>* stage0, bool valid_in,
+                                                bool special, int a, int tile, int c, int n1, int slot, int lt, int f_begin,
+                                                int f_end, const ApplyGeom& g) {
+  using TL = Tile<P>;
+  const bool valid = TL::SLOTS == 1 ? true : valid_in;
+  constexpr int N1 = TL::N1, N2 = TL::N2, HALF = TL::HALF, C = TL::C;
+  constexpr int STAGE = TL::SLOTS * P * C;
+  constexpr int CH = 16 / (int)sizeof(cplx<T>);
+  constexpr int ROW_CHUNKS = C / CH;
+  constexpr int PER_THREAD = (P * ROW_CHUNKS) / TL::SLOT_THREADS;
+  constexpr int ROWS_PER_PASS = TL::SLOT_THREADS / ROW_CHUNKS;
+  static_assert(C % CH == 0 && (P * ROW_CHUNKS) % TL::SLOT_THREADS == 0, "tile does not split into 16-byte chunks");
+  auto sync = []() { __syncthreads(); };
+  auto nosync = []() {};
+
+  const long long frame_stride = (long long)g.n_active * P * HALF;
+  const long long band_frame_stride = (long long)rb.frame_rows * HALF;
+  cplx<T>* tile_base = spec + ((long long)a * P) * HALF + tile * C;
+  const int row0 = lt / ROW_CHUNKS, part = lt % ROW_CHUNKS;
+  const cplx<T>* src0 = bands + ((long long)(valid ? rb.patch_row[a] : 0) + row0) * HALF + tile * C + part * CH;
+  const int dst0 = slot * (P * C) + row0 * C + part * CH;
+  const int n_it = f_end - f_begin;
+  auto issue = [&](int it, cplx<T>* stage) {
+    if (valid) {
+      const cplx<T>* src = src0 + (f_begin + it) * band_frame_stride;
+#pragma unroll
+      for (int i = 0; i < PER_THREAD; ++i)
+        cp_async16(stage + dst0 + i * (ROWS_PER_PASS * C), src + (long long)i * (ROWS_PER_PASS * HALF));
+    }
+    cp_async_commit();
+  };
+  auto ex = [=](int k2, int nn) { return ((slot * N2 + k2) * N1 + nn) * C + c; };
+
+  constexpr int NS = K2_STAGES;
+  int cur = 0;
+  grid_dependency_wait();
+  grid_launch_dependents();
+#pragma unroll
+  for (int s = 0; s < NS - 1; ++s) {
+    if (s < n_it) issue(s, stage0 + s * STAGE);
+    else cp_async_commit();
+  }
+  for (int it = 0; it < n_it; ++it, cur = (cur + 1 == NS ? 0 : cur + 1)) {
+    const int f = f_begin + it;
+    cplx<T>* xbuf = stage0 + cur * STAGE;
+    cp_async_wait_pending<NS - 2>();
+    __syncthreads();
+    {
+      const int nxt = cur + NS - 1 >= NS ? cur - 1 : cur + NS - 1;
+      if (it + NS - 1 < n_it) issue(it + NS - 1, stage0 + nxt * STAGE);
+      else cp_async_commit();
+    }
+    cplx<T> vf[N2];
+    static_for<0, N2>([&](auto jj) {
+      constexpr int j = decltype(jj)::value;
+      vf[j] = cscale_rn(xbuf[ex(j, n1)], wy[n1 + N1 * j]);
+    });
+    coop_fft_forward<P, T>(vf, n1, xbuf, tw, ex, sync);
+    cplx<T> zm[TILE0 ? N2 : 1];
+    if constexpr (TILE0) {
+      cplx<T>* zs = xbuf + slot * P;
+      if (special) {
+        static_for<0, N2>([&](auto ee) {
+          constexpr int e = decltype(ee)::value;
+          constexpr int m = e / N1, k1 = e % N1;
+          zs[(n1 + N1 * m) + N2 * k1] = vf[e];
+        });
+      }
+      __syncthreads();
+      static_for<0, N2>([&](auto ee) {
+        constexpr int e = decltype(ee)::value;
+        constexpr int m = e / N1, k1 = e % N1;
+        const int k = (n1 + N1 * m) + N2 * k1;
+        zm[e] = vf[e];
+        if (special) {
+          const cplx<T> zr = zs[(P - k) & (P - 1)];
+          zm[e] = mk<T>(zr.x, -zr.y);
+        }
+      });
+      __syncthreads();                                      // zs is read: the inverse transforms may reuse the buffer
+    }
+    for (int km = 0; km < n_kernels; ++km) {
+      const cplx<T>* kpm = kp + km * kmain_stride;
+      cplx<T> v[N2];
+      if constexpr (TILE0) {
+        const cplx<T>* knm = kn + km * knyq_stride;
+        static_for<0, N2>([&](auto ee) {
+          constexpr int e = decltype(ee)::value;
+          const cplx<T> kval = valid ? kpm[(long long)e * (N1 * C)] : mk<T>(T(0), T(0));
+          const cplx<T> kny = special ? knm[e * N1] : mk<T>(T(0), T(0));
+          const cplx<T> sum = mk<T>(T(0.5) * (vf[e].x + zm[e].x), T(0.5) * (vf[e].y + zm[e].y));
+          const cplx<T> dif = mk<T>(T(0.5) * (vf[e].x - zm[e].x), T(0.5) * (vf[e].y - zm[e].y));
+          v[e] = cadd(cmul(sum, kval), cmul(dif, kny));
+        });
+      } else {
+        static_for<0, N2>([&](auto ee) {
+          constexpr int e = decltype(ee)::value;
+          v[e] = cmul(vf[e], valid ? kpm[(long long)e * (N1 * C)] : mk<T>(T(0), T(0)));
+        });
+      }
+      // the exchange slots of one inverse transform are read before the next writes them (`sync` after the reads);
+      // after the last one, the next frame's top barrier orders them before the stage is refilled
+      if (km + 1 < n_kernels) coop_fft_inverse<P, T>(v, n1, xbuf, tw, ex, sync, sync);
+      else coop_fft_inverse<P, T>(v, n1, xbuf, tw, ex, sync, nosync);
+      if (valid) {
+        cplx<T>* base = tile_base + km * kspec_stride + f * frame_stride + c;
+        static_for<0, N2>([&](auto jj) {
+          constexpr int j = decltype(jj)::value;
+          base[(long long)(n1 + N1 * j) * HALF] = v[j];
+        });
+      }
+    }
+  }
+}
+
+template <int P, typename T>
+__global__ void __launch_bounds__(Tile<P>::K2_THREADS, 2)
+k2_stack(const cplx<T>* __restrict__ bands, const RowBands rb, cplx<T>* __restrict__ spec, long long kspec_stride,
+         const cplx<T>* __restrict__ kmain, long long kmain_stride, const cplx<T>* __restrict__ knyq, long long knyq_stride,
+         int n_kernels, const int* __restrict__ active, const cplx<T>* __restrict__ tw_g, const T* __restrict__ win_g,
+         int batch, int frames_per_cta, ApplyGeom g) {
+  using TL = Tile<P>;
+  constexpr int N1 = TL::N1, N2 = TL::N2, C = TL::C, NTILE = TL::NTILE;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  cplx<T>* tw = reinterpret_cast<cplx<T>*>(smem_raw);
+  T* wy = reinterpret_cast<T*>(tw + P);
+  cplx<T>* stage0 = reinterpret_cast<cplx<T>*>(wy + P);
+  for (int i = threadIdx.x; i < P; i += blockDim.x) { tw[i] = tw_g[i]; wy[i] = T(0.5) * win_g[i]; }
+
+  const int c = threadIdx.x % C;
+  const int n1 = (threadIdx.x / C) % N1;
+  const int slot = threadIdx.x / (C * N1);
+  const int lt = threadIdx.x % TL::SLOT_THREADS;
+  const long long first = (long long)blockIdx.x * TL::SLOTS;
+  const long long sitem = first + slot;
+  const long long total = (long long)g.n_active * NTILE;
+  const bool valid = sitem < total;
+  const int a = valid ? int(sitem / NTILE) : 0;
+  const int tile = valid ? int(sitem % NTILE) : 1;
+  bool any_tile0 = false;
+#pragma unroll
+  for (int s = 0; s < TL::SLOTS; ++s) any_tile0 |= (first + s < total) && ((first + s) % NTILE == 0);
+  if constexpr (TL::SLOTS == 1) { if (!valid) return; }
+  const bool special = valid && tile == 0 && c == 0;
+  const int gp = valid ? active[a] : 0;
+  const cplx<T>* kp = kmain + (((long long)gp * NTILE + (valid ? tile : 0)) * N2) * (N1 * C) + n1 * C + c;
+  const cplx<T>* kn = knyq + (long long)gp * P + n1;
+  const int f_begin = blockIdx.y * frames_per_cta;
+  const int f_end = min(batch, f_begin + frames_per_cta);
+  if (any_tile0)
+    k2_stack_frames<P, T, true>(bands, rb, spec, kspec_stride, kp, kmain_stride, kn, knyq_stride, n_kernels, tw, wy, stage0,
+                                valid, special, a, tile, c, n1, slot, lt, f_begin, f_end, g);
+  else
+    k2_stack_frames<P, T, false>(bands, rb, spec, kspec_stride, kp, kmain_stride, kn, knyq_stride, n_kernels, tw, wy, stage0,
+                                 valid, special, a, tile, c, n1, slot, lt, f_begin, f_end, g);
+}
+
 // ============================================================================ K3
 // row IFFT + window + overlap-add.  transform.py:164-177 (second IFFT axis, np.real, window,
 // `+=` into the canvas, crop).  Launched once per colour class: patches of one colour never
@@ -828,6 +996,36 @@ __global__ void construct_transfer_kernel(const cplx<T>* __restrict__ S, const c
     else { const T scl = T(1) / den; qx = nx * scl; qy = ny * scl; }
     // explicit non-fused complex product, same operation order as numpy
     K[i] = mk<T>(qx * tg.x - qy * tg.y, qx * tg.y + qy * tg.x);
+  }
+}
+
+// M kernels from one read of S and T: kernel m (m < n_kernels) goes to K + m * count, with (alpha, epsilon) =
+// pairs[2m], pairs[2m + 1] converted to T as construct_transfer_kernel's entry points convert theirs.  The per-bin
+// arithmetic is construct_transfer_kernel's, statement for statement, so every kernel is bit-identical to it.
+// DEV: `pairs` is device memory (rpsf_construct_kernels_dev); otherwise the host pairs arrive in `host_pairs`.
+constexpr int CONSTRUCT_BATCH = 64;     // kernels per launch: the host pairs travel as a 1 KB kernel parameter
+struct ConstructPairs { double v[2 * CONSTRUCT_BATCH]; };
+template <typename T, bool DEV = false>
+__global__ void construct_transfer_kernels(const cplx<T>* __restrict__ S, const cplx<T>* __restrict__ Tg,
+                                           cplx<T>* __restrict__ K, long long count, int n_kernels,
+                                           ConstructPairs host_pairs, const double* __restrict__ pairs) {
+  __shared__ T scalars[2 * CONSTRUCT_BATCH];
+  for (int j = threadIdx.x; j < 2 * n_kernels; j += blockDim.x) scalars[j] = T(DEV ? pairs[j] : host_pairs.v[j]);
+  __syncthreads();
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count;
+       i += (long long)gridDim.x * blockDim.x) {
+    const cplx<T> s = S[i], tg = Tg[i];
+    const T sa = hypot(s.x, s.y), ta = hypot(tg.x, tg.y);
+    for (int m = 0; m < n_kernels; ++m) {
+      const T alpha = scalars[2 * m], epsilon = scalars[2 * m + 1];
+      const T pw = pow_like_numpy<T>(sa, alpha - T(1));
+      const T nx = s.x * pw, ny = -s.y * pw;
+      const T den = pow_like_numpy<T>(sa, alpha + T(1)) + pow_like_numpy<T>(epsilon * ta, alpha + T(1));
+      T qx, qy;
+      if (den == T(0)) { qx = nx / fabs(den); qy = ny / fabs(den); }
+      else { const T scl = T(1) / den; qx = nx * scl; qy = ny * scl; }
+      K[(long long)m * count + i] = mk<T>(qx * tg.x - qy * tg.y, qx * tg.y + qy * tg.x);
+    }
   }
 }
 

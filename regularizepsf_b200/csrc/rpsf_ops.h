@@ -23,6 +23,13 @@ struct Ops {
   int (*k2)(int dt, const void* bands, const RowBands& rb, void* spec, const void* kmain, const void* knyq,
             const int* active, const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count,
             cudaStream_t s);
+  // the column pass of a transform stack (k2_stack): n_kernels kernels at kmain + m * kmain_stride / knyq + m *
+  // knyq_stride, spectra of kernel m at spec + m * kspec_stride (complex elements); k2s_ok(dt): it exists for this
+  // patch size and dtype (the pipelined stage ring fits)
+  int (*k2s)(int dt, const void* bands, const RowBands& rb, void* spec, long long kspec_stride, const void* kmain,
+             long long kmain_stride, const void* knyq, long long knyq_stride, int n_kernels, const int* active,
+             const void* tw, const void* win, const ApplyGeom& g, int batch, int sm_count, cudaStream_t s);
+  int (*k2s_ok)(int dt);
   int (*k3)(int dt, const void* spec, void* out, const int2* corners, const int* items, int n_items,
             const void* tw, const void* win, int store_only, const ApplyGeom& g, int batch, cudaStream_t s);
   // single-launch overlap-add: `teams` teams per CTA, `seg_w` output columns per CTA

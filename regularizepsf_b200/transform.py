@@ -305,6 +305,14 @@ class ArrayPSFTransform:
     #: the kernel tensor was made by construct / reconstruct, not given by the caller (reconstruct may write into it)
     _kernel_owned = False
 
+    @staticmethod
+    def stack(transforms) -> "TransformStack":
+        """A ``TransformStack`` of the kernels of ``transforms`` (copied into one (M, N, P, P) tensor), which must share
+        their coordinates (InvalidCoordinateError) and patch size (IncorrectShapeError); a sharded transform raises
+        NotImplementedError.  ``stack.apply(x)[m]`` is bit-identical to ``transforms[m].apply(x)``."""
+        from regularizepsf_b200.stack import TransformStack
+        return TransformStack.from_transforms(transforms)
+
     @classmethod
     def _constructed(cls, coordinates, kernel) -> "ArrayPSFTransform":
         obj = cls(DeviceCube(coordinates, kernel))
